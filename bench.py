@@ -2,6 +2,7 @@
 """Benchmark of the scan hot path: read-names/s scanned + matched (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--reads R] [--workload scan|demux]
+                    [--dump-outputs DIR]
 
 One step = one pass of the whole scan path over one synthetic NovaSeq-lane shaped input
 (config C2: 10+10 bp UDI, 384-sample sheet, `scan -n 1 -rc`): fused parse+pack+count kernel ->
@@ -21,6 +22,7 @@ lane: the first reads of the stream the e2e leg uses.
 After the timed loop the result is CHECKED: counts sum to the reads, shares of the ranks are disjoint, and the
 first 3 M reads of the lane -- tally, both matcher passes, orientation calls -- equal the C oracle's.
 `--scaling strong` (N > 1) deals the record chunks of ONE lane to the ranks instead of one lane each.
+`--dump-outputs DIR` (N = 1) writes what the last timed step computed as .npy files (see dump_outputs).
 At N = 1 the line also carries a `demux` object: BASELINE configs[3] through the record router as a stream
 (tools/bench_demux.py: 4 M pairs, 64 MB chunks cut anywhere, two in flight, every sink's byte stream compared with
 the C oracle's demux loop); `--workload demux` makes that the line, with the reference's frender_demux beside it.
@@ -45,6 +47,7 @@ CPU_SAMPLE_READS = 200_000     # bounded sample for the CPU arm (about 3 s of th
 E2E_MAX_BYTES = 6 << 30        # host-resident sample for the pinned-text leg (e2e_pcie)
 E2E_GZ_READS = 4_000_000       # reads in the .fastq.gz of the end-to-end leg
 CHECK_READS = 3_000_000        # prefix of the lane compared with the C oracle after the timed loop
+DUMP_ROWS = 1 << 19            # unique keys sampled by --dump-outputs (13 M at the default lane; 29 MB of .npy)
 
 
 def parse_args():
@@ -62,7 +65,15 @@ def parse_args():
     ap.add_argument("--workload", default="scan", choices=["scan", "demux"])
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: one lane per GPU; strong: ONE lane, its record chunks dealt to the GPUs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (float32/float64; "
+                         "a fixed, seeded sample of the unique keys) so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl == "reference" or args.workload != "scan"):
+        ap.error("--dump-outputs writes the outputs of the scan workload on the GPU (--workload scan, no --impl reference)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -257,12 +268,15 @@ def demux_files_equal(dir_a, dir_b):
     return all(digest(os.path.join(dir_a, n)) == digest(os.path.join(dir_b, n)) for n in names)
 
 
-def demux_cpu_baseline(with_cli=True):
+def demux_cpu_baseline(with_cli=True, steps=1, warmup=0):
+    """The reference's demux on the sample files: `warmup` untimed runs, then the mean of `steps` timed ones (each
+    into a directory of its own, as the reference writes into an empty one)."""
     cores = len(os.sched_getaffinity(0))
     ref = load_reference()
     with tempfile.TemporaryDirectory() as d:
         paths, res = demux_cpu_sample(d)
-        t_ref = demux_cpu_step(paths, res, os.path.join(d, "out_ref"), ref)
+        times = [demux_cpu_step(paths, res, os.path.join(d, f"out_ref{i}"), ref) for i in range(warmup + steps)]
+        t_ref = sum(times[warmup:]) / steps
         out = {"value": DEMUX_CPU_PAIRS / t_ref, "unit": "pairs/s", "cores": 1,
                "kind": "reference" if ref is not None else "port",
                "sample": f"frender_demux on the first {DEMUX_CPU_PAIRS} pairs of the C4 lane: R1/R2 .fastq.gz in, 387 "
@@ -273,7 +287,8 @@ def demux_cpu_baseline(with_cli=True):
             out["same_files_through_this_repo"] = {
                 "pairs_per_s": DEMUX_CPU_PAIRS / t_cli, "threads": cores,
                 "what": "frender_b200 demux on the same files (host inflate threads, device router stream, host deflate threads at the CLI's default level 6; includes creating the CUDA context)",
-                "sinks_identical_after_gunzip": demux_files_equal(os.path.join(d, "out_ref"), os.path.join(d, "out_b200"))}
+                "sinks_identical_after_gunzip": demux_files_equal(os.path.join(d, f"out_ref{warmup + steps - 1}"),
+                                                                  os.path.join(d, "out_b200"))}
     return out
 
 
@@ -284,9 +299,9 @@ def run_demux(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
         if rank == 0:
-            cpu = demux_cpu_baseline(with_cli=False)
+            cpu = demux_cpu_baseline(with_cli=False, steps=args.steps, warmup=args.warmup)
             print(json.dumps({"impl": "reference", "metric": "record_pairs_per_s_demuxed", "value": cpu["value"],
-                              "unit": "pairs/s", "n_gpus": args.gpus, "steps": 1, "warmup": 0,
+                              "unit": "pairs/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
                               "ms_per_step": 1e3 * DEMUX_CPU_PAIRS / cpu["value"], "higher_is_better": True,
                               "scaling": "weak", "vs_baseline": None, "dtype": "u8/u64", "data": "synthetic",
                               "config": demux_config(args.reads or DEMUX_PAIRS, args.gpus), "cpu_baseline": cpu,
@@ -444,6 +459,40 @@ class Clocks:
                 "reasons": sorted(self.reasons), "samples": len(sm), "source": self.source}
 
 
+def dump_outputs(out_dir, ctx, n_reads, res, last):
+    """--dump-outputs: what the last timed step computed, as a caller of the scan path receives it -- the unique-key
+    list (key, reads, first read) with each key's oriented-pass match (F:618-630), reads per read type and per sample
+    row over all keys, and the per-sample orientation sums and calls (F:354-388).  Per-key arrays hold a fixed, seeded
+    sample of DUMP_ROWS keys (rows of the first-appearance list, `key_row`); packed keys are split into 32-bit halves
+    so that float64 holds them exactly.  res: the matcher part of the step run once more with its per-key outputs
+    copied to the host (inside the timed loop they stay on the device); last: its orientation sums and calls."""
+    keys, counts, first = ctx.total_arrays()
+    n = len(keys)
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    weights = counts.astype(np.float64)
+    demuxable = res["srow"] >= 0
+    arrays = {
+        "totals": np.array([n_reads, n], np.float64),
+        "key_row": rows.astype(np.float64),
+        "key_hi": (keys[rows] >> np.uint64(32)).astype(np.float64),
+        "key_lo": (keys[rows] & np.uint64(0xFFFFFFFF)).astype(np.float64),
+        "reads": counts[rows].astype(np.float64),
+        "first_read": first[rows].astype(np.float64),
+        "matched_idx1_row": res["m1"][rows].astype(np.float32),
+        "matched_idx2_row": res["m2"][rows].astype(np.float32),
+        "read_type": res["type"][rows].astype(np.float32),
+        "sample_row": res["srow"][rows].astype(np.float32),
+        "reads_per_read_type": np.bincount(res["type"], weights, minlength=4),
+        "reads_per_sample_row": np.bincount(res["srow"][demuxable], weights[demuxable], minlength=len(ctx.sheet.ids)),
+        "orientation_reads_f": last["f_sum"].astype(np.float64),
+        "orientation_reads_rc": last["rc_sum"].astype(np.float64),
+        "orientation_rc_call": last["use"].astype(np.float32),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 def run_b200(args):
     from frender_b200 import _lib as L
     from frender_b200 import synth
@@ -452,6 +501,8 @@ def run_b200(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of one process (--gpus 1)")
     dist = None
     if world > 1:
         import torch.distributed as dist  # host-side rendezvous only (gloo); the data path is NCCL in the .so
@@ -470,9 +521,17 @@ def run_b200(args):
     bytes_per_read = 375.0
     table_log2 = args.table_log2 or (26 if reads > 100_000_000 else (24 if reads > 8_000_000 else 21))
     overhead = 2 * (32 << table_log2) + (8 << 30)
-    fit = int((free_b.value - overhead) / bytes_per_read)
+    # sized by the device's total memory, not by what is free at the moment: the same arguments on the same GPU model
+    # give the same lane, so that two runs (and two builds) compute on identical inputs
+    fit = int((total_b.value - overhead) / bytes_per_read)
     if reads > fit:
         reads = max(1_000_000, fit // 1_000_000 * 1_000_000)
+    cap = int(reads * 374.6) + (64 << 20)
+    need = cap + 2 * (32 << table_log2)           # the resident lane + the two unique-key tables
+    if need > free_b.value:                       # memory held by other processes on this GPU
+        raise SystemExit(f"bench.py: the {reads}-read lane needs {need / 1e9:.1f} GB of device memory, but only "
+                         f"{free_b.value / 1e9:.1f} GB of {total_b.value / 1e9:.1f} GB is free on GPU {local}; "
+                         f"free the GPU or pass a smaller --reads")
     ctx = Context(local, table_log2=table_log2)
     h = ctx._h
     ck = ctx._ck
@@ -484,7 +543,6 @@ def run_b200(args):
     vp = lambda a: a.ctypes.data_as(C.c_void_p)
     ck(lib.frb_synth_load(h, spec.seed, spec.l1, spec.l2, spec.n_samples, vp(emit_i7), vp(emit_i5), vp(cdf),
                           spec.lane, spec.read_len, spec.sub_t, spec.n_t, spec.rand_t, spec.hop_t))
-    cap = int(reads * 374.6) + (64 << 20)
     dbuf = C.c_void_p()
     ck(lib.frb_dev_alloc(h, cap, C.byref(dbuf)))
     g_base = rank * reads
@@ -512,6 +570,8 @@ def run_b200(args):
         if dist:
             dist.barrier()
 
+    last = {}       # orientation sums and calls of the latest step (--dump-outputs)
+
     def analyze(want_outputs):
         """matcher pass 1 (rc) -> orientation call -> pass 2; returns unique count"""
         r = ctx.match(N_SUBS, True, None, want_outputs=False)
@@ -519,6 +579,7 @@ def run_b200(args):
         if world > 1:   # every rank matched its share of the merged keys: the call is over the whole job
             f_sum, rc_sum = ctx.allreduce(f_sum), ctx.allreduce(rc_sum)
         use = np.array([f_sum[g] < rc_sum[g] for g in sheet.group], np.uint8)               # F:376
+        last.update(f_sum=f_sum, rc_sum=rc_sum, use=use)
         out = ctx.match(N_SUBS, False, use, want_outputs=want_outputs)
         return out
 
@@ -573,6 +634,10 @@ def run_b200(args):
     prof = {k: ctx.prof_read(k, reset=True) for k in range(L.K_NUM)}
     n_uniq = C.c_uint64()
     ck(lib.frb_total_finish(h, C.byref(n_uniq)))
+    if args.dump_outputs:
+        # the step's own matcher sequence on the list the last timed step left resident: rc pass -> orientation call
+        # -> oriented pass, which reuses the rc pass's idx1 verdicts exactly as inside the step
+        dump_outputs(args.dump_outputs, ctx, got_reads, analyze(True), last)
     if dist:    # the shares are disjoint: the job's unique keys are their sum
         box = [None] * world
         dist.all_gather_object(box, n_uniq.value)

@@ -41,6 +41,15 @@ SIGNATURES = {
     "frb_write_scan_csv": (C.c_int, [C.c_char_p, vp, vp, vp, vp, vp, vp, vp, u64, vp, vp, vp, u32, C.c_int]),
     "frb_pack_key": (C.c_int, [C.c_char_p, C.c_size_t, C.c_int, P(u64)]),
     "frb_unpack_key": (C.c_int, [u64, C.c_char_p]),
+    "frb_pack_key2": (C.c_int, [C.c_char_p, C.c_size_t, C.c_int, P(u64), P(u64)]),
+    "frb_unpack_key2": (C.c_int, [u64, u64, C.c_char_p]),
+    "frb_write_scan_csv2": (C.c_int, [C.c_char_p, vp, vp, vp, vp, vp, vp, vp, vp, u64, vp, vp, vp, u32, C.c_int]),
+    "frb_set_key_width": (C.c_int, [vp, u32]),
+    "frb_file_export_hi": (C.c_int, [vp, u32, vp, u64]),
+    "frb_total_export_hi": (C.c_int, [vp, vp, u64]),
+    "frb_total_load2": (C.c_int, [vp, vp, vp, vp, u64]),
+    "frb_sheet_load2": (C.c_int, [vp, vp, vp, vp, vp, vp, u32, u32, u32]),
+    "frb_route_load2": (C.c_int, [vp, vp, vp, vp, u64, u32]),
     "frb_scan_begin": (C.c_int, [vp, u32, u64]),
     "frb_scan_chunk_host": (C.c_int, [vp, vp, u64, u64, C.c_int]),
     "frb_scan_chunk_dev": (C.c_int, [vp, vp, u64, u64, C.c_int, vp, vp]),

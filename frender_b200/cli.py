@@ -19,7 +19,8 @@ from pathlib import Path
 import numpy as np
 
 from . import _lib
-from .engine import Context, FrbError, READ_TYPES, pack_keys, reverse_complement, unpack_keys
+from .engine import (Context, FrbError, MAX_SYMS as _MAX_SYMS, READ_TYPES, pack_keys, pack_keys2, reverse_complement,
+                     unpack_keys)
 
 STAMP = "%Y-%M-%d_%H%M_%Z"          # sic: minutes where the month should be (F:599, F:912)
 MIN_CHUNK = 1 << 20                  # smallest demux window (bytes per mate)
@@ -150,8 +151,10 @@ class ScanTables:
     """Results of the tally as arrays: total list + per-file lists (dict semantics of
     barcode_counter: a repeated basename keeps its first position and the last file's counts)."""
 
-    def __init__(self, names, total, per_file):
+    def __init__(self, names, total, per_file, keys_hi=None):
         self.keys, self.counts = total
+        self.keys_hi = keys_hi          # upper words of a wide context's keys, else None
+        self.names = list(names)
         slot = {}
         for i, name in enumerate(names):
             slot.setdefault(name, len(slot))
@@ -162,7 +165,8 @@ class ScanTables:
     @classmethod
     def from_ctx(cls, ctx, names):
         keys, counts, _ = ctx.total_arrays()
-        return cls(names, (keys, counts), [ctx.file_arrays(i)[:2] for i in range(len(names))])
+        keys_hi = ctx.total_keys_hi() if ctx.wide else None
+        return cls(names, (keys, counts), [ctx.file_arrays(i)[:2] for i in range(len(names))], keys_hi)
 
 
 def _scan_worker(rank, n_ranks, device, ident, jobs, sample, table_log2, conn):
@@ -350,7 +354,18 @@ def demux_ok_flags(ctx, tables, sheet_ids, prefix):
     files = tables.file_names
     if not files:
         return np.ones(len(tables.keys), bool), set()
-    ok, bad, err_row = ctx.demux_ok(class_file_matrix(files, sheet_ids, prefix), tables.files)
+    if ctx.wide:
+        # the context's own per-file lists, one per file scanned; a file whose basename a later file repeats is not
+        # part of barcode_counter (F:205) and fits every class
+        files = tables.names
+        match = class_file_matrix(files, sheet_ids, prefix)
+        last = {name: i for i, name in enumerate(files)}
+        for i, name in enumerate(files):
+            if last[name] != i:
+                match[:, i] = 1
+        ok, bad, err_row = ctx.demux_ok(match)
+    else:
+        ok, bad, err_row = ctx.demux_ok(class_file_matrix(files, sheet_ids, prefix), tables.files)
     if err_row is not None:
         re.compile(sheet_ids[err_row].removeprefix(prefix), re.I)   # raises what the reference's re.search raises
     return ok, {files[f] for f in np.flatnonzero(bad)}
@@ -426,6 +441,10 @@ def concurrent_streams(cores, files):
 
 def tally_files(ctx, files, names, sample, cores, n_gpus):
     """tally_barcodes (F:183-207) over the three ways of spreading the files: ranks, `-c` streams, one by one."""
+    if ctx.wide and (n_gpus > 1 or cores > 1):
+        print("Index fields longer than 21 symbols: one GPU, one inflate stream "
+              "(FRENDER_GPUS / -c over 128-bit keys are not supported yet).")
+        return tally_files(ctx, files, names, sample, 1, 1)
     if n_gpus > 1:
         per_file, total = scan_files_multi_gpu(files, sample, n_gpus, ctx.table_log2)
         for ordinal, name in enumerate(names):
@@ -500,6 +519,10 @@ def frender_scan(args, ctx=None):
             print(f"Sampling {sample} reads from the head of each file...")
         names = [os.path.basename(str(path)) for path in files]
         n_gpus = min(int(os.environ.get("FRENDER_GPUS", "1")), max(len(files), 1))
+        l1 = len(indexes["idx1"][0]) if len(indexes["idx1"]) else 0
+        l2 = len(indexes["idx2"][0]) if indexes.get("idx2") is not None and len(indexes["idx2"]) else 0
+        if l1 + (1 + l2 if l2 else 0) > _MAX_SYMS and not ctx.wide:
+            ctx.set_wide()        # the sheet's own keys need 128-bit keys
         while True:
             # A dict never refuses a key (F:172-177): when the unique-key tables turn out too small for the
             # input they are re-created four times as large and the tally starts over.
@@ -508,6 +531,13 @@ def frender_scan(args, ctx=None):
                 tables = tally_files(ctx, files, names, sample, cores, n_gpus)
                 break
             except (FrbError, SystemExit) as exc:
+                # a GPU worker of a multi-GPU run reports its error as text (SystemExit)
+                too_long = (isinstance(exc, FrbError) and exc.code == _lib.ERR_KEY_TOO_LONG) or (
+                    isinstance(exc, SystemExit) and "index field longer than 21 symbols" in str(exc))
+                if too_long and not ctx.wide:
+                    print("\nindex fields longer than 21 symbols: tallying again with 128-bit keys")
+                    ctx.set_wide()
+                    continue
                 full = (isinstance(exc, FrbError) and exc.code == _lib.ERR_TABLE_FULL) or "unique-key table full" in str(exc)
                 if not full or ctx.table_log2 + 2 > 32:
                     raise
@@ -561,13 +591,15 @@ def write_scan_csv(path, tables, res, sheet, idx2_used, ok):
             arr[i] = item.encode()
         return arr
 
+    hi = None if tables.keys_hi is None else np.ascontiguousarray(tables.keys_hi, np.uint64)
     arrays = [np.ascontiguousarray(tables.keys, np.uint64), np.ascontiguousarray(tables.counts, np.uint64),
               np.ascontiguousarray(res["m1"], np.int32), np.ascontiguousarray(res["m2"], np.int32),
               np.ascontiguousarray(res["type"], np.uint8), np.ascontiguousarray(res["srow"], np.int32),
               np.ascontiguousarray(ok, np.uint8)]
-    rc = _lib.lib.frb_write_scan_csv(os.fsencode(str(path)), *[a.ctypes.data_as(C.c_void_p) for a in arrays], n,
-                                     strings(sheet.idx1), strings(idx2_used), strings(sheet.ids), len(sheet.ids),
-                                     1 if sheet.single else 0)
+    ptrs = [a.ctypes.data_as(C.c_void_p) for a in arrays]
+    rc = _lib.lib.frb_write_scan_csv2(os.fsencode(str(path)), ptrs[0], None if hi is None else hi.ctypes.data_as(C.c_void_p),
+                                      *ptrs[1:], n, strings(sheet.idx1), strings(idx2_used), strings(sheet.ids),
+                                      len(sheet.ids), 1 if sheet.single else 0)
     _lib.check(None, rc)
 
 
@@ -766,11 +798,15 @@ def frender_demux(args, ctx=None):
             return undeter_sink
         return reject
 
-    keys = pack_keys(list(table.keys()))
     routes = np.array([route_of(*v) for v in table.values()], np.uint32)
 
     own_ctx = ctx is None
     ctx = ctx or Context(int(os.environ.get("FRENDER_DEVICE", "0")), table_log2=12)
+    # keys longer than 21 symbols in the results table: the router takes 128-bit keys
+    wide = any(len(k) > _MAX_SYMS for k in table)
+    if wide != ctx.wide:
+        ctx.set_wide(wide)
+    keys, keys_hi = pack_keys2(list(table.keys())) if wide else (pack_keys(list(table.keys())), None)
     chunk = max(int(os.environ.get("FRENDER_DEMUX_CHUNK_MB", "64")) << 20, MIN_CHUNK)
     # Host side of the router: inflate of the two mates and deflate of the sinks run on a thread pool (zlib
     # releases the GIL).  Every sink sees the same sequence of compress() calls as a serial loop would make,
@@ -797,7 +833,7 @@ def frender_demux(args, ctx=None):
                 writes.append(pool.submit(sinks[s]["R2"].write, o2[off2[s]:off2[s + 1]]))
 
     try:
-        ctx.route_load(keys, routes, n_sinks + 1)
+        ctx.route_load(keys, routes, n_sinks + 1, keys_hi)
         for r1_path, r2_path in pairs:
             print(f"Demultiplexing {r1_path.name}...")
             # The pair as a STREAM of chunks, two in flight: while chunk k is routed on the device and chunk k-1

@@ -34,6 +34,18 @@ struct DevState {
     unsigned long long spec_err_pos;  // composite position of the first parse error seen in a guessed tile
     int spec_err_code;                // ... and its code; promoted to err_code once the guesses are confirmed
     int spec_bad;                     // a guess of the current chunk was wrong: the chunk is redone by count
+    unsigned long long err_hi;        // wide context: upper word of the key of the first error (err_pos holds lo)
+};
+
+// Slot of a wide context's table (keys of up to 42 symbols, see frender_b200.h): same 32 bytes as Slot, so both
+// layouts share one allocation.  (lo, hi) is claimed with one 128-bit compare-and-swap; lo = FRB_EMPTY_KEY is free.
+struct __align__(32) WideSlot {
+    unsigned long long lo, hi;  // packed key: symbols 0..20 / 21..41
+    unsigned long long first;   // smallest read position seen
+    unsigned long long count;   // reads carrying the key
+};
+struct __align__(16) Key128 {
+    unsigned long long lo, hi;
 };
 
 // Position of a read inside a file as the speculative path records it: (tile index in the file << 13) | index of
@@ -43,6 +55,7 @@ constexpr int kCompositeShift = 13;  // a 30 KiB tile holds at most 7680 headers
 
 constexpr unsigned long long kEmpty = FRB_EMPTY_KEY;
 constexpr int kMaxSyms = 21;
+constexpr int kMaxWideSyms = 2 * kMaxSyms;
 constexpr uint32_t kMaxProbe = 1u << 15;
 
 // Symbol codes.  enc_read(): strict read alphabet, 0 = not allowed.
@@ -105,6 +118,39 @@ __device__ __noinline__ void table_add(Slot* __restrict__ tab, unsigned long lon
         h = (h + 1) & mask;
     }
     raise_error(st, FRB_ERR_TABLE_FULL, key);
+}
+
+// Wide keys: the first error also records the key's upper word.
+__device__ __forceinline__ void raise_error_wide(DevState* st, int code, unsigned long long pos, unsigned long long hi) {
+    if (atomicCAS(&st->err_code, 0, code) == 0) st->err_pos = pos, st->err_hi = hi;
+}
+
+// table_add for a wide context, inlined (a call would spill in the scan kernels).  A key with hi = 0 hashes as its
+// narrow twin.  One 16-byte load per probe;
+// a free slot is claimed with one 128-bit compare-and-swap on (lo, hi).
+__device__ __forceinline__ void table_add_wide(WideSlot* __restrict__ tab, unsigned long long mask, unsigned long long lo,
+                                            unsigned long long hi, unsigned long long cnt, unsigned long long pos,
+                                            unsigned long long* occupied, DevState* st) {
+    unsigned long long h = hash64(lo ^ (hi * 0x9E3779B97F4A7C15ULL)) & mask;
+    for (uint32_t probe = 0; probe < kMaxProbe; ++probe) {
+        unsigned long long klo, khi;
+        asm volatile("ld.volatile.global.v2.u64 {%0, %1}, [%2];" : "=l"(klo), "=l"(khi) : "l"(&tab[h].lo));
+        if (klo == kEmpty) {
+            const Key128 old = atomicCAS(reinterpret_cast<Key128*>(&tab[h].lo), Key128{kEmpty, 0ULL}, Key128{lo, hi});
+            klo = old.lo, khi = old.hi;
+            if (klo == kEmpty) {
+                atomicAdd(occupied, 1ULL);
+                klo = lo, khi = hi;
+            }
+        }
+        if (klo == lo && khi == hi) {
+            atomicAdd(&tab[h].count, cnt);
+            atomicMin(&tab[h].first, pos);
+            return;
+        }
+        h = (h + 1) & mask;
+    }
+    raise_error_wide(st, FRB_ERR_TABLE_FULL, lo, hi);
 }
 #endif
 

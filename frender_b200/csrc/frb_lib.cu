@@ -39,6 +39,7 @@ thread_local std::string g_last_error;
 
 struct KeyList {  // device arrays of one (key,count,first) list
     unsigned long long *keys = nullptr, *counts = nullptr, *first = nullptr;
+    unsigned long long* keys_hi = nullptr;  // upper key words, wide context only
     uint64_t n = 0, reads = 0;
     uint32_t ordinal = 0;
     bool sorted = true;   // in first-appearance order (a file's list is sorted when somebody first needs the order)
@@ -57,6 +58,7 @@ struct frb_ctx {
     cudaStream_t compute = nullptr, copy = nullptr;
     uint32_t log2 = 0;
     uint64_t cap = 0;
+    bool wide = false;  // keys of up to 42 symbols: WideSlot tables, (lo, hi) lists (frb_set_key_width)
     Slot *file_tab = nullptr, *total_tab = nullptr;
     DevState* st = nullptr;
     DevState* st_host = nullptr;  // pinned mirror
@@ -93,6 +95,7 @@ struct frb_ctx {
     uint64_t cur_limit = ~0ULL;
     // sheet
     unsigned long long *sheet_fwd = nullptr, *sheet_rc = nullptr;
+    unsigned long long *sheet_fwd_hi = nullptr, *sheet_rc_hi = nullptr;
     int* sheet_group = nullptr;
     unsigned char* sheet_use_rc = nullptr;
     unsigned long long *f_sum = nullptr, *rc_sum = nullptr;
@@ -213,8 +216,8 @@ int device_error_check(frb_ctx* c) {  // compute stream must be idle
     const int code = c->st_host->err_code;
     if (code == 0) return FRB_OK;
     const unsigned long long pos = c->st_host->err_pos;
-    char keytxt[24];
-    frb_unpack_key(pos, keytxt);
+    char keytxt[48];
+    frb_unpack_key2(pos, c->wide ? c->st_host->err_hi : 0ULL, keytxt);
     // clear so that the context stays usable after the caller handled the error
     CU(c, cudaMemsetAsync(&c->st->err_code, 0, sizeof(int), c->compute));
     switch (code) {
@@ -223,7 +226,7 @@ int device_error_check(frb_ctx* c) {  // compute stream must be idle
         case FRB_ERR_BAD_ALPHABET:
             return fail(c, code, "read %llu: index field holds a symbol outside ACGTN+", pos);
         case FRB_ERR_KEY_TOO_LONG:
-            return fail(c, code, "read %llu: index field longer than 21 symbols", pos);
+            return fail(c, code, "read %llu: index field longer than %d symbols", pos, c->wide ? kMaxWideSyms : kMaxSyms);
         case FRB_ERR_TABLE_FULL:
             return fail(c, code, "unique-key table full (2^%u slots): frb_resize_tables / FRENDER_TABLE_LOG2 for a larger one",
                         c->log2);
@@ -254,13 +257,17 @@ int free_list(frb_ctx* c, KeyList& l) {
     TRY(dfree(c, l.keys));
     TRY(dfree(c, l.counts));
     TRY(dfree(c, l.first));
+    TRY(dfree(c, l.keys_hi));
     l = KeyList{};
     return FRB_OK;
 }
 
 int clear_table(frb_ctx* c, Slot* tab) {
     ProfScope ps(c, FRB_K_OTHER);
-    clear_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(tab, c->cap);
+    if (c->wide)
+        clear_wide_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(reinterpret_cast<WideSlot*>(tab), c->cap);
+    else
+        clear_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(tab, c->cap);
     c->launches++;
     CU(c, cudaGetLastError());
     return FRB_OK;
@@ -280,7 +287,7 @@ int ensure_cub_tmp(frb_ctx* c, size_t bytes) {
 // Dense (key,count,first) arrays in arbitrary order -> list sorted by `first` (first-appearance order,
 // F:172-177 / F:199-205).  Takes over k0/c0/f0 (pool allocations) and frees them.
 int unsorted_to_sorted_list(frb_ctx* c, unsigned long long* k0, unsigned long long* c0, unsigned long long* f0,
-                            uint64_t n, KeyList* out, int first_bits = 64) {
+                            uint64_t n, KeyList* out, int first_bits = 64, unsigned long long* h0 = nullptr) {
     out->n = n;
     unsigned *i0 = nullptr, *i1 = nullptr;
     if (n) {
@@ -302,11 +309,17 @@ int unsorted_to_sorted_list(frb_ctx* c, unsigned long long* k0, unsigned long lo
         gather2_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(i1, k0, c0, out->keys,
                                                                                        out->counts, n);
         c->launches += 9;  // iota, cub radix sort passes (approximate), gather
+        if (h0) {  // a wide list: the upper key words follow the same permutation
+            TRY(dmalloc(c, &out->keys_hi, n * 8));
+            gather1_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(i1, h0, out->keys_hi, n);
+            c->launches++;
+        }
         CU(c, cudaGetLastError());
     }
     TRY(dfree(c, k0));
     TRY(dfree(c, c0));
     TRY(dfree(c, f0));
+    TRY(dfree(c, h0));
     if (i0) TRY(dfree(c, i0));
     if (i1) TRY(dfree(c, i1));
     return FRB_OK;
@@ -320,8 +333,8 @@ int ensure_sorted(frb_ctx* c, KeyList& l) {
     }
     KeyList tmp = l;
     KeyList out = l;
-    out.keys = out.counts = out.first = nullptr;
-    TRY(unsorted_to_sorted_list(c, tmp.keys, tmp.counts, tmp.first, tmp.n, &out, l.first_bits));  // frees tmp's arrays
+    out.keys = out.counts = out.first = out.keys_hi = nullptr;
+    TRY(unsorted_to_sorted_list(c, tmp.keys, tmp.counts, tmp.first, tmp.n, &out, l.first_bits, tmp.keys_hi));  // frees tmp's arrays
     out.sorted = true;
     l = out;
     return FRB_OK;
@@ -333,19 +346,24 @@ int table_to_sorted_list(frb_ctx* c, Slot* tab, uint64_t n, KeyList* out, int fi
     out->n = n;
     if (n == 0) return FRB_OK;
     if (n >= (1ULL << 32)) return fail(c, FRB_ERR_ARG, "more than 2^32 unique keys");
-    unsigned long long *k0 = nullptr, *c0 = nullptr, *f0 = nullptr;
+    unsigned long long *k0 = nullptr, *c0 = nullptr, *f0 = nullptr, *h0 = nullptr;
     TRY(dmalloc(c, &k0, n * 8));
     TRY(dmalloc(c, &c0, n * 8));
     TRY(dmalloc(c, &f0, n * 8));
+    if (c->wide) TRY(dmalloc(c, &h0, n * 8));
     {
         ProfScope ps(c, FRB_K_EXPORT);
         CU(c, cudaMemsetAsync(&c->st->scratch, 0, 8, c->compute));
-        compact_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(
-            tab, c->cap, k0, c0, f0, &c->st->scratch, n, tile_first);
+        if (c->wide)
+            compact_wide_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(
+                reinterpret_cast<const WideSlot*>(tab), c->cap, k0, h0, c0, f0, &c->st->scratch, n);
+        else
+            compact_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(
+                tab, c->cap, k0, c0, f0, &c->st->scratch, n, tile_first);
         c->launches++;
         CU(c, cudaGetLastError());
     }
-    return unsorted_to_sorted_list(c, k0, c0, f0, n, out, first_bits);
+    return unsorted_to_sorted_list(c, k0, c0, f0, n, out, first_bits, h0);
 }
 
 // The same when the number of occupied slots is not known: one pass over the table compacts and counts at once
@@ -354,15 +372,20 @@ int table_to_sorted_list_counting(frb_ctx* c, Slot* tab, uint64_t bound, KeyList
                                   const unsigned long long* tile_first) {
     bound = std::max<uint64_t>(std::min<uint64_t>(bound, c->cap), 1);
     if (bound >= (1ULL << 32)) return fail(c, FRB_ERR_ARG, "more than 2^32 unique keys");
-    unsigned long long *k0 = nullptr, *c0 = nullptr, *f0 = nullptr;
+    unsigned long long *k0 = nullptr, *c0 = nullptr, *f0 = nullptr, *h0 = nullptr;
     TRY(dmalloc(c, &k0, bound * 8));
     TRY(dmalloc(c, &c0, bound * 8));
     TRY(dmalloc(c, &f0, bound * 8));
+    if (c->wide) TRY(dmalloc(c, &h0, bound * 8));
     {
         ProfScope ps(c, FRB_K_EXPORT);
         CU(c, cudaMemsetAsync(&c->st->scratch, 0, 8, c->compute));
-        compact_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(
-            tab, c->cap, k0, c0, f0, &c->st->scratch, bound, tile_first);
+        if (c->wide)
+            compact_wide_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(
+                reinterpret_cast<const WideSlot*>(tab), c->cap, k0, h0, c0, f0, &c->st->scratch, bound);
+        else
+            compact_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(
+                tab, c->cap, k0, c0, f0, &c->st->scratch, bound, tile_first);
         c->launches++;
         CU(c, cudaGetLastError());
     }
@@ -373,7 +396,7 @@ int table_to_sorted_list_counting(frb_ctx* c, Slot* tab, uint64_t bound, KeyList
                                (unsigned long long)bound);
     // left in slot order: sorted by first appearance when somebody needs the order (ensure_sorted); a sharded
     // merge does not
-    out->keys = k0, out->counts = c0, out->first = f0, out->n = n;
+    out->keys = k0, out->counts = c0, out->first = f0, out->keys_hi = h0, out->n = n;
     out->sorted = false;
     out->first_bits = first_bits;
     return FRB_OK;
@@ -432,7 +455,7 @@ int launch_scan(frb_ctx* c, const unsigned char* dev, uint64_t nbytes, uint64_t 
     }
     // the lean (speculative) instantiation serves the tally of whole files: scan rule, no per-read outputs, no -s
     static const bool probe = getenv("FRB_SCAN_TIMING") && strcmp(getenv("FRB_SCAN_TIMING"), "spec") == 0;
-    const bool lean = lean_ok && (!a.timing || probe) && !no_guess && rule == FRB_RULE_SCAN && !keys_out && !rec_off_out && !skip_ptr &&
+    const bool lean = !c->wide && lean_ok && (!a.timing || probe) && !no_guess && rule == FRB_RULE_SCAN && !keys_out && !rec_off_out && !skip_ptr &&
                       c->cur_limit == ~0ULL && table != nullptr && table == c->file_tab && c->in_file;
     if (table == c->file_tab && c->in_file) {
         if (c->file_composite < 0) c->file_composite = lean ? 1 : 0;
@@ -442,10 +465,15 @@ int launch_scan(frb_ctx* c, const unsigned char* dev, uint64_t nbytes, uint64_t 
     if (!lean) {
         CU(c, cudaMemsetAsync(c->status, 0, (n_tiles + 1) * 8, c->compute));
         ProfScope ps(c, FRB_K_SCAN);
-        scan_ws_kernel<WsTile><<<grid, WsTile::threads, WsTile::smem, c->compute>>>(a);
         // tiles the kernel left out (empty list unless the input is not well-formed FASTQ or has lines shorter
-        // than 24 bytes on average)
-        scan_redo_kernel<<<c->sm_count, 64, 0, c->compute>>>(a);
+        // than 24 bytes on average) go to the redo kernel
+        if (c->wide && rule != kRuleOffsetsOnly) {  // record offsets alone need no key of either width
+            scan_ws_kernel<WsTileWide><<<grid, WsTileWide::threads, WsTileWide::smem, c->compute>>>(a);
+            scan_redo_wide_kernel<<<c->sm_count, 64, 0, c->compute>>>(a);
+        } else {
+            scan_ws_kernel<WsTile><<<grid, WsTile::threads, WsTile::smem, c->compute>>>(a);
+            scan_redo_kernel<<<c->sm_count, 64, 0, c->compute>>>(a);
+        }
         c->launches += 2;
     } else {
         // room for the first read ordinal of every tile of the file
@@ -605,11 +633,13 @@ int frb_create(int device, uint32_t table_log2, frb_ctx** out) {
     CU(c, cudaEventCreate(&c->t0));
     CU(c, cudaEventCreate(&c->t1));
     CU(c, cudaFuncSetAttribute(scan_ws_kernel<WsTile>, cudaFuncAttributeMaxDynamicSharedMemorySize, WsTile::smem));
+    CU(c, cudaFuncSetAttribute(scan_ws_kernel<WsTileWide>, cudaFuncAttributeMaxDynamicSharedMemorySize, WsTileWide::smem));
     CU(c, cudaFuncSetAttribute(scan_spec_kernel<WsTile>, cudaFuncAttributeMaxDynamicSharedMemorySize, WsTile::smem));
     CU(c, cudaFuncSetAttribute(scan_spec_kernel<WsTile, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, WsTile::smem));
     CU(c, cudaFuncSetAttribute(match_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     CU(c, cudaFuncSetAttribute(match_cand_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     CU(c, cudaFuncSetAttribute(match_idx1_cand_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    CU(c, cudaFuncSetAttribute(match_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
     TRY(clear_table(c, c->total_tab));
     CU(c, cudaStreamSynchronize(c->compute));
     *out = c;
@@ -630,6 +660,7 @@ void frb_destroy(frb_ctx* c) {
         if (c->ring[i]) cudaFreeHost(c->ring[i]);
     }
     cudaFree(c->sheet_fwd), cudaFree(c->sheet_rc), cudaFree(c->sheet_group), cudaFree(c->sheet_use_rc);
+    cudaFree(c->sheet_fwd_hi), cudaFree(c->sheet_rc_hi);
     cudaFree(c->f_sum), cudaFree(c->rc_sum);
     cudaFree(c->m1), cudaFree(c->m2), cudaFree(c->srow), cudaFree(c->m2rc), cudaFree(c->srowrc);
     cudaFree(c->type), cudaFree(c->typerc), cudaFree(c->work), cudaFree(c->work_n), cudaFree(c->cub_tmp), cudaFree(c->route_tab);
@@ -738,6 +769,40 @@ int frb_unpack_key(uint64_t key, char* out) {
     return n;
 }
 
+int frb_pack_key2(const char* s, size_t len, int sheet_mode, uint64_t* lo, uint64_t* hi) {
+    if (len > static_cast<size_t>(kMaxWideSyms)) return FRB_ERR_KEY_TOO_LONG;
+    const size_t n0 = std::min<size_t>(len, kMaxSyms);
+    TRY(frb_pack_key(s, n0, sheet_mode, lo));
+    return frb_pack_key(s + n0, len - n0, sheet_mode, hi);
+}
+int frb_unpack_key2(uint64_t lo, uint64_t hi, char* out) {
+    const int n = frb_unpack_key(lo, out);
+    return n < kMaxSyms ? n : n + frb_unpack_key(hi, out + n);
+}
+
+int frb_set_key_width(frb_ctx* c, uint32_t bits) {
+    CU(c, cudaSetDevice(c->device));
+    if (bits != 64 && bits != 128) return fail(c, FRB_ERR_ARG, "key width must be 64 or 128 bits");
+    TRY(frb_reset(c));
+    CU(c, cudaStreamSynchronize(c->compute));
+    c->wide = bits == 128;
+    // the tables change layout: the total table is cleared in the new one (the per-file table at every frb_scan_begin)
+    TRY(clear_table(c, c->total_tab));
+    c->total_tab_clean = true;
+    if (c->route_tab) CU(c, cudaFree(c->route_tab));
+    c->route_tab = nullptr, c->route_cap = 0, c->n_sinks = 0;
+    route_stream_destroy(c);  // its key buffer is sized for one width
+    // the sample sheet is packed for one width: it has to be loaded again
+    cudaFree(c->sheet_fwd), cudaFree(c->sheet_rc), cudaFree(c->sheet_group), cudaFree(c->sheet_use_rc);
+    cudaFree(c->f_sum), cudaFree(c->rc_sum), cudaFree(c->sheet_fwd_hi), cudaFree(c->sheet_rc_hi);
+    c->sheet_fwd = c->sheet_rc = nullptr, c->sheet_group = nullptr, c->sheet_use_rc = nullptr;
+    c->f_sum = c->rc_sum = nullptr, c->sheet_fwd_hi = c->sheet_rc_hi = nullptr;
+    c->rows = c->l1 = c->l2 = 0;
+    c->total_gen++, c->sheet_gen++;
+    CU(c, cudaStreamSynchronize(c->compute));
+    return FRB_OK;
+}
+
 // ---- hot path A -----------------------------------------------------------------------------
 int frb_scan_begin(frb_ctx* c, uint32_t file_ordinal, uint64_t read_limit) {
     CU(c, cudaSetDevice(c->device));
@@ -758,6 +823,8 @@ int frb_scan_chunk_dev(frb_ctx* c, const void* dev, uint64_t nbytes, uint64_t li
                        uint64_t* keys_out_dev, uint64_t* rec_off_out_dev) {
     CU(c, cudaSetDevice(c->device));
     if (!c->in_file) return fail(c, FRB_ERR_STATE, "frb_scan_chunk: no file begun");
+    if (c->wide && keys_out_dev)
+        return fail(c, FRB_ERR_STATE, "frb_scan_chunk_dev: per-read keys are not available on a wide (128-bit key) context");
     return launch_scan(c, static_cast<const unsigned char*>(dev), nbytes, line_base, rule,
                        reinterpret_cast<unsigned long long*>(keys_out_dev),
                        reinterpret_cast<unsigned long long*>(rec_off_out_dev), c->file_tab, 0);
@@ -823,7 +890,8 @@ int frb_file_size(frb_ctx* c, uint32_t i, uint64_t* n_unique, uint64_t* n_reads)
     if (n_reads) *n_reads = c->files[i].reads;
     return FRB_OK;
 }
-static int export_list(frb_ctx* c, KeyList& l, uint64_t* keys, uint64_t* counts, uint64_t* first, uint64_t cap) {
+static int export_list(frb_ctx* c, KeyList& l, uint64_t* keys, uint64_t* counts, uint64_t* first, uint64_t cap,
+                       uint64_t* keys_hi = nullptr) {
     TRY(ensure_sorted(c, l));
     if (cap < l.n) return fail(c, FRB_ERR_ARG, "export buffer too small (%llu < %llu)", (unsigned long long)cap,
                                (unsigned long long)l.n);
@@ -832,6 +900,10 @@ static int export_list(frb_ctx* c, KeyList& l, uint64_t* keys, uint64_t* counts,
     if (keys) CU(c, cudaMemcpyAsync(keys, l.keys, l.n * 8, cudaMemcpyDeviceToHost, c->compute));
     if (counts) CU(c, cudaMemcpyAsync(counts, l.counts, l.n * 8, cudaMemcpyDeviceToHost, c->compute));
     if (first) CU(c, cudaMemcpyAsync(first, l.first, l.n * 8, cudaMemcpyDeviceToHost, c->compute));
+    if (keys_hi) {
+        if (l.keys_hi) CU(c, cudaMemcpyAsync(keys_hi, l.keys_hi, l.n * 8, cudaMemcpyDeviceToHost, c->compute));
+        else memset(keys_hi, 0, l.n * 8);  // a narrow context: every key fits the lower word
+    }
     CU(c, cudaStreamSynchronize(c->compute));
     return FRB_OK;
 }
@@ -839,15 +911,24 @@ int frb_file_export(frb_ctx* c, uint32_t i, uint64_t* keys, uint64_t* counts, ui
     if (i >= c->files.size()) return fail(c, FRB_ERR_ARG, "file index out of range");
     return export_list(c, c->files[i], keys, counts, first_read, cap);
 }
+int frb_file_export_hi(frb_ctx* c, uint32_t i, uint64_t* keys_hi, uint64_t cap) {
+    if (i >= c->files.size()) return fail(c, FRB_ERR_ARG, "file index out of range");
+    return export_list(c, c->files[i], nullptr, nullptr, nullptr, cap, keys_hi);
+}
 
 static int merge_pending_files(frb_ctx* c) {  // fold file lists into total_tab (F:199-203)
     for (; c->merged_upto < c->files.size(); ++c->merged_upto) {
         const KeyList& fl = c->files[c->merged_upto];
         if (!fl.n) continue;
         ProfScope ps(c, FRB_K_EXPORT);
-        merge_list_kernel<<<static_cast<unsigned>((fl.n + 255) / 256), 256, 0, c->compute>>>(
-            c->total_tab, c->cap - 1, fl.keys, fl.counts, fl.first, fl.n,
-            static_cast<unsigned long long>(fl.ordinal) << 40, &c->st->occupied_total, c->st);
+        if (c->wide)
+            merge_wide_list_kernel<<<static_cast<unsigned>((fl.n + 255) / 256), 256, 0, c->compute>>>(
+                reinterpret_cast<WideSlot*>(c->total_tab), c->cap - 1, fl.keys, fl.keys_hi, fl.counts, fl.first, fl.n,
+                static_cast<unsigned long long>(fl.ordinal) << 40, &c->st->occupied_total, c->st);
+        else
+            merge_list_kernel<<<static_cast<unsigned>((fl.n + 255) / 256), 256, 0, c->compute>>>(
+                c->total_tab, c->cap - 1, fl.keys, fl.counts, fl.first, fl.n,
+                static_cast<unsigned long long>(fl.ordinal) << 40, &c->st->occupied_total, c->st);
         c->launches++;
         c->total_tab_clean = false;
         CU(c, cudaGetLastError());
@@ -874,6 +955,10 @@ static int total_build(frb_ctx* c, bool need_order) {
                 ProfScope ps(c, FRB_K_EXPORT);
                 CU(c, cudaMemcpyAsync(c->total.keys, fl.keys, fl.n * 8, cudaMemcpyDeviceToDevice, c->compute));
                 CU(c, cudaMemcpyAsync(c->total.counts, fl.counts, fl.n * 8, cudaMemcpyDeviceToDevice, c->compute));
+                if (fl.keys_hi) {
+                    TRY(dmalloc(c, &c->total.keys_hi, fl.n * 8));
+                    CU(c, cudaMemcpyAsync(c->total.keys_hi, fl.keys_hi, fl.n * 8, cudaMemcpyDeviceToDevice, c->compute));
+                }
                 add_offset_kernel<<<static_cast<unsigned>((fl.n + 255) / 256), 256, 0, c->compute>>>(
                     fl.first, c->total.first, fl.n, static_cast<unsigned long long>(fl.ordinal) << 40);
                 c->launches++;
@@ -903,14 +988,27 @@ int frb_total_export(frb_ctx* c, uint64_t* keys, uint64_t* counts, uint64_t* fir
     if (!c->total_ready) return fail(c, FRB_ERR_STATE, "frb_total_export: call frb_total_finish first");
     return export_list(c, c->total, keys, counts, first_pos, cap);
 }
+int frb_total_export_hi(frb_ctx* c, uint64_t* keys_hi, uint64_t cap) {
+    if (!c->total_ready) return fail(c, FRB_ERR_STATE, "frb_total_export_hi: call frb_total_finish first");
+    return export_list(c, c->total, nullptr, nullptr, nullptr, cap, keys_hi);
+}
 int frb_total_load(frb_ctx* c, const uint64_t* keys, const uint64_t* counts, uint64_t n) {
+    return frb_total_load2(c, keys, nullptr, counts, n);
+}
+int frb_total_load2(frb_ctx* c, const uint64_t* keys, const uint64_t* keys_hi, const uint64_t* counts, uint64_t n) {
     CU(c, cudaSetDevice(c->device));
+    if (keys_hi && !c->wide) return fail(c, FRB_ERR_STATE, "frb_total_load2: upper key words need a wide context (frb_set_key_width)");
     TRY(free_list(c, c->total));
     c->total.n = n;
     if (n) {
         TRY(dmalloc(c, &c->total.keys, n * 8));
         TRY(dmalloc(c, &c->total.counts, n * 8));
         TRY(dmalloc(c, &c->total.first, n * 8));
+        if (c->wide) {
+            TRY(dmalloc(c, &c->total.keys_hi, n * 8));
+            if (keys_hi) CU(c, cudaMemcpyAsync(c->total.keys_hi, keys_hi, n * 8, cudaMemcpyHostToDevice, c->compute));
+            else CU(c, cudaMemsetAsync(c->total.keys_hi, 0, n * 8, c->compute));
+        }
         CU(c, cudaMemcpyAsync(c->total.keys, keys, n * 8, cudaMemcpyHostToDevice, c->compute));
         CU(c, cudaMemcpyAsync(c->total.counts, counts, n * 8, cudaMemcpyHostToDevice, c->compute));
         CU(c, cudaMemsetAsync(c->total.first, 0, n * 8, c->compute));
@@ -923,6 +1021,7 @@ int frb_total_load(frb_ctx* c, const uint64_t* keys, const uint64_t* counts, uin
 int frb_total_merge(frb_ctx* c, const uint64_t* keys, const uint64_t* counts, const uint64_t* first_pos, uint64_t n) {
     CU(c, cudaSetDevice(c->device));
     if (c->in_file) return fail(c, FRB_ERR_STATE, "frb_total_merge: a file is still open");
+    if (c->wide) return fail(c, FRB_ERR_STATE, "frb_total_merge: not available on a wide (128-bit key) context");
     if (n) {
         unsigned long long *dk = nullptr, *dc = nullptr, *df = nullptr;
         TRY(dmalloc(c, &dk, n * 8));
@@ -1311,15 +1410,26 @@ int frb_gz_inflate(frb_ctx* c, const char* path, void* host_out, uint64_t cap, u
 // ---- hot path B -----------------------------------------------------------------------------
 int frb_sheet_load(frb_ctx* c, const uint64_t* fwd, const uint64_t* rc, const int32_t* group, uint32_t n_rows,
                    uint32_t l1, uint32_t l2) {
+    return frb_sheet_load2(c, fwd, nullptr, rc, nullptr, group, n_rows, l1, l2);
+}
+int frb_sheet_load2(frb_ctx* c, const uint64_t* fwd, const uint64_t* fwd_hi, const uint64_t* rc, const uint64_t* rc_hi,
+                    const int32_t* group, uint32_t n_rows, uint32_t l1, uint32_t l2) {
     CU(c, cudaSetDevice(c->device));
-    if (l1 == 0 || l1 + (l2 ? 1 + l2 : 0) > kMaxSyms) return fail(c, FRB_ERR_ARG, "index lengths %u+%u unsupported (max 21 symbols incl. '+')", l1, l2);
+    if ((fwd_hi || rc_hi) && !c->wide) return fail(c, FRB_ERR_STATE, "frb_sheet_load2: upper key words need a wide context (frb_set_key_width)");
+    if (c->wide) {
+        if (l1 == 0 || l1 > kMaxSyms || l2 > kMaxSyms || l1 + (l2 ? 1 + l2 : 0) > kMaxWideSyms)
+            return fail(c, FRB_ERR_ARG, "index lengths %u+%u unsupported (max 21 symbols per index, 42 incl. '+')", l1, l2);
+    } else if (l1 == 0 || l1 + (l2 ? 1 + l2 : 0) > kMaxSyms) {
+        return fail(c, FRB_ERR_ARG, "index lengths %u+%u unsupported (max 21 symbols incl. '+')", l1, l2);
+    }
     if (n_rows > 5000) return fail(c, FRB_ERR_ARG, "sample sheet with %u rows exceeds the 5000-row limit", n_rows);
     for (uint32_t r = 0; r < n_rows; ++r)
         if (group[r] < 0 || static_cast<uint32_t>(group[r]) >= n_rows) return fail(c, FRB_ERR_ARG, "bad group id");
     CU(c, cudaStreamSynchronize(c->compute));
     cudaFree(c->sheet_fwd), cudaFree(c->sheet_rc), cudaFree(c->sheet_group), cudaFree(c->sheet_use_rc);
-    cudaFree(c->f_sum), cudaFree(c->rc_sum);
+    cudaFree(c->f_sum), cudaFree(c->rc_sum), cudaFree(c->sheet_fwd_hi), cudaFree(c->sheet_rc_hi);
     c->sheet_fwd = c->sheet_rc = nullptr, c->sheet_group = nullptr, c->sheet_use_rc = nullptr;
+    c->sheet_fwd_hi = c->sheet_rc_hi = nullptr;
     c->f_sum = c->rc_sum = nullptr;
     const size_t n = std::max<uint32_t>(n_rows, 1);
     CU(c, cudaMalloc(&c->sheet_fwd, n * 8));
@@ -1328,6 +1438,14 @@ int frb_sheet_load(frb_ctx* c, const uint64_t* fwd, const uint64_t* rc, const in
     CU(c, cudaMalloc(&c->sheet_use_rc, n));
     CU(c, cudaMalloc(&c->f_sum, n * 8));
     CU(c, cudaMalloc(&c->rc_sum, n * 8));
+    if (c->wide) {
+        CU(c, cudaMalloc(&c->sheet_fwd_hi, n * 8));
+        CU(c, cudaMalloc(&c->sheet_rc_hi, n * 8));
+        CU(c, cudaMemset(c->sheet_fwd_hi, 0, n * 8));
+        CU(c, cudaMemset(c->sheet_rc_hi, 0, n * 8));
+        if (n_rows && fwd_hi) CU(c, cudaMemcpy(c->sheet_fwd_hi, fwd_hi, n_rows * 8, cudaMemcpyHostToDevice));
+        if (n_rows && rc_hi) CU(c, cudaMemcpy(c->sheet_rc_hi, rc_hi, n_rows * 8, cudaMemcpyHostToDevice));
+    }
     if (n_rows) {
         CU(c, cudaMemcpy(c->sheet_fwd, fwd, n_rows * 8, cudaMemcpyHostToDevice));
         CU(c, cudaMemcpy(c->sheet_rc, rc, n_rows * 8, cudaMemcpyHostToDevice));
@@ -1385,6 +1503,23 @@ int frb_match(frb_ctx* c, uint32_t n_subs, int rc_mode, const uint8_t* use_rc_ro
         c->m1_total_gen = c->total_gen, c->m1_sheet_gen = c->sheet_gen, c->m1_n_subs = n_subs;
         c->m1_from_rc = rc_mode != 0;
         ProfScope ps(c, FRB_K_MATCH);
+        if (c->wide) {  // sweeps over the split idx1 / idx2 words (no candidate tables for wide keys)
+            WideMatchArgs w{a, c->total.keys_hi, c->sheet_fwd_hi, c->sheet_rc_hi};
+            if (!reuse) {
+                CU(c, cudaMemsetAsync(c->work_n, 0, 8, c->compute));
+                match_idx1_wide_kernel<<<grid_for(n, kMatchThreads, c->sm_count, 8), kMatchThreads,
+                                         static_cast<size_t>(c->rows) * 8 + 16, c->compute>>>(w);
+                c->launches++;
+            } else {
+                CU(c, cudaMemsetAsync(c->m2, 0xFF, n * 4, c->compute));
+                CU(c, cudaMemsetAsync(c->srow, 0xFF, n * 4, c->compute));
+                CU(c, cudaMemsetAsync(c->type, 0, n, c->compute));
+            }
+            match_wide_kernel<<<grid_for(n, kMatchThreads, c->sm_count, 8), kMatchThreads,
+                                static_cast<size_t>(c->rows) * (5 * 8 + 4) + 16, c->compute>>>(w);
+            c->launches++;
+            CU(c, cudaGetLastError());
+        } else {
         // candidate rows from per-part tables instead of a sweep over the sheet, whenever the shape allows
         static const bool sweep_only = getenv("FRB_MATCH") && strcmp(getenv("FRB_MATCH"), "sweep") == 0;
         const unsigned parts = n_subs + 1;
@@ -1415,6 +1550,7 @@ int frb_match(frb_ctx* c, uint32_t n_subs, int rc_mode, const uint8_t* use_rc_ro
         }
         c->launches++;
         CU(c, cudaGetLastError());
+        }
     }
     if (n) {
         if (m1_row) CU(c, cudaMemcpyAsync(m1_row, c->m1, n * 4, cudaMemcpyDeviceToHost, c->compute));
@@ -1446,11 +1582,12 @@ int frb_demux_ok(frb_ctx* c, const uint8_t* match, uint32_t n_files, const uint6
     if (n > c->match_cap || c->m1_total_gen != c->total_gen)
         return fail(c, FRB_ERR_STATE, "frb_demux_ok: frb_match over the current total list first");
     if (!file_keys && n_files != c->files.size()) return fail(c, FRB_ERR_ARG, "frb_demux_ok: %u files, context holds %zu", n_files, c->files.size());
+    if (file_keys && c->wide) return fail(c, FRB_ERR_STATE, "frb_demux_ok: host file lists are not available on a wide (128-bit key) context");
     if (err_row_out) *err_row_out = 0x7FFFFFFF;
     if (n_files) memset(bad_files_out, 0, n_files);
     if (!n || !n_files) return FRB_OK;
     const size_t classes = 4 + static_cast<size_t>(c->rows);
-    unsigned long long* sorted_keys = nullptr;
+    unsigned long long *sorted_keys = nullptr, *sorted_hi = nullptr, *hi_by_lo = nullptr;
     unsigned *i0 = nullptr, *i1 = nullptr;
     unsigned char *d_match = nullptr, *d_ok = nullptr, *d_bad = nullptr;
     int* d_err = nullptr;
@@ -1474,6 +1611,18 @@ int frb_demux_ok(frb_ctx* c, const uint8_t* match, uint32_t n_files, const uint6
         TRY(ensure_cub_tmp(c, tmp));
         CU(c, cub::DeviceRadixSort::SortPairs(c->cub_tmp, tmp, c->total.keys, sorted_keys, i0, i1, static_cast<int>(n), 0, 63,
                                               c->compute));
+        if (c->wide) {
+            // second, stable pass on the upper words: sorted by (hi, lo); i1 ends as the permutation of that order
+            TRY(dmalloc(c, &hi_by_lo, n * 8));
+            TRY(dmalloc(c, &sorted_hi, n * 8));
+            gather1_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(i1, c->total.keys_hi, hi_by_lo, n);
+            CU(c, cub::DeviceRadixSort::SortPairs(nullptr, tmp, hi_by_lo, sorted_hi, i1, i0, static_cast<int>(n), 0, 63, c->compute));
+            TRY(ensure_cub_tmp(c, tmp));
+            CU(c, cub::DeviceRadixSort::SortPairs(c->cub_tmp, tmp, hi_by_lo, sorted_hi, i1, i0, static_cast<int>(n), 0, 63, c->compute));
+            std::swap(i0, i1);
+            gather1_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(i1, c->total.keys, sorted_keys, n);
+            c->launches += 2;
+        }
         for (uint32_t f = 0; f < n_files; ++f) {
             const unsigned long long *fk = nullptr, *fc = nullptr;
             unsigned long long *up_k = nullptr, *up_c = nullptr;
@@ -1493,8 +1642,13 @@ int frb_demux_ok(frb_ctx* c, const uint8_t* match, uint32_t n_files, const uint6
                 if (!nf) continue;
                 fk = c->files[f].keys, fc = c->files[f].counts;
             }
-            demux_ok_kernel<<<static_cast<unsigned>((nf + 255) / 256), 256, 0, c->compute>>>(
-                fk, fc, nf, sorted_keys, i1, n, c->type, c->srow, d_match, n_files, f, d_ok, d_bad, d_err);
+            if (c->wide)
+                demux_ok_wide_kernel<<<static_cast<unsigned>((nf + 255) / 256), 256, 0, c->compute>>>(
+                    fk, c->files[f].keys_hi, fc, nf, sorted_keys, sorted_hi, i1, n, c->type, c->srow, d_match, n_files, f,
+                    d_ok, d_bad, d_err);
+            else
+                demux_ok_kernel<<<static_cast<unsigned>((nf + 255) / 256), 256, 0, c->compute>>>(
+                    fk, fc, nf, sorted_keys, i1, n, c->type, c->srow, d_match, n_files, f, d_ok, d_bad, d_err);
             c->launches++;
             if (up_k) TRY(dfree(c, up_k));
             if (up_c) TRY(dfree(c, up_c));
@@ -1508,6 +1662,8 @@ int frb_demux_ok(frb_ctx* c, const uint8_t* match, uint32_t n_files, const uint6
     CU(c, cudaStreamSynchronize(c->compute));
     if (err_row_out) *err_row_out = err_row == 0x7F7F7F7F ? 0x7FFFFFFF : err_row;
     TRY(dfree(c, sorted_keys));
+    TRY(dfree(c, sorted_hi));
+    TRY(dfree(c, hi_by_lo));
     TRY(dfree(c, i0));
     TRY(dfree(c, i1));
     TRY(dfree(c, d_match));

@@ -453,3 +453,161 @@ __global__ void __launch_bounds__(kMatchThreads) match_cand_kernel(const MatchAr
 }
 
 }  // namespace frb
+
+// =================================================================================================
+// Wide context: keys of up to 42 symbols as (lo, hi).  Every key is split into an idx1 word (symbols [0, l1)) and
+// an idx2 word (symbols [l1 + 1, l1 + 1 + l2)), each <= 21 symbols, and the sweep of match_idx1_kernel /
+// match_kernel runs on the split words with one mask per index.  Same shape check, same classification.
+// =================================================================================================
+namespace frb {
+
+struct WideMatchArgs {
+    MatchArgs m;                       // keys / sheet_fwd / sheet_rc hold the lo words
+    const unsigned long long* keys_hi;
+    const unsigned long long* sheet_fwd_hi;
+    const unsigned long long* sheet_rc_hi;
+};
+
+// symbols [p, p + l) of the 126-bit key (lo | hi << 63) as one word, l <= 21
+__device__ __forceinline__ unsigned long long wide_field(unsigned long long lo, unsigned long long hi, unsigned p, unsigned l) {
+    const unsigned __int128 v = static_cast<unsigned __int128>(lo) | (static_cast<unsigned __int128>(hi) << 63);
+    return static_cast<unsigned long long>(v >> (3 * p)) & ((1ULL << (3 * l)) - 1ULL);
+}
+
+// kernel 1: shape check, first idx1 row, work list
+__global__ void __launch_bounds__(kMatchThreads) match_idx1_wide_kernel(const WideMatchArgs w) {
+    const MatchArgs& a = w.m;
+    extern __shared__ __align__(16) unsigned char msmem[];
+    unsigned long long* s_1 = reinterpret_cast<unsigned long long*>(msmem);  // idx1 word of every row
+    for (unsigned r = threadIdx.x; r < a.rows; r += blockDim.x) s_1[r] = wide_field(a.sheet_fwd[r], w.sheet_fwd_hi[r], 0, a.l1);
+    __syncthreads();
+    const unsigned long long B1 = ((1ULL << (3 * a.l1)) - 1) & kFoldLsb;
+    const unsigned n_subs = a.n_subs;
+    const int lane = threadIdx.x & 31;
+    const unsigned long long stride = static_cast<unsigned long long>(gridDim.x) * blockDim.x;
+    const unsigned long long n_up = (a.n + 31) & ~31ULL;
+    for (unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x; i < n_up;
+         i += stride) {
+        int first1 = -1;
+        if (i < a.n) {
+            const unsigned long long lo = a.keys[i], hi = w.keys_hi[i];
+            if (a.rows) {  // as in match_idx1_kernel: l1 symbols, '+', l2 symbols, then end or '+'
+                bool ok = true;
+                const unsigned total = a.l2 ? a.l1 + 1 + a.l2 : a.l1;
+                for (unsigned s = 0; s < total; ++s) {
+                    const unsigned sym = static_cast<unsigned>(wide_field(lo, hi, s, 1));
+                    if (a.l2 && s == a.l1) ok &= (sym == 6);
+                    else ok &= (sym >= 1 && sym <= 5);
+                }
+                if (total < kMaxWideSyms) {
+                    const unsigned nxt = static_cast<unsigned>(wide_field(lo, hi, total, 1));
+                    ok &= a.l2 ? (nxt == 0 || nxt == 6) : (nxt == 0);
+                }
+                if (!ok) raise_error_wide(a.st, FRB_ERR_BAD_LENGTH, lo, hi);
+            }
+            const unsigned long long k1 = wide_field(lo, hi, 0, a.l1);
+            for (unsigned r = 0; r < a.rows; ++r) {
+                const bool h1 = static_cast<unsigned>(__popcll(fold3(k1 ^ s_1[r]) & B1)) <= n_subs;
+                if (h1 && first1 < 0) first1 = r;
+            }
+            a.m1[i] = first1;
+            if (first1 < 0) {
+                a.m2[i] = -1, a.srow[i] = -1, a.type[i] = FRB_TYPE_UNDETERMINED;
+                if (a.rc_mode) a.m2rc[i] = -1, a.srowrc[i] = -1, a.typerc[i] = FRB_TYPE_UNDETERMINED;
+            }
+        }
+        const unsigned need = __ballot_sync(0xFFFFFFFFu, first1 >= 0);
+        if (need) {
+            unsigned long long base = 0;
+            const int leader = __ffs(need) - 1;
+            if (lane == leader) base = atomicAdd(a.work_n, static_cast<unsigned long long>(__popc(need)));
+            base = __shfl_sync(0xFFFFFFFFu, base, leader);
+            if (first1 >= 0) a.work[base + __popc(need & ((1u << lane) - 1u))] = static_cast<unsigned>(i);
+        }
+    }
+}
+
+// kernel 2: full classification of the keys on the work list (rc-mode cross-ambiguity rule and group sums included)
+__global__ void __launch_bounds__(kMatchThreads) match_wide_kernel(const WideMatchArgs w) {
+    const MatchArgs& a = w.m;
+    extern __shared__ __align__(16) unsigned char msmem[];
+    unsigned long long* s_1 = reinterpret_cast<unsigned long long*>(msmem);  // idx1
+    unsigned long long* s_a = s_1 + a.rows;                                  // idx2 as supplied / oriented
+    unsigned long long* s_b = s_a + a.rows;                                  // idx2 reverse-complemented
+    unsigned long long* s_f = s_b + a.rows;                                  // per-group forward reads
+    unsigned long long* s_r = s_f + a.rows;                                  // per-group rc reads
+    int* s_g = reinterpret_cast<int*>(s_r + a.rows);
+    const unsigned p2 = a.l1 + 1;
+    for (unsigned r = threadIdx.x; r < a.rows; r += blockDim.x) {
+        const bool flip = a.use_rc && a.use_rc[r];
+        s_1[r] = wide_field(a.sheet_fwd[r], w.sheet_fwd_hi[r], 0, a.l1);
+        s_a[r] = flip ? wide_field(a.sheet_rc[r], w.sheet_rc_hi[r], p2, a.l2) : wide_field(a.sheet_fwd[r], w.sheet_fwd_hi[r], p2, a.l2);
+        s_b[r] = wide_field(a.sheet_rc[r], w.sheet_rc_hi[r], p2, a.l2);
+        s_f[r] = 0, s_r[r] = 0;
+        s_g[r] = a.group[r];
+    }
+    __syncthreads();
+    const unsigned long long B1 = ((1ULL << (3 * a.l1)) - 1) & kFoldLsb;
+    const unsigned long long B2 = ((1ULL << (3 * a.l2)) - 1) & kFoldLsb;
+    const unsigned n_subs = a.n_subs;
+    const unsigned long long n_work = *a.work_n;
+    const unsigned long long stride = static_cast<unsigned long long>(gridDim.x) * blockDim.x;
+    for (unsigned long long j = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x; j < n_work;
+         j += stride) {
+        const unsigned long long i = a.work[j];
+        const unsigned long long lo = a.keys[i], hi = w.keys_hi[i];
+        const unsigned long long k1 = wide_field(lo, hi, 0, a.l1), k2 = wide_field(lo, hi, p2, a.l2);
+        const int first1 = a.m1[i];
+        int firstf = -1, firstr = -1, rowf = -1, rowr = -1;
+        unsigned nf = 0, nr = 0;
+        if (first1 >= 0) {
+            for (unsigned r = 0; r < a.rows; ++r) {
+                const bool h1 = static_cast<unsigned>(__popcll(fold3(k1 ^ s_1[r]) & B1)) <= n_subs;
+                const bool h2 = a.l2 ? (static_cast<unsigned>(__popcll(fold3(k2 ^ s_a[r]) & B2)) <= n_subs) : true;
+                if (h2 && firstf < 0) firstf = r;
+                if (h1 && h2) {
+                    ++nf;
+                    if (rowf < 0) rowf = r;
+                }
+                if (a.rc_mode) {
+                    const bool h3 = static_cast<unsigned>(__popcll(fold3(k2 ^ s_b[r]) & B2)) <= n_subs;
+                    if (h3 && firstr < 0) firstr = r;
+                    if (h1 && h3) {
+                        ++nr;
+                        if (rowr < 0) rowr = r;
+                    }
+                }
+            }
+        }
+        int m1, m2, type, srow;
+        classify_one(first1, firstf, nf, rowf, &m1, &m2, &type, &srow);
+        if (a.rc_mode) {
+            int m1r, m2r, typer, srowr;
+            classify_one(first1, firstr, nr, rowr, &m1r, &m2r, &typer, &srowr);
+            if (m1 < 0) m1 = m1r;  // F:319-323
+            if (type == FRB_TYPE_DEMUXABLE && typer == FRB_TYPE_DEMUXABLE && s_g[srow] != s_g[srowr]) {
+                type = typer = FRB_TYPE_AMBIGUOUS;  // F:336-349
+                srow = srowr = -1;
+            }
+            const unsigned long long c = a.counts[i];
+            if (srow >= 0) atomicAdd(&s_f[s_g[srow]], c);      // F:370-371
+            if (srowr >= 0) atomicAdd(&s_r[s_g[srowr]], c);    // F:372-373
+            a.m2rc[i] = m2r;
+            a.typerc[i] = static_cast<unsigned char>(typer);
+            a.srowrc[i] = srowr;
+        }
+        a.m1[i] = m1;
+        a.m2[i] = m2;
+        a.type[i] = static_cast<unsigned char>(type);
+        a.srow[i] = srow;
+    }
+    if (a.rc_mode) {
+        __syncthreads();
+        for (unsigned g = threadIdx.x; g < a.rows; g += blockDim.x) {
+            if (s_f[g]) atomicAdd(&a.f_sum[g], s_f[g]);
+            if (s_r[g]) atomicAdd(&a.rc_sum[g], s_r[g]);
+        }
+    }
+}
+
+}  // namespace frb

@@ -61,6 +61,28 @@ __global__ void __launch_bounds__(256) route_build_kernel(Slot* tab, unsigned lo
     raise_error(st, FRB_ERR_TABLE_FULL, key);
 }
 
+// route_build_kernel for a wide context: (lo, hi) -> sink id in WideSlot.count, claimed with one 128-bit
+// compare-and-swap on a table filled with ones (no real key has bit 63 of either word set).
+__global__ void __launch_bounds__(256) route_build_wide_kernel(WideSlot* tab, unsigned long long mask,
+                                                               const unsigned long long* __restrict__ keys,
+                                                               const unsigned long long* __restrict__ keys_hi,
+                                                               const unsigned* __restrict__ sinks, unsigned long long n,
+                                                               DevState* st) {
+    const unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x;
+    if (i >= n) return;
+    const unsigned long long lo = keys[i], hi = keys_hi[i];
+    unsigned long long h = hash64(lo ^ (hi * 0x9E3779B97F4A7C15ULL)) & mask;
+    for (unsigned probe = 0; probe < kMaxProbe; ++probe) {
+        const Key128 k = atomicCAS(reinterpret_cast<Key128*>(&tab[h].lo), Key128{kEmpty, kEmpty}, Key128{lo, hi});
+        if ((k.lo == kEmpty && k.hi == kEmpty) || (k.lo == lo && k.hi == hi)) {
+            tab[h].count = sinks[i];
+            return;
+        }
+        h = (h + 1) & mask;
+    }
+    raise_error_wide(st, FRB_ERR_TABLE_FULL, lo, hi);
+}
+
 // The parser left n_reads / line_carry of the mate it just scanned in DevState: move them into the stream state
 // and clear them for the next launch.  which = 1 / 2.
 __global__ void route_grab_kernel(DevState* st, RouteState* rs, int which) {
@@ -151,6 +173,78 @@ __global__ void __launch_bounds__(kRouteBlock) route_hist_kernel(const Slot* __r
                 break;
             }
             if (k == kEmpty) break;
+            h = (h + 1) & mask;
+        }
+        if (s == 0xFFFFFFFFu) {
+            atomicMin(&rs->bad, i);
+            s = 0;
+        }
+        l1 = static_cast<unsigned>(off1[i + 1] - off1[i]);
+        l2 = static_cast<unsigned>(off2[i + 1] - off2[i]);
+        sink[i] = s;
+    }
+    for (int w = 0; w < kRouteBlock / 32; ++w) {
+        if (warp == w && i < n) {
+            const unsigned active = __activemask();
+            const unsigned same = __match_any_sync(active, s);
+            // bytes of the lower lanes of my sink
+            unsigned before1 = 0, before2 = 0, tot1 = 0, tot2 = 0;
+            for (unsigned m = same; m; m &= m - 1) {
+                const int src = __ffs(m) - 1;
+                const unsigned a1 = __shfl_sync(same, l1, src), a2 = __shfl_sync(same, l2, src);
+                if (src < lane) before1 += a1, before2 += a2;
+                tot1 += a1, tot2 += a2;
+            }
+            local1[i] = s_acc[s] + before1;
+            local2[i] = s_acc[n_sinks + s] + before2;
+            __syncwarp(active);
+            if (lane == __ffs(same) - 1) s_acc[s] += tot1, s_acc[n_sinks + s] += tot2;
+        }
+        __syncthreads();
+    }
+    for (unsigned k = threadIdx.x; k < n_sinks; k += kRouteBlock) {
+        cell[static_cast<unsigned long long>(k) * n_blocks + b] = s_acc[k];
+        cell[static_cast<unsigned long long>(n_sinks + k) * n_blocks + b] = s_acc[n_sinks + k];
+        if (s_acc[k]) atomicAdd(&tot[k], static_cast<unsigned long long>(s_acc[k]));
+        if (s_acc[n_sinks + k]) atomicAdd(&tot[n_sinks + k], static_cast<unsigned long long>(s_acc[n_sinks + k]));
+    }
+}
+
+// route_hist_kernel for a wide context: key2 holds rec_cap lower words, then rec_cap upper words; the results table
+// is a WideSlot table (sink id in `count`, free slots all ones).  Kept apart from the narrow kernel, whose code this
+// leaves exactly as it is.
+// sink of every record, its offset inside its (block, sink) cell, and the cells' sizes.  cell[(s * n_blocks + b)]
+// for mate 1, the same + n_sinks * n_blocks for mate 2.  One warp-step after the other inside a block, so that
+// records of one sink keep their order.
+__global__ void __launch_bounds__(kRouteBlock) route_hist_wide_kernel(const WideSlot* __restrict__ tab, unsigned long long mask,
+                                                                 const unsigned long long* __restrict__ key2,
+                                                                 unsigned long long rec_cap,
+                                                                 const unsigned long long* __restrict__ off1,
+                                                                 const unsigned long long* __restrict__ off2,
+                                                                 RouteState* rs, unsigned n_sinks, unsigned n_blocks,
+                                                                 unsigned* __restrict__ sink, unsigned* __restrict__ local1,
+                                                                 unsigned* __restrict__ local2,
+                                                                 unsigned long long* __restrict__ cell,
+                                                                 unsigned long long* __restrict__ tot) {
+    extern __shared__ unsigned s_acc[];  // [2][n_sinks]
+    const unsigned long long n = rs->pairs;
+    const unsigned b = blockIdx.x;
+    if (static_cast<unsigned long long>(b) * kRouteBlock >= n) return;
+    for (unsigned i = threadIdx.x; i < 2 * n_sinks; i += kRouteBlock) s_acc[i] = 0;
+    __syncthreads();
+    const unsigned long long i = static_cast<unsigned long long>(b) * kRouteBlock + threadIdx.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    unsigned s = 0xFFFFFFFFu, l1 = 0, l2 = 0;
+    if (i < n) {
+        const unsigned long long lo = key2[i], hi = key2[rec_cap + i];
+        unsigned long long h = hash64(lo ^ (hi * 0x9E3779B97F4A7C15ULL)) & mask;
+        for (unsigned probe = 0; probe < kMaxProbe; ++probe) {
+            const ulonglong2 k = *reinterpret_cast<const ulonglong2*>(&tab[h].lo);
+            if (k.x == lo && k.y == hi) {
+                s = static_cast<unsigned>(tab[h].count);
+                break;
+            }
+            if (k.x == kEmpty) break;
             h = (h + 1) & mask;
         }
         if (s == 0xFFFFFFFFu) {

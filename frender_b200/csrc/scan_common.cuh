@@ -324,6 +324,96 @@ __device__ __forceinline__ int parse_header(const unsigned char* buf, const unsi
     return parse_serial(a.data + s_g, e_g - s_g, rule, key_out);
 }
 
+// ---- wide keys (up to 42 symbols: lo = symbols 0..20, hi = symbols 21..41) ---------------------------------------
+// parse_serial for a wide context.
+__host__ __device__ inline int parse_serial_wide(const unsigned char* s, unsigned long long len, int rule,
+                                                 unsigned long long* lo_out, unsigned long long* hi_out) {
+    unsigned long long i = 0;
+    if (rule == FRB_RULE_SCAN) {
+        while (i < len && s[i] != ' ') ++i;
+        if (i >= len) return FRB_ERR_BAD_HEADER;
+        ++i;
+    }
+    unsigned long long k0 = 0, k1 = 0;
+    int n = 0;
+    bool bad = false, too_long = false;
+    for (; i < len; ++i) {
+        unsigned c = s[i];
+        if (rule == FRB_RULE_SCAN && c == ' ') break;
+        if (c == ':') {
+            k0 = k1 = 0, n = 0, bad = false, too_long = false;
+            continue;
+        }
+        unsigned code = enc_read(c);
+        bad |= (code == 0);
+        if (n >= kMaxWideSyms) too_long = true;
+        else if (n < kMaxSyms) k0 |= static_cast<unsigned long long>(code) << (3 * n);
+        else k1 |= static_cast<unsigned long long>(code) << (3 * (n - kMaxSyms));
+        ++n;
+    }
+    if (bad) return FRB_ERR_BAD_ALPHABET;
+    if (too_long) return FRB_ERR_KEY_TOO_LONG;
+    *lo_out = k0, *hi_out = k1;
+    return 0;
+}
+
+// The order of the 21 3-bit groups of a word reversed (group j -> group 20 - j).
+__device__ __forceinline__ unsigned long long reverse21(unsigned long long w) {
+    const unsigned long long r = __brevll(w) >> 1;
+    return ((r & kFoldLsb3) << 2) | (r & (kFoldLsb3 << 1)) | ((r >> 2) & kFoldLsb3);
+}
+
+// parse_header for a wide context.  The fast path walks back over the last 43 bytes of the line.
+template <bool SUM = false>
+__device__ __forceinline__ int parse_header_wide(const unsigned char* buf, const unsigned char* lut, unsigned sb,
+                                                 unsigned eb, const ScanArgs& a, unsigned long long tile_off,
+                                                 unsigned long long* lo_out, unsigned long long* hi_out,
+                                                 unsigned long long* start_out) {
+    const bool scan_rule = (a.rule == FRB_RULE_SCAN);
+    if (sb != kUnknown) *start_out = tile_off + sb - kHalo;
+    if (sb != kUnknown && eb - sb > static_cast<unsigned>(kMaxWideSyms)) {
+        const int spaces = !scan_rule ? 1 : SUM ? count_spaces_sum(buf, sb, eb, a.pat_sp)
+                                               : count_spaces_fast(buf, sb, eb, a.pat_sp);
+        const unsigned char* const e = buf + eb;
+        unsigned long long delim = 0, r0 = 0, r1 = 0;  // r0 / r1: symbols 0..20 / 21..41 counted from the end
+#pragma unroll
+        for (int j = 0; j < kMaxWideSyms + 1; ++j) {
+            const unsigned v = lut[e[-1 - j]];
+            delim |= static_cast<unsigned long long>(v >> 3) << j;
+            if (j < kMaxSyms) r0 |= static_cast<unsigned long long>(v & 7u) << (3 * j);
+            else if (j < kMaxWideSyms) r1 |= static_cast<unsigned long long>(v & 7u) << (3 * (j - kMaxSyms));
+        }
+        if (spaces == 0) return FRB_ERR_BAD_HEADER;
+        if (spaces == 1 && delim != 0) {
+            const int len = __ffsll(static_cast<long long>(delim)) - 1;  // symbols in the key, <= 42
+            const unsigned long long want0 = len >= kMaxSyms ? kFoldLsb3 : (len ? (kFoldLsb3 & ((1ULL << (3 * len)) - 1ULL)) : 0ULL);
+            const unsigned long long want1 = len > kMaxSyms ? (kFoldLsb3 & ((1ULL << (3 * (len - kMaxSyms))) - 1ULL)) : 0ULL;
+            if (((r0 | (r0 >> 1) | (r0 >> 2)) & want0) != want0 || ((r1 | (r1 >> 1) | (r1 >> 2)) & want1) != want1)
+                return FRB_ERR_BAD_ALPHABET;
+            // the 42 symbols in text order, then shifted down by the 42 - len that are not part of the key
+            const unsigned long long f0 = reverse21(r1), f1 = reverse21(r0);
+            const int s = kMaxWideSyms - len;
+            if (s >= kMaxSyms) {
+                *lo_out = f1 >> (3 * (s - kMaxSyms)), *hi_out = 0;
+            } else {
+                *lo_out = s ? ((f0 >> (3 * s)) | (f1 << (3 * (kMaxSyms - s)))) & ((1ULL << 63) - 1ULL) : f0;
+                *hi_out = f1 >> (3 * s);
+            }
+            return 0;
+        }
+    }
+    const unsigned long long e_g = tile_off + eb - kHalo;
+    unsigned long long s_g;
+    if (sb != kUnknown) {
+        s_g = tile_off + sb - kHalo;
+    } else {
+        s_g = e_g;
+        while (s_g > a.skip && a.data[s_g - 1] != '\n') --s_g;
+    }
+    *start_out = s_g;
+    return parse_serial_wide(a.data + s_g, e_g - s_g, a.rule, lo_out, hi_out);
+}
+
 // ---- header parsing in two halves (speculative path) ------------------------------------------------------------
 // The tile buffer is wanted back as early as possible (its refill is a long-latency bulk copy), so an extractor
 // thread first LOADS what its header line needs -- the up to seven 16-byte segments the line touches (space

@@ -38,8 +38,13 @@ struct WsGeom {
     static constexpr bool split_regs = CTAS == 3 && threads == 256;
     static constexpr int regs_count = RC, regs_work = RW;  // their mean is the launch budget (80)
     static constexpr int smem = STAGES * buf + STAGES * nl_cap * (int)sizeof(uint16_t);
+    static constexpr bool wide = false;  // keys of up to 21 symbols in one word
 };
 using WsTile = WsGeom<15, 3, 3, 1280, 2>;  // 30 KiB tiles, two stages, 3 CTAs per SM
+// The same geometry for a wide context: keys of up to 42 symbols as (lo, hi), WideSlot table.
+struct WsTileWide : WsTile {
+    static constexpr bool wide = true;
+};
 
 // status[1 + t] of the speculative path: newlines of the tile (bits 0-19), unterminated last line (bit 20),
 // guessed list index of the first header end (bits 24-31, kNoGuess = none)

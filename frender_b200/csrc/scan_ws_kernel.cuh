@@ -44,6 +44,7 @@ __global__ void __launch_bounds__(G::threads) __maxnreg__(G::maxreg) scan_ws_ker
     __shared__ __align__(8) unsigned long long s_bfull[kBatches], s_bfree[kBatches];
     __shared__ unsigned long long s_keys[kBatches][kExt];  // kEmpty except on the first lane of every run of equal keys
     __shared__ unsigned char s_kcnt[kBatches][kExt];      // reads folded into that entry
+    __shared__ unsigned long long s_keys_hi[kBatches][G::wide ? kExt : 1];  // wide context: upper words
     __shared__ unsigned s_bmeta[kBatches][8];  // see BM_* below
     __shared__ unsigned s_berr[kBatches][kXWarps];
     __shared__ unsigned char s_lut[256];
@@ -125,10 +126,15 @@ __global__ void __launch_bounds__(G::threads) __maxnreg__(G::maxreg) scan_ws_ker
             // tile to scan_redo_kernel; without a guess the extractors ask the committer for the count
             // first.  Either way every tile is tallied by line COUNT, exactly as F:161-169 does.
             // The extractors issue no global atomics, so none of their barrier arrivals waits for one.
+            // a wide context's keys_out holds out_cap lower words, then out_cap upper words
+            unsigned long long key_hi = 0;  // wide context: upper word of this thread's key
             auto emit = [&](unsigned long long o, unsigned long long key, unsigned long long start_g) {
                 const unsigned long long slot = o - chunk_first_read;
                 if (slot < a.out_cap) {
                     if (a.keys_out) a.keys_out[slot] = key;
+                    if constexpr (G::wide) {
+                        if (a.keys_out) a.keys_out[a.out_cap + slot] = key < kBadKeyBase ? key_hi : 0ULL;
+                    }
                     if (a.rec_off_out) a.rec_off_out[slot] = start_g;
                 }
             };
@@ -162,13 +168,17 @@ __global__ void __launch_bounds__(G::threads) __maxnreg__(G::maxreg) scan_ws_ker
                 if (n) {
                     const unsigned grp = __ballot_sync(0xFFFFFFFFu, key != kEmpty);
                     if (key != kEmpty) {
-                        const unsigned same = __match_any_sync(grp, key);
+                        unsigned same = __match_any_sync(grp, key);
+                        if constexpr (G::wide) same &= __match_any_sync(grp, key_hi);
                         if (lane == __ffs(same) - 1) cnt = __popc(same);
                         else key = kEmpty;
                     }
                 }
                 mbar_wait(&s_bfree[b], ((nb / kBatches) & 1u) ^ 1u);
                 if (n) s_keys[b][pt] = key, s_kcnt[b][pt] = static_cast<unsigned char>(cnt);
+                if constexpr (G::wide) {
+                    if (n) s_keys_hi[b][pt] = key_hi;
+                }
                 const unsigned e = __reduce_min_sync(0xFFFFFFFFu, rc ? ((static_cast<unsigned>(pt) << 8) | static_cast<unsigned>(-rc)) : 0xFFFFFFFFu);
                 if (lane == 0) s_berr[b][pwarp] = e;
                 if (pt == 0) {
@@ -240,7 +250,11 @@ __global__ void __launch_bounds__(G::threads) __maxnreg__(G::maxreg) scan_ws_ker
                         if (have) {
                             const unsigned j = j0 + 4 * h;
                             const unsigned sb = j ? nl[j - 1] + 1u : halo_start;
-                            rc = parse_header<kRule, true>(buf, s_lut, sb, nl[j], a, tile_off, &key, &start_g);
+                            if constexpr (G::wide) {
+                                rc = parse_header_wide<true>(buf, s_lut, sb, nl[j], a, tile_off, &key, &key_hi, &start_g);
+                            } else {
+                                rc = parse_header<kRule, true>(buf, s_lut, sb, nl[j], a, tile_off, &key, &start_g);
+                            }
                             if (rc && a.rule == FRB_RULE_DEMUX && a.keys_out && !a.table) {  // the router decides whether it matters
                                 emit(of + h, kBadKeyBase + static_cast<unsigned long long>(-rc), start_g);
                                 key = kEmpty, rc = 0;
@@ -361,13 +375,14 @@ __global__ void __launch_bounds__(G::threads) __maxnreg__(G::maxreg) scan_ws_ker
                     }
                     ktick(k_look);
                 }
-                unsigned long long key[kRounds];
+                unsigned long long key[kRounds], key_hi[kRounds];
                 unsigned cnt[kRounds];
 #pragma unroll
                 for (int r = 0; r < kRounds; ++r) {
                     const unsigned idx = r * 32 + lane;
                     key[r] = (tile_ok && idx < n) ? s_keys[b][idx] : kEmpty;
                     cnt[r] = s_kcnt[b][idx];
+                    if constexpr (G::wide) key_hi[r] = s_keys_hi[b][idx];
                 }
                 unsigned err = 0xFFFFFFFFu;
 #pragma unroll
@@ -377,7 +392,17 @@ __global__ void __launch_bounds__(G::threads) __maxnreg__(G::maxreg) scan_ws_ker
                 if (tile_ok && n && err != 0xFFFFFFFFu && lane == 0) {
                     raise_error(a.st, -static_cast<int>(err & 0xFFu), of + h0 + (err >> 8));
                 }
-                if (a.table) {
+                if constexpr (G::wide) {
+                    if (!a.table) continue;
+                    // one probe loop per key (a 16-byte load, then the count / first updates or the claim)
+#pragma unroll
+                    for (int r = 0; r < kRounds; ++r) {
+                        if (key[r] != kEmpty) {
+                            table_add_wide(reinterpret_cast<WideSlot*>(a.table), a.table_mask, key[r], key_hi[r], cnt[r],
+                                           a.pos_base + of + h0 + r * 32 + lane, &a.st->occupied, a.st);
+                        }
+                    }
+                } else if (a.table) {
 #pragma unroll
                     for (int r = 0; r < kRounds; ++r) {
                         finish(r);  // the sets of the previous batch (their slot loads are long back)
@@ -390,10 +415,12 @@ __global__ void __launch_bounds__(G::threads) __maxnreg__(G::maxreg) scan_ws_ker
                 }
                 ktick(k_commit);
             }
+            if constexpr (!G::wide) {
 #pragma unroll 1
-            for (int k = 0; k < 2; ++k) {  // the second pass retires a CAS issued by the first
+                for (int k = 0; k < 2; ++k) {  // the second pass retires a CAS issued by the first
 #pragma unroll
-                for (int r = 0; r < kRounds; ++r) finish(r);
+                    for (int r = 0; r < kRounds; ++r) finish(r);
+                }
             }
             if (lane == 0 && my_reads) atomicAdd(&a.st->n_reads, my_reads);
             if (timing && lane == 0) {
@@ -463,6 +490,49 @@ __global__ void __launch_bounds__(64) scan_redo_kernel(const ScanArgs a_in) {
             if (reads) atomicAdd(&a.st->n_reads, reads);
             if (t == a.n_tiles - 1) a.st->line_carry = k;
         }
+    }
+}
+
+// scan_redo_kernel for a wide context (which never runs the speculative scan).  keys_out: out_cap lower words,
+// then out_cap upper words.
+__global__ void __launch_bounds__(64) scan_redo_wide_kernel(const ScanArgs a_in) {
+    ScanArgs a = a_in;
+    a.skip = a.skip_ptr ? *a.skip_ptr : 0ULL;
+    const unsigned long long n = a.st->redo_n;
+    const unsigned long long L0 = a.st->chunk_l0;
+    const unsigned long long chunk_first_read = (L0 + 3) >> 2;
+    for (unsigned long long idx = blockIdx.x * blockDim.x + threadIdx.x; idx < n;
+         idx += static_cast<unsigned long long>(gridDim.x) * blockDim.x) {
+        const unsigned t = a.redo[idx];
+        const unsigned long long off = static_cast<unsigned long long>(t) * a.tile_bytes;
+        const unsigned long long end = off + a.tile_bytes < a.nbytes ? off + a.tile_bytes : a.nbytes;
+        unsigned long long k = L0 + (t ? (a.status[t] & kValMask) : 0ULL);
+        unsigned long long prev = off > a.skip ? off : a.skip;
+        while (prev > a.skip && a.data[prev - 1] != '\n') --prev;
+        const bool vnl = t == a.n_tiles - 1 && end > off && end > a.skip && a.data[end - 1] != '\n';
+        unsigned long long reads = 0;
+        for (unsigned long long p = off > a.skip ? off : a.skip; p <= end; ++p) {
+            const bool is_end = p < end ? a.data[p] == '\n' : vnl;
+            if (!is_end) continue;
+            if ((k & 3) == 0 && (k >> 2) < a.read_limit) {
+                unsigned long long lo = 0, hi = 0;
+                const int rc = parse_serial_wide(a.data + prev, p - prev, a.rule, &lo, &hi);
+                ++reads;
+                const bool routed = a.rule == FRB_RULE_DEMUX && a.keys_out && !a.table;
+                if (rc && routed) lo = kBadKeyBase + static_cast<unsigned long long>(-rc), hi = 0;  // the router decides
+                else if (rc) raise_error(a.st, rc, k >> 2);
+                else if (a.table) table_add_wide(reinterpret_cast<WideSlot*>(a.table), a.table_mask, lo, hi, 1, a.pos_base + (k >> 2), &a.st->occupied, a.st);
+                const unsigned long long slot = (k >> 2) - chunk_first_read;
+                if ((!rc || routed) && slot < a.out_cap) {
+                    if (a.keys_out) a.keys_out[slot] = lo, a.keys_out[a.out_cap + slot] = hi;
+                    if (a.rec_off_out) a.rec_off_out[slot] = prev;
+                }
+            }
+            prev = p + 1;
+            ++k;
+        }
+        if (reads) atomicAdd(&a.st->n_reads, reads);
+        if (t == a.n_tiles - 1) a.st->line_carry = k;
     }
 }
 

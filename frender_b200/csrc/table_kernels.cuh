@@ -257,4 +257,102 @@ __global__ void __launch_bounds__(256) demux_ok_kernel(const unsigned long long*
     }
 }
 
+// ---- wide context (WideSlot tables, keys as lo / hi arrays) ---------------------------------------------------
+__global__ void __launch_bounds__(256) clear_wide_table_kernel(WideSlot* tab, unsigned long long cap) {
+    const unsigned long long stride = static_cast<unsigned long long>(gridDim.x) * blockDim.x;
+    ulonglong4* t4 = reinterpret_cast<ulonglong4*>(tab);
+    for (unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x; i < cap;
+         i += stride)
+        t4[i] = make_ulonglong4(kEmpty, 0ULL, ~0ULL, 0ULL);  // lo, hi, first, count
+}
+
+// compact_table_kernel for WideSlot tables (no composite positions: a wide context never runs the speculative scan)
+__global__ void __launch_bounds__(256) compact_wide_table_kernel(const WideSlot* __restrict__ tab, unsigned long long cap,
+                                                                 unsigned long long* __restrict__ keys,
+                                                                 unsigned long long* __restrict__ keys_hi,
+                                                                 unsigned long long* __restrict__ counts,
+                                                                 unsigned long long* __restrict__ first,
+                                                                 unsigned long long* counter, unsigned long long out_cap) {
+    __shared__ unsigned s_warp[8];
+    __shared__ unsigned long long s_base;
+    const unsigned long long stride = static_cast<unsigned long long>(gridDim.x) * blockDim.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned long long cap_up = (cap + 255) & ~255ULL;
+    for (unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x;
+         i < cap_up; i += stride) {
+        ulonglong4 s = make_ulonglong4(kEmpty, 0, 0, 0);
+        if (i < cap) s = reinterpret_cast<const ulonglong4*>(tab)[i];
+        const bool occ = s.x != kEmpty && s.w != 0;
+        const unsigned m = __ballot_sync(0xFFFFFFFFu, occ);
+        if (lane == 0) s_warp[warp] = __popc(m);
+        __syncthreads();
+        unsigned before = 0, total = 0;
+#pragma unroll
+        for (int w = 0; w < 8; ++w) {
+            const unsigned v = s_warp[w];
+            if (w < warp) before += v;
+            total += v;
+        }
+        if (threadIdx.x == 0 && total) s_base = atomicAdd(counter, static_cast<unsigned long long>(total));
+        __syncthreads();
+        if (occ) {
+            const unsigned long long idx = s_base + before + __popc(m & ((1u << lane) - 1u));
+            if (idx < out_cap) keys[idx] = s.x, keys_hi[idx] = s.y, counts[idx] = s.w, first[idx] = s.z;
+        }
+    }
+}
+
+__global__ void __launch_bounds__(256) gather1_kernel(const unsigned* __restrict__ perm,
+                                                      const unsigned long long* __restrict__ in,
+                                                      unsigned long long* __restrict__ out, unsigned long long n) {
+    const unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x;
+    if (i < n) out[i] = in[perm[i]];
+}
+
+// dst[(lo, hi)] += counts, first = min(first, pos_base + first_in)
+__global__ void __launch_bounds__(256) merge_wide_list_kernel(WideSlot* dst, unsigned long long mask,
+                                                              const unsigned long long* __restrict__ keys,
+                                                              const unsigned long long* __restrict__ keys_hi,
+                                                              const unsigned long long* __restrict__ counts,
+                                                              const unsigned long long* __restrict__ first,
+                                                              unsigned long long n, unsigned long long pos_base,
+                                                              unsigned long long* occupied, DevState* st) {
+    const unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x;
+    if (i < n) table_add_wide(dst, mask, keys[i], keys_hi[i], counts[i], first ? pos_base + first[i] : pos_base + i, occupied, st);
+}
+
+// demux_ok_kernel over wide keys: the total is sorted by (hi, lo).
+__global__ void __launch_bounds__(256) demux_ok_wide_kernel(const unsigned long long* __restrict__ fkeys,
+                                                            const unsigned long long* __restrict__ fkeys_hi,
+                                                            const unsigned long long* __restrict__ fcounts, unsigned long long nf,
+                                                            const unsigned long long* __restrict__ sorted_lo,
+                                                            const unsigned long long* __restrict__ sorted_hi,
+                                                            const unsigned* __restrict__ sorted_idx, unsigned long long n,
+                                                            const unsigned char* __restrict__ type, const int* __restrict__ srow,
+                                                            const unsigned char* __restrict__ match, unsigned n_files, unsigned f,
+                                                            unsigned char* __restrict__ ok, unsigned char* __restrict__ bad_file,
+                                                            int* err_row) {
+    const unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x;
+    if (i >= nf || (fcounts && fcounts[i] == 0)) return;
+    const unsigned long long klo = fkeys[i], khi = fkeys_hi[i];
+    unsigned long long lo = 0, hi = n;
+    while (lo < hi) {
+        const unsigned long long mid = (lo + hi) >> 1;
+        const unsigned long long mh = sorted_hi[mid];
+        if (mh < khi || (mh == khi && sorted_lo[mid] < klo)) lo = mid + 1;
+        else hi = mid;
+    }
+    if (lo >= n || sorted_lo[lo] != klo || sorted_hi[lo] != khi) return;
+    const unsigned idx = sorted_idx[lo];
+    const unsigned t = type[idx];
+    const unsigned cls = t == 2 ? 4u + static_cast<unsigned>(srow[idx]) : t;
+    const unsigned m = match[static_cast<unsigned long long>(cls) * n_files + f];
+    if (m == 2) {
+        atomicMin(err_row, static_cast<int>(cls) - 4);
+    } else if (m == 0) {
+        ok[idx] = 0;
+        bad_file[f] = 1;
+    }
+}
+
 }  // namespace frb

@@ -15,6 +15,7 @@ from . import _lib
 from ._lib import C, FrbError, READ_TYPES, check, lib
 
 MAX_SYMS = 21
+MAX_WIDE_SYMS = 2 * MAX_SYMS   # a wide context's keys: (lo, hi), see include/frender_b200.h
 _ENC = np.full(256, 255, np.uint8)
 for _ch, _code in zip(b"ACGTN+", range(1, 7)):
     _ENC[_ch] = _code
@@ -58,6 +59,35 @@ def unpack_keys(keys):
     return [t.decode() for t in txt.tolist()]
 
 
+def pack_keys2(strings, sheet_mode=False):
+    """list of index strings of up to 42 symbols -> (lo, hi) uint64 arrays (wide keys, include/frender_b200.h).
+    lo equals pack_keys() for strings of up to 21 symbols, whose hi is 0."""
+    if len(strings) == 0:
+        return np.zeros(0, np.uint64), np.zeros(0, np.uint64)
+    raw = [s.encode() if isinstance(s, str) else s for s in strings]
+    if max(len(r) for r in raw) > MAX_WIDE_SYMS:
+        raise FrbError(_lib.ERR_KEY_TOO_LONG, f"index field longer than {MAX_WIDE_SYMS} symbols")
+    mat = np.array(raw, dtype=f"S{MAX_WIDE_SYMS}").view(np.uint8).reshape(len(raw), MAX_WIDE_SYMS)
+    codes = (_ENC_SHEET if sheet_mode else _ENC)[mat]
+    if not sheet_mode and (codes == 255).any():
+        raise FrbError(_lib.ERR_BAD_ALPHABET, "index field holds a symbol outside ACGTN+")
+    codes = codes.astype(np.uint64)
+    lo = (codes[:, :MAX_SYMS] << _SHIFTS).sum(axis=1, dtype=np.uint64)
+    hi = (codes[:, MAX_SYMS:] << _SHIFTS).sum(axis=1, dtype=np.uint64)
+    return lo, hi
+
+
+def unpack_keys2(lo, hi):
+    """(lo, hi) uint64 arrays -> list of str (exact inverse of pack_keys2 for read keys)."""
+    lo = np.asarray(lo, dtype=np.uint64)
+    hi = np.asarray(hi, dtype=np.uint64)
+    if lo.size == 0:
+        return []
+    codes = np.concatenate([(lo[:, None] >> _SHIFTS) & np.uint64(7), (hi[:, None] >> _SHIFTS) & np.uint64(7)], axis=1)
+    txt = np.ascontiguousarray(_DEC[codes.astype(np.uint8)]).view(f"S{MAX_WIDE_SYMS}").ravel()
+    return [t.decode() for t in txt.tolist()]
+
+
 def _ptr(arr):
     return arr.ctypes.data_as(C.c_void_p) if arr is not None else None
 
@@ -65,7 +95,7 @@ def _ptr(arr):
 class PackedSheet:
     """Sample sheet in the matcher's layout (frb_sheet_load)."""
 
-    def __init__(self, indexes):
+    def __init__(self, indexes, wide=False):
         self.ids = list(indexes["id"])
         self.idx1 = list(indexes["idx1"])
         self.single = indexes.get("idx2") is None
@@ -80,8 +110,13 @@ class PackedSheet:
                 raise AssertionError(
                     f"Barcode lengths differ inside the sample sheet ({a!r}/{b!r} vs {self.l1}+{self.l2})")
         join = (lambda a, b: a) if self.single else (lambda a, b: a + "+" + b)
-        self.fwd = pack_keys([join(a, b) for a, b in zip(self.idx1, self.idx2)], sheet_mode=True)
-        self.rc = pack_keys([join(a, b) for a, b in zip(self.idx1, self.rc_idx2)], sheet_mode=True)
+        fwd = [join(a, b) for a, b in zip(self.idx1, self.idx2)]
+        rc = [join(a, b) for a, b in zip(self.idx1, self.rc_idx2)]
+        self.wide = wide
+        if wide:    # rows of up to 21+21 symbols (frb_sheet_load2)
+            (self.fwd, self.fwd_hi), (self.rc, self.rc_hi) = pack_keys2(fwd, True), pack_keys2(rc, True)
+        else:
+            self.fwd, self.rc = pack_keys(fwd, sheet_mode=True), pack_keys(rc, sheet_mode=True)
         first_row = {}
         self.group = np.array([first_row.setdefault(name, len(first_row)) for name in self.ids], np.int32)
         self.group_names = list(first_row)                                     # dict order, F:367
@@ -90,7 +125,7 @@ class PackedSheet:
 class Context:
     """One GPU context (frb_ctx).  Not thread-safe; use one per GPU."""
 
-    def __init__(self, device=0, table_log2=22):
+    def __init__(self, device=0, table_log2=22, wide=False):
         self._h = C.c_void_p()
         rc = lib.frb_create(device, table_log2, C.byref(self._h))
         if rc != _lib.OK:
@@ -100,6 +135,17 @@ class Context:
         self.table_log2 = table_log2
         self.sheet = None
         self.file_names = []
+        self.wide = False
+        if wide:
+            self.set_wide()
+
+    def set_wide(self, on=True):
+        """Keys of up to 42 symbols (128-bit keys, frb_set_key_width).  Forgets every file scanned so far."""
+        self._ck(lib.frb_set_key_width(self._h, 128 if on else 64))
+        self.wide = bool(on)
+        self.sheet = None
+        self.file_names = []
+        self._sharded = False
 
     def close(self):
         if self._h:
@@ -198,6 +244,26 @@ class Context:
         self._ck(lib.frb_file_size(self._h, i, C.byref(uniq), C.byref(reads)))
         return self._export(lambda k, c, f, n: lib.frb_file_export(self._h, i, k, c, f, n), uniq.value)
 
+    def file_keys_hi(self, i):
+        """Upper key words of file i, in the order of file_arrays (all zero on a narrow context)."""
+        uniq, reads = C.c_uint64(), C.c_uint64()
+        self._ck(lib.frb_file_size(self._h, i, C.byref(uniq), C.byref(reads)))
+        hi = np.empty(uniq.value, np.uint64)
+        self._ck(lib.frb_file_export_hi(self._h, i, _ptr(hi), uniq.value))
+        return hi
+
+    def total_keys_hi(self):
+        """Upper key words of "total", in the order of total_arrays (all zero on a narrow context)."""
+        uniq = C.c_uint64()
+        self._ck(lib.frb_total_finish(self._h, C.byref(uniq)))
+        hi = np.empty(uniq.value, np.uint64)
+        self._ck(lib.frb_total_export_hi(self._h, _ptr(hi), uniq.value))
+        return hi
+
+    def key_strings(self, keys, keys_hi=None):
+        """Packed keys of this context -> str."""
+        return unpack_keys2(keys, keys_hi) if self.wide else unpack_keys(keys)
+
     def total_arrays(self):
         """(keys, counts, first_pos) of "total", in first-appearance order (F:199-203)."""
         uniq = C.c_uint64()
@@ -207,16 +273,24 @@ class Context:
     def counter(self):
         """The reference's barcode_counter dict: {"total": {...}, basename: {...}} (F:200-207)."""
         keys, counts, _ = self.total_arrays()
-        out = {"total": dict(zip(unpack_keys(keys), counts.tolist()))}
+        hi = self.total_keys_hi() if self.wide else None
+        out = {"total": dict(zip(self.key_strings(keys, hi), counts.tolist()))}
         for i, name in enumerate(self.file_names):
             k, c, _ = self.file_arrays(i)
-            out[name] = dict(zip(unpack_keys(k), c.tolist()))      # same basename overwrites, F:205
+            hi = self.file_keys_hi(i) if self.wide else None
+            out[name] = dict(zip(self.key_strings(k, hi), c.tolist()))      # same basename overwrites, F:205
         return out
 
     # ---- hot path B -------------------------------------------------------------------------
     def load_sheet(self, indexes):
-        sh = indexes if isinstance(indexes, PackedSheet) else PackedSheet(indexes)
-        self._ck(lib.frb_sheet_load(self._h, _ptr(sh.fwd), _ptr(sh.rc), _ptr(sh.group), len(sh.ids), sh.l1, sh.l2))
+        sh = indexes if isinstance(indexes, PackedSheet) and indexes.wide == self.wide else PackedSheet(
+            indexes if not isinstance(indexes, PackedSheet) else
+            {"id": indexes.ids, "idx1": indexes.idx1, "idx2": None if indexes.single else indexes.idx2}, wide=self.wide)
+        if self.wide:
+            self._ck(lib.frb_sheet_load2(self._h, _ptr(sh.fwd), _ptr(sh.fwd_hi), _ptr(sh.rc), _ptr(sh.rc_hi),
+                                         _ptr(sh.group), len(sh.ids), sh.l1, sh.l2))
+        else:
+            self._ck(lib.frb_sheet_load(self._h, _ptr(sh.fwd), _ptr(sh.rc), _ptr(sh.group), len(sh.ids), sh.l1, sh.l2))
         self.sheet = sh
         return sh
 
@@ -224,15 +298,19 @@ class Context:
         """Use a caller-supplied {key: reads} dict as the unique-key list (process(), F:391).
         Only the first two '+' parts of a key take part in matching (F:306)."""
         if single:
-            keys = pack_keys(list(counter.keys()))
+            heads = list(counter.keys())
         else:
             heads = []
             for k in counter:
                 idx1, idx2 = k.split("+")[0:2]            # ValueError without a '+', as in F:306
                 heads.append(idx1 + "+" + idx2)
-            keys = pack_keys(heads)
         counts = np.fromiter(counter.values(), dtype=np.uint64, count=len(counter))
-        self._ck(lib.frb_total_load(self._h, _ptr(keys), _ptr(counts), len(keys)))
+        if self.wide:
+            keys, hi = pack_keys2(heads)
+            self._ck(lib.frb_total_load2(self._h, _ptr(keys), _ptr(hi), _ptr(counts), len(keys)))
+        else:
+            keys = pack_keys(heads)
+            self._ck(lib.frb_total_load(self._h, _ptr(keys), _ptr(counts), len(keys)))
 
     def load_total_arrays(self, keys, counts):
         """Use packed key / count arrays as the unique-key list (already in first-appearance order)."""
@@ -310,7 +388,8 @@ class Context:
         if counter is not None:
             self.load_total(counter, single=sh.single)
         keys, counts, _ = self.total_arrays()
-        names = list(counter.keys()) if counter is not None else unpack_keys(keys)
+        names = list(counter.keys()) if counter is not None else self.key_strings(
+            keys, self.total_keys_hi() if self.wide else None)
         r = self.match(num_subs, rc_mode, use_rc_rows)
         idx2 = sh.idx2
         if use_rc_rows is not None:
@@ -370,11 +449,16 @@ class Context:
         self._ck(lib.frb_demux_ok(self._h, _ptr(match), n_files, kp, cp, np_, _ptr(ok), _ptr(bad), C.byref(err)))
         return ok[:n.value].astype(bool), bad[:n_files].astype(bool), (None if err.value == 0x7FFFFFFF else err.value)
 
-    def route_load(self, keys, sink_ids, n_sinks):
-        """Results table for the demux router: packed key -> sink id (unique keys)."""
+    def route_load(self, keys, sink_ids, n_sinks, keys_hi=None):
+        """Results table for the demux router: packed key -> sink id (unique keys).  keys_hi: upper words of a wide
+        context's keys (pack_keys2)."""
         keys = np.ascontiguousarray(keys, np.uint64)
         sink_ids = np.ascontiguousarray(sink_ids, np.uint32)
-        self._ck(lib.frb_route_load(self._h, _ptr(keys), _ptr(sink_ids), len(keys), n_sinks))
+        if keys_hi is None:
+            self._ck(lib.frb_route_load(self._h, _ptr(keys), _ptr(sink_ids), len(keys), n_sinks))
+        else:
+            hi = np.ascontiguousarray(keys_hi, np.uint64)
+            self._ck(lib.frb_route_load2(self._h, _ptr(keys), _ptr(hi), _ptr(sink_ids), len(keys), n_sinks))
         self._n_sinks = n_sinks
 
     def route_pair(self, r1, r2, final=3):
@@ -450,8 +534,16 @@ def tally_barcodes(cores, files, sample=None, ctx=None):
     if sample:
         assert sample >= 1, "Number of reads to sample must be ≥ 1!"
     ctx.reset()
-    for ordinal, path in enumerate(files):
-        ctx.scan_gz(path, ordinal, sample)
+    try:
+        for ordinal, path in enumerate(files):
+            ctx.scan_gz(path, ordinal, sample)
+    except FrbError as exc:
+        if exc.code != _lib.ERR_KEY_TOO_LONG or ctx.wide:
+            raise
+        # a dict never refuses a key (F:172-177): index fields longer than 21 symbols take 128-bit keys
+        ctx.set_wide()
+        for ordinal, path in enumerate(files):
+            ctx.scan_gz(path, ordinal, sample)
     return ctx.counter()
 
 

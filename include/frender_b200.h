@@ -18,6 +18,16 @@
  * 21 symbols fit (10+1+10).  The map is injective, so counting packed keys equals
  * counting strings (F:172-177).  Anything else in a read's key is a hard error
  * (FRB_ERR_BAD_ALPHABET / FRB_ERR_KEY_TOO_LONG): documented deviation, DESIGN.md.
+ *
+ * Wide keys.  A context set to 128-bit keys (frb_set_key_width) takes index fields of up
+ * to 42 symbols as two words (lo, hi): symbol i < 21 at bits [3i, 3i+3) of lo, symbol
+ * 21 <= i < 42 at bits [3(i-21), 3(i-21)+3) of hi, same codes.  A key of <= 21 symbols
+ * has hi = 0 and lo = its narrow packing, so a wide context counts, orders and writes
+ * such keys exactly as a narrow one.  No real key sets bit 63 of lo (FRB_EMPTY_KEY stays
+ * free).  43 symbols or more are FRB_ERR_KEY_TOO_LONG.  On a wide context the narrow
+ * calls keep working and take hi = 0; frb_scan_chunk_dev with per-read keys_out,
+ * frb_total_merge, frb_allmerge, frb_shardmerge and frb_demux_ok with host file lists
+ * return FRB_ERR_STATE.
  */
 #ifndef FRENDER_B200_H
 #define FRENDER_B200_H
@@ -34,7 +44,7 @@ extern "C" {
 #define FRB_ERR_ARG (-2)           /* bad argument                                               */
 #define FRB_ERR_BAD_HEADER (-3)    /* header line without a 2nd space token (IndexError, F:169)  */
 #define FRB_ERR_BAD_ALPHABET (-4)  /* key symbol outside ACGTN+                                  */
-#define FRB_ERR_KEY_TOO_LONG (-5)  /* key longer than 21 symbols                                 */
+#define FRB_ERR_KEY_TOO_LONG (-5)  /* key longer than 21 symbols (42 on a wide context)          */
 #define FRB_ERR_TABLE_FULL (-6)    /* unique-key table exhausted: recreate with a larger log2    */
 #define FRB_ERR_BAD_LENGTH (-7)    /* key/sheet index lengths differ (AssertionError F:227) or a
                                       key has no '+' (ValueError F:306)                          */
@@ -85,6 +95,15 @@ int frb_write_scan_csv(const char* path, const uint64_t* keys, const uint64_t* c
                        int single_index);
 int frb_pack_key(const char* s, size_t len, int sheet_mode, uint64_t* out);
 int frb_unpack_key(uint64_t key, char* out23); /* writes <= 21 chars + NUL, returns length       */
+/* wide keys: (lo, hi), up to 42 symbols; frb_unpack_key2 writes <= 42 chars + NUL, returns length */
+int frb_pack_key2(const char* s, size_t len, int sheet_mode, uint64_t* lo, uint64_t* hi);
+int frb_unpack_key2(uint64_t lo, uint64_t hi, char* out44);
+/* frb_write_scan_csv with the upper words of wide keys (keys_hi NULL: all zero) */
+int frb_write_scan_csv2(const char* path, const uint64_t* keys, const uint64_t* keys_hi, const uint64_t* counts,
+                        const int32_t* m1, const int32_t* m2, const uint8_t* read_type, const int32_t* sample_row,
+                        const uint8_t* demux_ok, uint64_t n, const char* const* idx1_strings,
+                        const char* const* idx2_strings, const char* const* id_strings, uint32_t rows,
+                        int single_index);
 
 /* ---- hot path A: read-name parse + unique-combination counter ------------------------------
  * Replaces scan_file F:154-181 and tally_barcodes F:183-207.
@@ -138,6 +157,14 @@ int frb_total_load(frb_ctx* ctx, const uint64_t* keys, const uint64_t* counts, u
 int frb_total_merge(frb_ctx* ctx, const uint64_t* keys, const uint64_t* counts, const uint64_t* first_pos,
                     uint64_t n);
 int frb_reset(frb_ctx* ctx); /* forget all files and the total                                 */
+/* Key width of the context: 64 (narrow, the default) or 128 (wide, keys of up to 42 symbols).  Implies frb_reset,
+ * clears the route table and drops the sample sheet (load it again); frb_reset and frb_resize_tables keep the width.  The *_hi exports return the upper key
+ * words in the order of frb_file_export / frb_total_export (all zero on a narrow context); the *2 loads are the
+ * narrow calls with upper words added (wide context only).                                                       */
+int frb_set_key_width(frb_ctx* ctx, uint32_t bits);
+int frb_file_export_hi(frb_ctx* ctx, uint32_t file_idx, uint64_t* keys_hi, uint64_t cap);
+int frb_total_export_hi(frb_ctx* ctx, uint64_t* keys_hi, uint64_t cap);
+int frb_total_load2(frb_ctx* ctx, const uint64_t* keys, const uint64_t* keys_hi, const uint64_t* counts, uint64_t n);
 /* Re-create both unique-key tables with 2^table_log2 slots (implies frb_reset): the host's answer to
  * FRB_ERR_TABLE_FULL -- a Python dict never refuses a key (F:172-177), so the CLI resizes and tallies again. */
 int frb_resize_tables(frb_ctx* ctx, uint32_t table_log2);
@@ -158,6 +185,9 @@ int frb_resize_tables(frb_ctx* ctx, uint32_t table_log2);
  */
 int frb_sheet_load(frb_ctx* ctx, const uint64_t* fwd, const uint64_t* rc, const int32_t* group,
                    uint32_t n_rows, uint32_t l1, uint32_t l2);
+/* Wide context: rows packed as (lo, hi); l1 <= 21, l2 <= 21, l1 + 1 + l2 <= 42.                          */
+int frb_sheet_load2(frb_ctx* ctx, const uint64_t* fwd, const uint64_t* fwd_hi, const uint64_t* rc, const uint64_t* rc_hi,
+                    const int32_t* group, uint32_t n_rows, uint32_t l1, uint32_t l2);
 int frb_match(frb_ctx* ctx, uint32_t n_subs, int rc_mode, const uint8_t* use_rc_rows,
               int32_t* m1_row, int32_t* m2_row, uint8_t* type, int32_t* sample_row,
               int32_t* m2rc_row, uint8_t* type_rc, int32_t* sample_rc_row,
@@ -189,6 +219,10 @@ int frb_demux_ok(frb_ctx* ctx, const uint8_t* match, uint32_t n_files, const uin
  *                    partial record of that mate counts as a record (F:719-723).
  */
 int frb_route_load(frb_ctx* ctx, const uint64_t* keys, const uint32_t* sink_ids, uint64_t n, uint32_t n_sinks);
+/* frb_route_load with the upper words of wide keys (wide context only; the router then parses keys of up to 42
+ * symbols from the R2 headers).                                                                                  */
+int frb_route_load2(frb_ctx* ctx, const uint64_t* keys, const uint64_t* keys_hi, const uint32_t* sink_ids, uint64_t n,
+                    uint32_t n_sinks);
 int frb_route_pair(frb_ctx* ctx, const void* r1, uint64_t r1_bytes, const void* r2, uint64_t r2_bytes,
                    int final_chunk, void* out_r1, void* out_r2, uint64_t* off_r1, uint64_t* off_r2,
                    uint64_t* n_pairs, uint64_t* consumed_r1, uint64_t* consumed_r2, uint64_t* bad_key);

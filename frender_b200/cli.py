@@ -641,6 +641,27 @@ class GzSink:
         self.fh.close()
 
 
+class MemberSink:
+    """One output file of FRENDER_GZIP_LEVEL=gpu: the gzip members the device wrote for it, one per chunk, appended
+    as they come.  A file that received none gets the empty member, so that every sink decompresses."""
+
+    EMPTY = bytes.fromhex("1f8b080000000000000303000000000000000000")
+
+    def __init__(self, path):
+        self.fh = open(path, "wb")
+        self.empty = True
+
+    def write(self, data):
+        if len(data):
+            self.fh.write(data)
+            self.empty = False
+
+    def close(self):
+        if self.empty:
+            self.fh.write(self.EMPTY)
+        self.fh.close()
+
+
 class TextChunks:
     """Decompressed bytes of a fastq.gz with the newline translation of text mode (F:776), piece by piece."""
 
@@ -770,7 +791,10 @@ def frender_demux(args, ctx=None):
     n_gpus = int(os.environ.get("FRENDER_GPUS", "1"))
     if ctx is None and n_gpus > 1 and len(pairs) > 1:
         return demux_pairs_multi_gpu(args, pairs, min(n_gpus, len(pairs)), out_dir)
-    level = int(os.environ.get("FRENDER_GZIP_LEVEL", "6"))
+    # FRENDER_GZIP_LEVEL: a zlib level for the host deflate, or "gpu" for gzip members written on the device
+    level = os.environ.get("FRENDER_GZIP_LEVEL", "6").strip().lower()
+    gpu_gzip = level == "gpu"
+    level = None if gpu_gzip else int(level)
     infix = args.o + "_" if args.o else ""
     sink_names = []                                                             # sink id -> name
 
@@ -782,7 +806,8 @@ def frender_demux(args, ctx=None):
     undeter_sink = open_sink(undeter_name) if undeter else None
     hop_sink = open_sink("Index-hop") if index_hop else undeter_sink
     amb_sink = open_sink("Ambiguous") if ambiguous else undeter_sink
-    sinks = [{r: GzSink(f"{out_dir}{name}_frender-demux_{infix}{r}.fq.gz", level) for r in ("R1", "R2")}
+    sink_file = (lambda path: MemberSink(path)) if gpu_gzip else (lambda path: GzSink(path, level))
+    sinks = [{r: sink_file(f"{out_dir}{name}_frender-demux_{infix}{r}.fq.gz") for r in ("R1", "R2")}
              for name in sink_names]
     n_sinks = len(sink_names)
     reject = n_sinks                                                            # "Unrecognized read type" bucket
@@ -811,6 +836,7 @@ def frender_demux(args, ctx=None):
     # Host side of the router: inflate of the two mates and deflate of the sinks run on a thread pool (zlib
     # releases the GIL).  Every sink sees the same sequence of compress() calls as a serial loop would make,
     # so the output files are byte-identical to it; the writes of chunk k overlap the inflate of chunk k+1.
+    # With FRENDER_GZIP_LEVEL=gpu the device writes the members and the pool only appends them to the files.
     from concurrent.futures import ThreadPoolExecutor
     workers = max(2, int(os.environ.get("FRENDER_DEMUX_THREADS", str(len(os.sched_getaffinity(0))))))
     pool = ThreadPoolExecutor(max_workers=workers)
@@ -834,6 +860,7 @@ def frender_demux(args, ctx=None):
 
     try:
         ctx.route_load(keys, routes, n_sinks + 1, keys_hi)
+        ctx.route_gzip(gpu_gzip)
         for r1_path, r2_path in pairs:
             print(f"Demultiplexing {r1_path.name}...")
             # The pair as a STREAM of chunks, two in flight: while chunk k is routed on the device and chunk k-1

@@ -20,6 +20,7 @@
 #include <zlib.h>
 
 #include "common.cuh"
+#include "deflate_kernels.cuh"
 #include "gz_kernels.cuh"
 #include "match_kernel.cuh"
 #include "route_kernel.cuh"
@@ -118,6 +119,9 @@ struct frb_ctx {
     uint64_t route_cap = 0;
     uint32_t n_sinks = 0;
     struct RouteStreamHolder* route = nullptr;  // the demux stream (frb_route.inl)
+    bool route_gzip = false;                    // the demux stream returns gzip members (frb_route_set_gzip)
+    // device gzip writer of frb_gz_deflate (frb_deflate.inl)
+    struct DeflateHolder* deflate = nullptr;
     // device inflate (frb_gz.inl)
     struct GzBuffersHolder* gzbuf = nullptr;
     // synth
@@ -582,6 +586,7 @@ struct GzBuffersHolder {
 };
 
 static void route_stream_destroy(frb_ctx* c);  // frb_route.inl
+static void deflate_destroy(frb_ctx* c);       // frb_deflate.inl
 
 // ============================================================================================
 extern "C" {
@@ -665,6 +670,7 @@ void frb_destroy(frb_ctx* c) {
     cudaFree(c->m1), cudaFree(c->m2), cudaFree(c->srow), cudaFree(c->m2rc), cudaFree(c->srowrc);
     cudaFree(c->type), cudaFree(c->typerc), cudaFree(c->work), cudaFree(c->work_n), cudaFree(c->cub_tmp), cudaFree(c->route_tab);
     route_stream_destroy(c);
+    deflate_destroy(c);
     if (c->gzbuf) {
         gz_free(c->gzbuf->b);
         delete c->gzbuf;
@@ -1762,6 +1768,7 @@ uint64_t frb_launch_count(frb_ctx* c) { return c->launches; }
 
 }  // extern "C"
 
+#include "frb_deflate.inl"
 #include "frb_route.inl"
 #include "frb_nccl.inl"
 #include "frb_csv.inl"

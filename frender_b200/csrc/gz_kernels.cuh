@@ -24,6 +24,8 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "crc32.cuh"
+
 namespace frb {
 namespace gz {
 
@@ -61,11 +63,6 @@ struct Chunk {
 struct Trailer {
     unsigned int chunk, local_end, crc, isize;
     unsigned long long comp_end;   // byte behind the trailer in the piece buffer (which FILE of a batch ends here)
-};
-
-// x^(2^k) mod P for k < 32 (P = the CRC-32 polynomial, reflected; made by the host), kernel parameter
-struct CrcPowers {
-    unsigned int x2n[32];
 };
 
 // ---- bit access ---------------------------------------------------------------------------------------------
@@ -842,36 +839,7 @@ __global__ void __launch_bounds__(1024) gz_text_kernel(const unsigned char* __re
 // the block sums are prefix-combined (gz_crc_scan: F[b] = crc of text[0, 4096 b)), and every member end e gets
 // F(e) from F[e / 4096] and the bytes behind it (gz_crc_ends); a member [a, e) then has
 // crc = F(e) + x^(8 (e - a)) * F(a), which gz_crc_check compares with the trailer, as it does ISIZE.
-constexpr unsigned kCrcPoly = 0xEDB88320u;
 constexpr unsigned kCrcBlock = 4096;
-
-__device__ __forceinline__ unsigned crc_mul(unsigned a, unsigned b) {  // a * b mod P
-    unsigned p = 0;
-#pragma unroll 4
-    for (int k = 0; k < 32; ++k) {
-        p ^= b & (0u - ((a >> (31 - k)) & 1u));
-        b = (b >> 1) ^ (kCrcPoly & (0u - (b & 1u)));
-    }
-    return p;
-}
-__device__ inline unsigned crc_xpow8(const CrcPowers& pw, unsigned long long nbytes) {  // x^(8 nbytes) mod P
-    unsigned p = 0x80000000u;
-    for (int k = 3; nbytes; nbytes >>= 1, ++k)
-        if (nbytes & 1) p = crc_mul(pw.x2n[k & 31], p);
-    return p;
-}
-__device__ __forceinline__ unsigned crc_join(const CrcPowers& pw, unsigned crc_a, unsigned crc_b, unsigned long long len_b) {
-    return len_b ? (crc_mul(crc_xpow8(pw, len_b), crc_a) ^ crc_b) : crc_a;
-}
-__device__ inline unsigned crc_bytes(const unsigned char* __restrict__ p, unsigned n) {  // crc32 of n bytes, bit by bit
-    unsigned crc = 0xFFFFFFFFu;
-    for (unsigned i = 0; i < n; ++i) {
-        crc ^= p[i];
-#pragma unroll
-        for (int k = 0; k < 8; ++k) crc = (crc >> 1) ^ (kCrcPoly & (0u - (crc & 1u)));
-    }
-    return ~crc;
-}
 
 // blk[b] = crc32 of text[4096 b, min(4096 (b + 1), n)): one warp per block, 128 bytes per lane
 __global__ void __launch_bounds__(256) gz_crc_blocks_kernel(const unsigned char* __restrict__ text, unsigned long long n,

@@ -208,6 +208,16 @@ class Context:
         self._ck(lib.frb_gz_inflate(self._h, os.fsencode(str(path)), _ptr(out), cap, C.byref(n), C.byref(used)))
         return out[:n.value].tobytes() if used.value else None
 
+    def gz_deflate(self, data):
+        """One buffer -> one gzip member, encoded on the device (frb_gz_deflate); zlib.decompress(x, 31) inverts it."""
+        a = np.frombuffer(data, np.uint8) if len(data) else np.zeros(1, np.uint8)
+        n = len(data)
+        cap = lib.frb_gz_deflate_bound(n)
+        out = np.empty(cap, np.uint8)
+        got = C.c_uint64()
+        self._ck(lib.frb_gz_deflate(self._h, _ptr(a), n, _ptr(out), cap, C.byref(got)))
+        return out[:got.value].tobytes()
+
     def scan_bytes(self, data, ordinal=0, sample=None, rule=_lib.RULE_SCAN, name=None, chunk=None, line_base=0):
         """Decompressed FASTQ bytes from host memory, optionally fed in `chunk`-sized pieces cut
         at line ends.  line_base: lines of the FILE in front of `data` (a rank that scans only some chunks of a
@@ -482,6 +492,11 @@ class Context:
             self._ck(lib.frb_route_reserve(self._h, int(chunk_bytes)))
         else:
             self._ck(lib.frb_route_reset(self._h))
+
+    def route_gzip(self, on=True):
+        """Gzip mode of the demux stream (frb_route_set_gzip): route_pop then returns one gzip member per non-empty
+        sink and mate, compressed on the device.  Only between chunks; kept by route_reset."""
+        self._ck(lib.frb_route_set_gzip(self._h, 1 if on else 0))
 
     def route_push(self, r1, r2, final=0):
         """Queue one chunk pair of the demux stream (frb_route_push): bytes cut anywhere; what is not complete

@@ -234,3 +234,18 @@ def generate(spec, g0, g1, read_no=1):
 def generate_big(spec, g0, g1, read_no=1, step=200_000):
     """generate() in slices, to bound the temporary matrices."""
     return b"".join(generate(spec, a, min(a + step, g1), read_no) for a in range(g0, g1, step))
+
+
+def binned_qualities(data, seed=0):
+    """The same FASTQ with every quality symbol drawn from four binned values, as binned Illumina qualities look:
+    'F' 85 %, ':' 10 %, ',' 4 %, '#' 1 % (generate() writes all-'F' qualities).  Headers, bases and lengths stay."""
+    a = np.frombuffer(data, np.uint8).copy()
+    if not a.size:
+        return b""
+    line = np.empty(a.size, np.uint32)
+    line[0] = 0
+    np.cumsum(a[:-1] == 10, dtype=np.uint32, out=line[1:])
+    qual = (line % 4 == 3) & (a != 10)
+    rng = np.random.default_rng(seed)
+    a[qual] = rng.choice(np.frombuffer(b"F:,#", np.uint8), int(qual.sum()), p=[0.85, 0.10, 0.04, 0.01])
+    return a.tobytes()

@@ -143,6 +143,13 @@ int frb_scan_gz_batch(frb_ctx* ctx, const char* const* paths, const uint32_t* or
  * the stream (blocks larger than a chunk, '\r' in the text, ...) and nothing was written; frb_scan_gz falls back
  * to zlib on a host thread for such a file.                                                                */
 int frb_gz_inflate(frb_ctx* ctx, const char* path, void* host_out, uint64_t cap, uint64_t* nbytes, int* used_device);
+/* One buffer -> one gzip member (RFC 1952, zlib's wbits=31 header), encoded ON THE DEVICE (deflate_kernels.cuh:
+ * LZ77 + dynamic Huffman per 16 KiB piece, stored where that is not smaller).  host_in: n bytes, pinned or pageable;
+ * host_out: cap >= frb_gz_deflate_bound(n) bytes, else FRB_ERR_ARG; *out_n = bytes written.  n = 0 gives the
+ * 20-byte empty member.  The same input always gives the same bytes.                                          */
+int frb_gz_deflate(frb_ctx* ctx, const void* host_in, uint64_t n, void* host_out, uint64_t cap, uint64_t* out_n);
+/* Largest member frb_gz_deflate writes for n bytes: n + 5 per started 16 KiB piece + 20 (no context needed).   */
+uint64_t frb_gz_deflate_bound(uint64_t n);
 /* Per-file results (index = order of frb_scan_end calls) and the merged "total".            */
 int frb_file_count(frb_ctx* ctx, uint32_t* n_files);
 int frb_file_size(frb_ctx* ctx, uint32_t file_idx, uint64_t* n_unique, uint64_t* n_reads);
@@ -241,6 +248,12 @@ int frb_route_reserve(frb_ctx* ctx, uint64_t chunk_bytes);
 int frb_route_push(frb_ctx* ctx, const void* r1, uint64_t r1_bytes, const void* r2, uint64_t r2_bytes, int final_chunk);
 int frb_route_pop(frb_ctx* ctx, void** out_r1, void** out_r2, uint64_t* off_r1, uint64_t* off_r2, uint64_t* n_pairs,
                   uint64_t* carry_r1, uint64_t* carry_r2, uint64_t* bad_key);
+/* Gzip mode of the demux stream (on != 0): every chunk is compressed on the device behind the router, and only the
+ * compressed bytes cross to the host.  frb_route_pop keeps its meaning, except that out_m[off_m[s], off_m[s + 1]) is
+ * one gzip member holding exactly the bytes plain mode returns for sink s of mate m in that chunk; an empty cell stays
+ * empty.  Refused with FRB_ERR_STATE while chunks are in flight; kept by frb_route_reset.  frb_route_pair always
+ * returns plain bytes.                                                                                          */
+int frb_route_set_gzip(frb_ctx* ctx, int on);
 
 /* ---- multi-GPU: merge of the per-rank totals over NCCL (NVLink) ------------------------------
  * One process (or thread) per GPU.  Rank 0 makes the id, the host hands it to every rank.
@@ -270,7 +283,8 @@ int frb_synth_generate(frb_ctx* ctx, uint64_t g0, uint64_t g1, int read_no, void
 #define FRB_K_OTHER 4
 #define FRB_K_VERIFY 5 /* line phase of every tile by count (check of the speculative scan) */
 #define FRB_K_INFLATE 6 /* device-side gzip inflate */
-#define FRB_K_NUM 7
+#define FRB_K_DEFLATE 7 /* device-side gzip writer  */
+#define FRB_K_NUM 8
 int frb_timer_start(frb_ctx* ctx);            /* CUDA event on the compute stream              */
 int frb_timer_stop(frb_ctx* ctx, float* ms);  /* second event, synchronises, elapsed ms        */
 int frb_prof_enable(frb_ctx* ctx, int on);    /* per-kernel-class event pairs                  */

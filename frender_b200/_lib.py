@@ -57,6 +57,9 @@ SIGNATURES = {
     "frb_scan_gz": (C.c_int, [vp, C.c_char_p, u32, u64, P(u64), P(u64), P(u64)]),
     "frb_scan_gz_batch": (C.c_int, [vp, vp, vp, u32, vp, vp, vp, P(C.c_int)]),
     "frb_gz_inflate": (C.c_int, [vp, C.c_char_p, vp, u64, P(u64), P(C.c_int)]),
+    "frb_gz_open": (C.c_int, [vp, u32, C.c_char_p]),
+    "frb_gz_read": (C.c_int, [vp, u32, u64, P(vp), P(u64), P(C.c_int), P(C.c_int), P(u64), vp]),
+    "frb_gz_close": (C.c_int, [vp, u32]),
     "frb_gz_deflate": (C.c_int, [vp, vp, u64, vp, u64, P(u64)]),
     "frb_gz_deflate_bound": (u64, [u64]),
     "frb_file_count": (C.c_int, [vp, P(u32)]),

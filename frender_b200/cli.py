@@ -686,6 +686,48 @@ class TextChunks:
         return piece
 
 
+class DeviceTextChunks:
+    """TextChunks' interface over a span reader of `ctx` (Context.gz_read, mate `slot`): the text is inflated on the
+    device, and read() returns spans in device memory that route_push copies from there.  They are cut exactly where
+    TextChunks cuts (`size` bytes, fewer only at the end), and eof turns True on the read that returns nothing, so the
+    stream sees the same pushes.  When the device path hands the file back (FRB_GZ_RETRY_HOST causes, a damaged
+    file), a TextChunks takes over behind the text already returned; it raises whatever zlib raises."""
+
+    def __init__(self, ctx, slot, path):
+        self.ctx, self.slot, self.path = ctx, slot, path
+        self.eof = False
+        self.host = None                            # the TextChunks that took over
+        ctx.gz_open(slot, path)
+
+    @property
+    def on_device(self):
+        return self.host is None
+
+    def read(self, size):
+        if self.host is not None:
+            out = self.host.read(size)
+            self.eof = self.host.eof
+            return out
+        span = self.ctx.gz_read(self.slot, max(size, 1))
+        if span.declined:
+            self.ctx.gz_close(self.slot)
+            self.host = TextChunks(self.path)
+            left = span.delivered                   # checked text without '\r': the same bytes in text mode
+            while left:
+                got = len(self.host.fh.read(min(left, 1 << 24)))
+                if not got:
+                    break
+                left -= got
+            return self.read(size)
+        if span.size == 0:
+            self.eof = True
+        return span
+
+    def close(self):
+        if self.host is None:
+            self.ctx.gz_close(self.slot)
+
+
 def _demux_worker(rank, device, jobs, opts, out_dir, threads, conn):
     """One process per GPU: the file pairs `jobs` = [(ordinal, r1, r2)], each into its own part directory."""
     try:
@@ -833,6 +875,8 @@ def frender_demux(args, ctx=None):
         ctx.set_wide(wide)
     keys, keys_hi = pack_keys2(list(table.keys())) if wide else (pack_keys(list(table.keys())), None)
     chunk = max(int(os.environ.get("FRENDER_DEMUX_CHUNK_MB", "64")) << 20, MIN_CHUNK)
+    # FRB_GZ_DEVICE=0: the mates are inflated by zlib on the host, else on the device (DeviceTextChunks)
+    device_inflate = os.environ.get("FRB_GZ_DEVICE", "1") != "0"
     # Host side of the router: inflate of the two mates and deflate of the sinks run on a thread pool (zlib
     # releases the GIL).  Every sink sees the same sequence of compress() calls as a serial loop would make,
     # so the output files are byte-identical to it; the writes of chunk k overlap the inflate of chunk k+1.
@@ -858,6 +902,16 @@ def frender_demux(args, ctx=None):
             if off2[s + 1] > off2[s]:
                 writes.append(pool.submit(sinks[s]["R2"].write, o2[off2[s]:off2[s + 1]]))
 
+    mates = []
+
+    def fill(want):
+        """The next piece of both mates: host mates on the pool, device mates in this thread (a context is not
+        thread-safe)."""
+        jobs = [(m, 0 if m.eof else w) for m, w in zip(mates, want)]
+        futures = [None if getattr(m, "on_device", False) else pool.submit(m.read, n) for m, n in jobs]
+        got = [m.read(n) if f is None else None for (m, n), f in zip(jobs, futures)]
+        return [g if f is None else f.result() for g, f in zip(got, futures)]
+
     try:
         ctx.route_load(keys, routes, n_sinks + 1, keys_hi)
         ctx.route_gzip(gpu_gzip)
@@ -866,13 +920,14 @@ def frender_demux(args, ctx=None):
             # The pair as a STREAM of chunks, two in flight: while chunk k is routed on the device and chunk k-1
             # comes back and is deflated, chunk k+1 is inflated.  Chunks are cut anywhere; records that are not
             # complete yet (and the lead of one mate over the other) are carried on the device.
-            a, b = TextChunks(r1_path), TextChunks(r2_path)
+            mates[:] = ([DeviceTextChunks(ctx, 0, r1_path), DeviceTextChunks(ctx, 1, r2_path)] if device_inflate
+                        else [TextChunks(r1_path), TextChunks(r2_path)])
+            a, b = mates
             ctx.route_reset(chunk)
             flags, carry, over = [], (0, 0), False
             while not over:
                 want = [max(chunk - c, MIN_CHUNK // 4) for c in carry]   # carry + new bytes stay within the window
-                fills = [pool.submit(a.read, 0 if a.eof else want[0]), pool.submit(b.read, 0 if b.eof else want[1])]
-                da, db = (f.result() for f in fills)
+                da, db = fill(want)
                 flags.append((1 if a.eof else 0) | (2 if b.eof else 0))
                 ctx.route_push(da, db, flags[-1])
                 over = a.eof and b.eof
@@ -895,6 +950,9 @@ def frender_demux(args, ctx=None):
         finally:
             list(pool.map(lambda s: (s["R1"].close(), s["R2"].close()), sinks))
             pool.shutdown()
+        for m in mates:                             # the readers' buffers (a next gz_open would reuse the slot)
+            if isinstance(m, DeviceTextChunks):
+                m.close()
         if own_ctx:
             ctx.close()
 

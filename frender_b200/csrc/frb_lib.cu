@@ -11,6 +11,7 @@
 #include <cstdlib>
 #include <chrono>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -124,6 +125,8 @@ struct frb_ctx {
     struct DeflateHolder* deflate = nullptr;
     // device inflate (frb_gz.inl)
     struct GzBuffersHolder* gzbuf = nullptr;
+    // span readers of frb_gz_open / frb_gz_read, one per mate (frb_gz.inl)
+    struct GzReaderSlots* gzread = nullptr;
     // synth
     SynthArgs synth{};
     unsigned *synth_i7 = nullptr, *synth_i5 = nullptr;
@@ -584,6 +587,17 @@ int ensure_stages(frb_ctx* c) {
 struct GzBuffersHolder {
     GzBuffers b;
 };
+struct GzReaderSlots {
+    std::unique_ptr<GzTextReader> r[2];
+};
+
+static void gz_readers_destroy(frb_ctx* c) {
+    if (!c->gzread) return;
+    for (auto& r : c->gzread->r)
+        if (r) gz_text_free(c, *r);
+    delete c->gzread;
+    c->gzread = nullptr;
+}
 
 static void route_stream_destroy(frb_ctx* c);  // frb_route.inl
 static void deflate_destroy(frb_ctx* c);       // frb_deflate.inl
@@ -671,6 +685,7 @@ void frb_destroy(frb_ctx* c) {
     cudaFree(c->type), cudaFree(c->typerc), cudaFree(c->work), cudaFree(c->work_n), cudaFree(c->cub_tmp), cudaFree(c->route_tab);
     route_stream_destroy(c);
     deflate_destroy(c);
+    gz_readers_destroy(c);
     if (c->gzbuf) {
         gz_free(c->gzbuf->b);
         delete c->gzbuf;
@@ -1410,6 +1425,60 @@ int frb_gz_inflate(frb_ctx* c, const char* path, void* host_out, uint64_t cap, u
     if (rc == FRB_GZ_RETRY_HOST) return FRB_OK;
     if (rc != FRB_OK) return rc;
     *nbytes = off, *used_device = 1;
+    return FRB_OK;
+}
+
+// Span readers (GzTextReader, frb_gz.inl): the text of a .gz file in device memory, in spans of an exact size.
+int frb_gz_open(frb_ctx* c, uint32_t slot, const char* path) {
+    CU(c, cudaSetDevice(c->device));
+    if (slot >= 2 || !path) return fail(c, FRB_ERR_ARG, "frb_gz_open: slot must be 0 or 1, path not NULL");
+    TRY(frb_gz_close(c, slot));
+    if (!c->gzread) c->gzread = new GzReaderSlots();
+    std::unique_ptr<GzTextReader> r(new GzTextReader());
+    r->src.paths.emplace_back(path);
+    const int rc = r->src.open(c);
+    if (rc == FRB_ERR_IO) r->declined = true;  // zlib names the problem (FileNotFoundError, ...)
+    else TRY(rc);
+    c->gzread->r[slot] = std::move(r);
+    return FRB_OK;
+}
+
+int frb_gz_read(frb_ctx* c, uint32_t slot, uint64_t max_bytes, const void** dev_text, uint64_t* n, int* eof, int* declined,
+                uint64_t* delivered, void* host_copy) {
+    CU(c, cudaSetDevice(c->device));
+    if (!dev_text || !n || !eof || !declined || !delivered) return fail(c, FRB_ERR_ARG, "frb_gz_read: null output");
+    *dev_text = nullptr, *n = 0, *eof = 0, *declined = 0, *delivered = 0;
+    if (slot >= 2 || !c->gzread || !c->gzread->r[slot]) return fail(c, FRB_ERR_STATE, "frb_gz_read: slot %u is not open", slot);
+    if (max_bytes == 0) return fail(c, FRB_ERR_ARG, "frb_gz_read: max_bytes must be at least 1");
+    GzTextReader& R = *c->gzread->r[slot];
+    if (!R.declined) {
+        const unsigned char* text = nullptr;
+        bool end = false;
+        const int rc = gz_text_read(c, R, max_bytes, &text, n, &end);
+        if (rc == FRB_GZ_RETRY_HOST || rc == FRB_ERR_IO) {
+            R.declined = true;
+            R.p.reset();
+            *n = 0;
+        } else {
+            TRY(rc);
+            *dev_text = text, *eof = end ? 1 : 0;
+            if (host_copy && *n) {
+                CU(c, cudaMemcpyAsync(host_copy, text, *n, cudaMemcpyDeviceToHost, c->compute));
+                CU(c, cudaStreamSynchronize(c->compute));
+            }
+        }
+    }
+    *declined = R.declined ? 1 : 0;
+    *delivered = R.delivered;
+    return FRB_OK;
+}
+
+int frb_gz_close(frb_ctx* c, uint32_t slot) {
+    CU(c, cudaSetDevice(c->device));
+    if (slot >= 2) return fail(c, FRB_ERR_ARG, "frb_gz_close: slot must be 0 or 1");
+    if (!c->gzread || !c->gzread->r[slot]) return FRB_OK;
+    gz_text_free(c, *c->gzread->r[slot]);
+    c->gzread->r[slot].reset();
     return FRB_OK;
 }
 

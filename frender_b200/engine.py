@@ -92,6 +92,30 @@ def _ptr(arr):
     return arr.ctypes.data_as(C.c_void_p) if arr is not None else None
 
 
+class GzSpan:
+    """One frb_gz_read: `size` bytes of text at device address `ptr` (valid until the reader has inflated two more
+    pieces), `eof` when nothing follows them -- or `declined`: the device path handed the file back after
+    `delivered` bytes of text, and zlib goes on from there.  `data`: the same bytes on the host (read with copy=True)."""
+    __slots__ = ("ptr", "size", "eof", "declined", "delivered", "data")
+
+    def __init__(self, ptr, size, eof, declined, delivered, data=None):
+        self.ptr, self.size, self.eof = ptr, size, eof
+        self.declined, self.delivered, self.data = declined, delivered, data
+
+    def __len__(self):
+        return self.size
+
+
+def _chunk_arg(x):
+    """route_push's view of one mate: (pointer, bytes, keep-alive) for host bytes or a device GzSpan."""
+    if isinstance(x, GzSpan):
+        if x.declined:
+            raise ValueError("a declined GzSpan holds no text")
+        return C.c_void_p(x.ptr), x.size, None
+    a = np.frombuffer(x, np.uint8)
+    return _ptr(a), a.size, a
+
+
 class PackedSheet:
     """Sample sheet in the matcher's layout (frb_sheet_load)."""
 
@@ -207,6 +231,24 @@ class Context:
         n, used = C.c_uint64(), C.c_int()
         self._ck(lib.frb_gz_inflate(self._h, os.fsencode(str(path)), _ptr(out), cap, C.byref(n), C.byref(used)))
         return out[:n.value].tobytes() if used.value else None
+
+    def gz_open(self, slot, path):
+        """A span reader over the text of a .gz file, inflated on the device (frb_gz_open); slot 0 or 1."""
+        self._ck(lib.frb_gz_open(self._h, slot, os.fsencode(str(path))))
+
+    def gz_read(self, slot, max_bytes, copy=False):
+        """The next span of exactly max_bytes bytes (fewer only at the end of the text) as a GzSpan (frb_gz_read);
+        size 0 after the end.  copy=True also brings the bytes to the host (GzSpan.data)."""
+        ptr, n, eof, declined, delivered = C.c_void_p(), C.c_uint64(), C.c_int(), C.c_int(), C.c_uint64()
+        out = np.empty(max(max_bytes, 1), np.uint8) if copy else None
+        self._ck(lib.frb_gz_read(self._h, slot, max_bytes, C.byref(ptr), C.byref(n), C.byref(eof), C.byref(declined),
+                                 C.byref(delivered), _ptr(out)))
+        data = out[:n.value].tobytes() if copy else None
+        return GzSpan(ptr.value or 0, n.value, bool(eof.value), bool(declined.value), delivered.value, data)
+
+    def gz_close(self, slot):
+        """Free a span reader's thread and buffers (frb_gz_close)."""
+        self._ck(lib.frb_gz_close(self._h, slot))
 
     def gz_deflate(self, data):
         """One buffer -> one gzip member, encoded on the device (frb_gz_deflate); zlib.decompress(x, 31) inverts it."""
@@ -500,10 +542,10 @@ class Context:
 
     def route_push(self, r1, r2, final=0):
         """Queue one chunk pair of the demux stream (frb_route_push): bytes cut anywhere; what is not complete
-        yet is carried on the device.  Returns at once; at most two chunks may be in flight."""
-        a = np.frombuffer(r1, np.uint8)
-        b = np.frombuffer(r2, np.uint8)
-        self._ck(lib.frb_route_push(self._h, _ptr(a), a.size, _ptr(b), b.size, int(final)))
+        yet is carried on the device.  Either mate may be host bytes or a device GzSpan of this context (gz_read).
+        Returns at once; at most two chunks may be in flight."""
+        (pa, na, _ka), (pb, nb, _kb) = _chunk_arg(r1), _chunk_arg(r2)
+        self._ck(lib.frb_route_push(self._h, pa, na, pb, nb, int(final)))
 
     def route_pop(self):
         """The oldest chunk in flight (frb_route_pop): (out_r1, out_r2, off_r1, off_r2, pairs, carry_r1, carry_r2).

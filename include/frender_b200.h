@@ -143,6 +143,22 @@ int frb_scan_gz_batch(frb_ctx* ctx, const char* const* paths, const uint32_t* or
  * the stream (blocks larger than a chunk, '\r' in the text, ...) and nothing was written; frb_scan_gz falls back
  * to zlib on a host thread for such a file.                                                                */
 int frb_gz_inflate(frb_ctx* ctx, const char* path, void* host_out, uint64_t cap, uint64_t* nbytes, int* used_device);
+/* Span readers: the text of a .gz file inflated ON THE DEVICE and handed out in device memory, for the demux stream
+ * (frb_route_push takes the spans).  A context has two slots (0, 1), one per mate; frb_gz_open closes what the slot
+ * held, frb_gz_close frees a slot's thread and buffers (a no-op on a closed slot), frb_destroy closes both.
+ * frb_gz_read: *dev_text / *n = a span of EXACTLY max_bytes (>= 1) bytes of text, fewer only where the text ends;
+ * *eof = 1 when nothing follows the span; *n = 0 after the end.  A span stays valid until the reader has inflated
+ * two more pieces (FRB_GZ_PIECE_MB of compressed bytes each), and a copy of it that frb_route_push queued is always
+ * done before the reader writes its buffer again.  host_copy: NULL, or max_bytes bytes that receive the span too.
+ * *declined = 1: the device path handed the file back -- '\r' in the text, no block start found, not gzip, a
+ * truncated file, a CRC-32 / ISIZE mismatch, a read error -- and *n = 0.  *delivered = the text bytes handed out so
+ * far (always set); the caller goes on with zlib behind them, and zlib reports any error of the file.  Every read
+ * after that says declined again.  Staging overflow is handled inside: the reader starts over with larger staging
+ * areas and skips what it handed out.                                                                          */
+int frb_gz_open(frb_ctx* ctx, uint32_t slot, const char* path);
+int frb_gz_read(frb_ctx* ctx, uint32_t slot, uint64_t max_bytes, const void** dev_text, uint64_t* n, int* eof,
+                int* declined, uint64_t* delivered, void* host_copy);
+int frb_gz_close(frb_ctx* ctx, uint32_t slot);
 /* One buffer -> one gzip member (RFC 1952, zlib's wbits=31 header), encoded ON THE DEVICE (deflate_kernels.cuh:
  * LZ77 + dynamic Huffman per 16 KiB piece, stored where that is not smaller).  host_in: n bytes, pinned or pageable;
  * host_out: cap >= frb_gz_deflate_bound(n) bytes, else FRB_ERR_ARG; *out_n = bytes written.  n = 0 gives the
@@ -236,8 +252,10 @@ int frb_route_pair(frb_ctx* ctx, const void* r1, uint64_t r1_bytes, const void* 
 /* The same as a STREAM, two chunk pairs in flight: push queues a chunk pair and returns (H2D, kernels and the D2H
  * of the chunk before run at the same time); the inputs may be cut anywhere -- records that are not complete yet,
  * and the lead of one mate over the other, are carried on the device into the next chunk.  A stream's chunks may
- * not be larger than its first one.  final_chunk bit 0 / 1: the R1 / R2 file ends with this chunk.
- *   frb_route_pop   the oldest chunk in flight: *out_r1 / *out_r2 point into pinned memory of the library (valid
+ * not be larger than its first one.  final_chunk bit 0 / 1: the R1 / R2 file ends with this chunk.  Either mate may
+ * be host memory (pinned or pageable) or device memory of the context's device, e.g. a span of frb_gz_read (copied
+ * device to device on the copy stream); memory of another device is FRB_ERR_ARG.
+ *   frb_route_pop  the oldest chunk in flight: *out_r1 / *out_r2 point into pinned memory of the library (valid
  *                   until the chunk after next is pushed), sink s of mate m is out_m[off_m[s], off_m[s + 1]);
  *                   carry_r1 / carry_r2 = bytes pushed so far that are not routed yet.
  *   frb_route_reset a new stream begins (nothing carried).

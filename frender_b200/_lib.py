@@ -17,6 +17,7 @@ RULE_SCAN, RULE_DEMUX = 0, 1
 CARRY = 0xFFFFFFFFFFFFFFFF
 K_SCAN, K_EXPORT, K_MATCH, K_ROUTE, K_OTHER, K_VERIFY, K_INFLATE, K_DEFLATE = range(8)
 K_NUM = 8
+GZ_FORMAT_PLAIN, GZ_FORMAT_GZIP, GZ_FORMAT_BGZF = 0, 1, 2
 READ_TYPES = ("undetermined", "index_hop", "demuxable", "ambiguous")
 
 u64, u32, i32, u8 = C.c_uint64, C.c_uint32, C.c_int32, C.c_uint8
@@ -62,6 +63,8 @@ SIGNATURES = {
     "frb_gz_close": (C.c_int, [vp, u32]),
     "frb_gz_deflate": (C.c_int, [vp, vp, u64, vp, u64, P(u64)]),
     "frb_gz_deflate_bound": (u64, [u64]),
+    "frb_gz_deflate_bgzf": (C.c_int, [vp, vp, u64, vp, u64, P(u64)]),
+    "frb_gz_deflate_bgzf_bound": (u64, [u64]),
     "frb_file_count": (C.c_int, [vp, P(u32)]),
     "frb_file_size": (C.c_int, [vp, u32, P(u64), P(u64)]),
     "frb_file_export": (C.c_int, [vp, u32, vp, vp, vp, u64]),
@@ -81,6 +84,7 @@ SIGNATURES = {
     "frb_route_push": (C.c_int, [vp, vp, u64, vp, u64, C.c_int]),
     "frb_route_pop": (C.c_int, [vp, P(vp), P(vp), vp, vp, P(u64), P(u64), P(u64), P(u64)]),
     "frb_route_set_gzip": (C.c_int, [vp, C.c_int]),
+    "frb_route_set_gz_format": (C.c_int, [vp, C.c_int]),
     "frb_nccl_unique_id": (C.c_int, [C.c_char_p]),
     "frb_nccl_init": (C.c_int, [vp, C.c_char_p, C.c_int, C.c_int]),
     "frb_allmerge": (C.c_int, [vp, P(u64)]),

@@ -18,7 +18,7 @@ from pathlib import Path
 
 import numpy as np
 
-from . import _lib
+from . import _lib, bgzf
 from .engine import (Context, FrbError, MAX_SYMS as _MAX_SYMS, READ_TYPES, pack_keys, pack_keys2, reverse_complement,
                      unpack_keys)
 
@@ -662,6 +662,22 @@ class MemberSink:
         self.fh.close()
 
 
+class BgzfSink:
+    """One output file of FRENDER_GZIP_LEVEL=bgzf: the runs of BGZF blocks the device wrote for it, one per chunk,
+    appended as they come, and the EOF block at close.  A file that received none is the EOF block alone."""
+
+    def __init__(self, path):
+        self.fh = open(path, "wb")
+
+    def write(self, data):
+        if len(data):
+            self.fh.write(data)
+
+    def close(self):
+        self.fh.write(bgzf.EOF_BLOCK)
+        self.fh.close()
+
+
 class TextChunks:
     """Decompressed bytes of a fastq.gz with the newline translation of text mode (F:776), piece by piece."""
 
@@ -750,11 +766,25 @@ def _demux_worker(rank, device, jobs, opts, out_dir, threads, conn):
         conn.close()
 
 
+def join_parts(out_path, part_paths, bgzf_parts):
+    """One sink of a multi-GPU demux from its parts, in pair order: gzip members one after the other, or for BGZF
+    parts their blocks with one EOF block at the end (bgzf.join_files)."""
+    if bgzf_parts:
+        bgzf.join_files(out_path, part_paths)
+        return
+    import shutil
+    with open(out_path, "wb") as out:
+        for part in part_paths:
+            with open(part, "rb") as src:
+                shutil.copyfileobj(src, out, 1 << 22)
+
+
 def demux_pairs_multi_gpu(args, pairs, n_gpus, out_dir, worker=_demux_worker):
     """FRENDER_GPUS=N with several R1/R2 pairs (lanes): pair i is routed on GPU i % N into rank-local part files
     (SURVEY 8e: the demux outputs stay rank-local); the parts of every sink are then appended in pair order --
     gzip members one after the other, so every sink decompresses to exactly what the sequential loop over the
-    pairs (F:774) writes."""
+    pairs (F:774) writes.  With FRENDER_GZIP_LEVEL=bgzf the parts' EOF blocks but the last are dropped, and every
+    sink is byte for byte the file the sequential loop writes."""
     import multiprocessing as mp
     import shutil
     from multiprocessing.connection import wait
@@ -795,13 +825,18 @@ def demux_pairs_multi_gpu(args, pairs, n_gpus, out_dir, worker=_demux_worker):
     if failure is not None:
         raise SystemExit(failure)
     parts = [f"{out_dir}.part{i}" for i in range(len(pairs))]
+    bgzf_parts = gzip_level() == "bgzf"
     for name in sorted(os.listdir(parts[0])):
-        with open(out_dir + name, "wb") as out:
-            for part in parts:
-                with open(os.path.join(part, name), "rb") as src:
-                    shutil.copyfileobj(src, out, 1 << 22)
+        join_parts(out_dir + name, [os.path.join(part, name) for part in parts], bgzf_parts)
     for part in parts:
         shutil.rmtree(part)
+
+
+def gzip_level():
+    """FRENDER_GZIP_LEVEL: a zlib level for the host deflate (an int, default 6), "gpu" for gzip members written
+    on the device, or "bgzf" for BGZF blocks written on the device."""
+    level = os.environ.get("FRENDER_GZIP_LEVEL", "6").strip().lower()
+    return level if level in ("gpu", "bgzf") else int(level)
 
 
 def frender_demux(args, ctx=None):
@@ -833,10 +868,8 @@ def frender_demux(args, ctx=None):
     n_gpus = int(os.environ.get("FRENDER_GPUS", "1"))
     if ctx is None and n_gpus > 1 and len(pairs) > 1:
         return demux_pairs_multi_gpu(args, pairs, min(n_gpus, len(pairs)), out_dir)
-    # FRENDER_GZIP_LEVEL: a zlib level for the host deflate, or "gpu" for gzip members written on the device
-    level = os.environ.get("FRENDER_GZIP_LEVEL", "6").strip().lower()
-    gpu_gzip = level == "gpu"
-    level = None if gpu_gzip else int(level)
+    level = gzip_level()
+    gpu_gzip, gpu_bgzf = level == "gpu", level == "bgzf"
     infix = args.o + "_" if args.o else ""
     sink_names = []                                                             # sink id -> name
 
@@ -848,7 +881,7 @@ def frender_demux(args, ctx=None):
     undeter_sink = open_sink(undeter_name) if undeter else None
     hop_sink = open_sink("Index-hop") if index_hop else undeter_sink
     amb_sink = open_sink("Ambiguous") if ambiguous else undeter_sink
-    sink_file = (lambda path: MemberSink(path)) if gpu_gzip else (lambda path: GzSink(path, level))
+    sink_file = (MemberSink if gpu_gzip else BgzfSink if gpu_bgzf else (lambda path: GzSink(path, level)))
     sinks = [{r: sink_file(f"{out_dir}{name}_frender-demux_{infix}{r}.fq.gz") for r in ("R1", "R2")}
              for name in sink_names]
     n_sinks = len(sink_names)
@@ -880,7 +913,8 @@ def frender_demux(args, ctx=None):
     # Host side of the router: inflate of the two mates and deflate of the sinks run on a thread pool (zlib
     # releases the GIL).  Every sink sees the same sequence of compress() calls as a serial loop would make,
     # so the output files are byte-identical to it; the writes of chunk k overlap the inflate of chunk k+1.
-    # With FRENDER_GZIP_LEVEL=gpu the device writes the members and the pool only appends them to the files.
+    # With FRENDER_GZIP_LEVEL=gpu (or bgzf) the device writes the members (or blocks) and the pool only appends them
+    # to the files.
     from concurrent.futures import ThreadPoolExecutor
     workers = max(2, int(os.environ.get("FRENDER_DEMUX_THREADS", str(len(os.sched_getaffinity(0))))))
     pool = ThreadPoolExecutor(max_workers=workers)
@@ -914,7 +948,7 @@ def frender_demux(args, ctx=None):
 
     try:
         ctx.route_load(keys, routes, n_sinks + 1, keys_hi)
-        ctx.route_gzip(gpu_gzip)
+        ctx.route_gzip(gpu_gzip or gpu_bgzf, bgzf=gpu_bgzf)
         for r1_path, r2_path in pairs:
             print(f"Demultiplexing {r1_path.name}...")
             # The pair as a STREAM of chunks, two in flight: while chunk k is routed on the device and chunk k-1

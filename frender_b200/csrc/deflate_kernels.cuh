@@ -13,6 +13,12 @@
 //   deflate_cells_kernel   member offsets of the cells, gzip header and "03 00" + CRC-32 + ISIZE of every member
 //   deflate_gather_kernel  the piece bytes into place
 //
+// BGZF (the blocked gzip of htslib and bgzip) is a layout of the same pieces.  deflate_split_kernel cuts every cell
+// into blocks of at most kBgzfBlock bytes (three pieces), the five kernels above run over the blocks as if they were
+// cells -- so no back-reference crosses a block start and every block is a member of its own -- with htslib's
+// 18-byte header (the BC extra field holds the block's size), and deflate_cell_offsets_kernel gives every cell the
+// offset of its first block.  A cell is then a run of whole BGZF blocks; the 28-byte EOF block is the caller's.
+//
 // LZ77 of a piece: back-references reach into the kHist bytes of the same cell in front of the piece (never into
 // another cell), at most 32 KiB back, lengths 3..258.  Candidates come from a hash table of 4-byte prefixes in
 // shared memory that is filled in rounds of 256 positions: a position sees the latest earlier position of its hash
@@ -45,6 +51,9 @@ constexpr unsigned kSeg = kPiece / kLanes;
 constexpr int kMaxMatch = 258;
 constexpr unsigned kWindow = 32768;
 constexpr int kHeaderBytes = 10, kTrailerBytes = 10;  // gzip header; final empty block (2) + CRC-32 + ISIZE
+constexpr unsigned kBgzfBlock = 3 * kPiece;  // BGZF: input bytes per block (at most 49,195 bytes written)
+constexpr int kBgzfHeaderBytes = 18;         // gzip header with the 6-byte BC extra field
+constexpr int kBgzfEofBytes = 28;            // the empty block that ends a BGZF file
 
 struct PieceInfo {
     unsigned out;    // bytes of the piece in its scratch slot
@@ -222,6 +231,47 @@ __device__ inline void build_code(unsigned* freq, int n, int maxlen, unsigned ch
 }
 
 // ---- kernels ------------------------------------------------------------------------------------------------------
+// BGZF: block_off[0, n_blocks] = the cells cut into blocks of at most kBgzfBlock bytes, cell after cell; entries
+// behind the last block repeat the end offset (empty blocks: no output).  first_block[c] = blocks in front of cell c
+// (n_cells + 1 entries; the last is the block count).  A cell list that is not ordered, or reaches beyond max_bytes,
+// or a raised *skip, gives no blocks at all (every offset 0).  One block.
+__global__ void __launch_bounds__(1024) deflate_split_kernel(const unsigned long long* __restrict__ cell_off, unsigned n_cells,
+                                                             unsigned long long max_bytes, const int* __restrict__ skip,
+                                                             unsigned long long* __restrict__ block_off, unsigned n_blocks,
+                                                             unsigned* __restrict__ first_block) {
+    __shared__ unsigned s_sum[1024];
+    __shared__ unsigned s_bad;
+    const unsigned t = threadIdx.x;
+    if (t == 0) s_bad = (skip && *skip) || cell_off[n_cells] - cell_off[0] > max_bytes || cell_off[n_cells] < cell_off[0];
+    __syncthreads();
+    const unsigned per = (n_cells + 1023) / 1024, c0 = min(n_cells, t * per), c1 = min(n_cells, c0 + per);
+    unsigned local = 0;
+    for (unsigned c = c0; c < c1; ++c) {
+        if (cell_off[c + 1] < cell_off[c]) s_bad = 1;
+        local += static_cast<unsigned>((cell_off[c + 1] - cell_off[c] + kBgzfBlock - 1) / kBgzfBlock);
+    }
+    s_sum[t] = local;
+    __syncthreads();
+    for (unsigned d = 1; d < 1024; d <<= 1) {
+        const unsigned v = t >= d ? s_sum[t - d] : 0u;
+        __syncthreads();
+        s_sum[t] += v;
+        __syncthreads();
+    }
+    const bool bad = s_bad != 0 || s_sum[1023] > n_blocks;
+    unsigned run = bad ? 0u : s_sum[t] - local;
+    for (unsigned c = c0; c < c1; ++c) {
+        first_block[c] = run;
+        if (bad) continue;
+        const unsigned long long a = cell_off[c], len = cell_off[c + 1] - a;
+        for (unsigned long long j = 0; j * kBgzfBlock < len; ++j) block_off[run++] = a + j * kBgzfBlock;
+    }
+    const unsigned total = bad ? 0u : s_sum[1023];
+    const unsigned long long end = bad ? 0ull : cell_off[n_cells];
+    if (t == 1023) first_block[n_cells] = total;
+    for (unsigned b = total + t; b <= n_blocks; b += 1024) block_off[b] = end;
+}
+
 // first_piece[c] = pieces in front of cell c (n_cells + 1 entries; the last is the piece count).  A cell list that is
 // not ordered, or reaches beyond max_bytes, or a raised *skip, gives no pieces: the caller reports its own error.
 __global__ void __launch_bounds__(1024) deflate_plan_kernel(const unsigned long long* __restrict__ cell_off, unsigned n_cells,
@@ -516,19 +566,19 @@ __global__ void __launch_bounds__(kThreads, 2) deflate_piece_kernel(const unsign
     }
 }
 
-// start[p] = output bytes in front of piece p's part (header / trailer included), start[n] = all;
+// start[p] = output bytes in front of piece p's part (header of `hdr` bytes / trailer included), start[n] = all;
 // crc_pre[p] = CRC-32 of the input of pieces [0, p).  One block.
 __global__ void __launch_bounds__(1024) deflate_layout_kernel(const PieceInfo* __restrict__ info,
                                                               const unsigned* __restrict__ first_piece, unsigned n_cells,
                                                               unsigned long long* __restrict__ start,
-                                                              unsigned* __restrict__ crc_pre, gz::CrcPowers pw) {
+                                                              unsigned* __restrict__ crc_pre, gz::CrcPowers pw, int hdr) {
     __shared__ unsigned long long s_sum[1024], s_len[1024];
     __shared__ unsigned s_crc[1024];
     const unsigned t = threadIdx.x, n = first_piece[n_cells];
     const unsigned per = (n + 1023) / 1024, p0 = min(n, t * per), p1 = min(n, p0 + per);
     const unsigned xfull = gz::crc_xpow8(pw, kPiece);
     auto size = [&](const PieceInfo& f) {
-        return static_cast<unsigned long long>(f.out) + ((f.flags & 1) ? kHeaderBytes : 0) + ((f.flags & 2) ? kTrailerBytes : 0);
+        return static_cast<unsigned long long>(f.out) + ((f.flags & 1) ? hdr : 0) + ((f.flags & 2) ? kTrailerBytes : 0);
     };
     auto join = [&](unsigned crc, const PieceInfo& f) {
         return gz::crc_mul(f.in == kPiece ? xfull : gz::crc_xpow8(pw, f.in), crc) ^ f.crc;
@@ -566,12 +616,13 @@ __global__ void __launch_bounds__(1024) deflate_layout_kernel(const PieceInfo* _
     if (t == 1023) start[n] = s_sum[1023], crc_pre[n] = s_crc[1023];
 }
 
-// Member offsets (n_cells + 1), gzip header and trailer of every non-empty cell.
+// Member offsets (n_cells + 1), gzip header and trailer of every non-empty cell.  bgzf: htslib's header, whose BC
+// field holds the member's size - 1 (the cells are BGZF blocks here).
 __global__ void __launch_bounds__(128) deflate_cells_kernel(const unsigned long long* __restrict__ cell_off, unsigned n_cells,
                                                             const unsigned* __restrict__ first_piece,
                                                             const unsigned long long* __restrict__ start,
                                                             const unsigned* __restrict__ crc_pre, unsigned char* __restrict__ out,
-                                                            unsigned long long* __restrict__ out_off, gz::CrcPowers pw) {
+                                                            unsigned long long* __restrict__ out_off, gz::CrcPowers pw, bool bgzf) {
     const unsigned c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c > n_cells) return;
     const unsigned a = first_piece[c];
@@ -581,8 +632,15 @@ __global__ void __launch_bounds__(128) deflate_cells_kernel(const unsigned long 
     if (a == b) return;
     const unsigned long long len = cell_off[c + 1] - cell_off[c];
     unsigned char* const h = out + start[a];
-    const unsigned char head[kHeaderBytes] = {0x1f, 0x8b, 8, 0, 0, 0, 0, 0, 0, 3};  // zlib's, wbits = 31
-    for (int i = 0; i < kHeaderBytes; ++i) h[i] = head[i];
+    if (bgzf) {
+        const unsigned bsize = static_cast<unsigned>(start[b] - start[a] - 1);
+        const unsigned char head[kBgzfHeaderBytes] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0,
+                                                      static_cast<unsigned char>(bsize), static_cast<unsigned char>(bsize >> 8)};
+        for (int i = 0; i < kBgzfHeaderBytes; ++i) h[i] = head[i];
+    } else {
+        const unsigned char head[kHeaderBytes] = {0x1f, 0x8b, 8, 0, 0, 0, 0, 0, 0, 3};  // zlib's, wbits = 31
+        for (int i = 0; i < kHeaderBytes; ++i) h[i] = head[i];
+    }
     const unsigned crc = crc_pre[b] ^ gz::crc_mul(gz::crc_xpow8(pw, len), crc_pre[a]);
     const unsigned isize = static_cast<unsigned>(len);
     unsigned char* const e = out + start[b] - kTrailerBytes;
@@ -590,18 +648,27 @@ __global__ void __launch_bounds__(128) deflate_cells_kernel(const unsigned long 
     for (int i = 0; i < 4; ++i) e[2 + i] = static_cast<unsigned char>(crc >> (8 * i)), e[6 + i] = static_cast<unsigned char>(isize >> (8 * i));
 }
 
-// Piece bytes into place.  One CTA per piece (grid-stride).
+// Piece bytes into place (behind a header of `hdr` bytes for a cell's first piece).  One CTA per piece (grid-stride).
 __global__ void __launch_bounds__(256) deflate_gather_kernel(const unsigned* __restrict__ first_piece, unsigned n_cells,
                                                              const PieceInfo* __restrict__ info,
                                                              const unsigned long long* __restrict__ start,
-                                                             const unsigned char* __restrict__ scratch, unsigned char* __restrict__ out) {
+                                                             const unsigned char* __restrict__ scratch, unsigned char* __restrict__ out,
+                                                             int hdr) {
     const unsigned n = first_piece[n_cells];
     for (unsigned p = blockIdx.x; p < n; p += gridDim.x) {
         const PieceInfo f = info[p];
         const unsigned char* const s = scratch + static_cast<unsigned long long>(p) * kPieceCap;
-        unsigned char* const d = out + start[p] + ((f.flags & 1) ? kHeaderBytes : 0);
+        unsigned char* const d = out + start[p] + ((f.flags & 1) ? hdr : 0);
         for (unsigned i = threadIdx.x; i < f.out; i += blockDim.x) d[i] = s[i];
     }
+}
+
+// BGZF: out_off[c] = output offset of cell c's first block (n_cells + 1 entries), from the blocks' offsets.
+__global__ void __launch_bounds__(128) deflate_cell_offsets_kernel(const unsigned* __restrict__ first_block, unsigned n_cells,
+                                                                   const unsigned long long* __restrict__ block_out,
+                                                                   unsigned long long* __restrict__ out_off) {
+    const unsigned c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c <= n_cells) out_off[c] = block_out[first_block[c]];
 }
 
 }  // namespace dfl

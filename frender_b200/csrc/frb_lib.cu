@@ -120,7 +120,7 @@ struct frb_ctx {
     uint64_t route_cap = 0;
     uint32_t n_sinks = 0;
     struct RouteStreamHolder* route = nullptr;  // the demux stream (frb_route.inl)
-    bool route_gzip = false;                    // the demux stream returns gzip members (frb_route_set_gzip)
+    int route_gz = FRB_GZ_FORMAT_PLAIN;         // the demux stream returns gzip members / BGZF blocks (frb_route_set_gz_format)
     // device gzip writer of frb_gz_deflate (frb_deflate.inl)
     struct DeflateHolder* deflate = nullptr;
     // device inflate (frb_gz.inl)

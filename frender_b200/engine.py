@@ -250,14 +250,18 @@ class Context:
         """Free a span reader's thread and buffers (frb_gz_close)."""
         self._ck(lib.frb_gz_close(self._h, slot))
 
-    def gz_deflate(self, data):
-        """One buffer -> one gzip member, encoded on the device (frb_gz_deflate); zlib.decompress(x, 31) inverts it."""
+    def gz_deflate(self, data, bgzf=False):
+        """One buffer -> one gzip member, encoded on the device (frb_gz_deflate); zlib.decompress(x, 31) inverts it.
+        bgzf=True: a complete BGZF file instead, blocks and EOF block (frb_gz_deflate_bgzf); gzip.decompress
+        inverts it."""
         a = np.frombuffer(data, np.uint8) if len(data) else np.zeros(1, np.uint8)
         n = len(data)
-        cap = lib.frb_gz_deflate_bound(n)
+        bound, encode = ((lib.frb_gz_deflate_bgzf_bound, lib.frb_gz_deflate_bgzf) if bgzf
+                         else (lib.frb_gz_deflate_bound, lib.frb_gz_deflate))
+        cap = bound(n)
         out = np.empty(cap, np.uint8)
         got = C.c_uint64()
-        self._ck(lib.frb_gz_deflate(self._h, _ptr(a), n, _ptr(out), cap, C.byref(got)))
+        self._ck(encode(self._h, _ptr(a), n, _ptr(out), cap, C.byref(got)))
         return out[:got.value].tobytes()
 
     def scan_bytes(self, data, ordinal=0, sample=None, rule=_lib.RULE_SCAN, name=None, chunk=None, line_base=0):
@@ -535,10 +539,15 @@ class Context:
         else:
             self._ck(lib.frb_route_reset(self._h))
 
-    def route_gzip(self, on=True):
+    def route_gzip(self, on=True, bgzf=False):
         """Gzip mode of the demux stream (frb_route_set_gzip): route_pop then returns one gzip member per non-empty
-        sink and mate, compressed on the device.  Only between chunks; kept by route_reset."""
-        self._ck(lib.frb_route_set_gzip(self._h, 1 if on else 0))
+        sink and mate, compressed on the device.  bgzf=True (with on): a run of whole BGZF blocks per non-empty
+        sink and mate instead, without the EOF block (frb_route_set_gz_format).  Only between chunks; kept by
+        route_reset."""
+        if on and bgzf:
+            self._ck(lib.frb_route_set_gz_format(self._h, _lib.GZ_FORMAT_BGZF))
+        else:
+            self._ck(lib.frb_route_set_gzip(self._h, 1 if on else 0))
 
     def route_push(self, r1, r2, final=0):
         """Queue one chunk pair of the demux stream (frb_route_push): bytes cut anywhere; what is not complete

@@ -56,6 +56,10 @@ extern "C" {
 #define FRB_RULE_SCAN 0            /* 2nd space token, last ':' field (F:169)                    */
 #define FRB_RULE_DEMUX 1           /* last ':' field of the whole line (F:778)                   */
 
+#define FRB_GZ_FORMAT_PLAIN 0      /* demux stream: routed bytes as they are                     */
+#define FRB_GZ_FORMAT_GZIP 1       /* one gzip member per cell                                   */
+#define FRB_GZ_FORMAT_BGZF 2       /* BGZF blocks (htslib / bgzip) per cell                      */
+
 #define FRB_TYPE_UNDETERMINED 0
 #define FRB_TYPE_INDEX_HOP 1
 #define FRB_TYPE_DEMUXABLE 2
@@ -166,6 +170,15 @@ int frb_gz_close(frb_ctx* ctx, uint32_t slot);
 int frb_gz_deflate(frb_ctx* ctx, const void* host_in, uint64_t n, void* host_out, uint64_t cap, uint64_t* out_n);
 /* Largest member frb_gz_deflate writes for n bytes: n + 5 per started 16 KiB piece + 20 (no context needed).   */
 uint64_t frb_gz_deflate_bound(uint64_t n);
+/* One buffer -> one complete BGZF file (the blocked gzip of htslib and bgzip), encoded ON THE DEVICE: blocks of at
+ * most 49,152 input bytes, each a gzip member of its own with htslib's 18-byte header (the BC extra field holds the
+ * block's size - 1), no back-reference across a block start, then the 28-byte EOF block.  Plain multi-member gzip to
+ * any gzip reader.  n = 0 gives the EOF block alone.  cap >= frb_gz_deflate_bgzf_bound(n), else FRB_ERR_ARG.  The
+ * same input always gives the same bytes.                                                                      */
+int frb_gz_deflate_bgzf(frb_ctx* ctx, const void* host_in, uint64_t n, void* host_out, uint64_t cap, uint64_t* out_n);
+/* Largest file frb_gz_deflate_bgzf writes for n bytes: n + 5 per started 16 KiB piece + 28 per started 48 KiB block
+ * + 28 (no context needed).                                                                                     */
+uint64_t frb_gz_deflate_bgzf_bound(uint64_t n);
 /* Per-file results (index = order of frb_scan_end calls) and the merged "total".            */
 int frb_file_count(frb_ctx* ctx, uint32_t* n_files);
 int frb_file_size(frb_ctx* ctx, uint32_t file_idx, uint64_t* n_unique, uint64_t* n_reads);
@@ -272,6 +285,12 @@ int frb_route_pop(frb_ctx* ctx, void** out_r1, void** out_r2, uint64_t* off_r1, 
  * empty.  Refused with FRB_ERR_STATE while chunks are in flight; kept by frb_route_reset.  frb_route_pair always
  * returns plain bytes.                                                                                          */
 int frb_route_set_gzip(frb_ctx* ctx, int on);
+/* The output format of the demux stream: FRB_GZ_FORMAT_PLAIN, _GZIP (= frb_route_set_gzip(ctx, 1)) or _BGZF.  In
+ * BGZF format out_m[off_m[s], off_m[s + 1]) is a run of whole BGZF blocks (no EOF block) holding exactly the bytes
+ * plain mode returns for sink s of mate m in that chunk, so a sink's file is its runs appended chunk after chunk and
+ * the EOF block behind them; an empty cell stays empty.  The same rules as frb_route_set_gzip; any other format is
+ * FRB_ERR_ARG.                                                                                                  */
+int frb_route_set_gz_format(frb_ctx* ctx, int format);
 
 /* ---- multi-GPU: merge of the per-rank totals over NCCL (NVLink) ------------------------------
  * One process (or thread) per GPU.  Rank 0 makes the id, the host hands it to every rank.

@@ -88,14 +88,61 @@ __host__ __device__ __forceinline__ unsigned long long hash64(unsigned long long
 constexpr unsigned long long kBadKeyBase = ~0ULL - 256ULL;
 
 #ifdef __CUDACC__
-__device__ __forceinline__ void raise_error(DevState* st, int code, unsigned long long pos) {
-    if (atomicCAS(&st->err_code, 0, code) == 0) st->err_pos = pos;
+// ---- key width ---------------------------------------------------------------------------------------------------
+// A narrow key (up to 21 symbols) is one word and lives in a Slot; a wide key (up to 42 symbols) is (lo, hi) and
+// lives in a WideSlot.  Lists keep a wide key's words in two arrays, keys and keys_hi.  Kernels that serve both
+// widths take `bool Wide` and find here what differs between them; they take tables as the Slot arrays they are
+// allocated as, so that both instantiations have one signature.
+template <bool Wide> struct KeyWidth;
+
+template <> struct KeyWidth<false> {
+    using Slot = frb::Slot;
+    using Key = unsigned long long;
+    __device__ static Key at(const unsigned long long* keys, const unsigned long long*, unsigned long long i) {
+        return keys[i];
+    }
+    __device__ static unsigned long long hash(Key k) { return hash64(k); }
+    __device__ static Key ones() { return kEmpty; }  // key of a slot that was filled with ones
+    __device__ static ulonglong4 free_slot() { return make_ulonglong4(kEmpty, ~0ULL, 0ULL, 0ULL); }  // key, first, count, aux
+    __device__ static bool is_free(Key k) { return k == kEmpty; }
+    __device__ static bool same(Key a, Key b) { return a == b; }
+    __device__ static Key load(const Slot* s) { return s->key; }
+    __device__ static Key claim(Slot* s, Key expect, Key k) { return atomicCAS(&s->key, expect, k); }
+    __device__ static void record(DevState* st, Key k) { st->err_pos = k; }
+};
+
+// A key with hi = 0 hashes as its narrow twin.  A free slot is claimed with one 128-bit compare-and-swap on (lo, hi).
+template <> struct KeyWidth<true> {
+    using Slot = WideSlot;
+    using Key = Key128;
+    __device__ static Key at(const unsigned long long* keys, const unsigned long long* keys_hi, unsigned long long i) {
+        return Key128{keys[i], keys_hi[i]};
+    }
+    __device__ static unsigned long long hash(Key k) { return hash64(k.lo ^ (k.hi * 0x9E3779B97F4A7C15ULL)); }
+    __device__ static Key ones() { return Key128{kEmpty, kEmpty}; }
+    __device__ static ulonglong4 free_slot() { return make_ulonglong4(kEmpty, 0ULL, ~0ULL, 0ULL); }  // lo, hi, first, count
+    __device__ static bool is_free(Key k) { return k.lo == kEmpty; }
+    __device__ static bool same(Key a, Key b) { return a.lo == b.lo && a.hi == b.hi; }
+    __device__ static Key load(const Slot* s) {
+        const ulonglong2 k = *reinterpret_cast<const ulonglong2*>(&s->lo);
+        return Key128{k.x, k.y};
+    }
+    __device__ static Key claim(Slot* s, Key expect, Key k) { return atomicCAS(reinterpret_cast<Key128*>(&s->lo), expect, k); }
+    __device__ static void record(DevState* st, Key k) { st->err_pos = k.lo, st->err_hi = k.hi; }
+};
+
+// The first error raised on the device wins; `pos` is a read ordinal or the key the error is about.
+template <bool Wide = false>
+__device__ __forceinline__ void raise_error(DevState* st, int code, typename KeyWidth<Wide>::Key pos) {
+    if (atomicCAS(&st->err_code, 0, code) == 0) KeyWidth<Wide>::record(st, pos);
 }
 
-// count += cnt, first = min(first, pos) for `key`, inserting it if new.  Linear probing.
-// Cold path (collisions, first insertions that lost a race): out of line, so that the many places that
-// may need it do not each carry a copy of the probing loop (the scan kernels' SASS has to stay near the
-// instruction cache size).
+// count += cnt, first = min(first, pos) for `key`, inserting it if new.  Linear probing.  One overload per key width,
+// two bodies: the narrow one has to stay out of line and the wide one inlined, and one template body compiles the
+// narrow probing loop differently.
+// Narrow: the cold path (collisions, first insertions that lost a race), out of line, so that the many places that
+// may need it do not each carry a copy of the probing loop (the scan kernels' SASS has to stay near the instruction
+// cache size).
 __device__ __noinline__ void table_add(Slot* __restrict__ tab, unsigned long long mask,
                                           unsigned long long key, unsigned long long cnt,
                                           unsigned long long pos, unsigned long long* occupied,
@@ -120,23 +167,17 @@ __device__ __noinline__ void table_add(Slot* __restrict__ tab, unsigned long lon
     raise_error(st, FRB_ERR_TABLE_FULL, key);
 }
 
-// Wide keys: the first error also records the key's upper word.
-__device__ __forceinline__ void raise_error_wide(DevState* st, int code, unsigned long long pos, unsigned long long hi) {
-    if (atomicCAS(&st->err_code, 0, code) == 0) st->err_pos = pos, st->err_hi = hi;
-}
-
-// table_add for a wide context, inlined (a call would spill in the scan kernels).  A key with hi = 0 hashes as its
-// narrow twin.  One 16-byte load per probe;
-// a free slot is claimed with one 128-bit compare-and-swap on (lo, hi).
-__device__ __forceinline__ void table_add_wide(WideSlot* __restrict__ tab, unsigned long long mask, unsigned long long lo,
-                                            unsigned long long hi, unsigned long long cnt, unsigned long long pos,
-                                            unsigned long long* occupied, DevState* st) {
-    unsigned long long h = hash64(lo ^ (hi * 0x9E3779B97F4A7C15ULL)) & mask;
+// Wide: inlined (a call would spill in the scan kernels).  One 16-byte load per probe.
+__device__ __forceinline__ void table_add(WideSlot* __restrict__ tab, unsigned long long mask, Key128 key,
+                                          unsigned long long cnt, unsigned long long pos, unsigned long long* occupied,
+                                          DevState* st) {
+    const unsigned long long lo = key.lo, hi = key.hi;
+    unsigned long long h = KeyWidth<true>::hash(key) & mask;
     for (uint32_t probe = 0; probe < kMaxProbe; ++probe) {
         unsigned long long klo, khi;
         asm volatile("ld.volatile.global.v2.u64 {%0, %1}, [%2];" : "=l"(klo), "=l"(khi) : "l"(&tab[h].lo));
         if (klo == kEmpty) {
-            const Key128 old = atomicCAS(reinterpret_cast<Key128*>(&tab[h].lo), Key128{kEmpty, 0ULL}, Key128{lo, hi});
+            const Key128 old = atomicCAS(reinterpret_cast<Key128*>(&tab[h].lo), Key128{kEmpty, 0ULL}, key);
             klo = old.lo, khi = old.hi;
             if (klo == kEmpty) {
                 atomicAdd(occupied, 1ULL);
@@ -150,7 +191,7 @@ __device__ __forceinline__ void table_add_wide(WideSlot* __restrict__ tab, unsig
         }
         h = (h + 1) & mask;
     }
-    raise_error_wide(st, FRB_ERR_TABLE_FULL, lo, hi);
+    raise_error<true>(st, FRB_ERR_TABLE_FULL, key);
 }
 #endif
 

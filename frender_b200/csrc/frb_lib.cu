@@ -271,10 +271,8 @@ int free_list(frb_ctx* c, KeyList& l) {
 
 int clear_table(frb_ctx* c, Slot* tab) {
     ProfScope ps(c, FRB_K_OTHER);
-    if (c->wide)
-        clear_wide_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(reinterpret_cast<WideSlot*>(tab), c->cap);
-    else
-        clear_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(tab, c->cap);
+    const auto clear = c->wide ? clear_table_kernel<true> : clear_table_kernel<false>;
+    clear<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(tab, c->cap);
     c->launches++;
     CU(c, cudaGetLastError());
     return FRB_OK;
@@ -347,30 +345,31 @@ int ensure_sorted(frb_ctx* c, KeyList& l) {
     return FRB_OK;
 }
 
-// Table -> list sorted by `first`.
-int table_to_sorted_list(frb_ctx* c, Slot* tab, uint64_t n, KeyList* out, int first_bits = 64,
-                         const unsigned long long* tile_first = nullptr) {
+// Occupied slots of a table -> fresh arrays of `room` entries in `out`, in slot order; their number lands in
+// st->scratch.  tile_first: see compact_table_kernel.
+int compact_table(frb_ctx* c, Slot* tab, uint64_t room, const unsigned long long* tile_first, KeyList* out) {
+    TRY(dmalloc(c, &out->keys, room * 8));
+    TRY(dmalloc(c, &out->counts, room * 8));
+    TRY(dmalloc(c, &out->first, room * 8));
+    if (c->wide) TRY(dmalloc(c, &out->keys_hi, room * 8));
+    ProfScope ps(c, FRB_K_EXPORT);
+    CU(c, cudaMemsetAsync(&c->st->scratch, 0, 8, c->compute));
+    const auto compact = c->wide ? compact_table_kernel<true> : compact_table_kernel<false>;
+    compact<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(
+        tab, c->cap, out->keys, out->counts, out->first, &c->st->scratch, room, tile_first, out->keys_hi);
+    c->launches++;
+    CU(c, cudaGetLastError());
+    return FRB_OK;
+}
+
+// Table with n occupied slots -> list sorted by `first`.
+int table_to_sorted_list(frb_ctx* c, Slot* tab, uint64_t n, KeyList* out) {
     out->n = n;
     if (n == 0) return FRB_OK;
     if (n >= (1ULL << 32)) return fail(c, FRB_ERR_ARG, "more than 2^32 unique keys");
-    unsigned long long *k0 = nullptr, *c0 = nullptr, *f0 = nullptr, *h0 = nullptr;
-    TRY(dmalloc(c, &k0, n * 8));
-    TRY(dmalloc(c, &c0, n * 8));
-    TRY(dmalloc(c, &f0, n * 8));
-    if (c->wide) TRY(dmalloc(c, &h0, n * 8));
-    {
-        ProfScope ps(c, FRB_K_EXPORT);
-        CU(c, cudaMemsetAsync(&c->st->scratch, 0, 8, c->compute));
-        if (c->wide)
-            compact_wide_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(
-                reinterpret_cast<const WideSlot*>(tab), c->cap, k0, h0, c0, f0, &c->st->scratch, n);
-        else
-            compact_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(
-                tab, c->cap, k0, c0, f0, &c->st->scratch, n, tile_first);
-        c->launches++;
-        CU(c, cudaGetLastError());
-    }
-    return unsorted_to_sorted_list(c, k0, c0, f0, n, out, first_bits, h0);
+    KeyList l;
+    TRY(compact_table(c, tab, n, nullptr, &l));
+    return unsorted_to_sorted_list(c, l.keys, l.counts, l.first, n, out, 64, l.keys_hi);
 }
 
 // The same when the number of occupied slots is not known: one pass over the table compacts and counts at once
@@ -379,23 +378,7 @@ int table_to_sorted_list_counting(frb_ctx* c, Slot* tab, uint64_t bound, KeyList
                                   const unsigned long long* tile_first) {
     bound = std::max<uint64_t>(std::min<uint64_t>(bound, c->cap), 1);
     if (bound >= (1ULL << 32)) return fail(c, FRB_ERR_ARG, "more than 2^32 unique keys");
-    unsigned long long *k0 = nullptr, *c0 = nullptr, *f0 = nullptr, *h0 = nullptr;
-    TRY(dmalloc(c, &k0, bound * 8));
-    TRY(dmalloc(c, &c0, bound * 8));
-    TRY(dmalloc(c, &f0, bound * 8));
-    if (c->wide) TRY(dmalloc(c, &h0, bound * 8));
-    {
-        ProfScope ps(c, FRB_K_EXPORT);
-        CU(c, cudaMemsetAsync(&c->st->scratch, 0, 8, c->compute));
-        if (c->wide)
-            compact_wide_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(
-                reinterpret_cast<const WideSlot*>(tab), c->cap, k0, h0, c0, f0, &c->st->scratch, bound);
-        else
-            compact_table_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(
-                tab, c->cap, k0, c0, f0, &c->st->scratch, bound, tile_first);
-        c->launches++;
-        CU(c, cudaGetLastError());
-    }
+    TRY(compact_table(c, tab, bound, tile_first, out));
     CU(c, cudaStreamSynchronize(c->compute));
     TRY(device_error_check(c));
     const uint64_t n = c->st_host->scratch;
@@ -403,7 +386,7 @@ int table_to_sorted_list_counting(frb_ctx* c, Slot* tab, uint64_t bound, KeyList
                                (unsigned long long)bound);
     // left in slot order: sorted by first appearance when somebody needs the order (ensure_sorted); a sharded
     // merge does not
-    out->keys = k0, out->counts = c0, out->first = f0, out->keys_hi = h0, out->n = n;
+    out->n = n;
     out->sorted = false;
     out->first_bits = first_bits;
     return FRB_OK;
@@ -476,10 +459,10 @@ int launch_scan(frb_ctx* c, const unsigned char* dev, uint64_t nbytes, uint64_t 
         // than 24 bytes on average) go to the redo kernel
         if (c->wide && rule != kRuleOffsetsOnly) {  // record offsets alone need no key of either width
             scan_ws_kernel<WsTileWide><<<grid, WsTileWide::threads, WsTileWide::smem, c->compute>>>(a);
-            scan_redo_wide_kernel<<<c->sm_count, 64, 0, c->compute>>>(a);
+            scan_redo_kernel<WsTileWide><<<c->sm_count, 64, 0, c->compute>>>(a);
         } else {
             scan_ws_kernel<WsTile><<<grid, WsTile::threads, WsTile::smem, c->compute>>>(a);
-            scan_redo_kernel<<<c->sm_count, 64, 0, c->compute>>>(a);
+            scan_redo_kernel<WsTile><<<c->sm_count, 64, 0, c->compute>>>(a);
         }
         c->launches += 2;
     } else {
@@ -531,7 +514,7 @@ int launch_scan(frb_ctx* c, const unsigned char* dev, uint64_t nbytes, uint64_t 
             scan_spec_kernel<WsTile><<<grid, WsTile::threads, WsTile::smem, c->compute>>>(neg);
             spec_reset_first_kernel<<<grid_for(c->cap, 256, c->sm_count, 16), 256, 0, c->compute>>>(
                 table, c->cap, c->file_tiles << kCompositeShift, c->st);
-            scan_redo_kernel<<<c->sm_count, 64, 0, c->compute>>>(a);
+            scan_redo_kernel<WsTile><<<c->sm_count, 64, 0, c->compute>>>(a);
         }
         c->file_tiles += n_tiles;
         c->launches += 7;
@@ -942,14 +925,10 @@ static int merge_pending_files(frb_ctx* c) {  // fold file lists into total_tab 
         const KeyList& fl = c->files[c->merged_upto];
         if (!fl.n) continue;
         ProfScope ps(c, FRB_K_EXPORT);
-        if (c->wide)
-            merge_wide_list_kernel<<<static_cast<unsigned>((fl.n + 255) / 256), 256, 0, c->compute>>>(
-                reinterpret_cast<WideSlot*>(c->total_tab), c->cap - 1, fl.keys, fl.keys_hi, fl.counts, fl.first, fl.n,
-                static_cast<unsigned long long>(fl.ordinal) << 40, &c->st->occupied_total, c->st);
-        else
-            merge_list_kernel<<<static_cast<unsigned>((fl.n + 255) / 256), 256, 0, c->compute>>>(
-                c->total_tab, c->cap - 1, fl.keys, fl.counts, fl.first, fl.n,
-                static_cast<unsigned long long>(fl.ordinal) << 40, &c->st->occupied_total, c->st);
+        const auto merge = c->wide ? merge_list_kernel<true> : merge_list_kernel<false>;
+        merge<<<static_cast<unsigned>((fl.n + 255) / 256), 256, 0, c->compute>>>(
+            c->total_tab, c->cap - 1, fl.keys, fl.counts, fl.first, fl.n, static_cast<unsigned long long>(fl.ordinal) << 40,
+            &c->st->occupied_total, c->st, fl.keys_hi);
         c->launches++;
         c->total_tab_clean = false;
         CU(c, cudaGetLastError());
@@ -1053,8 +1032,8 @@ int frb_total_merge(frb_ctx* c, const uint64_t* keys, const uint64_t* counts, co
         CU(c, cudaMemcpyAsync(df, first_pos, n * 8, cudaMemcpyHostToDevice, c->compute));
         {
             ProfScope ps(c, FRB_K_EXPORT);
-            merge_list_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(
-                c->total_tab, c->cap - 1, dk, dc, df, n, 0ULL, &c->st->occupied_total, c->st);
+            merge_list_kernel<false><<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(
+                c->total_tab, c->cap - 1, dk, dc, df, n, 0ULL, &c->st->occupied_total, c->st, nullptr);
             c->launches++;
         }
         CU(c, cudaGetLastError());
@@ -1699,7 +1678,7 @@ int frb_demux_ok(frb_ctx* c, const uint8_t* match, uint32_t n_files, const uint6
             c->launches += 2;
         }
         for (uint32_t f = 0; f < n_files; ++f) {
-            const unsigned long long *fk = nullptr, *fc = nullptr;
+            const unsigned long long *fk = nullptr, *fc = nullptr, *fk_hi = nullptr;
             unsigned long long *up_k = nullptr, *up_c = nullptr;
             uint64_t nf = 0;
             if (file_keys) {
@@ -1715,15 +1694,12 @@ int frb_demux_ok(frb_ctx* c, const uint8_t* match, uint32_t n_files, const uint6
             } else {
                 nf = c->files[f].n;
                 if (!nf) continue;
-                fk = c->files[f].keys, fc = c->files[f].counts;
+                fk = c->files[f].keys, fc = c->files[f].counts, fk_hi = c->files[f].keys_hi;
             }
-            if (c->wide)
-                demux_ok_wide_kernel<<<static_cast<unsigned>((nf + 255) / 256), 256, 0, c->compute>>>(
-                    fk, c->files[f].keys_hi, fc, nf, sorted_keys, sorted_hi, i1, n, c->type, c->srow, d_match, n_files, f,
-                    d_ok, d_bad, d_err);
-            else
-                demux_ok_kernel<<<static_cast<unsigned>((nf + 255) / 256), 256, 0, c->compute>>>(
-                    fk, fc, nf, sorted_keys, i1, n, c->type, c->srow, d_match, n_files, f, d_ok, d_bad, d_err);
+            const auto demux_ok = c->wide ? demux_ok_kernel<true> : demux_ok_kernel<false>;
+            demux_ok<<<static_cast<unsigned>((nf + 255) / 256), 256, 0, c->compute>>>(
+                fk, fc, nf, sorted_keys, i1, n, c->type, c->srow, d_match, n_files, f, d_ok, d_bad, d_err,
+                fk_hi, sorted_hi);
             c->launches++;
             if (up_k) TRY(dfree(c, up_k));
             if (up_c) TRY(dfree(c, up_c));

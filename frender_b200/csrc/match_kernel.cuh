@@ -48,6 +48,84 @@ __device__ __forceinline__ void classify_one(int first1, int first2, unsigned bo
     }
 }
 
+// ---- pieces every matcher kernel shares ---------------------------------------------------------------------------
+// Shape check: idx1 of l1 symbols in 1..5, then '+' and idx2 of l2 symbols in 1..5, then end or another '+' (extra
+// parts ignored, F:306); single index: l1 symbols then end.  sym(s) = symbol s of the key, max_syms its capacity.
+template <class Sym>
+__device__ __forceinline__ bool shape_ok(const MatchArgs& a, unsigned max_syms, Sym sym) {
+    bool ok = true;
+    const unsigned total = a.l2 ? a.l1 + 1 + a.l2 : a.l1;
+    for (unsigned s = 0; s < total; ++s) {
+        const unsigned c = sym(s);
+        if (a.l2 && s == a.l1) ok &= (c == 6);
+        else ok &= (c >= 1 && c <= 5);
+    }
+    if (total < max_syms) {
+        const unsigned nxt = sym(total);
+        ok &= a.l2 ? (nxt == 0 || nxt == 6) : (nxt == 0);
+    }
+    return ok;
+}
+
+// A key without an idx1 row is undetermined whatever its idx2 does (F:259, F:280-284).
+__device__ __forceinline__ void mark_undetermined(const MatchArgs& a, unsigned long long i) {
+    a.m2[i] = -1, a.srow[i] = -1, a.type[i] = FRB_TYPE_UNDETERMINED;
+    if (a.rc_mode) a.m2rc[i] = -1, a.srowrc[i] = -1, a.typerc[i] = FRB_TYPE_UNDETERMINED;
+}
+
+// Keys of the warp with an idx1 row -> work list, one atomic per warp.  Every lane of the warp calls this.
+__device__ __forceinline__ void append_work(const MatchArgs& a, int lane, unsigned long long i, int first1) {
+    const unsigned need = __ballot_sync(0xFFFFFFFFu, first1 >= 0);
+    if (need) {
+        unsigned long long base = 0;
+        const int leader = __ffs(need) - 1;
+        if (lane == leader) base = atomicAdd(a.work_n, static_cast<unsigned long long>(__popc(need)));
+        base = __shfl_sync(0xFFFFFFFFu, base, leader);
+        if (first1 >= 0) a.work[base + __popc(need & ((1u << lane) - 1u))] = static_cast<unsigned>(i);
+    }
+}
+
+// Kernel 2's verdict on key i from the rows its sweep found: first idx2 row, rows matching both and the first of
+// them (-1: none), as supplied / oriented (f) and reverse-complemented (r, rc_mode only).  rc_mode also adds the
+// key's reads to the per-group sums in shared memory (s_f, s_r; s_g = group of every row).
+__device__ __forceinline__ void classify_store(const MatchArgs& a, unsigned long long i, int first1, int firstf,
+                                               unsigned nf, int rowf, int firstr, unsigned nr, int rowr,
+                                               unsigned long long* s_f, unsigned long long* s_r, const int* s_g) {
+    int m1, m2, type, srow;
+    classify_one(first1, firstf, nf, rowf, &m1, &m2, &type, &srow);
+    if (a.rc_mode) {
+        int m1r, m2r, typer, srowr;
+        classify_one(first1, firstr, nr, rowr, &m1r, &m2r, &typer, &srowr);
+        if (m1 < 0) m1 = m1r;  // F:319-323
+        if (type == FRB_TYPE_DEMUXABLE && typer == FRB_TYPE_DEMUXABLE && s_g[srow] != s_g[srowr]) {
+            type = typer = FRB_TYPE_AMBIGUOUS;  // F:336-349
+            srow = srowr = -1;
+        }
+        const unsigned long long c = a.counts[i];
+        if (srow >= 0) atomicAdd(&s_f[s_g[srow]], c);      // F:370-371
+        if (srowr >= 0) atomicAdd(&s_r[s_g[srowr]], c);    // F:372-373
+        a.m2rc[i] = m2r;
+        a.typerc[i] = static_cast<unsigned char>(typer);
+        a.srowrc[i] = srowr;
+    }
+    a.m1[i] = m1;
+    a.m2[i] = m2;
+    a.type[i] = static_cast<unsigned char>(type);
+    a.srow[i] = srow;
+}
+
+// The block's per-group sums -> f_sum / rc_sum (rc_mode only).  Every thread of the block calls this.
+__device__ __forceinline__ void flush_group_sums(const MatchArgs& a, const unsigned long long* s_f,
+                                                 const unsigned long long* s_r) {
+    if (a.rc_mode) {
+        __syncthreads();
+        for (unsigned g = threadIdx.x; g < a.rows; g += blockDim.x) {
+            if (s_f[g]) atomicAdd(&a.f_sum[g], s_f[g]);
+            if (s_r[g]) atomicAdd(&a.rc_sum[g], s_r[g]);
+        }
+    }
+}
+
 // ---- kernel 1: idx1 sweep over ALL unique keys, fully convergent --------------------------------
 // A key whose idx1 matches no row is undetermined whatever its idx2 does (F:259, F:280-284) -- the fate
 // of almost every unique key of a real lane (random index pairs dominate the unique set).  Those keys
@@ -68,22 +146,8 @@ __global__ void __launch_bounds__(kMatchThreads) match_idx1_kernel(const MatchAr
         int first1 = -1;
         if (i < a.n) {
             const unsigned long long key = a.keys[i];
-            // shape check: idx1 of l1 symbols in 1..5, then '+' and idx2 of l2 symbols in 1..5, then end
-            // or another '+' (extra parts ignored, F:306); single index: l1 symbols then end.
-            if (a.rows) {
-                bool ok = true;
-                const unsigned total = a.l2 ? a.l1 + 1 + a.l2 : a.l1;
-                for (unsigned s = 0; s < total; ++s) {
-                    const unsigned sym = static_cast<unsigned>(key >> (3 * s)) & 7u;
-                    if (a.l2 && s == a.l1) ok &= (sym == 6);
-                    else ok &= (sym >= 1 && sym <= 5);
-                }
-                if (total < kMaxSyms) {
-                    const unsigned nxt = static_cast<unsigned>(key >> (3 * total)) & 7u;
-                    ok &= a.l2 ? (nxt == 0 || nxt == 6) : (nxt == 0);
-                }
-                if (!ok) raise_error(a.st, FRB_ERR_BAD_LENGTH, key);
-            }
+            if (a.rows && !shape_ok(a, kMaxSyms, [&](unsigned s) { return static_cast<unsigned>(key >> (3 * s)) & 7u; }))
+                raise_error(a.st, FRB_ERR_BAD_LENGTH, key);
             if (a.l1 <= 10) {  // idx1 fits 30 bits: 32-bit compare, one LOP3 folds the three bit planes
                 const unsigned m = (1u << (3 * a.l1)) - 1u;
                 const unsigned k1 = static_cast<unsigned>(key) & m, b1 = static_cast<unsigned>(B1);
@@ -99,19 +163,9 @@ __global__ void __launch_bounds__(kMatchThreads) match_idx1_kernel(const MatchAr
                 }
             }
             a.m1[i] = first1;
-            if (first1 < 0) {
-                a.m2[i] = -1, a.srow[i] = -1, a.type[i] = FRB_TYPE_UNDETERMINED;
-                if (a.rc_mode) a.m2rc[i] = -1, a.srowrc[i] = -1, a.typerc[i] = FRB_TYPE_UNDETERMINED;
-            }
+            if (first1 < 0) mark_undetermined(a, i);
         }
-        const unsigned need = __ballot_sync(0xFFFFFFFFu, first1 >= 0);
-        if (need) {
-            unsigned long long base = 0;
-            const int leader = __ffs(need) - 1;
-            if (lane == leader) base = atomicAdd(a.work_n, static_cast<unsigned long long>(__popc(need)));
-            base = __shfl_sync(0xFFFFFFFFu, base, leader);
-            if (first1 >= 0) a.work[base + __popc(need & ((1u << lane) - 1u))] = static_cast<unsigned>(i);
-        }
+        append_work(a, lane, i, first1);
     }
 }
 
@@ -171,35 +225,9 @@ __global__ void __launch_bounds__(kMatchThreads) match_kernel(const MatchArgs a)
                 }
             }
         }
-        int m1, m2, type, srow;
-        classify_one(first1, firstf, nf, rowf, &m1, &m2, &type, &srow);
-        if (a.rc_mode) {
-            int m1r, m2r, typer, srowr;
-            classify_one(first1, firstr, nr, rowr, &m1r, &m2r, &typer, &srowr);
-            if (m1 < 0) m1 = m1r;  // F:319-323
-            if (type == FRB_TYPE_DEMUXABLE && typer == FRB_TYPE_DEMUXABLE && s_g[srow] != s_g[srowr]) {
-                type = typer = FRB_TYPE_AMBIGUOUS;  // F:336-349
-                srow = srowr = -1;
-            }
-            const unsigned long long c = a.counts[i];
-            if (srow >= 0) atomicAdd(&s_f[s_g[srow]], c);      // F:370-371
-            if (srowr >= 0) atomicAdd(&s_r[s_g[srowr]], c);    // F:372-373
-            a.m2rc[i] = m2r;
-            a.typerc[i] = static_cast<unsigned char>(typer);
-            a.srowrc[i] = srowr;
-        }
-        a.m1[i] = m1;
-        a.m2[i] = m2;
-        a.type[i] = static_cast<unsigned char>(type);
-        a.srow[i] = srow;
+        classify_store(a, i, first1, firstf, nf, rowf, firstr, nr, rowr, s_f, s_r, s_g);
     }
-    if (a.rc_mode) {
-        __syncthreads();
-        for (unsigned g = threadIdx.x; g < a.rows; g += blockDim.x) {
-            if (s_f[g]) atomicAdd(&a.f_sum[g], s_f[g]);
-            if (s_r[g]) atomicAdd(&a.rc_sum[g], s_r[g]);
-        }
-    }
+    flush_group_sums(a, s_f, s_r);
 }
 
 // =================================================================================================
@@ -322,20 +350,8 @@ __global__ void __launch_bounds__(kMatchThreads) match_idx1_cand_kernel(const Ma
         int first1 = -1;
         if (i < a.n) {
             const unsigned long long key = a.keys[i];
-            {   // shape check, as in the sweep kernel (F:306 / F:227)
-                bool ok = true;
-                const unsigned total = a.l2 ? a.l1 + 1 + a.l2 : a.l1;
-                for (unsigned s = 0; s < total; ++s) {
-                    const unsigned sym = static_cast<unsigned>(key >> (3 * s)) & 7u;
-                    if (a.l2 && s == a.l1) ok &= (sym == 6);
-                    else ok &= (sym >= 1 && sym <= 5);
-                }
-                if (total < kMaxSyms) {
-                    const unsigned nxt = static_cast<unsigned>(key >> (3 * total)) & 7u;
-                    ok &= a.l2 ? (nxt == 0 || nxt == 6) : (nxt == 0);
-                }
-                if (!ok) raise_error(a.st, FRB_ERR_BAD_LENGTH, key);
-            }
+            if (!shape_ok(a, kMaxSyms, [&](unsigned s) { return static_cast<unsigned>(key >> (3 * s)) & 7u; }))
+                raise_error(a.st, FRB_ERR_BAD_LENGTH, key);
             const unsigned k1 = static_cast<unsigned>(key) & m1mask;
             unsigned best = kNil;
             cand_visit(T, k1, [&](unsigned r) {
@@ -343,19 +359,9 @@ __global__ void __launch_bounds__(kMatchThreads) match_idx1_cand_kernel(const Ma
             });
             first1 = best == kNil ? -1 : static_cast<int>(best);
             a.m1[i] = first1;
-            if (first1 < 0) {
-                a.m2[i] = -1, a.srow[i] = -1, a.type[i] = FRB_TYPE_UNDETERMINED;
-                if (a.rc_mode) a.m2rc[i] = -1, a.srowrc[i] = -1, a.typerc[i] = FRB_TYPE_UNDETERMINED;
-            }
+            if (first1 < 0) mark_undetermined(a, i);
         }
-        const unsigned need = __ballot_sync(0xFFFFFFFFu, first1 >= 0);
-        if (need) {
-            unsigned long long base = 0;
-            const int leader = __ffs(need) - 1;
-            if (lane == leader) base = atomicAdd(a.work_n, static_cast<unsigned long long>(__popc(need)));
-            base = __shfl_sync(0xFFFFFFFFu, base, leader);
-            if (first1 >= 0) a.work[base + __popc(need & ((1u << lane) - 1u))] = static_cast<unsigned>(i);
-        }
+        append_work(a, lane, i, first1);
     }
 }
 
@@ -421,6 +427,7 @@ __global__ void __launch_bounds__(kMatchThreads) match_cand_kernel(const MatchAr
                 });
             }
         }
+        // classify_store written out: called here, it changes how the compiler schedules this kernel's epilogue
         int m1, m2, type, srow;
         classify_one(first1, static_cast<int>(firstf), nf, static_cast<int>(rowf), &m1, &m2, &type, &srow);
         if (a.rc_mode) {
@@ -443,13 +450,7 @@ __global__ void __launch_bounds__(kMatchThreads) match_cand_kernel(const MatchAr
         a.type[i] = static_cast<unsigned char>(type);
         a.srow[i] = srow;
     }
-    if (a.rc_mode) {
-        __syncthreads();
-        for (unsigned g = threadIdx.x; g < a.rows; g += blockDim.x) {
-            if (s_f[g]) atomicAdd(&a.f_sum[g], s_f[g]);
-            if (s_r[g]) atomicAdd(&a.rc_sum[g], s_r[g]);
-        }
-    }
+    flush_group_sums(a, s_f, s_r);
 }
 
 }  // namespace frb
@@ -491,39 +492,18 @@ __global__ void __launch_bounds__(kMatchThreads) match_idx1_wide_kernel(const Wi
         int first1 = -1;
         if (i < a.n) {
             const unsigned long long lo = a.keys[i], hi = w.keys_hi[i];
-            if (a.rows) {  // as in match_idx1_kernel: l1 symbols, '+', l2 symbols, then end or '+'
-                bool ok = true;
-                const unsigned total = a.l2 ? a.l1 + 1 + a.l2 : a.l1;
-                for (unsigned s = 0; s < total; ++s) {
-                    const unsigned sym = static_cast<unsigned>(wide_field(lo, hi, s, 1));
-                    if (a.l2 && s == a.l1) ok &= (sym == 6);
-                    else ok &= (sym >= 1 && sym <= 5);
-                }
-                if (total < kMaxWideSyms) {
-                    const unsigned nxt = static_cast<unsigned>(wide_field(lo, hi, total, 1));
-                    ok &= a.l2 ? (nxt == 0 || nxt == 6) : (nxt == 0);
-                }
-                if (!ok) raise_error_wide(a.st, FRB_ERR_BAD_LENGTH, lo, hi);
-            }
+            if (a.rows &&
+                !shape_ok(a, kMaxWideSyms, [&](unsigned s) { return static_cast<unsigned>(wide_field(lo, hi, s, 1)); }))
+                raise_error<true>(a.st, FRB_ERR_BAD_LENGTH, Key128{lo, hi});
             const unsigned long long k1 = wide_field(lo, hi, 0, a.l1);
             for (unsigned r = 0; r < a.rows; ++r) {
                 const bool h1 = static_cast<unsigned>(__popcll(fold3(k1 ^ s_1[r]) & B1)) <= n_subs;
                 if (h1 && first1 < 0) first1 = r;
             }
             a.m1[i] = first1;
-            if (first1 < 0) {
-                a.m2[i] = -1, a.srow[i] = -1, a.type[i] = FRB_TYPE_UNDETERMINED;
-                if (a.rc_mode) a.m2rc[i] = -1, a.srowrc[i] = -1, a.typerc[i] = FRB_TYPE_UNDETERMINED;
-            }
+            if (first1 < 0) mark_undetermined(a, i);
         }
-        const unsigned need = __ballot_sync(0xFFFFFFFFu, first1 >= 0);
-        if (need) {
-            unsigned long long base = 0;
-            const int leader = __ffs(need) - 1;
-            if (lane == leader) base = atomicAdd(a.work_n, static_cast<unsigned long long>(__popc(need)));
-            base = __shfl_sync(0xFFFFFFFFu, base, leader);
-            if (first1 >= 0) a.work[base + __popc(need & ((1u << lane) - 1u))] = static_cast<unsigned>(i);
-        }
+        append_work(a, lane, i, first1);
     }
 }
 
@@ -579,35 +559,9 @@ __global__ void __launch_bounds__(kMatchThreads) match_wide_kernel(const WideMat
                 }
             }
         }
-        int m1, m2, type, srow;
-        classify_one(first1, firstf, nf, rowf, &m1, &m2, &type, &srow);
-        if (a.rc_mode) {
-            int m1r, m2r, typer, srowr;
-            classify_one(first1, firstr, nr, rowr, &m1r, &m2r, &typer, &srowr);
-            if (m1 < 0) m1 = m1r;  // F:319-323
-            if (type == FRB_TYPE_DEMUXABLE && typer == FRB_TYPE_DEMUXABLE && s_g[srow] != s_g[srowr]) {
-                type = typer = FRB_TYPE_AMBIGUOUS;  // F:336-349
-                srow = srowr = -1;
-            }
-            const unsigned long long c = a.counts[i];
-            if (srow >= 0) atomicAdd(&s_f[s_g[srow]], c);      // F:370-371
-            if (srowr >= 0) atomicAdd(&s_r[s_g[srowr]], c);    // F:372-373
-            a.m2rc[i] = m2r;
-            a.typerc[i] = static_cast<unsigned char>(typer);
-            a.srowrc[i] = srowr;
-        }
-        a.m1[i] = m1;
-        a.m2[i] = m2;
-        a.type[i] = static_cast<unsigned char>(type);
-        a.srow[i] = srow;
+        classify_store(a, i, first1, firstf, nf, rowf, firstr, nr, rowr, s_f, s_r, s_g);
     }
-    if (a.rc_mode) {
-        __syncthreads();
-        for (unsigned g = threadIdx.x; g < a.rows; g += blockDim.x) {
-            if (s_f[g]) atomicAdd(&a.f_sum[g], s_f[g]);
-            if (s_r[g]) atomicAdd(&a.rc_sum[g], s_r[g]);
-        }
-    }
+    flush_group_sums(a, s_f, s_r);
 }
 
 }  // namespace frb

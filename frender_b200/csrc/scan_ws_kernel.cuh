@@ -398,8 +398,8 @@ __global__ void __launch_bounds__(G::threads) __maxnreg__(G::maxreg) scan_ws_ker
 #pragma unroll
                     for (int r = 0; r < kRounds; ++r) {
                         if (key[r] != kEmpty) {
-                            table_add_wide(reinterpret_cast<WideSlot*>(a.table), a.table_mask, key[r], key_hi[r], cnt[r],
-                                           a.pos_base + of + h0 + r * 32 + lane, &a.st->occupied, a.st);
+                            table_add(reinterpret_cast<WideSlot*>(a.table), a.table_mask, Key128{key[r], key_hi[r]}, cnt[r],
+                                      a.pos_base + of + h0 + r * 32 + lane, &a.st->occupied, a.st);
                         }
                     }
                 } else if (a.table) {
@@ -433,16 +433,22 @@ __global__ void __launch_bounds__(G::threads) __maxnreg__(G::maxreg) scan_ws_ker
 // Tiles the warp-specialised kernel left out -- a guessed line phase that turned out wrong (input that is
 // not well-formed FASTQ), or more newlines than a tile's position list holds -- tallied strictly by line
 // count, one thread per tile, from the bytes in global memory.  status[] holds every tile's inclusive
-// newline prefix by now.  Slow and exact; the list is empty for ordinary input.
+// newline prefix by now.  Slow and exact; the list is empty for ordinary input.  A wide context (G::wide) never
+// runs the speculative scan; its keys_out holds out_cap lower words, then out_cap upper words.
+template <class G>
 __global__ void __launch_bounds__(64) scan_redo_kernel(const ScanArgs a_in) {
+    using K = KeyWidth<G::wide>;
     ScanArgs a = a_in;
     a.skip = a.skip_ptr ? *a.skip_ptr : 0ULL;
     // speculative path: a wrong guess somewhere in the chunk -> every tile is redone (the negate pass took the
     // guessed keys out again); a parse error of a guessed tile stands once all guesses are confirmed
-    const bool all = a.composite && a.st->spec_bad;
-    if (a.composite && !all && blockIdx.x == 0 && threadIdx.x == 0 && a.st->spec_err_code) {
-        const unsigned long long p = a.st->spec_err_pos;
-        raise_error(a.st, a.st->spec_err_code, a.tile_first[p >> kCompositeShift] + (p & ((1ULL << kCompositeShift) - 1)));
+    bool all = false;
+    if constexpr (!G::wide) {
+        all = a.composite && a.st->spec_bad;
+        if (a.composite && !all && blockIdx.x == 0 && threadIdx.x == 0 && a.st->spec_err_code) {
+            const unsigned long long p = a.st->spec_err_pos;
+            raise_error(a.st, a.st->spec_err_code, a.tile_first[p >> kCompositeShift] + (p & ((1ULL << kCompositeShift) - 1)));
+        }
     }
     const unsigned long long n = all ? a.n_tiles : a.st->redo_n;
     const unsigned long long L0 = a.st->chunk_l0;
@@ -461,24 +467,32 @@ __global__ void __launch_bounds__(64) scan_redo_kernel(const ScanArgs a_in) {
             const bool is_end = p < end ? a.data[p] == '\n' : vnl;
             if (!is_end) continue;
             if ((k & 3) == 0 && (k >> 2) < a.read_limit) {
-                unsigned long long key = 0;
-                const int rc = a.rule == kRuleOffsetsOnly ? 0 : parse_serial(a.data + prev, p - prev, a.rule, &key);
+                typename K::Key key{};
+                int rc;
+                if constexpr (G::wide) rc = parse_serial_wide(a.data + prev, p - prev, a.rule, &key.lo, &key.hi);
+                else rc = a.rule == kRuleOffsetsOnly ? 0 : parse_serial(a.data + prev, p - prev, a.rule, &key);
                 const unsigned long long pos =
-                    a.composite ? (((a.tile_base + t) << kCompositeShift) | reads) : a.pos_base + (k >> 2);
+                    !G::wide && a.composite ? (((a.tile_base + t) << kCompositeShift) | reads) : a.pos_base + (k >> 2);
                 ++reads;
+                // per-read key: the lower word, and for a wide context the upper word out_cap entries further on
+                auto emit = [&](unsigned long long slot, typename K::Key out) {
+                    if constexpr (G::wide) a.keys_out[slot] = out.lo, a.keys_out[a.out_cap + slot] = out.hi;
+                    else a.keys_out[slot] = out;
+                };
                 if (rc && a.rule == FRB_RULE_DEMUX && a.keys_out && !a.table) {
                     const unsigned long long slot = (k >> 2) - chunk_first_read;
                     if (slot < a.out_cap) {
-                        if (a.keys_out) a.keys_out[slot] = kBadKeyBase + static_cast<unsigned long long>(-rc);
+                        if (a.keys_out) emit(slot, typename K::Key{kBadKeyBase + static_cast<unsigned long long>(-rc)});
                         if (a.rec_off_out) a.rec_off_out[slot] = prev;
                     }
                 } else if (rc) {
                     raise_error(a.st, rc, k >> 2);
                 } else {
-                    if (a.table) table_add(a.table, a.table_mask, key, 1, pos, &a.st->occupied, a.st);
+                    if (a.table)
+                        table_add(reinterpret_cast<typename K::Slot*>(a.table), a.table_mask, key, 1, pos, &a.st->occupied, a.st);
                     const unsigned long long slot = (k >> 2) - chunk_first_read;
                     if (slot < a.out_cap) {
-                        if (a.keys_out) a.keys_out[slot] = key;
+                        if (a.keys_out) emit(slot, key);
                         if (a.rec_off_out) a.rec_off_out[slot] = prev;
                     }
                 }
@@ -486,53 +500,10 @@ __global__ void __launch_bounds__(64) scan_redo_kernel(const ScanArgs a_in) {
             prev = p + 1;
             ++k;
         }
-        if (!a.composite) {  // the speculative path takes both from the summed counts (spec_scan_kernel)
+        if (G::wide || !a.composite) {  // the speculative path takes both from the summed counts (spec_scan_kernel)
             if (reads) atomicAdd(&a.st->n_reads, reads);
             if (t == a.n_tiles - 1) a.st->line_carry = k;
         }
-    }
-}
-
-// scan_redo_kernel for a wide context (which never runs the speculative scan).  keys_out: out_cap lower words,
-// then out_cap upper words.
-__global__ void __launch_bounds__(64) scan_redo_wide_kernel(const ScanArgs a_in) {
-    ScanArgs a = a_in;
-    a.skip = a.skip_ptr ? *a.skip_ptr : 0ULL;
-    const unsigned long long n = a.st->redo_n;
-    const unsigned long long L0 = a.st->chunk_l0;
-    const unsigned long long chunk_first_read = (L0 + 3) >> 2;
-    for (unsigned long long idx = blockIdx.x * blockDim.x + threadIdx.x; idx < n;
-         idx += static_cast<unsigned long long>(gridDim.x) * blockDim.x) {
-        const unsigned t = a.redo[idx];
-        const unsigned long long off = static_cast<unsigned long long>(t) * a.tile_bytes;
-        const unsigned long long end = off + a.tile_bytes < a.nbytes ? off + a.tile_bytes : a.nbytes;
-        unsigned long long k = L0 + (t ? (a.status[t] & kValMask) : 0ULL);
-        unsigned long long prev = off > a.skip ? off : a.skip;
-        while (prev > a.skip && a.data[prev - 1] != '\n') --prev;
-        const bool vnl = t == a.n_tiles - 1 && end > off && end > a.skip && a.data[end - 1] != '\n';
-        unsigned long long reads = 0;
-        for (unsigned long long p = off > a.skip ? off : a.skip; p <= end; ++p) {
-            const bool is_end = p < end ? a.data[p] == '\n' : vnl;
-            if (!is_end) continue;
-            if ((k & 3) == 0 && (k >> 2) < a.read_limit) {
-                unsigned long long lo = 0, hi = 0;
-                const int rc = parse_serial_wide(a.data + prev, p - prev, a.rule, &lo, &hi);
-                ++reads;
-                const bool routed = a.rule == FRB_RULE_DEMUX && a.keys_out && !a.table;
-                if (rc && routed) lo = kBadKeyBase + static_cast<unsigned long long>(-rc), hi = 0;  // the router decides
-                else if (rc) raise_error(a.st, rc, k >> 2);
-                else if (a.table) table_add_wide(reinterpret_cast<WideSlot*>(a.table), a.table_mask, lo, hi, 1, a.pos_base + (k >> 2), &a.st->occupied, a.st);
-                const unsigned long long slot = (k >> 2) - chunk_first_read;
-                if ((!rc || routed) && slot < a.out_cap) {
-                    if (a.keys_out) a.keys_out[slot] = lo, a.keys_out[a.out_cap + slot] = hi;
-                    if (a.rec_off_out) a.rec_off_out[slot] = prev;
-                }
-            }
-            prev = p + 1;
-            ++k;
-        }
-        if (reads) atomicAdd(&a.st->n_reads, reads);
-        if (t == a.n_tiles - 1) a.st->line_carry = k;
     }
 }
 

@@ -5,25 +5,30 @@
 
 namespace frb {
 
+template <bool Wide>
 __global__ void __launch_bounds__(256) clear_table_kernel(Slot* tab, unsigned long long cap) {
     const unsigned long long stride = static_cast<unsigned long long>(gridDim.x) * blockDim.x;
     ulonglong4* t4 = reinterpret_cast<ulonglong4*>(tab);
     for (unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x; i < cap;
          i += stride)
-        t4[i] = make_ulonglong4(kEmpty, ~0ULL, 0ULL, 0ULL);  // key, first, count, aux
+        t4[i] = KeyWidth<Wide>::free_slot();
 }
 
 // Occupied slots (key present, count not taken back to 0 by a negate pass) -> dense arrays in arbitrary order;
 // *counter receives their number (the scan kernel does not keep it: knowing who won a slot would mean waiting for
 // every compare-and-swap's result).  One atomic per
 // block and pass (a per-warp atomic on the one counter was the kernel's bound: 2 M atomics for 2^26 slots).
+// tile_first (narrow only, may be null): turns composite positions into read ordinals; a wide context never runs the
+// speculative scan.  keys_hi (wide only): the upper key words.
+template <bool Wide>
 __global__ void __launch_bounds__(256) compact_table_kernel(const Slot* __restrict__ tab, unsigned long long cap,
                                                             unsigned long long* __restrict__ keys,
                                                             unsigned long long* __restrict__ counts,
                                                             unsigned long long* __restrict__ first,
                                                             unsigned long long* counter,
                                                             unsigned long long out_cap,
-                                                            const unsigned long long* __restrict__ tile_first = nullptr) {
+                                                            const unsigned long long* __restrict__ tile_first,
+                                                            unsigned long long* __restrict__ keys_hi) {
     __shared__ unsigned s_warp[8];
     __shared__ unsigned long long s_base;
     const unsigned long long stride = static_cast<unsigned long long>(gridDim.x) * blockDim.x;
@@ -33,7 +38,7 @@ __global__ void __launch_bounds__(256) compact_table_kernel(const Slot* __restri
          i < cap_up; i += stride) {
         ulonglong4 s = make_ulonglong4(kEmpty, 0, 0, 0);
         if (i < cap) s = reinterpret_cast<const ulonglong4*>(tab)[i];
-        const bool occ = s.x != kEmpty && s.z != 0;
+        const bool occ = s.x != kEmpty && (Wide ? s.w : s.z) != 0;  // key present, count
         const unsigned m = __ballot_sync(0xFFFFFFFFu, occ);
         if (lane == 0) s_warp[warp] = __popc(m);
         __syncthreads();
@@ -49,10 +54,14 @@ __global__ void __launch_bounds__(256) compact_table_kernel(const Slot* __restri
         if (occ) {
             const unsigned long long idx = s_base + before + __popc(m & ((1u << lane) - 1u));
             if (idx < out_cap) {
-                keys[idx] = s.x;
-                counts[idx] = s.z;
-                // composite position (tile << 13 | header index) -> read ordinal
-                first[idx] = tile_first ? tile_first[s.y >> kCompositeShift] + (s.y & ((1ULL << kCompositeShift) - 1)) : s.y;
+                if constexpr (Wide) {
+                    keys[idx] = s.x, keys_hi[idx] = s.y, counts[idx] = s.w, first[idx] = s.z;
+                } else {
+                    keys[idx] = s.x;
+                    counts[idx] = s.z;
+                    // composite position (tile << 13 | header index) -> read ordinal
+                    first[idx] = tile_first ? tile_first[s.y >> kCompositeShift] + (s.y & ((1ULL << kCompositeShift) - 1)) : s.y;
+                }
             }
         }
     }
@@ -83,15 +92,19 @@ __global__ void __launch_bounds__(256) add_offset_kernel(const unsigned long lon
     if (i < n) out[i] = in[i] + off;
 }
 
-// dst[key] += counts, first = min(first, pos_base + first_in)
+// dst[key] += counts, first = min(first, pos_base + first_in).  keys_hi: upper key words (wide only).
+template <bool Wide>
 __global__ void __launch_bounds__(256) merge_list_kernel(Slot* dst, unsigned long long mask,
                                                          const unsigned long long* __restrict__ keys,
                                                          const unsigned long long* __restrict__ counts,
                                                          const unsigned long long* __restrict__ first,
                                                          unsigned long long n, unsigned long long pos_base,
-                                                         unsigned long long* occupied, DevState* st) {
+                                                         unsigned long long* occupied, DevState* st,
+                                                         const unsigned long long* __restrict__ keys_hi) {
     const unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x;
-    if (i < n) table_add(dst, mask, keys[i], counts[i], first ? pos_base + first[i] : pos_base + i, occupied, st);
+    if (i < n)
+        table_add(reinterpret_cast<typename KeyWidth<Wide>::Slot*>(dst), mask, KeyWidth<Wide>::at(keys, keys_hi, i), counts[i],
+                  first ? pos_base + first[i] : pos_base + i, occupied, st);
 }
 
 // Entries sorted by key (ks) with their original positions (perm): every run of equal keys becomes one entry
@@ -227,6 +240,8 @@ __global__ void __launch_bounds__(256) gather3_kernel(const unsigned* __restrict
 // One thread per entry of one file's list: find the key in the total list (binary search in the key-sorted view),
 // take its class -- read type 0/1/3, or 4 + sample row for a demuxable key -- and look up class x file in the
 // match matrix the host made with the reference's regexes (0 no, 1 yes, 2 the regex does not compile).
+// Wide keys: fkeys_hi / sorted_hi hold the upper words, and the total is sorted by (hi, lo).
+template <bool Wide>
 __global__ void __launch_bounds__(256) demux_ok_kernel(const unsigned long long* __restrict__ fkeys,
                                                        const unsigned long long* __restrict__ fcounts, unsigned long long nf,
                                                        const unsigned long long* __restrict__ sorted_keys,
@@ -234,17 +249,29 @@ __global__ void __launch_bounds__(256) demux_ok_kernel(const unsigned long long*
                                                        const unsigned char* __restrict__ type, const int* __restrict__ srow,
                                                        const unsigned char* __restrict__ match, unsigned n_files, unsigned f,
                                                        unsigned char* __restrict__ ok, unsigned char* __restrict__ bad_file,
-                                                       int* err_row) {
+                                                       int* err_row, const unsigned long long* __restrict__ fkeys_hi,
+                                                       const unsigned long long* __restrict__ sorted_hi) {
     const unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x;
     if (i >= nf || (fcounts && fcounts[i] == 0)) return;
-    const unsigned long long key = fkeys[i];
+    const auto key = KeyWidth<Wide>::at(fkeys, fkeys_hi, i);
     unsigned long long lo = 0, hi = n;
     while (lo < hi) {
         const unsigned long long mid = (lo + hi) >> 1;
-        if (sorted_keys[mid] < key) lo = mid + 1;
-        else hi = mid;
+        if constexpr (Wide) {
+            const unsigned long long mh = sorted_hi[mid];
+            if (mh < key.hi || (mh == key.hi && sorted_keys[mid] < key.lo)) lo = mid + 1;
+            else hi = mid;
+        } else {
+            if (sorted_keys[mid] < key) lo = mid + 1;
+            else hi = mid;
+        }
     }
-    if (lo >= n || sorted_keys[lo] != key) return;  // not part of the total: nothing to flag
+    if (lo >= n) return;  // not part of the total: nothing to flag
+    if constexpr (Wide) {
+        if (sorted_keys[lo] != key.lo || sorted_hi[lo] != key.hi) return;
+    } else {
+        if (sorted_keys[lo] != key) return;
+    }
     const unsigned idx = sorted_idx[lo];
     const unsigned t = type[idx];
     const unsigned cls = t == 2 ? 4u + static_cast<unsigned>(srow[idx]) : t;
@@ -254,51 +281,6 @@ __global__ void __launch_bounds__(256) demux_ok_kernel(const unsigned long long*
     } else if (m == 0) {
         ok[idx] = 0;
         bad_file[f] = 1;
-    }
-}
-
-// ---- wide context (WideSlot tables, keys as lo / hi arrays) ---------------------------------------------------
-__global__ void __launch_bounds__(256) clear_wide_table_kernel(WideSlot* tab, unsigned long long cap) {
-    const unsigned long long stride = static_cast<unsigned long long>(gridDim.x) * blockDim.x;
-    ulonglong4* t4 = reinterpret_cast<ulonglong4*>(tab);
-    for (unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x; i < cap;
-         i += stride)
-        t4[i] = make_ulonglong4(kEmpty, 0ULL, ~0ULL, 0ULL);  // lo, hi, first, count
-}
-
-// compact_table_kernel for WideSlot tables (no composite positions: a wide context never runs the speculative scan)
-__global__ void __launch_bounds__(256) compact_wide_table_kernel(const WideSlot* __restrict__ tab, unsigned long long cap,
-                                                                 unsigned long long* __restrict__ keys,
-                                                                 unsigned long long* __restrict__ keys_hi,
-                                                                 unsigned long long* __restrict__ counts,
-                                                                 unsigned long long* __restrict__ first,
-                                                                 unsigned long long* counter, unsigned long long out_cap) {
-    __shared__ unsigned s_warp[8];
-    __shared__ unsigned long long s_base;
-    const unsigned long long stride = static_cast<unsigned long long>(gridDim.x) * blockDim.x;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const unsigned long long cap_up = (cap + 255) & ~255ULL;
-    for (unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x;
-         i < cap_up; i += stride) {
-        ulonglong4 s = make_ulonglong4(kEmpty, 0, 0, 0);
-        if (i < cap) s = reinterpret_cast<const ulonglong4*>(tab)[i];
-        const bool occ = s.x != kEmpty && s.w != 0;
-        const unsigned m = __ballot_sync(0xFFFFFFFFu, occ);
-        if (lane == 0) s_warp[warp] = __popc(m);
-        __syncthreads();
-        unsigned before = 0, total = 0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) {
-            const unsigned v = s_warp[w];
-            if (w < warp) before += v;
-            total += v;
-        }
-        if (threadIdx.x == 0 && total) s_base = atomicAdd(counter, static_cast<unsigned long long>(total));
-        __syncthreads();
-        if (occ) {
-            const unsigned long long idx = s_base + before + __popc(m & ((1u << lane) - 1u));
-            if (idx < out_cap) keys[idx] = s.x, keys_hi[idx] = s.y, counts[idx] = s.w, first[idx] = s.z;
-        }
     }
 }
 
@@ -307,52 +289,6 @@ __global__ void __launch_bounds__(256) gather1_kernel(const unsigned* __restrict
                                                       unsigned long long* __restrict__ out, unsigned long long n) {
     const unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x;
     if (i < n) out[i] = in[perm[i]];
-}
-
-// dst[(lo, hi)] += counts, first = min(first, pos_base + first_in)
-__global__ void __launch_bounds__(256) merge_wide_list_kernel(WideSlot* dst, unsigned long long mask,
-                                                              const unsigned long long* __restrict__ keys,
-                                                              const unsigned long long* __restrict__ keys_hi,
-                                                              const unsigned long long* __restrict__ counts,
-                                                              const unsigned long long* __restrict__ first,
-                                                              unsigned long long n, unsigned long long pos_base,
-                                                              unsigned long long* occupied, DevState* st) {
-    const unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x;
-    if (i < n) table_add_wide(dst, mask, keys[i], keys_hi[i], counts[i], first ? pos_base + first[i] : pos_base + i, occupied, st);
-}
-
-// demux_ok_kernel over wide keys: the total is sorted by (hi, lo).
-__global__ void __launch_bounds__(256) demux_ok_wide_kernel(const unsigned long long* __restrict__ fkeys,
-                                                            const unsigned long long* __restrict__ fkeys_hi,
-                                                            const unsigned long long* __restrict__ fcounts, unsigned long long nf,
-                                                            const unsigned long long* __restrict__ sorted_lo,
-                                                            const unsigned long long* __restrict__ sorted_hi,
-                                                            const unsigned* __restrict__ sorted_idx, unsigned long long n,
-                                                            const unsigned char* __restrict__ type, const int* __restrict__ srow,
-                                                            const unsigned char* __restrict__ match, unsigned n_files, unsigned f,
-                                                            unsigned char* __restrict__ ok, unsigned char* __restrict__ bad_file,
-                                                            int* err_row) {
-    const unsigned long long i = blockIdx.x * static_cast<unsigned long long>(blockDim.x) + threadIdx.x;
-    if (i >= nf || (fcounts && fcounts[i] == 0)) return;
-    const unsigned long long klo = fkeys[i], khi = fkeys_hi[i];
-    unsigned long long lo = 0, hi = n;
-    while (lo < hi) {
-        const unsigned long long mid = (lo + hi) >> 1;
-        const unsigned long long mh = sorted_hi[mid];
-        if (mh < khi || (mh == khi && sorted_lo[mid] < klo)) lo = mid + 1;
-        else hi = mid;
-    }
-    if (lo >= n || sorted_lo[lo] != klo || sorted_hi[lo] != khi) return;
-    const unsigned idx = sorted_idx[lo];
-    const unsigned t = type[idx];
-    const unsigned cls = t == 2 ? 4u + static_cast<unsigned>(srow[idx]) : t;
-    const unsigned m = match[static_cast<unsigned long long>(cls) * n_files + f];
-    if (m == 2) {
-        atomicMin(err_row, static_cast<int>(cls) - 4);
-    } else if (m == 0) {
-        ok[idx] = 0;
-        bad_file[f] = 1;
-    }
 }
 
 }  // namespace frb

@@ -173,7 +173,8 @@ def _scan_worker(rank, n_ranks, device, ident, jobs, sample, table_log2, conn):
     """One process per GPU (FRENDER_GPUS > 1): scan this rank's files, report, and -- once the parent has heard
     from every rank that its scans went through -- merge the per-rank tables over NCCL and send the per-file
     lists (and, from rank 0, the merged total) to the parent.  A rank that fails never enters the collective,
-    and neither does anybody else: the parent only says "go" when all ranks are ready for it."""
+    and neither does anybody else: the parent only says "go" when all ranks are ready for it.  The rank's own total
+    is built before it reports, so that a table too small for the union of its files fails here too."""
     try:
         ctx = Context(device, table_log2=table_log2)
         ctx.nccl_init(ident, rank, n_ranks)
@@ -190,6 +191,7 @@ def _scan_worker(rank, n_ranks, device, ident, jobs, sample, table_log2, conn):
                 fk, fc, _ = ctx.file_arrays(k + j)
                 out.append((jobs[k + j][0], reads, uniq, fk, fc))
             k += len(done)
+        ctx.total_arrays()
         conn.send(("scanned", None, None))
         if not conn.recv():                     # another rank failed: no collective
             return

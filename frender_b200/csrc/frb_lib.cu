@@ -93,6 +93,8 @@ struct frb_ctx {
     unsigned long long* xchg[3] = {nullptr, nullptr, nullptr};  // send parts, received parts, histograms
     size_t xchg_cap[3] = {0, 0, 0};
     bool total_tab_clean = true;   // total_tab holds no keys
+    int total_err = FRB_OK;        // a merge into total_tab failed (it holds part of the total): kept until frb_reset
+    std::string total_err_msg;
     uint32_t cur_ordinal = 0;
     uint64_t cur_limit = ~0ULL;
     // sheet
@@ -245,6 +247,18 @@ int device_error_check(frb_ctx* c) {  // compute stream must be idle
         default:
             return fail(c, code, "device error %d at %llu", code, pos);
     }
+}
+
+// device_error_check after a merge into total_tab (compute stream idle).  The merge cannot be undone, so its error is
+// returned again by every later call until frb_reset, instead of the partial total.
+int total_tab_check(frb_ctx* c) {
+    if (c->total_err == FRB_OK) {
+        const int rc = device_error_check(c);
+        if (rc == FRB_OK) return FRB_OK;
+        c->total_err = rc;
+        c->total_err_msg = c->err;
+    }
+    return fail(c, c->total_err, "%s", c->total_err_msg.c_str());
 }
 
 // Stream-ordered allocations for everything sized by the number of unique keys: served from the
@@ -938,6 +952,7 @@ static int merge_pending_files(frb_ctx* c) {  // fold file lists into total_tab 
 
 // need_order = false: the caller (a sharded merge) regroups the entries anyway
 static int total_build(frb_ctx* c, bool need_order) {
+    if (c->total_err != FRB_OK) return total_tab_check(c);
     if (!c->total_ready) {
         TRY(free_list(c, c->total));
         if (c->files.size() == 1 && c->merged_upto == 0 && !c->ext_merged) {
@@ -967,7 +982,7 @@ static int total_build(frb_ctx* c, bool need_order) {
         } else {
             TRY(merge_pending_files(c));
             CU(c, cudaStreamSynchronize(c->compute));
-            TRY(device_error_check(c));
+            TRY(total_tab_check(c));
             TRY(table_to_sorted_list(c, c->total_tab, c->st_host->occupied_total, &c->total));
         }
         c->total_ready = true;
@@ -1045,7 +1060,7 @@ int frb_total_merge(frb_ctx* c, const uint64_t* keys, const uint64_t* counts, co
     }
     c->ext_merged = true;
     c->total_ready = false;
-    return FRB_OK;
+    return total_tab_check(c);
 }
 int frb_reset(frb_ctx* c) {
     CU(c, cudaSetDevice(c->device));
@@ -1059,6 +1074,7 @@ int frb_reset(frb_ctx* c) {
     c->merged_upto = 0;
     c->ext_merged = false;
     c->sharded = false;
+    c->total_err = FRB_OK;
     if (!c->total_tab_clean) {
         TRY(clear_table(c, c->total_tab));
         c->total_tab_clean = true;

@@ -189,7 +189,10 @@ int frb_total_export(frb_ctx* ctx, uint64_t* keys, uint64_t* counts, uint64_t* f
 /* Load a (key,count) list as the total instead of scanning (process() on a caller's dict).  */
 int frb_total_load(frb_ctx* ctx, const uint64_t* keys, const uint64_t* counts, uint64_t n);
 /* Fold a (key,count,first_pos) list produced elsewhere (another context scanning other files of
- * the same run, F:199-203) into this context's total; first_pos must already be global.          */
+ * the same run, F:199-203) into this context's total; first_pos must already be global.
+ * A merge into the total table that fails (FRB_ERR_TABLE_FULL) leaves part of the total behind: this call,
+ * frb_total_finish and everything built on the total return that error again until frb_reset /
+ * frb_resize_tables.                                                                              */
 int frb_total_merge(frb_ctx* ctx, const uint64_t* keys, const uint64_t* counts, const uint64_t* first_pos,
                     uint64_t n);
 int frb_reset(frb_ctx* ctx); /* forget all files and the total                                 */

@@ -85,6 +85,7 @@ SIGNATURES = {
     "frb_route_pop": (C.c_int, [vp, P(vp), P(vp), vp, vp, P(u64), P(u64), P(u64), P(u64)]),
     "frb_route_set_gzip": (C.c_int, [vp, C.c_int]),
     "frb_route_set_gz_format": (C.c_int, [vp, C.c_int]),
+    "frb_route_set_mates": (C.c_int, [vp, C.c_int]),
     "frb_nccl_unique_id": (C.c_int, [C.c_char_p]),
     "frb_nccl_init": (C.c_int, [vp, C.c_char_p, C.c_int, C.c_int]),
     "frb_allmerge": (C.c_int, [vp, P(u64)]),

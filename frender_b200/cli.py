@@ -144,6 +144,28 @@ def get_paired_files(files):
     return pairs
 
 
+def get_single_end_files(files):
+    """[R1] of a single-end run (FRENDER_SINGLE_END=1): the files get_paired_files takes as read 1 (_R1_), each
+    routed alone.  An R1 with a read 2 file is refused (half of a paired input would be dropped silently), and so
+    is an input without any R1."""
+    r1s = [p for p in files if re.search("_R1_", str(p), re.I)]
+    if not r1s:
+        raise SystemExit("FRENDER_SINGLE_END=1: no read 1 file (a name with _R1_) among the inputs")
+    for r1 in r1s:
+        # only names with _R1_ / _R2_ can be mates (is_read_mate reads the mate number from both; an I1 index file
+        # one character away from an R1 has none)
+        mates = [q for q in files if re.search("_R[12]_", str(q)) and is_read_mate(str(r1), str(q))]
+        if mates:
+            raise SystemExit(f"FRENDER_SINGLE_END=1: {r1} has a read 2 file ({mates[0]}); paired input is "
+                             "demultiplexed without FRENDER_SINGLE_END")
+    return r1s
+
+
+def single_end():
+    """FRENDER_SINGLE_END: set (and not 0), frender demux routes R1 files alone, by their own headers."""
+    return os.environ.get("FRENDER_SINGLE_END", "0").strip() not in ("", "0")
+
+
 # ---------------------------------------------------------------------------------------------
 # scan (F:567-642)
 # ---------------------------------------------------------------------------------------------
@@ -747,7 +769,8 @@ class DeviceTextChunks:
 
 
 def _demux_worker(rank, device, jobs, opts, out_dir, threads, conn):
-    """One process per GPU: the file pairs `jobs` = [(ordinal, r1, r2)], each into its own part directory."""
+    """One process per GPU: the file pairs `jobs` = [(ordinal, r1, r2)], each into its own part directory (r2 is
+    None in a single-end run)."""
     try:
         os.environ["FRENDER_DEVICE"] = str(device)
         os.environ["FRENDER_GPUS"] = "1"
@@ -755,7 +778,8 @@ def _demux_worker(rank, device, jobs, opts, out_dir, threads, conn):
         ctx = Context(device, table_log2=12)
         try:
             for ordinal, r1, r2 in jobs:
-                ns = argparse.Namespace(**opts, files=[str(r1), str(r2)], d=f"{out_dir}.part{ordinal}")
+                files = [str(p) for p in (r1, r2) if p is not None]
+                ns = argparse.Namespace(**opts, files=files, d=f"{out_dir}.part{ordinal}")
                 frender_demux(ns, ctx=ctx)
         finally:
             ctx.close()
@@ -782,7 +806,8 @@ def join_parts(out_path, part_paths, bgzf_parts):
 
 
 def demux_pairs_multi_gpu(args, pairs, n_gpus, out_dir, worker=_demux_worker):
-    """FRENDER_GPUS=N with several R1/R2 pairs (lanes): pair i is routed on GPU i % N into rank-local part files
+    """FRENDER_GPUS=N with several R1/R2 pairs (lanes), or R1 files of a single-end run as (R1, None) pairs: pair i
+    is routed on GPU i % N into rank-local part files
     (SURVEY 8e: the demux outputs stay rank-local); the parts of every sink are then appended in pair order --
     gzip members one after the other, so every sink decompresses to exactly what the sequential loop over the
     pairs (F:774) writes.  With FRENDER_GZIP_LEVEL=bgzf the parts' EOF blocks but the last are dropped, and every
@@ -863,7 +888,10 @@ def frender_demux(args, ctx=None):
             raise SystemExit("Specified directory or file path doesn't seem to exist!")
     else:
         files = {"file": [Path(f) for f in args.files]}
-    pairs = get_paired_files(parse_files(files, just_r1=False))
+    single = single_end()
+    inputs = parse_files(files, just_r1=False)
+    # single-end: R1 files alone, as (R1, None) pairs
+    pairs = [(r1, None) for r1 in get_single_end_files(inputs)] if single else get_paired_files(inputs)
 
     out_dir = args.d if args.d.endswith("/") else args.d + "/"
     os.mkdir(args.d)                                                            # FileExistsError as in F:755
@@ -884,8 +912,8 @@ def frender_demux(args, ctx=None):
     hop_sink = open_sink("Index-hop") if index_hop else undeter_sink
     amb_sink = open_sink("Ambiguous") if ambiguous else undeter_sink
     sink_file = (MemberSink if gpu_gzip else BgzfSink if gpu_bgzf else (lambda path: GzSink(path, level)))
-    sinks = [{r: sink_file(f"{out_dir}{name}_frender-demux_{infix}{r}.fq.gz") for r in ("R1", "R2")}
-             for name in sink_names]
+    reads = ("R1",) if single else ("R1", "R2")
+    sinks = [{r: sink_file(f"{out_dir}{name}_frender-demux_{infix}{r}.fq.gz") for r in reads} for name in sink_names]
     n_sinks = len(sink_names)
     reject = n_sinks                                                            # "Unrecognized read type" bucket
 
@@ -941,7 +969,7 @@ def frender_demux(args, ctx=None):
     mates = []
 
     def fill(want):
-        """The next piece of both mates: host mates on the pool, device mates in this thread (a context is not
+        """The next piece of every mate: host mates on the pool, device mates in this thread (a context is not
         thread-safe)."""
         jobs = [(m, 0 if m.eof else w) for m, w in zip(mates, want)]
         futures = [None if getattr(m, "on_device", False) else pool.submit(m.read, n) for m, n in jobs]
@@ -951,29 +979,30 @@ def frender_demux(args, ctx=None):
     try:
         ctx.route_load(keys, routes, n_sinks + 1, keys_hi)
         ctx.route_gzip(gpu_gzip or gpu_bgzf, bgzf=gpu_bgzf)
+        ctx.route_mates(1 if single else 2)
         for r1_path, r2_path in pairs:
             print(f"Demultiplexing {r1_path.name}...")
             # The pair as a STREAM of chunks, two in flight: while chunk k is routed on the device and chunk k-1
             # comes back and is deflated, chunk k+1 is inflated.  Chunks are cut anywhere; records that are not
-            # complete yet (and the lead of one mate over the other) are carried on the device.
-            mates[:] = ([DeviceTextChunks(ctx, 0, r1_path), DeviceTextChunks(ctx, 1, r2_path)] if device_inflate
-                        else [TextChunks(r1_path), TextChunks(r2_path)])
-            a, b = mates
+            # complete yet (and the lead of one mate over the other) are carried on the device.  A single-end
+            # stream is the same with R1 alone (mate slot 0).
+            paths = [p for p in (r1_path, r2_path) if p is not None]
+            mates[:] = [DeviceTextChunks(ctx, m, p) if device_inflate else TextChunks(p) for m, p in enumerate(paths)]
             ctx.route_reset(chunk)
             flags, carry, over = [], (0, 0), False
             while not over:
-                want = [max(chunk - c, MIN_CHUNK // 4) for c in carry]   # carry + new bytes stay within the window
-                da, db = fill(want)
-                flags.append((1 if a.eof else 0) | (2 if b.eof else 0))
-                ctx.route_push(da, db, flags[-1])
-                over = a.eof and b.eof
+                # carry + new bytes stay within the window
+                got = fill([max(chunk - c, MIN_CHUNK // 4) for c in carry[:len(mates)]])
+                flags.append(sum(1 << m for m, reader in enumerate(mates) if reader.eof))
+                ctx.route_push(got[0], got[1] if len(got) > 1 else None, flags[-1])
+                over = all(reader.eof for reader in mates)
                 if len(flags) == 2:
                     popped, was = ctx.route_pop(), flags.pop(0)
                     write_out(popped)
                     carry = popped[5:7]
                     # zip() ends with the shorter mate (F:777): that file is over and nothing of it is left on
                     # the device (which ignores the chunk that is already queued behind this one)
-                    over = over or bool(was & 1 and carry[0] == 0) or bool(was & 2 and carry[1] == 0)
+                    over = over or any(was >> m & 1 and carry[m] == 0 for m in range(len(mates)))
             for _ in flags:
                 write_out(ctx.route_pop())
     except FrbError as exc:
@@ -984,7 +1013,7 @@ def frender_demux(args, ctx=None):
         try:
             drain()
         finally:
-            list(pool.map(lambda s: (s["R1"].close(), s["R2"].close()), sinks))
+            list(pool.map(lambda s: [f.close() for f in s.values()], sinks))
             pool.shutdown()
         for m in mates:                             # the readers' buffers (a next gz_open would reuse the slot)
             if isinstance(m, DeviceTextChunks):

@@ -123,6 +123,7 @@ struct frb_ctx {
     uint32_t n_sinks = 0;
     struct RouteStreamHolder* route = nullptr;  // the demux stream (frb_route.inl)
     int route_gz = FRB_GZ_FORMAT_PLAIN;         // the demux stream returns gzip members / BGZF blocks (frb_route_set_gz_format)
+    int route_mates = 2;                        // 1: single-end demux stream, R1 alone (frb_route_set_mates)
     // device gzip writer of frb_gz_deflate (frb_deflate.inl)
     struct DeflateHolder* deflate = nullptr;
     // device inflate (frb_gz.inl)

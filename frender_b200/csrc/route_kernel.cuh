@@ -15,7 +15,10 @@
 //   route_copy_kernel   one warp per record and mate: 16-byte stores, source realigned with funnel shifts
 //   route_carry_kernel  the unconsumed tails to the front of the next chunk's buffers
 // Algorithmic bytes = 2 x (R1 + R2): every byte read once by the parser and written once into its sink (the copy
-// re-reads the chunk, which is still in L2).  Nothing here depends on a host-side count: grids are sized by
+// re-reads the chunk, which is still in L2).
+// A single-end stream (Mates = 1, frb_route_set_mates) is the same with R1 alone: the parser takes the keys from the
+// R1 headers, the routed records are R1's complete records (no zip), the scan runs on a (S, 1) grid and the copy,
+// the carry and the deflate on R1 only -- 2 x R1 algorithmic bytes.  Nothing here depends on a host-side count: grids are sized by
 // capacity and the kernels take the record counts from device memory.
 #pragma once
 #include "common.cuh"
@@ -75,7 +78,9 @@ __global__ void route_grab_kernel(DevState* st, RouteState* rs, int which) {
 }
 
 // pairs, bytes used, and the terminators of the offset lists.  end1 / end2 = bytes in the chunk buffers;
-// final bit 0 / 1: the R1 / R2 stream ends with this chunk.
+// final bit 0 / 1: the R1 / R2 stream ends with this chunk.  Mates = 1 (single-end): R1 alone, its complete records
+// are routed (a trailing partial one once bit 0 is set); off2 / in2 / end2 are not read.
+template <int Mates>
 __global__ void route_plan_kernel(RouteState* rs, DevState* st, unsigned long long* off1, unsigned long long* off2,
                                   const unsigned char* __restrict__ in1, const unsigned char* __restrict__ in2,
                                   unsigned long long end1, unsigned long long end2, int final_chunk,
@@ -97,27 +102,27 @@ __global__ void route_plan_kernel(RouteState* rs, DevState* st, unsigned long lo
         rs->pairs = 0;
         return;
     }
-    if (rs->n1 > rec_cap || rs->n2 > rec_cap) {
+    if (rs->n1 > rec_cap || (Mates == 2 && rs->n2 > rec_cap)) {
         rs->error = FRB_ERR_ARG;  // records shorter than 16 bytes
         rs->pairs = 0;
         return;
     }
     off1[rs->n1] = end1;
-    off2[rs->n2] = end2;
+    if constexpr (Mates == 2) off2[rs->n2] = end2;
     // zip() of the 4-line groupers stops at the shorter mate (F:777); a trailing partial record only exists at the
     // end of a file (F:719-723)
     // (the parser counts a last line without '\n' as a line; before the end of the file it is not complete)
     const unsigned long long open1 = (end1 > rs->skip1 && in1[end1 - 1] != '\n') ? 1 : 0;
-    const unsigned long long open2 = (end2 > rs->skip2 && in2[end2 - 1] != '\n') ? 1 : 0;
+    const unsigned long long open2 = (Mates == 2 && end2 > rs->skip2 && in2[end2 - 1] != '\n') ? 1 : 0;
     const unsigned long long e1 = (final_chunk & 1) ? rs->n1 : (rs->lines1 - open1) / 4;
-    const unsigned long long e2 = (final_chunk & 2) ? rs->n2 : (rs->lines2 - open2) / 4;
+    const unsigned long long e2 = Mates == 1 ? ~0ull : (final_chunk & 2) ? rs->n2 : (rs->lines2 - open2) / 4;
     const unsigned long long n = e1 < e2 ? e1 : e2;
     rs->pairs = n;
     rs->used1 = n ? off1[n] : rs->skip1;
-    rs->used2 = n ? off2[n] : rs->skip2;
+    rs->used2 = Mates == 1 ? end2 : n ? off2[n] : rs->skip2;
     rs->bad = ~0ull;
     // a mate that has ended and is used up ends the stream (F:777): what the other one still holds is never read
-    if (((final_chunk & 1) && n == rs->n1) || ((final_chunk & 2) && n == rs->n2)) {
+    if (((final_chunk & 1) && n == rs->n1) || (Mates == 2 && (final_chunk & 2) && n == rs->n2)) {
         rs->done = 1;
         rs->used1 = end1, rs->used2 = end2;
     }
@@ -125,9 +130,10 @@ __global__ void route_plan_kernel(RouteState* rs, DevState* st, unsigned long lo
 }
 
 // sink of every record, its offset inside its (block, sink) cell, and the cells' sizes.  cell[(s * n_blocks + b)]
-// for mate 1, the same + n_sinks * n_blocks for mate 2.  One warp-step after the other inside a block, so that
-// records of one sink keep their order.  key2_hi: upper key words (wide only).
-template <bool Wide>
+// for mate 1, the same + n_sinks * n_blocks for mate 2 (Mates = 2 only).  One warp-step after the other inside a
+// block, so that records of one sink keep their order.  key2: the keys of the routed records (parsed from R2, or
+// from R1 when Mates = 1); key2_hi: their upper words (wide only).
+template <bool Wide, int Mates>
 __global__ void __launch_bounds__(kRouteBlock) route_hist_kernel(const Slot* __restrict__ table, unsigned long long mask,
                                                                  const unsigned long long* __restrict__ key2,
                                                                  const unsigned long long* __restrict__ off1,
@@ -140,11 +146,11 @@ __global__ void __launch_bounds__(kRouteBlock) route_hist_kernel(const Slot* __r
                                                                  const unsigned long long* __restrict__ key2_hi) {
     using K = KeyWidth<Wide>;
     const typename K::Slot* __restrict__ const tab = reinterpret_cast<const typename K::Slot*>(table);
-    extern __shared__ unsigned s_acc[];  // [2][n_sinks]
+    extern __shared__ unsigned s_acc[];  // [Mates][n_sinks]
     const unsigned long long n = rs->pairs;
     const unsigned b = blockIdx.x;
     if (static_cast<unsigned long long>(b) * kRouteBlock >= n) return;
-    for (unsigned i = threadIdx.x; i < 2 * n_sinks; i += kRouteBlock) s_acc[i] = 0;
+    for (unsigned i = threadIdx.x; i < Mates * n_sinks; i += kRouteBlock) s_acc[i] = 0;
     __syncthreads();
     const unsigned long long i = static_cast<unsigned long long>(b) * kRouteBlock + threadIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -166,7 +172,7 @@ __global__ void __launch_bounds__(kRouteBlock) route_hist_kernel(const Slot* __r
             s = 0;
         }
         l1 = static_cast<unsigned>(off1[i + 1] - off1[i]);
-        l2 = static_cast<unsigned>(off2[i + 1] - off2[i]);
+        if constexpr (Mates == 2) l2 = static_cast<unsigned>(off2[i + 1] - off2[i]);
         sink[i] = s;
     }
     for (int w = 0; w < kRouteBlock / 32; ++w) {
@@ -177,22 +183,25 @@ __global__ void __launch_bounds__(kRouteBlock) route_hist_kernel(const Slot* __r
             unsigned before1 = 0, before2 = 0, tot1 = 0, tot2 = 0;
             for (unsigned m = same; m; m &= m - 1) {
                 const int src = __ffs(m) - 1;
-                const unsigned a1 = __shfl_sync(same, l1, src), a2 = __shfl_sync(same, l2, src);
+                const unsigned a1 = __shfl_sync(same, l1, src), a2 = Mates == 2 ? __shfl_sync(same, l2, src) : 0;
                 if (src < lane) before1 += a1, before2 += a2;
                 tot1 += a1, tot2 += a2;
             }
             local1[i] = s_acc[s] + before1;
-            local2[i] = s_acc[n_sinks + s] + before2;
+            if constexpr (Mates == 2) local2[i] = s_acc[n_sinks + s] + before2;
             __syncwarp(active);
-            if (lane == __ffs(same) - 1) s_acc[s] += tot1, s_acc[n_sinks + s] += tot2;
+            if (lane == __ffs(same) - 1) {
+                s_acc[s] += tot1;
+                if constexpr (Mates == 2) s_acc[n_sinks + s] += tot2;
+            }
         }
         __syncthreads();
     }
     for (unsigned k = threadIdx.x; k < n_sinks; k += kRouteBlock) {
         cell[static_cast<unsigned long long>(k) * n_blocks + b] = s_acc[k];
-        cell[static_cast<unsigned long long>(n_sinks + k) * n_blocks + b] = s_acc[n_sinks + k];
+        if constexpr (Mates == 2) cell[static_cast<unsigned long long>(n_sinks + k) * n_blocks + b] = s_acc[n_sinks + k];
         if (s_acc[k]) atomicAdd(&tot[k], static_cast<unsigned long long>(s_acc[k]));
-        if (s_acc[n_sinks + k]) atomicAdd(&tot[n_sinks + k], static_cast<unsigned long long>(s_acc[n_sinks + k]));
+        if (Mates == 2 && s_acc[n_sinks + k]) atomicAdd(&tot[n_sinks + k], static_cast<unsigned long long>(s_acc[n_sinks + k]));
     }
 }
 

@@ -549,11 +549,17 @@ class Context:
         else:
             self._ck(lib.frb_route_set_gzip(self._h, 1 if on else 0))
 
+    def route_mates(self, n):
+        """Paired (2) or single-end (1) demux stream (frb_route_set_mates): a single-end stream routes R1 alone, by
+        the keys of its own headers; route_push then takes r2=None and route_pop returns empty R2 offsets.  Only
+        between chunks; kept by route_reset."""
+        self._ck(lib.frb_route_set_mates(self._h, int(n)))
+
     def route_push(self, r1, r2, final=0):
         """Queue one chunk pair of the demux stream (frb_route_push): bytes cut anywhere; what is not complete
-        yet is carried on the device.  Either mate may be host bytes or a device GzSpan of this context (gz_read).
-        Returns at once; at most two chunks may be in flight."""
-        (pa, na, _ka), (pb, nb, _kb) = _chunk_arg(r1), _chunk_arg(r2)
+        yet is carried on the device.  Either mate may be host bytes or a device GzSpan of this context (gz_read);
+        r2 is None in a single-end stream (route_mates(1)).  Returns at once; at most two chunks may be in flight."""
+        (pa, na, _ka), (pb, nb, _kb) = _chunk_arg(r1), (None, 0, None) if r2 is None else _chunk_arg(r2)
         self._ck(lib.frb_route_push(self._h, pa, na, pb, nb, int(final)))
 
     def route_pop(self):
@@ -567,7 +573,8 @@ class Context:
                                    C.byref(c1), C.byref(c2), C.byref(bad)))
         n1, n2 = int(off1[-1]), int(off2[-1])
         v1 = np.ctypeslib.as_array((C.c_uint8 * max(n1, 1)).from_address(o1.value))[:n1]
-        v2 = np.ctypeslib.as_array((C.c_uint8 * max(n2, 1)).from_address(o2.value))[:n2]
+        v2 = (np.ctypeslib.as_array((C.c_uint8 * max(n2, 1)).from_address(o2.value))[:n2] if o2.value
+              else np.empty(0, np.uint8))                 # a single-end stream returns no R2
         return v1, v2, off1.astype(np.int64), off2.astype(np.int64), pairs.value, c1.value, c2.value
 
     # ---- measurement ------------------------------------------------------------------------

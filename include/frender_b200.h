@@ -294,6 +294,15 @@ int frb_route_set_gzip(frb_ctx* ctx, int on);
  * the EOF block behind them; an empty cell stays empty.  The same rules as frb_route_set_gzip; any other format is
  * FRB_ERR_ARG.                                                                                                  */
 int frb_route_set_gz_format(frb_ctx* ctx, int format);
+/* Paired (mates = 2, the default) or single-end (mates = 1) demux stream; any other value is FRB_ERR_ARG.  The same
+ * rules as frb_route_set_gz_format: refused with FRB_ERR_STATE while chunks are in flight, kept by frb_route_reset.
+ * A single-end stream routes the records of R1 alone, each by the key of its own header (the demux rule, F:778
+ * applied to the R1 header line); every output format and wide contexts (frb_route_load2) work as in a paired one.
+ *   frb_route_push  takes r2 = NULL, r2_bytes = 0 (anything else is FRB_ERR_ARG); only bit 0 of final_chunk counts,
+ *                   and a trailing partial record of R1 is routed once it is set.
+ *   frb_route_pop   *n_pairs = records routed; *out_r2 = NULL, off_r2 all zero, carry_r2 = 0.
+ * frb_route_pair always routes pairs: it saves the setting, routes with mates = 2 and restores it.                */
+int frb_route_set_mates(frb_ctx* ctx, int mates);
 
 /* ---- multi-GPU: merge of the per-rank totals over NCCL (NVLink) ------------------------------
  * One process (or thread) per GPU.  Rank 0 makes the id, the host hands it to every rank.

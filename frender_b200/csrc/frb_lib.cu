@@ -22,6 +22,7 @@
 
 #include "common.cuh"
 #include "deflate_kernels.cuh"
+#include "frb_own.h"
 #include "gz_kernels.cuh"
 #include "match_kernel.cuh"
 #include "route_kernel.cuh"
@@ -39,9 +40,9 @@ namespace {
 constexpr int kHostStages = 3;
 thread_local std::string g_last_error;
 
-struct KeyList {  // device arrays of one (key,count,first) list
-    unsigned long long *keys = nullptr, *counts = nullptr, *first = nullptr;
-    unsigned long long* keys_hi = nullptr;  // upper key words, wide context only
+struct KeyList {  // device arrays of one (key,count,first) list, from the memory pool
+    PoolBuf<unsigned long long> keys, counts, first;
+    PoolBuf<unsigned long long> keys_hi;  // upper key words, wide context only
     uint64_t n = 0, reads = 0;
     uint32_t ordinal = 0;
     bool sorted = true;   // in first-appearance order (a file's list is sorted when somebody first needs the order)
@@ -49,99 +50,102 @@ struct KeyList {  // device arrays of one (key,count,first) list
 };
 
 struct ProfPair {
-    cudaEvent_t a, b;
+    Event a, b;
     int cls;
 };
+
+// defined in the frb_*.inl files
+struct GzBuffers;
+struct GzTextReader;
+struct DeflateBuffers;
+struct RouteStream;
 
 }  // namespace
 
 struct frb_ctx {
+    // first, so that they are destroyed last: the pool buffers below queue their frees on `compute`
+    Stream compute, copy;
     int device = 0, sm_count = 0;
-    cudaStream_t compute = nullptr, copy = nullptr;
     uint32_t log2 = 0;
     uint64_t cap = 0;
     bool wide = false;  // keys of up to 42 symbols: WideSlot tables, (lo, hi) lists (frb_set_key_width)
-    Slot *file_tab = nullptr, *total_tab = nullptr;
-    DevState* st = nullptr;
-    DevState* st_host = nullptr;  // pinned mirror
-    unsigned long long* status = nullptr;
-    unsigned int* redo = nullptr;  // tiles left to scan_redo_kernel (same capacity as status)
-    size_t status_cap = 0;
+    DevBuf<Slot> file_tab, total_tab;
+    DevBuf<DevState> st;
+    PinnedBuf<DevState> st_host;  // pinned mirror
+    DevBuf<unsigned long long> status;
+    DevBuf<unsigned int> redo;  // tiles left to scan_redo_kernel (same capacity as status)
     // speculative scan path: first read ordinal of every tile of the current file (composite -> ordinal)
-    unsigned long long* tile_first = nullptr;
-    size_t tile_first_cap = 0;
+    DevBuf<unsigned long long> tile_first;
     uint64_t file_tiles = 0;            // tiles of the current file scanned so far
     int file_composite = -1;            // -1 undecided, 0 read ordinals, 1 composite positions in file_tab
-    unsigned long long* block_sums = nullptr;
-    size_t block_sums_cap = 0;
+    DevBuf<unsigned long long> block_sums;
+    DevBuf<unsigned long long> scan_timing;  // FRB_SCAN_TIMING: the scan kernels' clock sums
     // host-chunk staging
-    unsigned char* stage[kHostStages] = {nullptr, nullptr, nullptr};
-    cudaEvent_t stage_copied[kHostStages], stage_done[kHostStages];
+    DevBuf<unsigned char> stage[kHostStages];
+    Event stage_copied[kHostStages], stage_done[kHostStages];
     size_t stage_cap = 0;
     int stage_next = 0;
     // gz pipeline ring (pinned)
-    unsigned char* ring[kHostStages] = {nullptr, nullptr, nullptr};
+    PinnedBuf<unsigned char> ring[kHostStages];
     // results
     std::vector<KeyList> files;
     KeyList total;
-    unsigned long long* skip_slot = nullptr;  // device word: where the text begins in the buffer of a batch segment
+    DevBuf<unsigned long long> skip_slot;  // device word: where the text begins in the buffer of a batch segment
     bool total_ready = false, in_file = false;
     size_t merged_upto = 0;        // file lists already folded into total_tab
     bool ext_merged = false;       // lists from other contexts were folded in (frb_total_merge)
     bool sharded = false;          // total holds this rank's share of a sharded merge (no table behind it)
     // exchange buffers of the sharded merge: kept (grow-only) so that NCCL sees the same addresses every step
-    unsigned long long* xchg[3] = {nullptr, nullptr, nullptr};  // send parts, received parts, histograms
-    size_t xchg_cap[3] = {0, 0, 0};
+    DevBuf<unsigned char> xchg[3];  // send parts, received parts, histograms
     bool total_tab_clean = true;   // total_tab holds no keys
     int total_err = FRB_OK;        // a merge into total_tab failed (it holds part of the total): kept until frb_reset
     std::string total_err_msg;
     uint32_t cur_ordinal = 0;
     uint64_t cur_limit = ~0ULL;
-    // sheet
-    unsigned long long *sheet_fwd = nullptr, *sheet_rc = nullptr;
-    unsigned long long *sheet_fwd_hi = nullptr, *sheet_rc_hi = nullptr;
-    int* sheet_group = nullptr;
-    unsigned char* sheet_use_rc = nullptr;
-    unsigned long long *f_sum = nullptr, *rc_sum = nullptr;
+    // sheet (packed for one key width) and the per-row sums of the matcher
+    struct Sheet {
+        DevBuf<unsigned long long> fwd, rc, fwd_hi, rc_hi;
+        DevBuf<int> group;
+        DevBuf<unsigned char> use_rc;
+        DevBuf<unsigned long long> f_sum, rc_sum;
+    } sheet;
     uint32_t rows = 0, l1 = 0, l2 = 0;
-    // matcher outputs (device, grown on demand)
-    int *m1 = nullptr, *m2 = nullptr, *srow = nullptr, *m2rc = nullptr, *srowrc = nullptr;
-    unsigned char *type = nullptr, *typerc = nullptr;
-    unsigned* work = nullptr;             // keys with an idx1 match (matcher work list)
-    unsigned long long* work_n = nullptr;
-    uint64_t match_cap = 0;
+    // matcher outputs (device, grown on demand; `work` is allocated last, so it holds room for as many keys as all do)
+    struct Matcher {
+        DevBuf<unsigned long long> work_n;
+        DevBuf<int> m1, m2, srow, m2rc, srowrc;
+        DevBuf<unsigned char> type, typerc;
+        DevBuf<unsigned> work;  // keys with an idx1 match (matcher work list)
+    } matcher;
     uint64_t total_gen = 0, sheet_gen = 0;            // bumped whenever the total list / sheet changes
     uint64_t m1_total_gen = ~0ULL, m1_sheet_gen = ~0ULL;  // what c->m1 currently describes
     uint32_t m1_n_subs = ~0u;
     bool m1_from_rc = false;                              // ... and it came from an rc_mode pass
     // temp for sort
-    void* cub_tmp = nullptr;
-    size_t cub_tmp_bytes = 0;
+    DevBuf<unsigned char> cub_tmp;
     // route
-    Slot* route_tab = nullptr;
-    uint64_t route_cap = 0;
+    DevBuf<Slot> route_tab;
     uint32_t n_sinks = 0;
-    struct RouteStreamHolder* route = nullptr;  // the demux stream (frb_route.inl)
+    std::unique_ptr<RouteStream> route;  // the demux stream (frb_route.inl)
     int route_gz = FRB_GZ_FORMAT_PLAIN;         // the demux stream returns gzip members / BGZF blocks (frb_route_set_gz_format)
     int route_mates = 2;                        // 1: single-end demux stream, R1 alone (frb_route_set_mates)
     // device gzip writer of frb_gz_deflate (frb_deflate.inl)
-    struct DeflateHolder* deflate = nullptr;
+    std::unique_ptr<DeflateBuffers> deflate;
     // device inflate (frb_gz.inl)
-    struct GzBuffersHolder* gzbuf = nullptr;
+    std::unique_ptr<GzBuffers> gzbuf;
     // span readers of frb_gz_open / frb_gz_read, one per mate (frb_gz.inl)
-    struct GzReaderSlots* gzread = nullptr;
+    std::unique_ptr<GzTextReader> gzread[2];
     // synth
     SynthArgs synth{};
-    unsigned *synth_i7 = nullptr, *synth_i5 = nullptr;
-    unsigned long long* synth_cdf = nullptr;
-    unsigned long long *synth_len = nullptr, *synth_off = nullptr;
-    uint64_t synth_cap = 0;
+    DevBuf<unsigned> synth_i7, synth_i5;
+    DevBuf<unsigned long long> synth_cdf;
+    DevBuf<unsigned long long> synth_len, synth_off;
     bool synth_ready = false;
     // nccl
     void* nccl_comm = nullptr;
     int rank = 0, n_ranks = 1;
     // measurement
-    cudaEvent_t t0 = nullptr, t1 = nullptr;
+    Event t0, t1;
     bool prof = false;
     std::vector<ProfPair> prof_pending;
     std::vector<ProfPair> prof_free;
@@ -150,6 +154,8 @@ struct frb_ctx {
     uint64_t launches = 0;
     uint64_t gz_device_files = 0;  // files inflated on the device
     std::string err;
+
+    ~frb_ctx();  // defined behind the frb_*.inl files, where the types of the members above are complete
 };
 
 namespace {
@@ -185,11 +191,11 @@ struct ProfScope {  // brackets a kernel (class) with events when profiling is o
     ProfScope(frb_ctx* ctx, int cls) : c(ctx), on(ctx->prof) {
         if (!on) return;
         if (!c->prof_free.empty()) {
-            p = c->prof_free.back();
+            p = std::move(c->prof_free.back());
             c->prof_free.pop_back();
         } else {
-            cudaEventCreate(&p.a);
-            cudaEventCreate(&p.b);
+            p.a.create(cudaEventDefault);
+            p.b.create(cudaEventDefault);
         }
         p.cls = cls;
         cudaEventRecord(p.a, c->compute);
@@ -197,7 +203,7 @@ struct ProfScope {  // brackets a kernel (class) with events when profiling is o
     ~ProfScope() {
         if (!on) return;
         cudaEventRecord(p.b, c->compute);
-        c->prof_pending.push_back(p);
+        c->prof_pending.push_back(std::move(p));
     }
 };
 
@@ -208,7 +214,7 @@ void prof_collect(frb_ctx* c) {  // call after the compute stream is idle
             c->prof_ms[p.cls] += ms;
             c->prof_n[p.cls] += 1;
         }
-        c->prof_free.push_back(p);
+        c->prof_free.push_back(std::move(p));
     }
     c->prof_pending.clear();
 }
@@ -262,28 +268,6 @@ int total_tab_check(frb_ctx* c) {
     return fail(c, c->total_err, "%s", c->total_err_msg.c_str());
 }
 
-// Stream-ordered allocations for everything sized by the number of unique keys: served from the
-// device's memory pool (release threshold = never), so a steady-state step makes no driver calls
-// that synchronise the device.
-template <typename T>
-int dmalloc(frb_ctx* c, T** p, size_t bytes) {
-    CU(c, cudaMallocAsync(reinterpret_cast<void**>(p), bytes ? bytes : 8, c->compute));
-    return FRB_OK;
-}
-int dfree(frb_ctx* c, void* p) {
-    if (p) CU(c, cudaFreeAsync(p, c->compute));
-    return FRB_OK;
-}
-
-int free_list(frb_ctx* c, KeyList& l) {
-    TRY(dfree(c, l.keys));
-    TRY(dfree(c, l.counts));
-    TRY(dfree(c, l.first));
-    TRY(dfree(c, l.keys_hi));
-    l = KeyList{};
-    return FRB_OK;
-}
-
 int clear_table(frb_ctx* c, Slot* tab) {
     ProfScope ps(c, FRB_K_OTHER);
     const auto clear = c->wide ? clear_table_kernel<true> : clear_table_kernel<false>;
@@ -294,54 +278,42 @@ int clear_table(frb_ctx* c, Slot* tab) {
 }
 
 int ensure_cub_tmp(frb_ctx* c, size_t bytes) {
-    if (bytes <= c->cub_tmp_bytes) return FRB_OK;
-    bytes += bytes / 2;
-    if (c->cub_tmp) CU(c, cudaFree(c->cub_tmp));
-    c->cub_tmp = nullptr;
-    c->cub_tmp_bytes = 0;
-    CU(c, cudaMalloc(&c->cub_tmp, bytes));
-    c->cub_tmp_bytes = bytes;
+    if (bytes > c->cub_tmp.size()) CU(c, c->cub_tmp.alloc(bytes + bytes / 2));
     return FRB_OK;
 }
 
-// Dense (key,count,first) arrays in arbitrary order -> list sorted by `first` (first-appearance order,
-// F:172-177 / F:199-205).  Takes over k0/c0/f0 (pool allocations) and frees them.
-int unsorted_to_sorted_list(frb_ctx* c, unsigned long long* k0, unsigned long long* c0, unsigned long long* f0,
-                            uint64_t n, KeyList* out, int first_bits = 64, unsigned long long* h0 = nullptr) {
+// The n entries of `in`, (key,count,first) in arbitrary order -> list sorted by `first` (first-appearance order,
+// F:172-177 / F:199-205).
+int unsorted_to_sorted_list(frb_ctx* c, const KeyList& in, KeyList* out, int first_bits = 64) {
+    const uint64_t n = in.n;
     out->n = n;
-    unsigned *i0 = nullptr, *i1 = nullptr;
     if (n) {
-        TRY(dmalloc(c, &i0, n * 4));
-        TRY(dmalloc(c, &i1, n * 4));
-        TRY(dmalloc(c, &out->keys, n * 8));
-        TRY(dmalloc(c, &out->counts, n * 8));
-        TRY(dmalloc(c, &out->first, n * 8));
+        PoolBuf<unsigned> i0, i1;
+        CU(c, i0.alloc(n, c->compute));
+        CU(c, i1.alloc(n, c->compute));
+        CU(c, out->keys.alloc(n, c->compute));
+        CU(c, out->counts.alloc(n, c->compute));
+        CU(c, out->first.alloc(n, c->compute));
         ProfScope ps(c, FRB_K_EXPORT);
         iota_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(i0, n);
         size_t tmp = 0;
         // first_bits: significant bits of `first` (a file's read ordinals stay below 2^40: five radix passes
         // instead of eight)
-        CU(c, cub::DeviceRadixSort::SortPairs(nullptr, tmp, f0, out->first, i0, i1, static_cast<int>(n), 0,
-                                              first_bits, c->compute));
+        CU(c, cub::DeviceRadixSort::SortPairs(nullptr, tmp, in.first.get(), out->first.get(), i0.get(), i1.get(),
+                                              static_cast<int>(n), 0, first_bits, c->compute));
         TRY(ensure_cub_tmp(c, tmp));
-        CU(c, cub::DeviceRadixSort::SortPairs(c->cub_tmp, tmp, f0, out->first, i0, i1, static_cast<int>(n), 0,
-                                              first_bits, c->compute));
-        gather2_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(i1, k0, c0, out->keys,
+        CU(c, cub::DeviceRadixSort::SortPairs(c->cub_tmp, tmp, in.first.get(), out->first.get(), i0.get(), i1.get(),
+                                              static_cast<int>(n), 0, first_bits, c->compute));
+        gather2_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(i1, in.keys, in.counts, out->keys,
                                                                                        out->counts, n);
         c->launches += 9;  // iota, cub radix sort passes (approximate), gather
-        if (h0) {  // a wide list: the upper key words follow the same permutation
-            TRY(dmalloc(c, &out->keys_hi, n * 8));
-            gather1_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(i1, h0, out->keys_hi, n);
+        if (in.keys_hi) {  // a wide list: the upper key words follow the same permutation
+            CU(c, out->keys_hi.alloc(n, c->compute));
+            gather1_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(i1, in.keys_hi, out->keys_hi, n);
             c->launches++;
         }
         CU(c, cudaGetLastError());
     }
-    TRY(dfree(c, k0));
-    TRY(dfree(c, c0));
-    TRY(dfree(c, f0));
-    TRY(dfree(c, h0));
-    if (i0) TRY(dfree(c, i0));
-    if (i1) TRY(dfree(c, i1));
     return FRB_OK;
 }
 
@@ -351,22 +323,20 @@ int ensure_sorted(frb_ctx* c, KeyList& l) {
         l.sorted = true;
         return FRB_OK;
     }
-    KeyList tmp = l;
-    KeyList out = l;
-    out.keys = out.counts = out.first = out.keys_hi = nullptr;
-    TRY(unsorted_to_sorted_list(c, tmp.keys, tmp.counts, tmp.first, tmp.n, &out, l.first_bits, tmp.keys_hi));  // frees tmp's arrays
-    out.sorted = true;
-    l = out;
+    KeyList out;
+    out.reads = l.reads, out.ordinal = l.ordinal, out.first_bits = l.first_bits;
+    TRY(unsorted_to_sorted_list(c, l, &out, l.first_bits));
+    l = std::move(out);
     return FRB_OK;
 }
 
 // Occupied slots of a table -> fresh arrays of `room` entries in `out`, in slot order; their number lands in
 // st->scratch.  tile_first: see compact_table_kernel.
 int compact_table(frb_ctx* c, Slot* tab, uint64_t room, const unsigned long long* tile_first, KeyList* out) {
-    TRY(dmalloc(c, &out->keys, room * 8));
-    TRY(dmalloc(c, &out->counts, room * 8));
-    TRY(dmalloc(c, &out->first, room * 8));
-    if (c->wide) TRY(dmalloc(c, &out->keys_hi, room * 8));
+    CU(c, out->keys.alloc(room, c->compute));
+    CU(c, out->counts.alloc(room, c->compute));
+    CU(c, out->first.alloc(room, c->compute));
+    if (c->wide) CU(c, out->keys_hi.alloc(room, c->compute));
     ProfScope ps(c, FRB_K_EXPORT);
     CU(c, cudaMemsetAsync(&c->st->scratch, 0, 8, c->compute));
     const auto compact = c->wide ? compact_table_kernel<true> : compact_table_kernel<false>;
@@ -383,8 +353,9 @@ int table_to_sorted_list(frb_ctx* c, Slot* tab, uint64_t n, KeyList* out) {
     if (n == 0) return FRB_OK;
     if (n >= (1ULL << 32)) return fail(c, FRB_ERR_ARG, "more than 2^32 unique keys");
     KeyList l;
+    l.n = n;
     TRY(compact_table(c, tab, n, nullptr, &l));
-    return unsorted_to_sorted_list(c, l.keys, l.counts, l.first, n, out, 64, l.keys_hi);
+    return unsorted_to_sorted_list(c, l, out);
 }
 
 // The same when the number of occupied slots is not known: one pass over the table compacts and counts at once
@@ -417,16 +388,10 @@ int launch_scan(frb_ctx* c, const unsigned char* dev, uint64_t nbytes, uint64_t 
     const uint64_t tile = static_cast<uint64_t>(WsTile::tile);
     const uint64_t n_tiles = (nbytes + tile - 1) / tile;
     if (n_tiles >= 0xFFFFFFFFULL || nbytes >= (1ULL << 40)) return fail(c, FRB_ERR_ARG, "chunk too large");
-    if (n_tiles + 1 > c->status_cap) {
-        if (c->status) CU(c, cudaFree(c->status));
-        c->status = nullptr;
-        c->status_cap = 0;
+    if (n_tiles + 1 > std::min(c->status.size(), c->redo.size())) {
         const size_t want = std::max<size_t>(n_tiles + 1, 1 << 16);
-        CU(c, cudaMalloc(&c->status, want * 8));
-        if (c->redo) CU(c, cudaFree(c->redo));
-        c->redo = nullptr;
-        CU(c, cudaMalloc(&c->redo, want * 4));
-        c->status_cap = want;
+        CU(c, c->status.alloc(want));
+        CU(c, c->redo.alloc(want));
     }
     ScanArgs a{};
     a.data = dev;
@@ -452,11 +417,10 @@ int launch_scan(frb_ctx* c, const unsigned char* dev, uint64_t nbytes, uint64_t 
     a.pat_nl = 0x0A0A0A0Au;
     a.pat_sp = 0x20202020u;
     CU(c, cudaMemsetAsync(&c->st->redo_n, 0, 8, c->compute));
-    static unsigned long long* timing = nullptr;
     if (getenv("FRB_SCAN_TIMING")) {
-        if (!timing) cudaMalloc(&timing, 2048);
-        cudaMemsetAsync(timing, 0, 2048, c->compute);
-        a.timing = timing;
+        if (!c->scan_timing) c->scan_timing.alloc(256);
+        cudaMemsetAsync(c->scan_timing, 0, 2048, c->compute);
+        a.timing = c->scan_timing;
     }
     // the lean (speculative) instantiation serves the tally of whole files: scan rule, no per-read outputs, no -s
     static const bool probe = getenv("FRB_SCAN_TIMING") && strcmp(getenv("FRB_SCAN_TIMING"), "spec") == 0;
@@ -482,26 +446,16 @@ int launch_scan(frb_ctx* c, const unsigned char* dev, uint64_t nbytes, uint64_t 
         c->launches += 2;
     } else {
         // room for the first read ordinal of every tile of the file
-        if (c->file_tiles + n_tiles > c->tile_first_cap) {
-            const size_t want = std::max<size_t>((c->file_tiles + n_tiles) * 2, 1 << 16);
-            unsigned long long* grown = nullptr;
-            CU(c, cudaMalloc(&grown, want * 8));
+        if (c->file_tiles + n_tiles > c->tile_first.size()) {
+            DevBuf<unsigned long long> grown;
+            CU(c, grown.alloc(std::max<size_t>((c->file_tiles + n_tiles) * 2, 1 << 16)));
             if (c->file_tiles)
                 CU(c, cudaMemcpyAsync(grown, c->tile_first, c->file_tiles * 8, cudaMemcpyDeviceToDevice, c->compute));
             CU(c, cudaStreamSynchronize(c->compute));
-            if (c->tile_first) CU(c, cudaFree(c->tile_first));
-            c->tile_first = grown;
-            c->tile_first_cap = want;
+            c->tile_first = std::move(grown);
         }
         const unsigned n_blocks = static_cast<unsigned>((n_tiles + kVerifyTiles - 1) / kVerifyTiles);
-        if (n_blocks > c->block_sums_cap) {
-            if (c->block_sums) CU(c, cudaFree(c->block_sums));
-            c->block_sums = nullptr;
-            c->block_sums_cap = 0;
-            const size_t want = std::max<size_t>(n_blocks * 2, 1024);
-            CU(c, cudaMalloc(&c->block_sums, want * 8));
-            c->block_sums_cap = want;
-        }
+        if (n_blocks > c->block_sums.size()) CU(c, c->block_sums.alloc(std::max<size_t>(n_blocks * 2, 1024)));
         a.tile_base = c->file_tiles;
         a.tile_first = c->tile_first;
         a.composite = 1;
@@ -568,13 +522,13 @@ int launch_scan(frb_ctx* c, const unsigned char* dev, uint64_t nbytes, uint64_t 
 }
 
 int ensure_stages(frb_ctx* c) {
-    if (c->stage[0]) return FRB_OK;
+    if (c->stage_done[kHostStages - 1]) return FRB_OK;  // created last
     const char* env = getenv("FRB_STAGE_MB");
     c->stage_cap = static_cast<size_t>(env ? atoi(env) : 64) << 20;
     for (int i = 0; i < kHostStages; ++i) {
-        CU(c, cudaMalloc(&c->stage[i], c->stage_cap + 64));
-        CU(c, cudaEventCreateWithFlags(&c->stage_copied[i], cudaEventDisableTiming));
-        CU(c, cudaEventCreateWithFlags(&c->stage_done[i], cudaEventDisableTiming));
+        CU(c, c->stage[i].alloc(c->stage_cap + 64));
+        CU(c, c->stage_copied[i].create(cudaEventDisableTiming));
+        CU(c, c->stage_done[i].create(cudaEventDisableTiming));
     }
     return FRB_OK;
 }
@@ -582,23 +536,6 @@ int ensure_stages(frb_ctx* c) {
 }  // namespace
 
 #include "frb_gz.inl"
-struct GzBuffersHolder {
-    GzBuffers b;
-};
-struct GzReaderSlots {
-    std::unique_ptr<GzTextReader> r[2];
-};
-
-static void gz_readers_destroy(frb_ctx* c) {
-    if (!c->gzread) return;
-    for (auto& r : c->gzread->r)
-        if (r) gz_text_free(c, *r);
-    delete c->gzread;
-    c->gzread = nullptr;
-}
-
-static void route_stream_destroy(frb_ctx* c);  // frb_route.inl
-static void deflate_destroy(frb_ctx* c);       // frb_deflate.inl
 
 // ============================================================================================
 extern "C" {
@@ -628,7 +565,8 @@ int frb_create(int device, uint32_t table_log2, frb_ctx** out) {
     if (prop.major < 10)
         return fail(nullptr, FRB_ERR_CUDA, "device %d is sm_%d%d; this library is built for sm_100a only", device,
                     prop.major, prop.minor);
-    frb_ctx* c = new frb_ctx();
+    std::unique_ptr<frb_ctx> owner(new frb_ctx());  // released on every early return below
+    frb_ctx* c = owner.get();
     c->device = device;
     c->sm_count = prop.multiProcessorCount;
     c->log2 = table_log2;
@@ -640,15 +578,15 @@ int frb_create(int device, uint32_t table_log2, frb_ctx** out) {
         CU(c, cudaDeviceGetDefaultMemPool(&pool, device));
         CU(c, cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep));
     }
-    CU(c, cudaStreamCreateWithFlags(&c->compute, cudaStreamNonBlocking));
-    CU(c, cudaStreamCreateWithFlags(&c->copy, cudaStreamNonBlocking));
-    CU(c, cudaMalloc(&c->file_tab, c->cap * sizeof(Slot)));
-    CU(c, cudaMalloc(&c->total_tab, c->cap * sizeof(Slot)));
-    CU(c, cudaMalloc(&c->st, sizeof(DevState)));
+    CU(c, c->compute.create(cudaStreamNonBlocking));
+    CU(c, c->copy.create(cudaStreamNonBlocking));
+    CU(c, c->file_tab.alloc(c->cap));
+    CU(c, c->total_tab.alloc(c->cap));
+    CU(c, c->st.alloc(1));
     CU(c, cudaMemset(c->st, 0, sizeof(DevState)));
-    CU(c, cudaMallocHost(&c->st_host, sizeof(DevState)));
-    CU(c, cudaEventCreate(&c->t0));
-    CU(c, cudaEventCreate(&c->t1));
+    CU(c, c->st_host.alloc(1));
+    CU(c, c->t0.create(cudaEventDefault));
+    CU(c, c->t1.create(cudaEventDefault));
     CU(c, cudaFuncSetAttribute(scan_ws_kernel<WsTile>, cudaFuncAttributeMaxDynamicSharedMemorySize, WsTile::smem));
     CU(c, cudaFuncSetAttribute(scan_ws_kernel<WsTileWide>, cudaFuncAttributeMaxDynamicSharedMemorySize, WsTileWide::smem));
     CU(c, cudaFuncSetAttribute(scan_spec_kernel<WsTile>, cudaFuncAttributeMaxDynamicSharedMemorySize, WsTile::smem));
@@ -659,7 +597,7 @@ int frb_create(int device, uint32_t table_log2, frb_ctx** out) {
     CU(c, cudaFuncSetAttribute(match_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
     TRY(clear_table(c, c->total_tab));
     CU(c, cudaStreamSynchronize(c->compute));
-    *out = c;
+    *out = owner.release();
     return FRB_OK;
 }
 
@@ -667,32 +605,6 @@ void frb_destroy(frb_ctx* c) {
     if (!c) return;
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
-    for (auto& f : c->files) free_list(c, f);
-    free_list(c, c->total);
-    cudaFree(c->skip_slot);
-    cudaFree(c->file_tab), cudaFree(c->total_tab), cudaFree(c->st), cudaFreeHost(c->st_host), cudaFree(c->status), cudaFree(c->redo), cudaFree(c->tile_first), cudaFree(c->block_sums);
-    for (auto* p : c->xchg) cudaFree(p);
-    for (int i = 0; i < kHostStages; ++i) {
-        if (c->stage[i]) cudaFree(c->stage[i]), cudaEventDestroy(c->stage_copied[i]), cudaEventDestroy(c->stage_done[i]);
-        if (c->ring[i]) cudaFreeHost(c->ring[i]);
-    }
-    cudaFree(c->sheet_fwd), cudaFree(c->sheet_rc), cudaFree(c->sheet_group), cudaFree(c->sheet_use_rc);
-    cudaFree(c->sheet_fwd_hi), cudaFree(c->sheet_rc_hi);
-    cudaFree(c->f_sum), cudaFree(c->rc_sum);
-    cudaFree(c->m1), cudaFree(c->m2), cudaFree(c->srow), cudaFree(c->m2rc), cudaFree(c->srowrc);
-    cudaFree(c->type), cudaFree(c->typerc), cudaFree(c->work), cudaFree(c->work_n), cudaFree(c->cub_tmp), cudaFree(c->route_tab);
-    route_stream_destroy(c);
-    deflate_destroy(c);
-    gz_readers_destroy(c);
-    if (c->gzbuf) {
-        gz_free(c->gzbuf->b);
-        delete c->gzbuf;
-    }
-    cudaFree(c->synth_i7), cudaFree(c->synth_i5), cudaFree(c->synth_cdf), cudaFree(c->synth_len), cudaFree(c->synth_off);
-    for (auto& p : c->prof_pending) cudaEventDestroy(p.a), cudaEventDestroy(p.b);
-    for (auto& p : c->prof_free) cudaEventDestroy(p.a), cudaEventDestroy(p.b);
-    cudaEventDestroy(c->t0), cudaEventDestroy(c->t1);
-    cudaStreamDestroy(c->compute), cudaStreamDestroy(c->copy);
     delete c;
 }
 
@@ -701,13 +613,12 @@ int frb_resize_tables(frb_ctx* c, uint32_t table_log2) {
     if (table_log2 < 10 || table_log2 > 32) return fail(c, FRB_ERR_ARG, "table_log2 must be in [10, 32]");
     TRY(frb_reset(c));  // forgets every file and the total: a table cannot be re-hashed under a running tally
     CU(c, cudaStreamSynchronize(c->compute));
-    CU(c, cudaFree(c->file_tab));
-    CU(c, cudaFree(c->total_tab));
-    c->file_tab = c->total_tab = nullptr;
+    c->file_tab.reset();  // both go before the new ones are allocated
+    c->total_tab.reset();
     c->log2 = table_log2;
     c->cap = 1ULL << table_log2;
-    CU(c, cudaMalloc(&c->file_tab, c->cap * sizeof(Slot)));
-    CU(c, cudaMalloc(&c->total_tab, c->cap * sizeof(Slot)));
+    CU(c, c->file_tab.alloc(c->cap));
+    CU(c, c->total_tab.alloc(c->cap));
     TRY(clear_table(c, c->total_tab));
     c->total_tab_clean = true;
     CU(c, cudaStreamSynchronize(c->compute));
@@ -722,22 +633,23 @@ int frb_sync(frb_ctx* c) {
 }
 
 // ---- memory ---------------------------------------------------------------------------------
+// the caller's buffers: acquired and released as the owners of frb_own.h do, but owned by the caller
 int frb_host_alloc(void** p, size_t nbytes) {
-    CU(nullptr, cudaMallocHost(p, nbytes));
+    CU(nullptr, PinnedMem::acquire(p, nbytes, nullptr));
     return FRB_OK;
 }
 int frb_host_free(void* p) {
-    CU(nullptr, cudaFreeHost(p));
+    CU(nullptr, PinnedMem::release(p, nullptr));
     return FRB_OK;
 }
 int frb_dev_alloc(frb_ctx* c, size_t nbytes, void** dptr) {
     CU(c, cudaSetDevice(c->device));
-    CU(c, cudaMalloc(dptr, nbytes));
+    CU(c, DeviceMem::acquire(dptr, nbytes, nullptr));
     return FRB_OK;
 }
 int frb_dev_free(frb_ctx* c, void* dptr) {
     CU(c, cudaSetDevice(c->device));
-    CU(c, cudaFree(dptr));
+    CU(c, DeviceMem::release(dptr, nullptr));
     return FRB_OK;
 }
 int frb_h2d(frb_ctx* c, void* dptr, const void* host, size_t nbytes) {
@@ -808,14 +720,10 @@ int frb_set_key_width(frb_ctx* c, uint32_t bits) {
     // the tables change layout: the total table is cleared in the new one (the per-file table at every frb_scan_begin)
     TRY(clear_table(c, c->total_tab));
     c->total_tab_clean = true;
-    if (c->route_tab) CU(c, cudaFree(c->route_tab));
-    c->route_tab = nullptr, c->route_cap = 0, c->n_sinks = 0;
-    route_stream_destroy(c);  // its key buffer is sized for one width
+    c->route_tab.reset(), c->n_sinks = 0;
+    c->route.reset();  // its key buffer is sized for one width
     // the sample sheet is packed for one width: it has to be loaded again
-    cudaFree(c->sheet_fwd), cudaFree(c->sheet_rc), cudaFree(c->sheet_group), cudaFree(c->sheet_use_rc);
-    cudaFree(c->f_sum), cudaFree(c->rc_sum), cudaFree(c->sheet_fwd_hi), cudaFree(c->sheet_rc_hi);
-    c->sheet_fwd = c->sheet_rc = nullptr, c->sheet_group = nullptr, c->sheet_use_rc = nullptr;
-    c->f_sum = c->rc_sum = nullptr, c->sheet_fwd_hi = c->sheet_rc_hi = nullptr;
+    c->sheet = {};
     c->rows = c->l1 = c->l2 = 0;
     c->total_gen++, c->sheet_gen++;
     CU(c, cudaStreamSynchronize(c->compute));
@@ -891,8 +799,8 @@ int frb_scan_end(frb_ctx* c, uint64_t* n_reads, uint64_t* n_unique) {
     fl.ordinal = c->cur_ordinal;
     // Unique keys of the file = occupied slots of its table (at most one per read): compacted and counted in one
     // pass.  Read ordinals of one file stay below 2^40; composite positions become ordinals here.
-    TRY(table_to_sorted_list_counting(c, c->file_tab, fl.reads, &fl, 40, c->file_composite == 1 ? c->tile_first : nullptr));
-    c->files.push_back(fl);
+    TRY(table_to_sorted_list_counting(c, c->file_tab, fl.reads, &fl, 40, c->file_composite == 1 ? c->tile_first.get() : nullptr));
+    c->files.push_back(std::move(fl));
     c->total_ready = false;
     if (n_reads) *n_reads = fl.reads;
     if (n_unique) *n_unique = fl.n;
@@ -955,7 +863,7 @@ static int merge_pending_files(frb_ctx* c) {  // fold file lists into total_tab 
 static int total_build(frb_ctx* c, bool need_order) {
     if (c->total_err != FRB_OK) return total_tab_check(c);
     if (!c->total_ready) {
-        TRY(free_list(c, c->total));
+        c->total = KeyList{};
         if (c->files.size() == 1 && c->merged_upto == 0 && !c->ext_merged) {
             // one file: "total" is that file's list (F:199-203 degenerates to a copy); only `first`
             // gets the file ordinal in its high bits
@@ -965,14 +873,14 @@ static int total_build(frb_ctx* c, bool need_order) {
             c->total.first_bits = 64;
             c->total.n = fl.n;
             if (fl.n) {
-                TRY(dmalloc(c, &c->total.keys, fl.n * 8));
-                TRY(dmalloc(c, &c->total.counts, fl.n * 8));
-                TRY(dmalloc(c, &c->total.first, fl.n * 8));
+                CU(c, c->total.keys.alloc(fl.n, c->compute));
+                CU(c, c->total.counts.alloc(fl.n, c->compute));
+                CU(c, c->total.first.alloc(fl.n, c->compute));
                 ProfScope ps(c, FRB_K_EXPORT);
                 CU(c, cudaMemcpyAsync(c->total.keys, fl.keys, fl.n * 8, cudaMemcpyDeviceToDevice, c->compute));
                 CU(c, cudaMemcpyAsync(c->total.counts, fl.counts, fl.n * 8, cudaMemcpyDeviceToDevice, c->compute));
                 if (fl.keys_hi) {
-                    TRY(dmalloc(c, &c->total.keys_hi, fl.n * 8));
+                    CU(c, c->total.keys_hi.alloc(fl.n, c->compute));
                     CU(c, cudaMemcpyAsync(c->total.keys_hi, fl.keys_hi, fl.n * 8, cudaMemcpyDeviceToDevice, c->compute));
                 }
                 add_offset_kernel<<<static_cast<unsigned>((fl.n + 255) / 256), 256, 0, c->compute>>>(
@@ -1014,14 +922,14 @@ int frb_total_load(frb_ctx* c, const uint64_t* keys, const uint64_t* counts, uin
 int frb_total_load2(frb_ctx* c, const uint64_t* keys, const uint64_t* keys_hi, const uint64_t* counts, uint64_t n) {
     CU(c, cudaSetDevice(c->device));
     if (keys_hi && !c->wide) return fail(c, FRB_ERR_STATE, "frb_total_load2: upper key words need a wide context (frb_set_key_width)");
-    TRY(free_list(c, c->total));
+    c->total = KeyList{};
     c->total.n = n;
     if (n) {
-        TRY(dmalloc(c, &c->total.keys, n * 8));
-        TRY(dmalloc(c, &c->total.counts, n * 8));
-        TRY(dmalloc(c, &c->total.first, n * 8));
+        CU(c, c->total.keys.alloc(n, c->compute));
+        CU(c, c->total.counts.alloc(n, c->compute));
+        CU(c, c->total.first.alloc(n, c->compute));
         if (c->wide) {
-            TRY(dmalloc(c, &c->total.keys_hi, n * 8));
+            CU(c, c->total.keys_hi.alloc(n, c->compute));
             if (keys_hi) CU(c, cudaMemcpyAsync(c->total.keys_hi, keys_hi, n * 8, cudaMemcpyHostToDevice, c->compute));
             else CU(c, cudaMemsetAsync(c->total.keys_hi, 0, n * 8, c->compute));
         }
@@ -1039,10 +947,10 @@ int frb_total_merge(frb_ctx* c, const uint64_t* keys, const uint64_t* counts, co
     if (c->in_file) return fail(c, FRB_ERR_STATE, "frb_total_merge: a file is still open");
     if (c->wide) return fail(c, FRB_ERR_STATE, "frb_total_merge: not available on a wide (128-bit key) context");
     if (n) {
-        unsigned long long *dk = nullptr, *dc = nullptr, *df = nullptr;
-        TRY(dmalloc(c, &dk, n * 8));
-        TRY(dmalloc(c, &dc, n * 8));
-        TRY(dmalloc(c, &df, n * 8));
+        PoolBuf<unsigned long long> dk, dc, df;
+        CU(c, dk.alloc(n, c->compute));
+        CU(c, dc.alloc(n, c->compute));
+        CU(c, df.alloc(n, c->compute));
         CU(c, cudaMemcpyAsync(dk, keys, n * 8, cudaMemcpyHostToDevice, c->compute));
         CU(c, cudaMemcpyAsync(dc, counts, n * 8, cudaMemcpyHostToDevice, c->compute));
         CU(c, cudaMemcpyAsync(df, first_pos, n * 8, cudaMemcpyHostToDevice, c->compute));
@@ -1054,9 +962,6 @@ int frb_total_merge(frb_ctx* c, const uint64_t* keys, const uint64_t* counts, co
         }
         CU(c, cudaGetLastError());
         CU(c, cudaStreamSynchronize(c->compute));  // the host arrays may be reused by the caller
-        TRY(dfree(c, dk));
-        TRY(dfree(c, dc));
-        TRY(dfree(c, df));
         c->total_tab_clean = false;
     }
     c->ext_merged = true;
@@ -1066,9 +971,8 @@ int frb_total_merge(frb_ctx* c, const uint64_t* keys, const uint64_t* counts, co
 int frb_reset(frb_ctx* c) {
     CU(c, cudaSetDevice(c->device));
     CU(c, cudaStreamSynchronize(c->compute));
-    for (auto& f : c->files) TRY(free_list(c, f));
     c->files.clear();
-    TRY(free_list(c, c->total));
+    c->total = KeyList{};
     c->total_ready = false;
     c->in_file = false;
     CU(c, cudaMemsetAsync(c->st, 0, sizeof(DevState), c->compute));
@@ -1113,7 +1017,7 @@ static int scan_gz_host(frb_ctx* c, const char* path, uint32_t file_ordinal, uin
     CU(c, cudaSetDevice(c->device));
     TRY(ensure_stages(c));
     for (int i = 0; i < kHostStages; ++i)
-        if (!c->ring[i]) CU(c, cudaMallocHost(&c->ring[i], c->stage_cap));
+        if (!c->ring[i]) CU(c, c->ring[i].alloc(c->stage_cap));
     gzFile gz = gzopen(path, "rb");
     if (!gz) return fail(c, FRB_ERR_IO, "cannot open %s", path);
     gzbuffer(gz, 1 << 20);
@@ -1263,12 +1167,12 @@ int frb_scan_gz(frb_ctx* c, const char* path, uint32_t file_ordinal, uint64_t re
     CU(c, cudaSetDevice(c->device));
     static const bool device_ok = !(getenv("FRB_GZ_DEVICE") && atoi(getenv("FRB_GZ_DEVICE")) == 0);
     if (device_ok && !read_limit) {  // -s reads a head sample only: the host path stops early
-        if (!c->gzbuf) c->gzbuf = new GzBuffersHolder();
+        if (!c->gzbuf) c->gzbuf.reset(new GzBuffers());
         TRY(frb_scan_begin(c, file_ordinal, 0));
         bool first = true;
         uint64_t raw = 0;
         const int rc = gz_device_inflate(
-            c, c->gzbuf->b, path, &raw,
+            c, *c->gzbuf, path, &raw,
             [&](unsigned char* dev, uint64_t n, bool) {
                 const int r = launch_scan(c, dev, n, first ? 0 : FRB_CARRY, FRB_RULE_SCAN, nullptr, nullptr, c->file_tab, 0);
                 first = false;
@@ -1315,8 +1219,8 @@ int frb_scan_gz_batch(frb_ctx* c, const char* const* paths, const uint32_t* ordi
             magic[2] != 8)
             return FRB_OK;
     }
-    if (!c->gzbuf) c->gzbuf = new GzBuffersHolder();
-    if (!c->skip_slot) CU(c, cudaMalloc(&c->skip_slot, 8));
+    if (!c->gzbuf) c->gzbuf.reset(new GzBuffers());
+    if (!c->skip_slot) CU(c, c->skip_slot.alloc(1));
     const size_t files_before = c->files.size();
     std::vector<uint64_t> text_end(n_files, ~0ULL);  // where the text of file i ends in the stream's text
     uint32_t closed = 0;      // files whose end is known
@@ -1328,10 +1232,7 @@ int frb_scan_gz_batch(frb_ctx* c, const char* const* paths, const uint32_t* ordi
         c->in_file = false;
         cudaStreamSynchronize(c->compute);
         cudaMemsetAsync(&c->st->err_code, 0, sizeof(int), c->compute);
-        while (c->files.size() > files_before) {
-            free_list(c, c->files.back());
-            c->files.pop_back();
-        }
+        while (c->files.size() > files_before) c->files.pop_back();
         std::fill(text_end.begin(), text_end.end(), ~0ULL);
         closed = cur = 0, open = false, first_chunk = true, scanned = 0, file_text_start = 0;
     };
@@ -1378,7 +1279,7 @@ int frb_scan_gz_batch(frb_ctx* c, const char* const* paths, const uint32_t* ordi
         return FRB_OK;
     };
     uint64_t raw = 0;
-    const int rc = gz_device_inflate_source(c, c->gzbuf->b, src, &raw, sink,
+    const int rc = gz_device_inflate_source(c, *c->gzbuf, src, &raw, sink,
                                             [&]() {
                                                 rollback();
                                                 return FRB_OK;
@@ -1402,11 +1303,11 @@ int frb_scan_gz_batch(frb_ctx* c, const char* const* paths, const uint32_t* ordi
 // declined the stream (nothing is written then).
 int frb_gz_inflate(frb_ctx* c, const char* path, void* host_out, uint64_t cap, uint64_t* nbytes, int* used_device) {
     CU(c, cudaSetDevice(c->device));
-    if (!c->gzbuf) c->gzbuf = new GzBuffersHolder();
+    if (!c->gzbuf) c->gzbuf.reset(new GzBuffers());
     uint64_t off = 0, raw = 0;
     *nbytes = 0, *used_device = 0;
     const int rc = gz_device_inflate(
-        c, c->gzbuf->b, path, &raw,
+        c, *c->gzbuf, path, &raw,
         [&](unsigned char* dev, uint64_t n, bool) {
             if (off + n > cap) return fail(c, FRB_ERR_ARG, "frb_gz_inflate: output buffer too small");
             CU(c, cudaMemcpyAsync(static_cast<unsigned char*>(host_out) + off, dev, n, cudaMemcpyDeviceToHost, c->compute));
@@ -1429,13 +1330,12 @@ int frb_gz_open(frb_ctx* c, uint32_t slot, const char* path) {
     CU(c, cudaSetDevice(c->device));
     if (slot >= 2 || !path) return fail(c, FRB_ERR_ARG, "frb_gz_open: slot must be 0 or 1, path not NULL");
     TRY(frb_gz_close(c, slot));
-    if (!c->gzread) c->gzread = new GzReaderSlots();
     std::unique_ptr<GzTextReader> r(new GzTextReader());
     r->src.paths.emplace_back(path);
     const int rc = r->src.open(c);
     if (rc == FRB_ERR_IO) r->declined = true;  // zlib names the problem (FileNotFoundError, ...)
     else TRY(rc);
-    c->gzread->r[slot] = std::move(r);
+    c->gzread[slot] = std::move(r);
     return FRB_OK;
 }
 
@@ -1444,9 +1344,9 @@ int frb_gz_read(frb_ctx* c, uint32_t slot, uint64_t max_bytes, const void** dev_
     CU(c, cudaSetDevice(c->device));
     if (!dev_text || !n || !eof || !declined || !delivered) return fail(c, FRB_ERR_ARG, "frb_gz_read: null output");
     *dev_text = nullptr, *n = 0, *eof = 0, *declined = 0, *delivered = 0;
-    if (slot >= 2 || !c->gzread || !c->gzread->r[slot]) return fail(c, FRB_ERR_STATE, "frb_gz_read: slot %u is not open", slot);
+    if (slot >= 2 || !c->gzread[slot]) return fail(c, FRB_ERR_STATE, "frb_gz_read: slot %u is not open", slot);
     if (max_bytes == 0) return fail(c, FRB_ERR_ARG, "frb_gz_read: max_bytes must be at least 1");
-    GzTextReader& R = *c->gzread->r[slot];
+    GzTextReader& R = *c->gzread[slot];
     if (!R.declined) {
         const unsigned char* text = nullptr;
         bool end = false;
@@ -1472,9 +1372,7 @@ int frb_gz_read(frb_ctx* c, uint32_t slot, uint64_t max_bytes, const void** dev_
 int frb_gz_close(frb_ctx* c, uint32_t slot) {
     CU(c, cudaSetDevice(c->device));
     if (slot >= 2) return fail(c, FRB_ERR_ARG, "frb_gz_close: slot must be 0 or 1");
-    if (!c->gzread || !c->gzread->r[slot]) return FRB_OK;
-    gz_text_free(c, *c->gzread->r[slot]);
-    c->gzread->r[slot].reset();
+    gz_text_free(c, c->gzread[slot]);
     return FRB_OK;
 }
 
@@ -1497,30 +1395,27 @@ int frb_sheet_load2(frb_ctx* c, const uint64_t* fwd, const uint64_t* fwd_hi, con
     for (uint32_t r = 0; r < n_rows; ++r)
         if (group[r] < 0 || static_cast<uint32_t>(group[r]) >= n_rows) return fail(c, FRB_ERR_ARG, "bad group id");
     CU(c, cudaStreamSynchronize(c->compute));
-    cudaFree(c->sheet_fwd), cudaFree(c->sheet_rc), cudaFree(c->sheet_group), cudaFree(c->sheet_use_rc);
-    cudaFree(c->f_sum), cudaFree(c->rc_sum), cudaFree(c->sheet_fwd_hi), cudaFree(c->sheet_rc_hi);
-    c->sheet_fwd = c->sheet_rc = nullptr, c->sheet_group = nullptr, c->sheet_use_rc = nullptr;
-    c->sheet_fwd_hi = c->sheet_rc_hi = nullptr;
-    c->f_sum = c->rc_sum = nullptr;
+    c->sheet = {};  // the old arrays go before the new ones are allocated
+    auto& sh = c->sheet;
     const size_t n = std::max<uint32_t>(n_rows, 1);
-    CU(c, cudaMalloc(&c->sheet_fwd, n * 8));
-    CU(c, cudaMalloc(&c->sheet_rc, n * 8));
-    CU(c, cudaMalloc(&c->sheet_group, n * 4));
-    CU(c, cudaMalloc(&c->sheet_use_rc, n));
-    CU(c, cudaMalloc(&c->f_sum, n * 8));
-    CU(c, cudaMalloc(&c->rc_sum, n * 8));
+    CU(c, sh.fwd.alloc(n));
+    CU(c, sh.rc.alloc(n));
+    CU(c, sh.group.alloc(n));
+    CU(c, sh.use_rc.alloc(n));
+    CU(c, sh.f_sum.alloc(n));
+    CU(c, sh.rc_sum.alloc(n));
     if (c->wide) {
-        CU(c, cudaMalloc(&c->sheet_fwd_hi, n * 8));
-        CU(c, cudaMalloc(&c->sheet_rc_hi, n * 8));
-        CU(c, cudaMemset(c->sheet_fwd_hi, 0, n * 8));
-        CU(c, cudaMemset(c->sheet_rc_hi, 0, n * 8));
-        if (n_rows && fwd_hi) CU(c, cudaMemcpy(c->sheet_fwd_hi, fwd_hi, n_rows * 8, cudaMemcpyHostToDevice));
-        if (n_rows && rc_hi) CU(c, cudaMemcpy(c->sheet_rc_hi, rc_hi, n_rows * 8, cudaMemcpyHostToDevice));
+        CU(c, sh.fwd_hi.alloc(n));
+        CU(c, sh.rc_hi.alloc(n));
+        CU(c, cudaMemset(sh.fwd_hi, 0, n * 8));
+        CU(c, cudaMemset(sh.rc_hi, 0, n * 8));
+        if (n_rows && fwd_hi) CU(c, cudaMemcpy(sh.fwd_hi, fwd_hi, n_rows * 8, cudaMemcpyHostToDevice));
+        if (n_rows && rc_hi) CU(c, cudaMemcpy(sh.rc_hi, rc_hi, n_rows * 8, cudaMemcpyHostToDevice));
     }
     if (n_rows) {
-        CU(c, cudaMemcpy(c->sheet_fwd, fwd, n_rows * 8, cudaMemcpyHostToDevice));
-        CU(c, cudaMemcpy(c->sheet_rc, rc, n_rows * 8, cudaMemcpyHostToDevice));
-        CU(c, cudaMemcpy(c->sheet_group, group, n_rows * 4, cudaMemcpyHostToDevice));
+        CU(c, cudaMemcpy(sh.fwd, fwd, n_rows * 8, cudaMemcpyHostToDevice));
+        CU(c, cudaMemcpy(sh.rc, rc, n_rows * 8, cudaMemcpyHostToDevice));
+        CU(c, cudaMemcpy(sh.group, group, n_rows * 4, cudaMemcpyHostToDevice));
     }
     c->rows = n_rows, c->l1 = l1, c->l2 = l2;
     c->sheet_gen++;
@@ -1532,41 +1427,39 @@ int frb_match(frb_ctx* c, uint32_t n_subs, int rc_mode, const uint8_t* use_rc_ro
               uint64_t* f_sum, uint64_t* rc_sum) {
     CU(c, cudaSetDevice(c->device));
     if (!c->total_ready) return fail(c, FRB_ERR_STATE, "frb_match: no total list (frb_total_finish / frb_total_load)");
-    if (!c->sheet_fwd) return fail(c, FRB_ERR_STATE, "frb_match: no sample sheet loaded");
+    if (!c->sheet.fwd) return fail(c, FRB_ERR_STATE, "frb_match: no sample sheet loaded");
     if (rc_mode && c->l2 == 0) return fail(c, FRB_ERR_ARG, "frb_match: rc_mode needs a dual-index sheet");
     const uint64_t n = c->total.n;
-    if (n > c->match_cap) {
+    auto& mo = c->matcher;
+    if (n > mo.work.size()) {
         CU(c, cudaStreamSynchronize(c->compute));
-        cudaFree(c->m1), cudaFree(c->m2), cudaFree(c->srow), cudaFree(c->m2rc), cudaFree(c->srowrc);
-        cudaFree(c->type), cudaFree(c->typerc), cudaFree(c->work), cudaFree(c->work_n);
-        c->match_cap = 0;
-        CU(c, cudaMalloc(&c->m1, n * 4));
-        CU(c, cudaMalloc(&c->m2, n * 4));
-        CU(c, cudaMalloc(&c->srow, n * 4));
-        CU(c, cudaMalloc(&c->m2rc, n * 4));
-        CU(c, cudaMalloc(&c->srowrc, n * 4));
-        CU(c, cudaMalloc(&c->type, n));
-        CU(c, cudaMalloc(&c->typerc, n));
-        CU(c, cudaMalloc(&c->work, n * 4));
-        CU(c, cudaMalloc(&c->work_n, 8));
-        c->match_cap = n;
+        mo = {};  // the old arrays go before the new ones are allocated
+        CU(c, mo.work_n.alloc(1));
+        CU(c, mo.m1.alloc(n));
+        CU(c, mo.m2.alloc(n));
+        CU(c, mo.srow.alloc(n));
+        CU(c, mo.m2rc.alloc(n));
+        CU(c, mo.srowrc.alloc(n));
+        CU(c, mo.type.alloc(n));
+        CU(c, mo.typerc.alloc(n));
+        CU(c, mo.work.alloc(n));
         c->m1_total_gen = ~0ULL;
     }
     const size_t rows1 = std::max<uint32_t>(c->rows, 1);
     if (use_rc_rows && c->rows)
-        CU(c, cudaMemcpyAsync(c->sheet_use_rc, use_rc_rows, c->rows, cudaMemcpyHostToDevice, c->compute));
-    CU(c, cudaMemsetAsync(c->f_sum, 0, rows1 * 8, c->compute));
-    CU(c, cudaMemsetAsync(c->rc_sum, 0, rows1 * 8, c->compute));
+        CU(c, cudaMemcpyAsync(c->sheet.use_rc, use_rc_rows, c->rows, cudaMemcpyHostToDevice, c->compute));
+    CU(c, cudaMemsetAsync(c->sheet.f_sum, 0, rows1 * 8, c->compute));
+    CU(c, cudaMemsetAsync(c->sheet.rc_sum, 0, rows1 * 8, c->compute));
     if (n) {
         MatchArgs a{};
         a.keys = c->total.keys, a.counts = c->total.counts, a.n = n;
-        a.sheet_fwd = c->sheet_fwd, a.sheet_rc = c->sheet_rc, a.group = c->sheet_group;
-        a.use_rc = use_rc_rows ? c->sheet_use_rc : nullptr;
+        a.sheet_fwd = c->sheet.fwd, a.sheet_rc = c->sheet.rc, a.group = c->sheet.group;
+        a.use_rc = use_rc_rows ? c->sheet.use_rc.get() : nullptr;
         a.rows = c->rows, a.l1 = c->l1, a.l2 = c->l2, a.n_subs = n_subs, a.rc_mode = rc_mode;
-        a.m1 = c->m1, a.m2 = c->m2, a.srow = c->srow, a.type = c->type;
-        a.m2rc = c->m2rc, a.srowrc = c->srowrc, a.typerc = c->typerc;
-        a.f_sum = c->f_sum, a.rc_sum = c->rc_sum, a.st = c->st;
-        a.work = c->work, a.work_n = c->work_n;
+        a.m1 = mo.m1, a.m2 = mo.m2, a.srow = mo.srow, a.type = mo.type;
+        a.m2rc = mo.m2rc, a.srowrc = mo.srowrc, a.typerc = mo.typerc;
+        a.f_sum = c->sheet.f_sum, a.rc_sum = c->sheet.rc_sum, a.st = c->st;
+        a.work = mo.work, a.work_n = mo.work_n;
         // An rc pass tried both orientations of every row, so its idx1 verdicts (and its work list) carry
         // over to any per-row choice of orientation over the same keys / sheet / n (F:618-630).
         const bool reuse = !rc_mode && c->m1_from_rc && c->m1_total_gen == c->total_gen &&
@@ -1575,16 +1468,16 @@ int frb_match(frb_ctx* c, uint32_t n_subs, int rc_mode, const uint8_t* use_rc_ro
         c->m1_from_rc = rc_mode != 0;
         ProfScope ps(c, FRB_K_MATCH);
         if (c->wide) {  // sweeps over the split idx1 / idx2 words (no candidate tables for wide keys)
-            WideMatchArgs w{a, c->total.keys_hi, c->sheet_fwd_hi, c->sheet_rc_hi};
+            WideMatchArgs w{a, c->total.keys_hi, c->sheet.fwd_hi, c->sheet.rc_hi};
             if (!reuse) {
-                CU(c, cudaMemsetAsync(c->work_n, 0, 8, c->compute));
+                CU(c, cudaMemsetAsync(mo.work_n, 0, 8, c->compute));
                 match_idx1_wide_kernel<<<grid_for(n, kMatchThreads, c->sm_count, 8), kMatchThreads,
                                          static_cast<size_t>(c->rows) * 8 + 16, c->compute>>>(w);
                 c->launches++;
             } else {
-                CU(c, cudaMemsetAsync(c->m2, 0xFF, n * 4, c->compute));
-                CU(c, cudaMemsetAsync(c->srow, 0xFF, n * 4, c->compute));
-                CU(c, cudaMemsetAsync(c->type, 0, n, c->compute));
+                CU(c, cudaMemsetAsync(mo.m2, 0xFF, n * 4, c->compute));
+                CU(c, cudaMemsetAsync(mo.srow, 0xFF, n * 4, c->compute));
+                CU(c, cudaMemsetAsync(mo.type, 0, n, c->compute));
             }
             match_wide_kernel<<<grid_for(n, kMatchThreads, c->sm_count, 8), kMatchThreads,
                                 static_cast<size_t>(c->rows) * (5 * 8 + 4) + 16, c->compute>>>(w);
@@ -1598,7 +1491,7 @@ int frb_match(frb_ctx* c, uint32_t n_subs, int rc_mode, const uint8_t* use_rc_ro
         const bool cand = !sweep_only && c->rows > 0 && c->l2 > 0 && parts_usable(c->l1, n_subs, c->rows, slots) &&
                           parts_usable(c->l2, n_subs, c->rows, slots);
         if (!reuse) {
-            CU(c, cudaMemsetAsync(c->work_n, 0, 8, c->compute));
+            CU(c, cudaMemsetAsync(mo.work_n, 0, 8, c->compute));
             if (cand)
                 match_idx1_cand_kernel<<<grid_for(n, kMatchThreads, c->sm_count, 4), kMatchThreads,
                                          cand_bytes(c->rows, parts, slots) + 16, c->compute>>>(a, slots);
@@ -1608,9 +1501,9 @@ int frb_match(frb_ctx* c, uint32_t n_subs, int rc_mode, const uint8_t* use_rc_ro
             c->launches++;
         } else {
             // keys off the work list stay undetermined; m1 is already -1 for them
-            CU(c, cudaMemsetAsync(c->m2, 0xFF, n * 4, c->compute));
-            CU(c, cudaMemsetAsync(c->srow, 0xFF, n * 4, c->compute));
-            CU(c, cudaMemsetAsync(c->type, 0, n, c->compute));
+            CU(c, cudaMemsetAsync(mo.m2, 0xFF, n * 4, c->compute));
+            CU(c, cudaMemsetAsync(mo.srow, 0xFF, n * 4, c->compute));
+            CU(c, cudaMemsetAsync(mo.type, 0, n, c->compute));
         }
         if (cand) {
             const size_t smem = static_cast<size_t>(c->rows) * 24 + 32 + (rc_mode ? 2 : 1) * cand_bytes(c->rows, parts, slots);
@@ -1624,18 +1517,18 @@ int frb_match(frb_ctx* c, uint32_t n_subs, int rc_mode, const uint8_t* use_rc_ro
         }
     }
     if (n) {
-        if (m1_row) CU(c, cudaMemcpyAsync(m1_row, c->m1, n * 4, cudaMemcpyDeviceToHost, c->compute));
-        if (m2_row) CU(c, cudaMemcpyAsync(m2_row, c->m2, n * 4, cudaMemcpyDeviceToHost, c->compute));
-        if (type) CU(c, cudaMemcpyAsync(type, c->type, n, cudaMemcpyDeviceToHost, c->compute));
-        if (sample_row) CU(c, cudaMemcpyAsync(sample_row, c->srow, n * 4, cudaMemcpyDeviceToHost, c->compute));
+        if (m1_row) CU(c, cudaMemcpyAsync(m1_row, mo.m1, n * 4, cudaMemcpyDeviceToHost, c->compute));
+        if (m2_row) CU(c, cudaMemcpyAsync(m2_row, mo.m2, n * 4, cudaMemcpyDeviceToHost, c->compute));
+        if (type) CU(c, cudaMemcpyAsync(type, mo.type, n, cudaMemcpyDeviceToHost, c->compute));
+        if (sample_row) CU(c, cudaMemcpyAsync(sample_row, mo.srow, n * 4, cudaMemcpyDeviceToHost, c->compute));
         if (rc_mode) {
-            if (m2rc_row) CU(c, cudaMemcpyAsync(m2rc_row, c->m2rc, n * 4, cudaMemcpyDeviceToHost, c->compute));
-            if (type_rc) CU(c, cudaMemcpyAsync(type_rc, c->typerc, n, cudaMemcpyDeviceToHost, c->compute));
-            if (sample_rc_row) CU(c, cudaMemcpyAsync(sample_rc_row, c->srowrc, n * 4, cudaMemcpyDeviceToHost, c->compute));
+            if (m2rc_row) CU(c, cudaMemcpyAsync(m2rc_row, mo.m2rc, n * 4, cudaMemcpyDeviceToHost, c->compute));
+            if (type_rc) CU(c, cudaMemcpyAsync(type_rc, mo.typerc, n, cudaMemcpyDeviceToHost, c->compute));
+            if (sample_rc_row) CU(c, cudaMemcpyAsync(sample_rc_row, mo.srowrc, n * 4, cudaMemcpyDeviceToHost, c->compute));
         }
     }
-    if (f_sum && c->rows) CU(c, cudaMemcpyAsync(f_sum, c->f_sum, c->rows * 8, cudaMemcpyDeviceToHost, c->compute));
-    if (rc_sum && c->rows) CU(c, cudaMemcpyAsync(rc_sum, c->rc_sum, c->rows * 8, cudaMemcpyDeviceToHost, c->compute));
+    if (f_sum && c->rows) CU(c, cudaMemcpyAsync(f_sum, c->sheet.f_sum, c->rows * 8, cudaMemcpyDeviceToHost, c->compute));
+    if (rc_sum && c->rows) CU(c, cudaMemcpyAsync(rc_sum, c->sheet.rc_sum, c->rows * 8, cudaMemcpyDeviceToHost, c->compute));
     CU(c, cudaStreamSynchronize(c->compute));
     return device_error_check(c);
 }
@@ -1650,7 +1543,7 @@ int frb_demux_ok(frb_ctx* c, const uint8_t* match, uint32_t n_files, const uint6
     CU(c, cudaSetDevice(c->device));
     if (!c->total_ready) return fail(c, FRB_ERR_STATE, "frb_demux_ok: no total list");
     const uint64_t n = c->total.n;
-    if (n > c->match_cap || c->m1_total_gen != c->total_gen)
+    if (n > c->matcher.work.size() || c->m1_total_gen != c->total_gen)
         return fail(c, FRB_ERR_STATE, "frb_demux_ok: frb_match over the current total list first");
     if (!file_keys && n_files != c->files.size()) return fail(c, FRB_ERR_ARG, "frb_demux_ok: %u files, context holds %zu", n_files, c->files.size());
     if (file_keys && c->wide) return fail(c, FRB_ERR_STATE, "frb_demux_ok: host file lists are not available on a wide (128-bit key) context");
@@ -1658,17 +1551,17 @@ int frb_demux_ok(frb_ctx* c, const uint8_t* match, uint32_t n_files, const uint6
     if (n_files) memset(bad_files_out, 0, n_files);
     if (!n || !n_files) return FRB_OK;
     const size_t classes = 4 + static_cast<size_t>(c->rows);
-    unsigned long long *sorted_keys = nullptr, *sorted_hi = nullptr, *hi_by_lo = nullptr;
-    unsigned *i0 = nullptr, *i1 = nullptr;
-    unsigned char *d_match = nullptr, *d_ok = nullptr, *d_bad = nullptr;
-    int* d_err = nullptr;
-    TRY(dmalloc(c, &sorted_keys, n * 8));
-    TRY(dmalloc(c, &i0, n * 4));
-    TRY(dmalloc(c, &i1, n * 4));
-    TRY(dmalloc(c, &d_match, classes * n_files));
-    TRY(dmalloc(c, &d_ok, n));
-    TRY(dmalloc(c, &d_bad, n_files));
-    TRY(dmalloc(c, &d_err, 4));
+    PoolBuf<unsigned long long> sorted_keys, sorted_hi, hi_by_lo;
+    PoolBuf<unsigned> i0, i1;
+    PoolBuf<unsigned char> d_match, d_ok, d_bad;
+    PoolBuf<int> d_err;
+    CU(c, sorted_keys.alloc(n, c->compute));
+    CU(c, i0.alloc(n, c->compute));
+    CU(c, i1.alloc(n, c->compute));
+    CU(c, d_match.alloc(classes * n_files, c->compute));
+    CU(c, d_ok.alloc(n, c->compute));
+    CU(c, d_bad.alloc(n_files, c->compute));
+    CU(c, d_err.alloc(1, c->compute));
     CU(c, cudaMemcpyAsync(d_match, match, classes * n_files, cudaMemcpyHostToDevice, c->compute));
     CU(c, cudaMemsetAsync(d_ok, 1, n, c->compute));
     CU(c, cudaMemsetAsync(d_bad, 0, n_files, c->compute));
@@ -1677,34 +1570,36 @@ int frb_demux_ok(frb_ctx* c, const uint8_t* match, uint32_t n_files, const uint6
         ProfScope ps(c, FRB_K_EXPORT);
         iota_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(i0, n);
         size_t tmp = 0;
-        CU(c, cub::DeviceRadixSort::SortPairs(nullptr, tmp, c->total.keys, sorted_keys, i0, i1, static_cast<int>(n), 0, 63,
-                                              c->compute));
+        CU(c, cub::DeviceRadixSort::SortPairs(nullptr, tmp, c->total.keys.get(), sorted_keys.get(), i0.get(), i1.get(),
+                                              static_cast<int>(n), 0, 63, c->compute));
         TRY(ensure_cub_tmp(c, tmp));
-        CU(c, cub::DeviceRadixSort::SortPairs(c->cub_tmp, tmp, c->total.keys, sorted_keys, i0, i1, static_cast<int>(n), 0, 63,
-                                              c->compute));
+        CU(c, cub::DeviceRadixSort::SortPairs(c->cub_tmp, tmp, c->total.keys.get(), sorted_keys.get(), i0.get(), i1.get(),
+                                              static_cast<int>(n), 0, 63, c->compute));
         if (c->wide) {
             // second, stable pass on the upper words: sorted by (hi, lo); i1 ends as the permutation of that order
-            TRY(dmalloc(c, &hi_by_lo, n * 8));
-            TRY(dmalloc(c, &sorted_hi, n * 8));
+            CU(c, hi_by_lo.alloc(n, c->compute));
+            CU(c, sorted_hi.alloc(n, c->compute));
             gather1_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(i1, c->total.keys_hi, hi_by_lo, n);
-            CU(c, cub::DeviceRadixSort::SortPairs(nullptr, tmp, hi_by_lo, sorted_hi, i1, i0, static_cast<int>(n), 0, 63, c->compute));
+            CU(c, cub::DeviceRadixSort::SortPairs(nullptr, tmp, hi_by_lo.get(), sorted_hi.get(), i1.get(), i0.get(),
+                                                  static_cast<int>(n), 0, 63, c->compute));
             TRY(ensure_cub_tmp(c, tmp));
-            CU(c, cub::DeviceRadixSort::SortPairs(c->cub_tmp, tmp, hi_by_lo, sorted_hi, i1, i0, static_cast<int>(n), 0, 63, c->compute));
+            CU(c, cub::DeviceRadixSort::SortPairs(c->cub_tmp, tmp, hi_by_lo.get(), sorted_hi.get(), i1.get(), i0.get(),
+                                                  static_cast<int>(n), 0, 63, c->compute));
             std::swap(i0, i1);
             gather1_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(i1, c->total.keys, sorted_keys, n);
             c->launches += 2;
         }
         for (uint32_t f = 0; f < n_files; ++f) {
             const unsigned long long *fk = nullptr, *fc = nullptr, *fk_hi = nullptr;
-            unsigned long long *up_k = nullptr, *up_c = nullptr;
+            PoolBuf<unsigned long long> up_k, up_c;
             uint64_t nf = 0;
             if (file_keys) {
                 nf = file_n[f];
                 if (!nf) continue;
-                TRY(dmalloc(c, &up_k, nf * 8));
+                CU(c, up_k.alloc(nf, c->compute));
                 CU(c, cudaMemcpyAsync(up_k, file_keys[f], nf * 8, cudaMemcpyHostToDevice, c->compute));
                 if (file_counts && file_counts[f]) {
-                    TRY(dmalloc(c, &up_c, nf * 8));
+                    CU(c, up_c.alloc(nf, c->compute));
                     CU(c, cudaMemcpyAsync(up_c, file_counts[f], nf * 8, cudaMemcpyHostToDevice, c->compute));
                 }
                 fk = up_k, fc = up_c;
@@ -1715,11 +1610,9 @@ int frb_demux_ok(frb_ctx* c, const uint8_t* match, uint32_t n_files, const uint6
             }
             const auto demux_ok = c->wide ? demux_ok_kernel<true> : demux_ok_kernel<false>;
             demux_ok<<<static_cast<unsigned>((nf + 255) / 256), 256, 0, c->compute>>>(
-                fk, fc, nf, sorted_keys, i1, n, c->type, c->srow, d_match, n_files, f, d_ok, d_bad, d_err,
+                fk, fc, nf, sorted_keys, i1, n, c->matcher.type, c->matcher.srow, d_match, n_files, f, d_ok, d_bad, d_err,
                 fk_hi, sorted_hi);
             c->launches++;
-            if (up_k) TRY(dfree(c, up_k));
-            if (up_c) TRY(dfree(c, up_c));
         }
         CU(c, cudaGetLastError());
     }
@@ -1729,15 +1622,6 @@ int frb_demux_ok(frb_ctx* c, const uint8_t* match, uint32_t n_files, const uint6
     CU(c, cudaMemcpyAsync(&err_row, d_err, 4, cudaMemcpyDeviceToHost, c->compute));
     CU(c, cudaStreamSynchronize(c->compute));
     if (err_row_out) *err_row_out = err_row == 0x7F7F7F7F ? 0x7FFFFFFF : err_row;
-    TRY(dfree(c, sorted_keys));
-    TRY(dfree(c, sorted_hi));
-    TRY(dfree(c, hi_by_lo));
-    TRY(dfree(c, i0));
-    TRY(dfree(c, i1));
-    TRY(dfree(c, d_match));
-    TRY(dfree(c, d_ok));
-    TRY(dfree(c, d_bad));
-    TRY(dfree(c, d_err));
     return device_error_check(c);
 }
 
@@ -1747,10 +1631,10 @@ int frb_synth_load(frb_ctx* c, uint64_t seed, uint32_t l1, uint32_t l2, uint32_t
                    uint32_t n_t, uint64_t rand_t, uint64_t hop_t) {
     CU(c, cudaSetDevice(c->device));
     if (l1 > 12 || l2 > 12 || n_samples == 0 || lane > 9) return fail(c, FRB_ERR_ARG, "frb_synth_load: bad shape");
-    cudaFree(c->synth_i7), cudaFree(c->synth_i5), cudaFree(c->synth_cdf);
-    CU(c, cudaMalloc(&c->synth_i7, n_samples * 4));
-    CU(c, cudaMalloc(&c->synth_i5, n_samples * 4));
-    CU(c, cudaMalloc(&c->synth_cdf, n_samples * 8));
+    c->synth_ready = false;  // until the new arrays are in place
+    CU(c, c->synth_i7.alloc(n_samples));
+    CU(c, c->synth_i5.alloc(n_samples));
+    CU(c, c->synth_cdf.alloc(n_samples));
     CU(c, cudaMemcpy(c->synth_i7, emit_i7, n_samples * 4, cudaMemcpyHostToDevice));
     CU(c, cudaMemcpy(c->synth_i5, emit_i5, n_samples * 4, cudaMemcpyHostToDevice));
     CU(c, cudaMemcpy(c->synth_cdf, cdf, n_samples * 8, cudaMemcpyHostToDevice));
@@ -1770,20 +1654,18 @@ int frb_synth_generate(frb_ctx* c, uint64_t g0, uint64_t g1, int read_no, void* 
     const uint64_t n = g1 - g0;
     *nbytes = 0;
     if (n == 0) return FRB_OK;
-    if (n > c->synth_cap) {
-        cudaFree(c->synth_len), cudaFree(c->synth_off);
-        c->synth_cap = 0;
-        CU(c, cudaMalloc(&c->synth_len, n * 8));
-        CU(c, cudaMalloc(&c->synth_off, n * 8));
-        c->synth_cap = n;
+    if (n > std::min(c->synth_len.size(), c->synth_off.size())) {
+        c->synth_len.reset(), c->synth_off.reset();
+        CU(c, c->synth_len.alloc(n));
+        CU(c, c->synth_off.alloc(n));
     }
     SynthArgs a = c->synth;
     a.g0 = g0, a.n = n, a.read_no = read_no;
     synth_len_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->compute>>>(a, c->synth_len);
     size_t tmp = 0;
-    CU(c, cub::DeviceScan::ExclusiveSum(nullptr, tmp, c->synth_len, c->synth_off, static_cast<int>(n), c->compute));
+    CU(c, cub::DeviceScan::ExclusiveSum(nullptr, tmp, c->synth_len.get(), c->synth_off.get(), static_cast<int>(n), c->compute));
     TRY(ensure_cub_tmp(c, tmp));
-    CU(c, cub::DeviceScan::ExclusiveSum(c->cub_tmp, tmp, c->synth_len, c->synth_off, static_cast<int>(n), c->compute));
+    CU(c, cub::DeviceScan::ExclusiveSum(c->cub_tmp, tmp, c->synth_len.get(), c->synth_off.get(), static_cast<int>(n), c->compute));
     unsigned long long last_off = 0, last_len = 0;
     CU(c, cudaMemcpyAsync(&last_off, c->synth_off + (n - 1), 8, cudaMemcpyDeviceToHost, c->compute));
     CU(c, cudaMemcpyAsync(&last_len, c->synth_len + (n - 1), 8, cudaMemcpyDeviceToHost, c->compute));
@@ -1834,3 +1716,7 @@ uint64_t frb_launch_count(frb_ctx* c) { return c->launches; }
 #include "frb_route.inl"
 #include "frb_nccl.inl"
 #include "frb_csv.inl"
+
+frb_ctx::~frb_ctx() {
+    for (auto& r : gzread) gz_text_free(this, r);  // their read-ahead threads stop before the buffers go
+}

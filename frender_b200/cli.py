@@ -21,6 +21,7 @@ import numpy as np
 from . import _lib, bgzf
 from .engine import (Context, FrbError, MAX_SYMS as _MAX_SYMS, READ_TYPES, pack_keys, pack_keys2, reverse_complement,
                      unpack_keys)
+from .shard import Ranks, WorkerFailed, assign
 
 STAMP = "%Y-%M-%d_%H%M_%Z"          # sic: minutes where the month should be (F:599, F:912)
 MIN_CHUNK = 1 << 20                  # smallest demux window (bytes per mate)
@@ -191,43 +192,46 @@ class ScanTables:
         return cls(names, (keys, counts), [ctx.file_arrays(i)[:2] for i in range(len(names))], keys_hi)
 
 
+def scan_in_runs(ctx, paths, ordinals, sample):
+    """Scan `paths` (file ordinals `ordinals`) on ctx: a run of small files goes through the device as ONE gzip
+    stream of several members (small_file_run), any other file -- and every file when sampling -- on its own.
+    Yields (index into paths, reads, unique keys) per file, each run's files once the run is done."""
+    k = 0
+    while k < len(paths):
+        run = small_file_run(paths, k) if not sample else 1
+        done = ctx.scan_gz_batch(paths[k:k + run], ordinals[k:k + run]) if run > 1 else None
+        if done is None:
+            done = [ctx.scan_gz(paths[k], ordinals[k], sample)[:2]]
+        for j, (reads, uniq, *_) in enumerate(done):
+            yield k + j, reads, uniq
+        k += len(done)
+
+
+def print_tally(name, reads, uniq):
+    print(f"Tallying barcodes from {name}...found {uniq} new barcode{'' if uniq == 1 else 's'} in {reads} reads.")
+
+
 def _scan_worker(rank, n_ranks, device, ident, jobs, sample, table_log2, conn):
     """One process per GPU (FRENDER_GPUS > 1): scan this rank's files, report, and -- once the parent has heard
     from every rank that its scans went through -- merge the per-rank tables over NCCL and send the per-file
     lists (and, from rank 0, the merged total) to the parent.  A rank that fails never enters the collective,
     and neither does anybody else: the parent only says "go" when all ranks are ready for it.  The rank's own total
     is built before it reports, so that a table too small for the union of its files fails here too."""
-    try:
-        ctx = Context(device, table_log2=table_log2)
-        ctx.nccl_init(ident, rank, n_ranks)
-        ctx.reset()
-        out = []
-        k = 0
-        while k < len(jobs):                    # runs of small files as one stream, like the one-GPU path
-            paths = [path for _, path in jobs]
-            run = small_file_run(paths, k) if not sample else 1
-            done = ctx.scan_gz_batch(paths[k:k + run], [o for o, _ in jobs[k:k + run]]) if run > 1 else None
-            if done is None:
-                done = [ctx.scan_gz(jobs[k][1], jobs[k][0], sample)[:2]]
-            for j, (reads, uniq, *_) in enumerate(done):
-                fk, fc, _ = ctx.file_arrays(k + j)
-                out.append((jobs[k + j][0], reads, uniq, fk, fc))
-            k += len(done)
-        ctx.total_arrays()
-        conn.send(("scanned", None, None))
-        if not conn.recv():                     # another rank failed: no collective
-            return
-        ctx.allmerge()
-        total = ctx.total_arrays()[:2] if rank == 0 else None
-        conn.send(("ok", out, total))
-        ctx.close()
-    except BaseException as exc:            # forwarded: the parent re-raises
-        try:
-            conn.send(("error", repr(exc), None))
-        except OSError:
-            pass
-    finally:
-        conn.close()
+    ctx = Context(device, table_log2=table_log2)
+    ctx.nccl_init(ident, rank, n_ranks)
+    ctx.reset()
+    ordinals, paths = [o for o, _ in jobs], [p for _, p in jobs]
+    out = []
+    for k, reads, uniq in scan_in_runs(ctx, paths, ordinals, sample):
+        fk, fc, _ = ctx.file_arrays(k)
+        out.append((ordinals[k], reads, uniq, fk, fc))
+    ctx.total_arrays()
+    conn.send(("scanned", None))
+    if not conn.recv():                     # another rank failed: no collective
+        return
+    ctx.allmerge()
+    conn.send(("ok", (out, ctx.total_arrays()[:2] if rank == 0 else None)))
+    ctx.close()
 
 
 def scan_files_concurrent(files, sample, streams, device, table_log2, main_ctx):
@@ -284,69 +288,16 @@ def scan_files_concurrent(files, sample, streams, device, table_log2, main_ctx):
 def scan_files_multi_gpu(files, sample, n_gpus, table_log2, worker=_scan_worker):
     """File-level sharding over n_gpus GPUs (SURVEY 8e): file i goes to rank i % n_gpus.  The parent listens to
     all ranks at once (and to their exit): the first failure, or a rank that dies, ends the job with that rank's
-    error instead of leaving the others in a collective that can never complete."""
-    import multiprocessing as mp
-    from multiprocessing.connection import wait
-
-    from .shard import assign
-    mpc = mp.get_context("spawn")
+    error (WorkerFailed) instead of leaving the others in a collective that can never complete."""
     ident = Context.nccl_unique_id()
     jobs = list(enumerate(files))
-    procs, pipes = [], []
-    for rank in range(n_gpus):
-        parent, child = mpc.Pipe(duplex=True)
-        p = mpc.Process(target=worker, args=(rank, n_gpus, rank, ident, assign(jobs, rank, n_gpus), sample,
-                                             table_log2, child))
-        p.start()
-        child.close()
-        procs.append(p)
-        pipes.append(parent)
-
-    def stop_all(message):
-        for conn in pipes:
-            try:
-                conn.send(False)
-            except OSError:
-                pass
-        for p in procs:
-            p.join(timeout=5)
-            if p.is_alive():
-                p.terminate()
-        raise SystemExit(message)
-
-    def collect(expect):
-        """one message of kind `expect` from every rank"""
-        got = {}
-        while len(got) < n_gpus:
-            pending = [r for r in range(n_gpus) if r not in got]
-            ready = wait([pipes[r] for r in pending] + [procs[r].sentinel for r in pending])
-            for r in pending:
-                if pipes[r] in ready:
-                    try:
-                        status, payload, tot = pipes[r].recv()
-                    except EOFError:
-                        stop_all(f"GPU worker {r} exited without a result")
-                    if status != expect:
-                        stop_all(f"GPU worker {r} failed: {payload}")
-                    got[r] = (payload, tot)
-                elif procs[r].sentinel in ready and not pipes[r].poll():
-                    stop_all(f"GPU worker {r} exited without a result")
-        return got
-
-    collect("scanned")
-    for conn in pipes:
-        conn.send(True)
-    results = collect("ok")
-    per_file, total = {}, None
-    for rank in range(n_gpus):
-        payload, tot = results[rank]
-        for ordinal, reads, uniq, fk, fc in payload:
-            per_file[ordinal] = (reads, uniq, fk, fc)
-        if tot is not None:
-            total = tot
-    for p in procs:
-        p.join()
-    return per_file, total
+    with Ranks(worker, [(rank, n_gpus, rank, ident, assign(jobs, rank, n_gpus), sample, table_log2)
+                        for rank in range(n_gpus)]) as ranks:
+        ranks.collect("scanned")
+        ranks.send_all(True)
+        results = ranks.collect("ok")
+    per_file = {ordinal: (reads, uniq, fk, fc) for out, _ in results for ordinal, reads, uniq, fk, fc in out}
+    return per_file, results[0][1]
 
 
 def class_file_matrix(files, sheet_ids, prefix):
@@ -471,34 +422,18 @@ def tally_files(ctx, files, names, sample, cores, n_gpus):
         return tally_files(ctx, files, names, sample, 1, 1)
     if n_gpus > 1:
         per_file, total = scan_files_multi_gpu(files, sample, n_gpus, ctx.table_log2)
-        for ordinal, name in enumerate(names):
-            reads, uniq = per_file[ordinal][:2]
-            print(f"Tallying barcodes from {name}...found {uniq} new barcode{'' if uniq == 1 else 's'} "
-                  f"in {reads} reads.")
-        tables = ScanTables(names, total, [per_file[i][2:] for i in range(len(names))])
-        ctx.load_total_arrays(*total)
     elif cores > 1 and len(files) > 1 and concurrent_streams(cores, files) > 1:
         streams = concurrent_streams(cores, files)
         per_file, total = scan_files_concurrent(files, sample, streams, ctx.device, ctx.table_log2, ctx)
-        for ordinal, name in enumerate(names):
-            reads, uniq = per_file[ordinal][:2]
-            print(f"Tallying barcodes from {name}...found {uniq} new barcode{'' if uniq == 1 else 's'} "
-                  f"in {reads} reads.")
-        tables = ScanTables(names, total, [per_file[i][2:4] for i in range(len(names))])
     else:
-        ordinal = 0
-        while ordinal < len(files):
-            # a run of small files goes through the device as ONE gzip stream of several members
-            run = small_file_run(files, ordinal) if not sample else 1
-            done = ctx.scan_gz_batch(files[ordinal:ordinal + run], ordinal) if run > 1 else None
-            if done is None:
-                done = [ctx.scan_gz(files[ordinal], ordinal, sample)[:2]]
-            for k, (reads, uniq, *_) in enumerate(done):
-                print(f"Tallying barcodes from {names[ordinal + k]}...found {uniq} new barcode{'' if uniq == 1 else 's'} "
-                      f"in {reads} reads.")
-            ordinal += len(done)
-        tables = ScanTables.from_ctx(ctx, names)
-    return tables
+        for k, reads, uniq in scan_in_runs(ctx, files, range(len(files)), sample):
+            print_tally(names[k], reads, uniq)
+        return ScanTables.from_ctx(ctx, names)
+    for ordinal, name in enumerate(names):
+        print_tally(name, *per_file[ordinal][:2])
+    if n_gpus > 1:
+        ctx.load_total_arrays(*total)
+    return ScanTables(names, total, [per_file[i][2:4] for i in range(len(names))])
 
 
 def frender_scan(args, ctx=None):
@@ -554,16 +489,13 @@ def frender_scan(args, ctx=None):
                 ctx.reset()
                 tables = tally_files(ctx, files, names, sample, cores, n_gpus)
                 break
-            except (FrbError, SystemExit) as exc:
-                # a GPU worker of a multi-GPU run reports its error as text (SystemExit)
-                too_long = (isinstance(exc, FrbError) and exc.code == _lib.ERR_KEY_TOO_LONG) or (
-                    isinstance(exc, SystemExit) and "index field longer than 21 symbols" in str(exc))
-                if too_long and not ctx.wide:
+            except (FrbError, WorkerFailed) as exc:
+                code = exc.code if isinstance(exc, FrbError) else exc.frb_code
+                if code == _lib.ERR_KEY_TOO_LONG and not ctx.wide:
                     print("\nindex fields longer than 21 symbols: tallying again with 128-bit keys")
                     ctx.set_wide()
                     continue
-                full = (isinstance(exc, FrbError) and exc.code == _lib.ERR_TABLE_FULL) or "unique-key table full" in str(exc)
-                if not full or ctx.table_log2 + 2 > 32:
+                if code != _lib.ERR_TABLE_FULL or ctx.table_log2 + 2 > 32:
                     raise
                 print(f"\nunique-key tables of 2^{ctx.table_log2} slots are full: tallying again with "
                       f"2^{ctx.table_log2 + 2}")
@@ -771,25 +703,18 @@ class DeviceTextChunks:
 def _demux_worker(rank, device, jobs, opts, out_dir, threads, conn):
     """One process per GPU: the file pairs `jobs` = [(ordinal, r1, r2)], each into its own part directory (r2 is
     None in a single-end run)."""
+    os.environ["FRENDER_DEVICE"] = str(device)
+    os.environ["FRENDER_GPUS"] = "1"
+    os.environ["FRENDER_DEMUX_THREADS"] = str(threads)
+    ctx = Context(device, table_log2=12)
     try:
-        os.environ["FRENDER_DEVICE"] = str(device)
-        os.environ["FRENDER_GPUS"] = "1"
-        os.environ["FRENDER_DEMUX_THREADS"] = str(threads)
-        ctx = Context(device, table_log2=12)
-        try:
-            for ordinal, r1, r2 in jobs:
-                files = [str(p) for p in (r1, r2) if p is not None]
-                ns = argparse.Namespace(**opts, files=files, d=f"{out_dir}.part{ordinal}")
-                frender_demux(ns, ctx=ctx)
-        finally:
-            ctx.close()
-        conn.send(("ok", None))
-    except SystemExit as exc:
-        conn.send(("error", str(exc)))
-    except BaseException as exc:
-        conn.send(("error", repr(exc)))
+        for ordinal, r1, r2 in jobs:
+            files = [str(p) for p in (r1, r2) if p is not None]
+            ns = argparse.Namespace(**opts, files=files, d=f"{out_dir}.part{ordinal}")
+            frender_demux(ns, ctx=ctx)
     finally:
-        conn.close()
+        ctx.close()
+    conn.send(("ok", None))
 
 
 def join_parts(out_path, part_paths, bgzf_parts):
@@ -811,52 +736,23 @@ def demux_pairs_multi_gpu(args, pairs, n_gpus, out_dir, worker=_demux_worker):
     (SURVEY 8e: the demux outputs stay rank-local); the parts of every sink are then appended in pair order --
     gzip members one after the other, so every sink decompresses to exactly what the sequential loop over the
     pairs (F:774) writes.  With FRENDER_GZIP_LEVEL=bgzf the parts' EOF blocks but the last are dropped, and every
-    sink is byte for byte the file the sequential loop writes."""
-    import multiprocessing as mp
+    sink is byte for byte the file the sequential loop writes.  The part directories are removed whether the run
+    succeeds or fails."""
     import shutil
-    from multiprocessing.connection import wait
-
-    from .shard import assign
-    mpc = mp.get_context("spawn")
     opts = {k: getattr(args, k) for k in ("no_index_hop", "no_ambiguous", "no_undeter", "no_samples", "o", "r")}
     jobs = [(i, r1, r2) for i, (r1, r2) in enumerate(pairs)]
     threads = max(2, len(os.sched_getaffinity(0)) // n_gpus)
-    procs, pipes = [], []
-    for rank in range(n_gpus):
-        parent, child = mpc.Pipe(duplex=False)
-        p = mpc.Process(target=worker, args=(rank, rank, assign(jobs, rank, n_gpus), opts, out_dir, threads, child))
-        p.start()
-        child.close()
-        procs.append(p)
-        pipes.append(parent)
-    failure = None
-    pending = set(range(n_gpus))
-    while pending and failure is None:
-        ready = wait([pipes[r] for r in pending] + [procs[r].sentinel for r in pending])
-        for r in list(pending):
-            if pipes[r] in ready or (procs[r].sentinel in ready and pipes[r].poll()):
-                try:
-                    status, payload = pipes[r].recv()
-                except EOFError:
-                    status, payload = "error", "exited without a result"
-                if status != "ok":
-                    failure = f"GPU worker {r} failed: {payload}"
-                pending.discard(r)
-            elif procs[r].sentinel in ready:
-                failure = f"GPU worker {r} exited without a result"
-                pending.discard(r)
-    for p in procs:
-        if failure is not None and p.is_alive():
-            p.terminate()
-        p.join()
-    if failure is not None:
-        raise SystemExit(failure)
     parts = [f"{out_dir}.part{i}" for i in range(len(pairs))]
-    bgzf_parts = gzip_level() == "bgzf"
-    for name in sorted(os.listdir(parts[0])):
-        join_parts(out_dir + name, [os.path.join(part, name) for part in parts], bgzf_parts)
-    for part in parts:
-        shutil.rmtree(part)
+    try:
+        with Ranks(worker, [(rank, rank, assign(jobs, rank, n_gpus), opts, out_dir, threads)
+                            for rank in range(n_gpus)]) as ranks:
+            ranks.collect("ok")
+        bgzf_parts = gzip_level() == "bgzf"
+        for name in sorted(os.listdir(parts[0])):
+            join_parts(out_dir + name, [os.path.join(part, name) for part in parts], bgzf_parts)
+    finally:
+        for part in parts:
+            shutil.rmtree(part, ignore_errors=True)
 
 
 def gzip_level():

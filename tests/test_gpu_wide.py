@@ -355,9 +355,11 @@ def test_cli_wide_scan_takes_one_gpu(lane_12x12, tmp_path, monkeypatch, capsys):
     assert "one GPU, one inflate stream" in capsys.readouterr().out
 
 
-def test_cli_narrow_multi_gpu_worker_too_long_goes_wide(lane_12x12, tmp_path, monkeypatch, capsys):
-    """A multi-GPU worker that reports KEY_TOO_LONG (as text) sends the CLI to 128-bit keys on one GPU."""
+def test_cli_narrow_multi_gpu_worker_key_too_long_code_goes_wide(lane_12x12, tmp_path, monkeypatch, capsys):
+    """A multi-GPU worker that reports KEY_TOO_LONG sends the CLI to 128-bit keys on one GPU."""
+    import frender_b200._lib as L
     import frender_b200.cli as cli
+    from frender_b200.shard import WorkerFailed
     spec, path, _ = lane_12x12
     short = dataclasses.replace(spec, l1=10, l2=10, sheet_i7=spec.sheet_i7[:, :10], sheet_i5=spec.sheet_i5[:, :10])
     (tmp_path / "SampleSheet.csv").write_text(short.sheet_csv())
@@ -368,8 +370,8 @@ def test_cli_narrow_multi_gpu_worker_too_long_goes_wide(lane_12x12, tmp_path, mo
         files.append(str(dst))
 
     def worker_fails(*a, **k):
-        raise SystemExit("GPU worker 0 failed: FrbError('frender_b200 error -5: read 0: index field longer than 21 "
-                         "symbols')")
+        raise WorkerFailed(0, "FrbError('frender_b200 error -5: read 0: index field longer than 21 symbols')",
+                           frb_code=L.ERR_KEY_TOO_LONG)
     monkeypatch.setattr(cli, "scan_files_multi_gpu", worker_fails)
     monkeypatch.setenv("FRENDER_GPUS", "2")
     with pytest.raises(AssertionError):      # the 10+10 sheet against 12+12 keys, F:227

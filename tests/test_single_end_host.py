@@ -120,18 +120,13 @@ def test_single_end_cli_refusals_come_before_any_device_work(tmp_path, monkeypat
 # ---- multi-GPU join ----------------------------------------------------------------------------------------------
 def _stub_single_end_worker(rank, device, jobs, opts, out_dir, threads, conn):
     """Stands in for cli._demux_worker without a GPU: one gzip member per R1 sink and job; jobs carry no R2."""
-    try:
-        for ordinal, r1, r2 in jobs:
-            assert r2 is None
-            os.mkdir(f"{out_dir}.part{ordinal}")
-            for sink in ("S1_frender-demux_R1.fq.gz", "Undetermined_frender-demux_R1.fq.gz"):
-                with open(os.path.join(f"{out_dir}.part{ordinal}", sink), "wb") as fh:
-                    fh.write(gzip.compress(f"{sink}:{ordinal}:{rank}:{os.path.basename(str(r1))}\n".encode()))
-        conn.send(("ok", None))
-    except BaseException as exc:
-        conn.send(("error", repr(exc)))
-    finally:
-        conn.close()
+    for ordinal, r1, r2 in jobs:
+        assert r2 is None
+        os.mkdir(f"{out_dir}.part{ordinal}")
+        for sink in ("S1_frender-demux_R1.fq.gz", "Undetermined_frender-demux_R1.fq.gz"):
+            with open(os.path.join(f"{out_dir}.part{ordinal}", sink), "wb") as fh:
+                fh.write(gzip.compress(f"{sink}:{ordinal}:{rank}:{os.path.basename(str(r1))}\n".encode()))
+    conn.send(("ok", None))
 
 
 def test_multi_gpu_single_end_appends_the_parts_in_file_order(tmp_path):

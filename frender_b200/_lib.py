@@ -86,6 +86,9 @@ SIGNATURES = {
     "frb_route_set_gzip": (C.c_int, [vp, C.c_int]),
     "frb_route_set_gz_format": (C.c_int, [vp, C.c_int]),
     "frb_route_set_mates": (C.c_int, [vp, C.c_int]),
+    "frb_route_set_mates2": (C.c_int, [vp, C.c_int, C.c_int]),
+    "frb_route_pushv": (C.c_int, [vp, vp, vp, C.c_int]),
+    "frb_route_popv": (C.c_int, [vp, vp, vp, P(u64), vp, P(u64)]),
     "frb_nccl_unique_id": (C.c_int, [C.c_char_p]),
     "frb_nccl_init": (C.c_int, [vp, C.c_char_p, C.c_int, C.c_int]),
     "frb_allmerge": (C.c_int, [vp, P(u64)]),

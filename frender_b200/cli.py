@@ -167,6 +167,56 @@ def single_end():
     return os.environ.get("FRENDER_SINGLE_END", "0").strip() not in ("", "0")
 
 
+INDEX_READS = ("I1", "I2")
+
+
+def index_reads():
+    """FRENDER_INDEX_READS: set (and not 0), frender demux also routes every R1's index-read files (I1 / I2)."""
+    return os.environ.get("FRENDER_INDEX_READS", "0").strip() not in ("", "0")
+
+
+def get_index_files(files):
+    """FRENDER_INDEX_READS=1: (the inputs without their index-read files, the kinds of index file of the run, and
+    {R1: [its index files in I1, I2 order]}).  Index-read files are the inputs whose name ends in _I1_ or _I2_, a
+    three-digit number and the fastq.gz suffix (Illumina's _I1_001.fastq.gz); an R1's index files are the ones beside
+    it whose name is the R1's with its last _R1_ replaced by _I1_ or _I2_.  Every R1 must have the same kinds, so
+    that the run has one set of sinks; an R1 that lacks one, an index file without an R1 and an input without any
+    index file are refused."""
+    # Illumina index-read names end in _I1_001.fastq.gz / _I2_001.fastq.gz: a sample name holding "_I1_" is no index
+    index = [p for p in files if re.search(r"_I[12]_\d{3}\.f[ast]*q\.gz$", os.path.basename(str(p)), re.I)]
+    if not index:
+        raise SystemExit("FRENDER_INDEX_READS=1: no index read file (a name ending in _I1_001.fastq.gz or "
+                         "_I2_001.fastq.gz) among the inputs")
+    rest = [p for p in files if p not in index]
+    found, wanted = {}, {}
+    for r1 in (p for p in rest if re.search("_R1_", str(p), re.I)):
+        r1 = Path(r1)
+        wanted[r1] = {k: r1.with_name(re.sub("_R1_(?!.*_R1_)", f"_{k}_", r1.name, flags=re.I)) for k in INDEX_READS}
+        found[r1] = {k: p for k, p in wanted[r1].items() if p in index}
+    claimed = {p for have in found.values() for p in have.values()}
+    for p in index:
+        if Path(p) not in claimed:
+            raise SystemExit(f"FRENDER_INDEX_READS=1: index read file {p} has no read 1 file")
+    kinds = [k for k in INDEX_READS if any(k in have for have in found.values())]
+    for r1, have in found.items():
+        for k in kinds:
+            if k not in have:
+                raise SystemExit(f"FRENDER_INDEX_READS=1: {r1} has no {k} file ({wanted[r1][k].name}), which other "
+                                 "read 1 files have")
+    return rest, kinds, {r1: [have[k] for k in kinds] for r1, have in found.items()}
+
+
+def demux_lanes(inputs, single, indexed):
+    """The files frender demux routes together, one tuple per lane: (R1, R2 or None, index files...), and the read
+    names of the tuple's files that are there ("R1", "R2", "I1", "I2")."""
+    kinds, index_of = [], {}
+    if indexed:
+        inputs, kinds, index_of = get_index_files(inputs)
+    pairs = [(r1, None) for r1 in get_single_end_files(inputs)] if single else get_paired_files(inputs)
+    lanes = [(r1, r2, *index_of[Path(r1)]) for r1, r2 in pairs] if indexed else pairs
+    return lanes, ["R1"] + ([] if single else ["R2"]) + kinds
+
+
 # ---------------------------------------------------------------------------------------------
 # scan (F:567-642)
 # ---------------------------------------------------------------------------------------------
@@ -701,15 +751,15 @@ class DeviceTextChunks:
 
 
 def _demux_worker(rank, device, jobs, opts, out_dir, threads, conn):
-    """One process per GPU: the file pairs `jobs` = [(ordinal, r1, r2)], each into its own part directory (r2 is
-    None in a single-end run)."""
+    """One process per GPU: the file pairs `jobs` = [(ordinal, r1, r2, index files...)], each into its own part
+    directory (r2 is None in a single-end run; index files come with FRENDER_INDEX_READS=1)."""
     os.environ["FRENDER_DEVICE"] = str(device)
     os.environ["FRENDER_GPUS"] = "1"
     os.environ["FRENDER_DEMUX_THREADS"] = str(threads)
     ctx = Context(device, table_log2=12)
     try:
-        for ordinal, r1, r2 in jobs:
-            files = [str(p) for p in (r1, r2) if p is not None]
+        for ordinal, r1, r2, *index in jobs:
+            files = [str(p) for p in (r1, r2, *index) if p is not None]
             ns = argparse.Namespace(**opts, files=files, d=f"{out_dir}.part{ordinal}")
             frender_demux(ns, ctx=ctx)
     finally:
@@ -731,8 +781,9 @@ def join_parts(out_path, part_paths, bgzf_parts):
 
 
 def demux_pairs_multi_gpu(args, pairs, n_gpus, out_dir, worker=_demux_worker):
-    """FRENDER_GPUS=N with several R1/R2 pairs (lanes), or R1 files of a single-end run as (R1, None) pairs: pair i
-    is routed on GPU i % N into rank-local part files
+    """FRENDER_GPUS=N with several R1/R2 pairs (lanes), or R1 files of a single-end run as (R1, None) pairs, each
+    followed by its index-read files with FRENDER_INDEX_READS=1: pair i is routed on GPU i % N into rank-local part
+    files
     (SURVEY 8e: the demux outputs stay rank-local); the parts of every sink are then appended in pair order --
     gzip members one after the other, so every sink decompresses to exactly what the sequential loop over the
     pairs (F:774) writes.  With FRENDER_GZIP_LEVEL=bgzf the parts' EOF blocks but the last are dropped, and every
@@ -740,7 +791,7 @@ def demux_pairs_multi_gpu(args, pairs, n_gpus, out_dir, worker=_demux_worker):
     succeeds or fails."""
     import shutil
     opts = {k: getattr(args, k) for k in ("no_index_hop", "no_ambiguous", "no_undeter", "no_samples", "o", "r")}
-    jobs = [(i, r1, r2) for i, (r1, r2) in enumerate(pairs)]
+    jobs = [(i, *pair) for i, pair in enumerate(pairs)]
     threads = max(2, len(os.sched_getaffinity(0)) // n_gpus)
     parts = [f"{out_dir}.part{i}" for i in range(len(pairs))]
     try:
@@ -786,8 +837,8 @@ def frender_demux(args, ctx=None):
         files = {"file": [Path(f) for f in args.files]}
     single = single_end()
     inputs = parse_files(files, just_r1=False)
-    # single-end: R1 files alone, as (R1, None) pairs
-    pairs = [(r1, None) for r1 in get_single_end_files(inputs)] if single else get_paired_files(inputs)
+    # single-end: R1 files alone, as (R1, None) pairs; with index reads every pair is followed by its I1 / I2 files
+    pairs, reads = demux_lanes(inputs, single, index_reads())
 
     out_dir = args.d if args.d.endswith("/") else args.d + "/"
     os.mkdir(args.d)                                                            # FileExistsError as in F:755
@@ -808,7 +859,6 @@ def frender_demux(args, ctx=None):
     hop_sink = open_sink("Index-hop") if index_hop else undeter_sink
     amb_sink = open_sink("Ambiguous") if ambiguous else undeter_sink
     sink_file = (MemberSink if gpu_gzip else BgzfSink if gpu_bgzf else (lambda path: GzSink(path, level)))
-    reads = ("R1",) if single else ("R1", "R2")
     sinks = [{r: sink_file(f"{out_dir}{name}_frender-demux_{infix}{r}.fq.gz") for r in reads} for name in sink_names]
     n_sinks = len(sink_names)
     reject = n_sinks                                                            # "Unrecognized read type" bucket
@@ -852,15 +902,14 @@ def frender_demux(args, ctx=None):
         writes.clear()
 
     def write_out(popped):
-        o1, o2, off1, off2 = popped[:4]
-        if off1[reject + 1] > off1[reject]:
+        outs, offs = popped[:2]
+        if offs[0][reject + 1] > offs[0][reject]:
             raise SystemExit("Unrecognized read type found in supplied frender result file!")
         drain()                                     # a sink's compress() calls stay in order
         for s in range(n_sinks):
-            if off1[s + 1] > off1[s]:
-                writes.append(pool.submit(sinks[s]["R1"].write, o1[off1[s]:off1[s + 1]]))
-            if off2[s + 1] > off2[s]:
-                writes.append(pool.submit(sinks[s]["R2"].write, o2[off2[s]:off2[s + 1]]))
+            for read, out, off in zip(reads, outs, offs):
+                if off[s + 1] > off[s]:
+                    writes.append(pool.submit(sinks[s][read].write, out[off[s]:off[s + 1]]))
 
     mates = []
 
@@ -868,39 +917,49 @@ def frender_demux(args, ctx=None):
         """The next piece of every mate: host mates on the pool, device mates in this thread (a context is not
         thread-safe)."""
         jobs = [(m, 0 if m.eof else w) for m, w in zip(mates, want)]
-        futures = [None if getattr(m, "on_device", False) else pool.submit(m.read, n) for m, n in jobs]
-        got = [m.read(n) if f is None else None for (m, n), f in zip(jobs, futures)]
+        idle = [not m.eof and n == 0 for m, n in jobs]          # an index mate that is far enough ahead
+        futures = [None if getattr(m, "on_device", False) or i else pool.submit(m.read, n)
+                   for (m, n), i in zip(jobs, idle)]
+        got = [b"" if i else m.read(n) if f is None else None for (m, n), f, i in zip(jobs, futures, idle)]
         return [g if f is None else f.result() for g, f in zip(got, futures)]
 
     try:
         ctx.route_load(keys, routes, n_sinks + 1, keys_hi)
         ctx.route_gzip(gpu_gzip or gpu_bgzf, bgzf=gpu_bgzf)
-        ctx.route_mates(1 if single else 2)
-        for r1_path, r2_path in pairs:
-            print(f"Demultiplexing {r1_path.name}...")
-            # The pair as a STREAM of chunks, two in flight: while chunk k is routed on the device and chunk k-1
+        # the keys come from R2's headers, or from R1's in a single-end run; index reads follow as mates 3 and 4
+        ctx.route_mates(len(reads), key_mate=0 if single else 1)
+        for lane in pairs:
+            print(f"Demultiplexing {lane[0].name}...")
+            # The lane as a STREAM of chunks, two in flight: while chunk k is routed on the device and chunk k-1
             # comes back and is deflated, chunk k+1 is inflated.  Chunks are cut anywhere; records that are not
-            # complete yet (and the lead of one mate over the other) are carried on the device.  A single-end
-            # stream is the same with R1 alone (mate slot 0).
-            paths = [p for p in (r1_path, r2_path) if p is not None]
+            # complete yet (and the lead of one mate over another) are carried on the device.  Mate m reads into
+            # span-reader slot m: R1, R2 (absent when single-end), then the index reads.
+            paths = [p for p in lane if p is not None]
             mates[:] = [DeviceTextChunks(ctx, m, p) if device_inflate else TextChunks(p) for m, p in enumerate(paths)]
             ctx.route_reset(chunk)
-            flags, carry, over = [], (0, 0), False
+            flags, sizes, carry, over = [], [], [0] * len(mates), False
             while not over:
-                # carry + new bytes stay within the window
-                got = fill([max(chunk - c, MIN_CHUNK // 4) for c in carry[:len(mates)]])
+                # carry + new bytes stay within the window.  An index record is several times shorter than a read
+                # record, so an index mate given the same bytes would run ahead of its reads by more than the carry
+                # area holds: it reads only what keeps its bytes not yet routed, the chunk in flight included,
+                # within the window.
+                ahead = [sum(s[m] for s in sizes) for m in range(len(mates))]
+                got = fill([max(chunk - c, MIN_CHUNK // 4) if read in ("R1", "R2") else max(chunk - c - a, 0)
+                            for read, c, a in zip(reads, carry, ahead)])
                 flags.append(sum(1 << m for m, reader in enumerate(mates) if reader.eof))
-                ctx.route_push(got[0], got[1] if len(got) > 1 else None, flags[-1])
+                sizes.append([len(g) for g in got])
+                ctx.route_pushv(got, flags[-1])
                 over = all(reader.eof for reader in mates)
                 if len(flags) == 2:
-                    popped, was = ctx.route_pop(), flags.pop(0)
+                    popped, was = ctx.route_popv(), flags.pop(0)
+                    sizes.pop(0)
                     write_out(popped)
-                    carry = popped[5:7]
+                    carry = popped[3]
                     # zip() ends with the shorter mate (F:777): that file is over and nothing of it is left on
                     # the device (which ignores the chunk that is already queued behind this one)
                     over = over or any(was >> m & 1 and carry[m] == 0 for m in range(len(mates)))
             for _ in flags:
-                write_out(ctx.route_pop())
+                write_out(ctx.route_popv())
     except FrbError as exc:
         if exc.code == _lib.ERR_KEY_NOT_FOUND:
             raise SystemExit(exc.message)

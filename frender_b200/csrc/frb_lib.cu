@@ -128,13 +128,14 @@ struct frb_ctx {
     uint32_t n_sinks = 0;
     std::unique_ptr<RouteStream> route;  // the demux stream (frb_route.inl)
     int route_gz = FRB_GZ_FORMAT_PLAIN;         // the demux stream returns gzip members / BGZF blocks (frb_route_set_gz_format)
-    int route_mates = 2;                        // 1: single-end demux stream, R1 alone (frb_route_set_mates)
+    int route_mates = 2;                        // mates of the demux stream: 1 single-end, 3 / 4 with index reads (frb_route_set_mates2)
+    int route_key_mate = 1;                     // the mate whose headers give the keys: R2, or R1 when single-end
     // device gzip writer of frb_gz_deflate (frb_deflate.inl)
     std::unique_ptr<DeflateBuffers> deflate;
     // device inflate (frb_gz.inl)
     std::unique_ptr<GzBuffers> gzbuf;
-    // span readers of frb_gz_open / frb_gz_read, one per mate (frb_gz.inl)
-    std::unique_ptr<GzTextReader> gzread[2];
+    // span readers of frb_gz_open / frb_gz_read, one per mate: R1, R2, I1, I2 (frb_gz.inl)
+    std::unique_ptr<GzTextReader> gzread[4];
     // synth
     SynthArgs synth{};
     DevBuf<unsigned> synth_i7, synth_i5;
@@ -1328,7 +1329,7 @@ int frb_gz_inflate(frb_ctx* c, const char* path, void* host_out, uint64_t cap, u
 // Span readers (GzTextReader, frb_gz.inl): the text of a .gz file in device memory, in spans of an exact size.
 int frb_gz_open(frb_ctx* c, uint32_t slot, const char* path) {
     CU(c, cudaSetDevice(c->device));
-    if (slot >= 2 || !path) return fail(c, FRB_ERR_ARG, "frb_gz_open: slot must be 0 or 1, path not NULL");
+    if (slot >= 4 || !path) return fail(c, FRB_ERR_ARG, "frb_gz_open: slot must be 0 to 3, path not NULL");
     TRY(frb_gz_close(c, slot));
     std::unique_ptr<GzTextReader> r(new GzTextReader());
     r->src.paths.emplace_back(path);
@@ -1344,7 +1345,7 @@ int frb_gz_read(frb_ctx* c, uint32_t slot, uint64_t max_bytes, const void** dev_
     CU(c, cudaSetDevice(c->device));
     if (!dev_text || !n || !eof || !declined || !delivered) return fail(c, FRB_ERR_ARG, "frb_gz_read: null output");
     *dev_text = nullptr, *n = 0, *eof = 0, *declined = 0, *delivered = 0;
-    if (slot >= 2 || !c->gzread[slot]) return fail(c, FRB_ERR_STATE, "frb_gz_read: slot %u is not open", slot);
+    if (slot >= 4 || !c->gzread[slot]) return fail(c, FRB_ERR_STATE, "frb_gz_read: slot %u is not open", slot);
     if (max_bytes == 0) return fail(c, FRB_ERR_ARG, "frb_gz_read: max_bytes must be at least 1");
     GzTextReader& R = *c->gzread[slot];
     if (!R.declined) {
@@ -1371,7 +1372,7 @@ int frb_gz_read(frb_ctx* c, uint32_t slot, uint64_t max_bytes, const void** dev_
 
 int frb_gz_close(frb_ctx* c, uint32_t slot) {
     CU(c, cudaSetDevice(c->device));
-    if (slot >= 2) return fail(c, FRB_ERR_ARG, "frb_gz_close: slot must be 0 or 1");
+    if (slot >= 4) return fail(c, FRB_ERR_ARG, "frb_gz_close: slot must be 0 to 3");
     gz_text_free(c, c->gzread[slot]);
     return FRB_OK;
 }

@@ -1,6 +1,6 @@
 // Hot path C: demux record router (reference loop F:774-810, write_reads F:726-730, grouper F:719-723).
 //
-// A STREAM of chunk pairs (R1 bytes, R2 bytes, cut anywhere) goes through the device without a host round trip
+// A STREAM of chunks (R1 bytes, R2 bytes, ..., cut anywhere) goes through the device without a host round trip
 // in between:
 //   scan_ws_kernel (general form) on R2: key of every record under the demux rule (F:778) + record offsets;
 //   on R1: record offsets only.  A record that is not complete yet (and the surplus records of the mate that
@@ -18,29 +18,47 @@
 // re-reads the chunk, which is still in L2).
 // A single-end stream (Mates = 1, frb_route_set_mates) is the same with R1 alone: the parser takes the keys from the
 // R1 headers, the routed records are R1's complete records (no zip), the scan runs on a (S, 1) grid and the copy,
-// the carry and the deflate on R1 only -- 2 x R1 algorithmic bytes.  Nothing here depends on a host-side count: grids are sized by
-// capacity and the kernels take the record counts from device memory.
+// the carry and the deflate on R1 only -- 2 x R1 algorithmic bytes.
+// Index reads (frb_route_set_mates2, Mates = 3 or 4) add the I1 / I2 files as more mates behind R1 (and R2): the key
+// still comes from one mate (R2, or R1 in a single-end stream), every other mate is parsed for record offsets only,
+// and record i of every mate goes to the sink of record i's key.  The zip() runs over all Mates files; the scan runs
+// on a (S, Mates) grid, the carry on (64, Mates), the copy and the deflate once per mate.  Nothing here depends on a
+// host-side count: grids are sized by capacity and the kernels take the record counts from device memory.
 #pragma once
 #include "common.cuh"
 
 namespace frb {
 
 constexpr int kRouteBlock = 256;                    // records per histogram block
+constexpr int kRouteMaxMates = 4;                   // R1, R2, I1, I2
+// Shared memory a block may have on sm_90 / sm_100 (the opt-in limit): the histogram keeps [Mates][n_sinks] u32
+// counters in it, so a stream of m mates takes at most kRouteSmemMax / (4 m) sinks (14,528 at 4 mates).
+constexpr unsigned kRouteSmemMax = 227u << 10;
 
-// Device-resident state of the stream (one per context; the `out` part is copied to the host per chunk).
+// Device-resident state of the stream (one per context; copied to the host per chunk).  Per-mate arrays: mate m is
+// the m-th buffer of frb_route_pushv (R1, R2, then the index reads).
 struct RouteState {
     // carried into the next chunk
-    unsigned long long skip1, skip2;      // where the text begins in the next chunk's buffers (carry area - carry)
+    unsigned long long skip[kRouteMaxMates];   // where the text begins in the next chunk's buffers (carry area - carry)
     // this chunk
-    unsigned long long n1, n2;            // records parsed (a trailing partial one included)
-    unsigned long long lines1, lines2;    // lines parsed
-    unsigned long long pairs;             // records routed
-    unsigned long long used1, used2;      // end of the routed records in the chunk buffers (buffer offsets)
-    unsigned long long out1, out2;        // bytes written to the sinks, per mate
-    unsigned long long bad;               // smallest record with a key the results table does not hold (~0: none)
+    unsigned long long n[kRouteMaxMates];      // records parsed (a trailing partial one included)
+    unsigned long long lines[kRouteMaxMates];  // lines parsed
+    unsigned long long pairs;                  // records routed (of every mate)
+    unsigned long long used[kRouteMaxMates];   // end of the routed records in the chunk buffers (buffer offsets)
+    unsigned long long out[kRouteMaxMates];    // bytes written to the sinks, per mate
+    unsigned long long bad;                    // smallest record with a key the results table does not hold (~0: none)
     unsigned long long bad_key;
-    int error;                            // FRB_ERR_* raised by the plan (a record longer than the carry area)
-    int done;                             // one mate has ended and is used up: zip() is over, later chunks are ignored
+    int error;                                 // FRB_ERR_* raised by the plan (a record longer than the carry area)
+    int done;                                  // one mate has ended and is used up: zip() is over, later chunks are ignored
+};
+
+// Per-mate device pointers and sizes of one chunk, passed by value (mates >= Mates are not read).
+struct RouteMates {
+    unsigned long long* off[kRouteMaxMates];   // record offsets (rec_cap + 1 each)
+    unsigned* local[kRouteMaxMates];           // offset of every record inside its (block, sink) cell
+    const unsigned char* in[kRouteMaxMates];   // the chunk buffers: [carry area | new bytes]
+    unsigned char* next[kRouteMaxMates];       // the next chunk's buffers (the carry goes there)
+    unsigned long long end[kRouteMaxMates];    // bytes in the chunk buffers (carry area included)
 };
 
 // results-table build: key -> sink id stored in the slot's `count` (keys are unique: the host keeps the last CSV row
@@ -69,21 +87,18 @@ __global__ void __launch_bounds__(256) route_build_kernel(Slot* table, unsigned 
 }
 
 // The parser left n_reads / line_carry of the mate it just scanned in DevState: move them into the stream state
-// and clear them for the next launch.  which = 1 / 2.
-__global__ void route_grab_kernel(DevState* st, RouteState* rs, int which) {
+// and clear them for the next launch.
+__global__ void route_grab_kernel(DevState* st, RouteState* rs, int mate) {
     if (threadIdx.x || blockIdx.x) return;
-    if (which == 2) rs->n2 = st->n_reads, rs->lines2 = st->line_carry;
-    else rs->n1 = st->n_reads, rs->lines1 = st->line_carry;
+    rs->n[mate] = st->n_reads, rs->lines[mate] = st->line_carry;
     st->n_reads = 0, st->line_carry = 0;
 }
 
-// pairs, bytes used, and the terminators of the offset lists.  end1 / end2 = bytes in the chunk buffers;
-// final bit 0 / 1: the R1 / R2 stream ends with this chunk.  Mates = 1 (single-end): R1 alone, its complete records
-// are routed (a trailing partial one once bit 0 is set); off2 / in2 / end2 are not read.
+// pairs, bytes used, and the terminators of the offset lists.  m.end[k] = bytes in the chunk buffers of mate k;
+// final bit k: mate k's file ends with this chunk.  The routed records are the ones every mate has complete (the
+// zip() of the 4-line groupers, F:777, over Mates files; Mates = 1: R1's complete records).
 template <int Mates>
-__global__ void route_plan_kernel(RouteState* rs, DevState* st, unsigned long long* off1, unsigned long long* off2,
-                                  const unsigned char* __restrict__ in1, const unsigned char* __restrict__ in2,
-                                  unsigned long long end1, unsigned long long end2, int final_chunk,
+__global__ void route_plan_kernel(RouteState* rs, DevState* st, RouteMates m, int final_chunk,
                                   unsigned long long rec_cap, unsigned long long carry_cap, unsigned long long* tot,
                                   unsigned n_tot) {
     for (unsigned k = threadIdx.x; k < n_tot; k += blockDim.x) tot[k] = 0;  // per-sink bytes, summed by the histogram
@@ -92,7 +107,8 @@ __global__ void route_plan_kernel(RouteState* rs, DevState* st, unsigned long lo
     if (rs->done) {  // chunks the host had already queued when the shorter mate ran out
         st->err_code = 0;
         rs->pairs = 0;
-        rs->used1 = end1, rs->used2 = end2;
+#pragma unroll
+        for (int k = 0; k < Mates; ++k) rs->used[k] = m.end[k];
         return;
     }
     if (st->err_code) {  // raised by the parser (a key outside the alphabet, ...)
@@ -102,48 +118,53 @@ __global__ void route_plan_kernel(RouteState* rs, DevState* st, unsigned long lo
         rs->pairs = 0;
         return;
     }
-    if (rs->n1 > rec_cap || (Mates == 2 && rs->n2 > rec_cap)) {
-        rs->error = FRB_ERR_ARG;  // records shorter than 16 bytes
-        rs->pairs = 0;
-        return;
-    }
-    off1[rs->n1] = end1;
-    if constexpr (Mates == 2) off2[rs->n2] = end2;
+#pragma unroll
+    for (int k = 0; k < Mates; ++k)
+        if (rs->n[k] > rec_cap) {
+            rs->error = FRB_ERR_ARG;  // records shorter than 16 bytes
+            rs->pairs = 0;
+            return;
+        }
     // zip() of the 4-line groupers stops at the shorter mate (F:777); a trailing partial record only exists at the
     // end of a file (F:719-723)
     // (the parser counts a last line without '\n' as a line; before the end of the file it is not complete)
-    const unsigned long long open1 = (end1 > rs->skip1 && in1[end1 - 1] != '\n') ? 1 : 0;
-    const unsigned long long open2 = (Mates == 2 && end2 > rs->skip2 && in2[end2 - 1] != '\n') ? 1 : 0;
-    const unsigned long long e1 = (final_chunk & 1) ? rs->n1 : (rs->lines1 - open1) / 4;
-    const unsigned long long e2 = Mates == 1 ? ~0ull : (final_chunk & 2) ? rs->n2 : (rs->lines2 - open2) / 4;
-    const unsigned long long n = e1 < e2 ? e1 : e2;
-    rs->pairs = n;
-    rs->used1 = n ? off1[n] : rs->skip1;
-    rs->used2 = Mates == 1 ? end2 : n ? off2[n] : rs->skip2;
-    rs->bad = ~0ull;
-    // a mate that has ended and is used up ends the stream (F:777): what the other one still holds is never read
-    if (((final_chunk & 1) && n == rs->n1) || (Mates == 2 && (final_chunk & 2) && n == rs->n2)) {
-        rs->done = 1;
-        rs->used1 = end1, rs->used2 = end2;
+    unsigned long long n = ~0ull;
+#pragma unroll
+    for (int k = 0; k < Mates; ++k) {
+        m.off[k][rs->n[k]] = m.end[k];
+        const unsigned long long open = (m.end[k] > rs->skip[k] && m.in[k][m.end[k] - 1] != '\n') ? 1 : 0;
+        const unsigned long long e = (final_chunk >> k & 1) ? rs->n[k] : (rs->lines[k] - open) / 4;
+        n = e < n ? e : n;
     }
-    if (end1 - rs->used1 > carry_cap || end2 - rs->used2 > carry_cap) rs->error = FRB_ERR_ARG;
+    rs->pairs = n;
+    rs->bad = ~0ull;
+    // a mate that has ended and is used up ends the stream (F:777): what the others still hold is never read
+    bool over = false;
+#pragma unroll
+    for (int k = 0; k < Mates; ++k) {
+        rs->used[k] = n ? m.off[k][n] : rs->skip[k];
+        over = over || ((final_chunk >> k & 1) && n == rs->n[k]);
+    }
+    if (over) rs->done = 1;
+#pragma unroll
+    for (int k = 0; k < Mates; ++k) {
+        if (over) rs->used[k] = m.end[k];
+        if (m.end[k] - rs->used[k] > carry_cap) rs->error = FRB_ERR_ARG;
+    }
 }
 
-// sink of every record, its offset inside its (block, sink) cell, and the cells' sizes.  cell[(s * n_blocks + b)]
-// for mate 1, the same + n_sinks * n_blocks for mate 2 (Mates = 2 only).  One warp-step after the other inside a
-// block, so that records of one sink keep their order.  key2: the keys of the routed records (parsed from R2, or
-// from R1 when Mates = 1); key2_hi: their upper words (wide only).
+// sink of every record, its offset inside its (block, sink) cell, and the cells' sizes.  cell[(k * n_sinks + s) *
+// n_blocks + b] for mate k.  One warp-step after the other inside a block, so that records of one sink keep their
+// order.  key: the keys of the routed records (parsed from the key mate's headers: R2, or R1 in a single-end stream);
+// key_hi: their upper words (wide only).
 template <bool Wide, int Mates>
 __global__ void __launch_bounds__(kRouteBlock) route_hist_kernel(const Slot* __restrict__ table, unsigned long long mask,
-                                                                 const unsigned long long* __restrict__ key2,
-                                                                 const unsigned long long* __restrict__ off1,
-                                                                 const unsigned long long* __restrict__ off2,
-                                                                 RouteState* rs, unsigned n_sinks, unsigned n_blocks,
-                                                                 unsigned* __restrict__ sink, unsigned* __restrict__ local1,
-                                                                 unsigned* __restrict__ local2,
+                                                                 const unsigned long long* __restrict__ key,
+                                                                 const RouteMates m, RouteState* rs, unsigned n_sinks,
+                                                                 unsigned n_blocks, unsigned* __restrict__ sink,
                                                                  unsigned long long* __restrict__ cell,
                                                                  unsigned long long* __restrict__ tot,
-                                                                 const unsigned long long* __restrict__ key2_hi) {
+                                                                 const unsigned long long* __restrict__ key_hi) {
     using K = KeyWidth<Wide>;
     const typename K::Slot* __restrict__ const tab = reinterpret_cast<const typename K::Slot*>(table);
     extern __shared__ unsigned s_acc[];  // [Mates][n_sinks]
@@ -154,25 +175,27 @@ __global__ void __launch_bounds__(kRouteBlock) route_hist_kernel(const Slot* __r
     __syncthreads();
     const unsigned long long i = static_cast<unsigned long long>(b) * kRouteBlock + threadIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    unsigned s = 0xFFFFFFFFu, l1 = 0, l2 = 0;
+    unsigned s = 0xFFFFFFFFu, len[Mates];
+#pragma unroll
+    for (int k = 0; k < Mates; ++k) len[k] = 0;
     if (i < n) {
-        const auto key = K::at(key2, key2_hi, i);
-        unsigned long long h = K::hash(key) & mask;
+        const auto k = K::at(key, key_hi, i);
+        unsigned long long h = K::hash(k) & mask;
         for (unsigned probe = 0; probe < kMaxProbe; ++probe) {
-            const auto k = K::load(&tab[h]);
-            if (K::same(k, key)) {
+            const auto t = K::load(&tab[h]);
+            if (K::same(t, k)) {
                 s = static_cast<unsigned>(tab[h].count);
                 break;
             }
-            if (K::is_free(k)) break;
+            if (K::is_free(t)) break;
             h = (h + 1) & mask;
         }
         if (s == 0xFFFFFFFFu) {
             atomicMin(&rs->bad, i);
             s = 0;
         }
-        l1 = static_cast<unsigned>(off1[i + 1] - off1[i]);
-        if constexpr (Mates == 2) l2 = static_cast<unsigned>(off2[i + 1] - off2[i]);
+#pragma unroll
+        for (int q = 0; q < Mates; ++q) len[q] = static_cast<unsigned>(m.off[q][i + 1] - m.off[q][i]);
         sink[i] = s;
     }
     for (int w = 0; w < kRouteBlock / 32; ++w) {
@@ -180,28 +203,35 @@ __global__ void __launch_bounds__(kRouteBlock) route_hist_kernel(const Slot* __r
             const unsigned active = __activemask();
             const unsigned same = __match_any_sync(active, s);
             // bytes of the lower lanes of my sink
-            unsigned before1 = 0, before2 = 0, tot1 = 0, tot2 = 0;
-            for (unsigned m = same; m; m &= m - 1) {
-                const int src = __ffs(m) - 1;
-                const unsigned a1 = __shfl_sync(same, l1, src), a2 = Mates == 2 ? __shfl_sync(same, l2, src) : 0;
-                if (src < lane) before1 += a1, before2 += a2;
-                tot1 += a1, tot2 += a2;
+            unsigned before[Mates], all[Mates];
+#pragma unroll
+            for (int q = 0; q < Mates; ++q) before[q] = 0, all[q] = 0;
+            for (unsigned bits = same; bits; bits &= bits - 1) {
+                const int src = __ffs(bits) - 1;
+#pragma unroll
+                for (int q = 0; q < Mates; ++q) {
+                    const unsigned a = __shfl_sync(same, len[q], src);
+                    if (src < lane) before[q] += a;
+                    all[q] += a;
+                }
             }
-            local1[i] = s_acc[s] + before1;
-            if constexpr (Mates == 2) local2[i] = s_acc[n_sinks + s] + before2;
+#pragma unroll
+            for (int q = 0; q < Mates; ++q) m.local[q][i] = s_acc[q * n_sinks + s] + before[q];
             __syncwarp(active);
             if (lane == __ffs(same) - 1) {
-                s_acc[s] += tot1;
-                if constexpr (Mates == 2) s_acc[n_sinks + s] += tot2;
+#pragma unroll
+                for (int q = 0; q < Mates; ++q) s_acc[q * n_sinks + s] += all[q];
             }
         }
         __syncthreads();
     }
     for (unsigned k = threadIdx.x; k < n_sinks; k += kRouteBlock) {
-        cell[static_cast<unsigned long long>(k) * n_blocks + b] = s_acc[k];
-        if constexpr (Mates == 2) cell[static_cast<unsigned long long>(n_sinks + k) * n_blocks + b] = s_acc[n_sinks + k];
-        if (s_acc[k]) atomicAdd(&tot[k], static_cast<unsigned long long>(s_acc[k]));
-        if (Mates == 2 && s_acc[n_sinks + k]) atomicAdd(&tot[n_sinks + k], static_cast<unsigned long long>(s_acc[n_sinks + k]));
+#pragma unroll
+        for (int q = 0; q < Mates; ++q) {
+            const unsigned v = s_acc[q * n_sinks + k];
+            cell[(static_cast<unsigned long long>(q) * n_sinks + k) * n_blocks + b] = v;
+            if (v) atomicAdd(&tot[q * n_sinks + k], static_cast<unsigned long long>(v));
+        }
     }
 }
 
@@ -246,8 +276,7 @@ __global__ void __launch_bounds__(kRouteBlock) route_scan_kernel(unsigned long l
         if (s == n_sinks - 1) {
             const unsigned long long end = base + t[s];
             sink_off[static_cast<unsigned long long>(mate) * (n_sinks + 1) + n_sinks] = end;
-            if (mate == 0) rs->out1 = end;
-            else rs->out2 = end;
+            rs->out[mate] = end;
         }
     }
     for (unsigned long long b0 = 0; b0 < used_blocks; b0 += kRouteBlock) {
@@ -301,24 +330,23 @@ __global__ void __launch_bounds__(256) route_copy_kernel(const RouteState* __res
     }
 }
 
-// The unconsumed tails in front of the next chunk's buffers (they end where the host puts the new
-// bytes), and where the text begins there.
-__global__ void __launch_bounds__(1024) route_carry_kernel(RouteState* rs, const unsigned char* __restrict__ in1,
-                                                           const unsigned char* __restrict__ in2, unsigned long long end1,
-                                                           unsigned long long end2, unsigned char* __restrict__ next1,
-                                                           unsigned char* __restrict__ next2, unsigned long long carry_cap) {
-    const unsigned long long c1 = end1 - rs->used1, c2 = end2 - rs->used2;
+// The unconsumed tails in front of the next chunk's buffers (they end where the host puts the new bytes), and
+// where the text begins there.  Grid (64, mates): blockIdx.y is the mate.
+__global__ void __launch_bounds__(1024) route_carry_kernel(RouteState* rs, const RouteMates m, unsigned long long carry_cap) {
+    const unsigned k = blockIdx.y;
+    const unsigned char* in = nullptr;
+    unsigned char* next = nullptr;
+    unsigned long long end = 0;
+#pragma unroll
+    for (unsigned q = 0; q < kRouteMaxMates; ++q)  // selects, not an indexed copy of the parameters in local memory
+        if (q == k) in = m.in[q], next = m.next[q], end = m.end[q];
+    const unsigned long long c = end - rs->used[k];
     if (rs->error) return;
-    const unsigned char* const src = blockIdx.y ? in2 + rs->used2 : in1 + rs->used1;
-    unsigned char* const dst = blockIdx.y ? next2 + (carry_cap - c2) : next1 + (carry_cap - c1);
-    const unsigned long long c = blockIdx.y ? c2 : c1;
+    const unsigned char* const src = in + rs->used[k];
+    unsigned char* const dst = next + (carry_cap - c);
     for (unsigned long long i = blockIdx.x * 1024ull + threadIdx.x; i < c; i += gridDim.x * 1024ull) dst[i] = src[i];
     __syncthreads();
-    if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) {
-        // read by the NEXT chunk's kernels only (stream order)
-        rs->skip1 = carry_cap - c1;
-        rs->skip2 = carry_cap - c2;
-    }
+    if (blockIdx.x == 0 && threadIdx.x == 0) rs->skip[k] = carry_cap - c;  // read by the NEXT chunk's kernels only
 }
 
 }  // namespace frb

@@ -160,6 +160,7 @@ class Context:
         self.sheet = None
         self.file_names = []
         self.wide = False
+        self._route_mates = 2
         if wide:
             self.set_wide()
 
@@ -233,7 +234,8 @@ class Context:
         return out[:n.value].tobytes() if used.value else None
 
     def gz_open(self, slot, path):
-        """A span reader over the text of a .gz file, inflated on the device (frb_gz_open); slot 0 or 1."""
+        """A span reader over the text of a .gz file, inflated on the device (frb_gz_open); slot 0 to 3, one per
+        mate (R1, R2, I1, I2)."""
         self._ck(lib.frb_gz_open(self._h, slot, os.fsencode(str(path))))
 
     def gz_read(self, slot, max_bytes, copy=False):
@@ -549,11 +551,18 @@ class Context:
         else:
             self._ck(lib.frb_route_set_gzip(self._h, 1 if on else 0))
 
-    def route_mates(self, n):
+    def route_mates(self, n, key_mate=None):
         """Paired (2) or single-end (1) demux stream (frb_route_set_mates): a single-end stream routes R1 alone, by
-        the keys of its own headers; route_push then takes r2=None and route_pop returns empty R2 offsets.  Only
-        between chunks; kept by route_reset."""
-        self._ck(lib.frb_route_set_mates(self._h, int(n)))
+        the keys of its own headers; route_push then takes r2=None and route_pop returns empty R2 offsets.  With
+        index reads, 3 or 4 mates (R1, R2, I1, I2 in that order, R2 absent when single-end) and the mate whose
+        headers give the keys (frb_route_set_mates2; key_mate=None: R2, or R1 when n is 1); such a stream goes
+        through route_pushv / route_popv.  Only between chunks; kept by route_reset."""
+        if key_mate is None and n in (1, 2):
+            self._ck(lib.frb_route_set_mates(self._h, int(n)))
+        else:
+            key = min(int(n), 2) - 1 if key_mate is None else int(key_mate)
+            self._ck(lib.frb_route_set_mates2(self._h, int(n), key))
+        self._route_mates = int(n)
 
     def route_push(self, r1, r2, final=0):
         """Queue one chunk pair of the demux stream (frb_route_push): bytes cut anywhere; what is not complete
@@ -576,6 +585,31 @@ class Context:
         v2 = (np.ctypeslib.as_array((C.c_uint8 * max(n2, 1)).from_address(o2.value))[:n2] if o2.value
               else np.empty(0, np.uint8))                 # a single-end stream returns no R2
         return v1, v2, off1.astype(np.int64), off2.astype(np.int64), pairs.value, c1.value, c2.value
+
+    def route_pushv(self, chunks, final=0):
+        """Queue one chunk of every mate (frb_route_pushv): chunks[m] is host bytes or a device GzSpan of this
+        context, for each of the route_mates() mates; bit m of final: mate m's file ends with this chunk."""
+        args = [_chunk_arg(x) for x in chunks]
+        ptrs = (C.c_void_p * max(len(args), 1))(*[a[0] for a in args])
+        sizes = np.array([a[1] for a in args] or [0], np.uint64)
+        self._ck(lib.frb_route_pushv(self._h, ptrs, _ptr(sizes), int(final)))
+
+    def route_popv(self):
+        """The oldest chunk in flight (frb_route_popv): (outs, offs, records, carries) with one entry per mate;
+        sink s of mate m is outs[m][offs[m][s]:offs[m][s+1]].  outs are views of the library's pinned memory, valid
+        until the chunk after next is pushed."""
+        m = self._route_mates
+        outs = (C.c_void_p * m)()
+        offs = np.zeros((m, self._n_sinks + 1), np.uint64)
+        carry = np.zeros(m, np.uint64)
+        records, bad = C.c_uint64(), C.c_uint64()
+        self._ck(lib.frb_route_popv(self._h, outs, _ptr(offs), C.byref(records), _ptr(carry), C.byref(bad)))
+        views = []
+        for k in range(m):
+            n = int(offs[k, -1])
+            views.append(np.ctypeslib.as_array((C.c_uint8 * max(n, 1)).from_address(outs[k]))[:n] if n
+                         else np.empty(0, np.uint8))
+        return views, offs.astype(np.int64), records.value, [int(c) for c in carry]
 
     # ---- measurement ------------------------------------------------------------------------
     def launches(self):

@@ -182,8 +182,11 @@ def keys_of(spec, g0, g1):
     return out
 
 
-def generate(spec, g0, g1, read_no=1):
-    """FASTQ bytes of reads g0..g1-1 of mate `read_no` (1 or 2)."""
+def generate(spec, g0, g1, read_no=1, index_read=None):
+    """FASTQ bytes of reads g0..g1-1 of mate `read_no` (1 or 2).  index_read=1 / 2: the records of the I1 / I2 file
+    instead -- the header of mate `read_no`, the i7 / i5 that header carries as the sequence, and 'F' qualities."""
+    if index_read not in (None, 1, 2) or (index_read == 2 and not spec.l2):
+        raise ValueError(f"index read {index_read!r} of a spec with l2 = {spec.l2}")
     n = g1 - g0
     if n <= 0:
         return b""
@@ -220,6 +223,12 @@ def generate(spec, g0, g1, read_no=1):
         for p in range(spec.l2):
             cols.append(SYMS[i5[:, p]]); valid.append(np.ones(n, bool))
     const(b"\n")
+    if index_read:
+        seq = i7 if index_read == 1 else i5
+        for p in range(seq.shape[1]):
+            cols.append(SYMS[seq[:, p]]); valid.append(np.ones(n, bool))
+        const(b"\n+\n" + b"F" * seq.shape[1] + b"\n")
+        return np.stack(cols, axis=1)[np.stack(valid, axis=1)].tobytes()
     j0 = J_SEQ1 if read_no == 1 else J_SEQ2
     words = [draw(spec.seed, g, j0 + k) for k in range((spec.read_len + 31) // 32)]
     for i in range(spec.read_len):
@@ -231,9 +240,9 @@ def generate(spec, g0, g1, read_no=1):
     return mat[msk].tobytes()
 
 
-def generate_big(spec, g0, g1, read_no=1, step=200_000):
+def generate_big(spec, g0, g1, read_no=1, step=200_000, index_read=None):
     """generate() in slices, to bound the temporary matrices."""
-    return b"".join(generate(spec, a, min(a + step, g1), read_no) for a in range(g0, g1, step))
+    return b"".join(generate(spec, a, min(a + step, g1), read_no, index_read) for a in range(g0, g1, step))
 
 
 def binned_qualities(data, seed=0):

@@ -148,8 +148,9 @@ int frb_scan_gz_batch(frb_ctx* ctx, const char* const* paths, const uint32_t* or
  * to zlib on a host thread for such a file.                                                                */
 int frb_gz_inflate(frb_ctx* ctx, const char* path, void* host_out, uint64_t cap, uint64_t* nbytes, int* used_device);
 /* Span readers: the text of a .gz file inflated ON THE DEVICE and handed out in device memory, for the demux stream
- * (frb_route_push takes the spans).  A context has two slots (0, 1), one per mate; frb_gz_open closes what the slot
- * held, frb_gz_close frees a slot's thread and buffers (a no-op on a closed slot), frb_destroy closes both.
+ * (frb_route_push takes the spans).  A context has four slots (0 to 3), one per mate (R1, R2, I1, I2); a slot costs
+ * nothing until it is opened.  frb_gz_open closes what the slot held, frb_gz_close frees a slot's thread and buffers
+ * (a no-op on a closed slot), frb_destroy closes all of them.
  * frb_gz_read: *dev_text / *n = a span of EXACTLY max_bytes (>= 1) bytes of text, fewer only where the text ends;
  * *eof = 1 when nothing follows the span; *n = 0 after the end.  A span stays valid until the reader has inflated
  * two more pieces (FRB_GZ_PIECE_MB of compressed bytes each), and a copy of it that frb_route_push queued is always
@@ -259,7 +260,8 @@ int frb_demux_ok(frb_ctx* ctx, const uint8_t* match, uint32_t n_files, const uin
  */
 int frb_route_load(frb_ctx* ctx, const uint64_t* keys, const uint32_t* sink_ids, uint64_t n, uint32_t n_sinks);
 /* frb_route_load with the upper words of wide keys (wide context only; the router then parses keys of up to 42
- * symbols from the R2 headers).                                                                                  */
+ * symbols from the R2 headers -- from the key mate's headers in a stream of frb_route_set_mates2, index reads
+ * included).                                                                                                     */
 int frb_route_load2(frb_ctx* ctx, const uint64_t* keys, const uint64_t* keys_hi, const uint32_t* sink_ids, uint64_t n,
                     uint32_t n_sinks);
 int frb_route_pair(frb_ctx* ctx, const void* r1, uint64_t r1_bytes, const void* r2, uint64_t r2_bytes,
@@ -303,6 +305,27 @@ int frb_route_set_gz_format(frb_ctx* ctx, int format);
  *   frb_route_pop   *n_pairs = records routed; *out_r2 = NULL, off_r2 all zero, carry_r2 = 0.
  * frb_route_pair always routes pairs: it saves the setting, routes with mates = 2 and restores it.                */
 int frb_route_set_mates(frb_ctx* ctx, int mates);
+/* Index reads: a stream of 1 to 4 mates, the keys taken from the headers of mate key_mate (0-based).  The caller
+ * orders the mates R1, R2 (absent when single-end), then I1 and / or I2, with key_mate = 1 (R2) or 0 (single-end R1);
+ * frb_route_set_mates(ctx, m) is frb_route_set_mates2(ctx, m, m - 1).  Every other mate is parsed for its record
+ * offsets alone, and record i of every mate goes to the sink of record i's key; the zip() of F:777 runs over all the
+ * mates (a record is routed once every mate has it complete, a trailing partial record counts once its file has
+ * ended, and the stream ends once any mate has ended and is used up).  Every output format and wide contexts work as
+ * in a paired stream.  mates outside 1..4 or key_mate outside 0..mates-1 is FRB_ERR_ARG; the same rules as
+ * frb_route_set_mates otherwise.  The buffers of mates 3 and 4 are allocated when such a stream is first set (or with
+ * the stream's other buffers; after frb_route_pair rebuilt the stream for a pair, at the next push).  A stream's
+ * histogram keeps one 32-bit counter per sink and mate in the 227 KiB of shared memory a block may have, so a 4-mate stream takes at most 14,528 sinks (3 mates: the usual 16,384): a
+ * results table with more is FRB_ERR_ARG, here or at frb_route_load.
+ *   frb_route_pushv  in[m] / n[m] = the chunk of mate m (host or device memory, as frb_route_push), for every mate;
+ *                    bit m of final_bits: mate m's file ends with this chunk.
+ *   frb_route_popv   out[m] = the routed bytes of mate m (pinned memory of the library, valid as for frb_route_pop),
+ *                    off[m * (n_sinks + 1) + s] = start of sink s in out[m]; carry[m] (may be NULL) = bytes of mate m
+ *                    pushed so far that are not routed yet; *n_records = records routed (of every mate).
+ * frb_route_push / frb_route_pop are their one- and two-mate forms; on a stream of 3 or 4 mates they are
+ * FRB_ERR_STATE.  frb_route_pair stays two-mate.                                                                   */
+int frb_route_set_mates2(frb_ctx* ctx, int mates, int key_mate);
+int frb_route_pushv(frb_ctx* ctx, const void* const* in, const uint64_t* n, int final_bits);
+int frb_route_popv(frb_ctx* ctx, void** out, uint64_t* off, uint64_t* n_records, uint64_t* carry, uint64_t* bad_key);
 
 /* ---- multi-GPU: merge of the per-rank totals over NCCL (NVLink) ------------------------------
  * One process (or thread) per GPU.  Rank 0 makes the id, the host hands it to every rank.

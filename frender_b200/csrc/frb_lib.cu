@@ -592,10 +592,10 @@ int frb_create(int device, uint32_t table_log2, frb_ctx** out) {
     CU(c, cudaFuncSetAttribute(scan_ws_kernel<WsTileWide>, cudaFuncAttributeMaxDynamicSharedMemorySize, WsTileWide::smem));
     CU(c, cudaFuncSetAttribute(scan_spec_kernel<WsTile>, cudaFuncAttributeMaxDynamicSharedMemorySize, WsTile::smem));
     CU(c, cudaFuncSetAttribute(scan_spec_kernel<WsTile, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, WsTile::smem));
-    CU(c, cudaFuncSetAttribute(match_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    CU(c, cudaFuncSetAttribute(match_cand_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    CU(c, cudaFuncSetAttribute(match_idx1_cand_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    CU(c, cudaFuncSetAttribute(match_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+    CU(c, cudaFuncSetAttribute(match_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMatchSmemMax));
+    CU(c, cudaFuncSetAttribute(match_cand_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMatchSmemMax));
+    CU(c, cudaFuncSetAttribute(match_idx1_cand_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMatchSmemMax));
+    CU(c, cudaFuncSetAttribute(match_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMatchWideSmemMax));
     TRY(clear_table(c, c->total_tab));
     CU(c, cudaStreamSynchronize(c->compute));
     *out = owner.release();
@@ -1465,57 +1465,47 @@ int frb_match(frb_ctx* c, uint32_t n_subs, int rc_mode, const uint8_t* use_rc_ro
         // over to any per-row choice of orientation over the same keys / sheet / n (F:618-630).
         const bool reuse = !rc_mode && c->m1_from_rc && c->m1_total_gen == c->total_gen &&
                            c->m1_sheet_gen == c->sheet_gen && c->m1_n_subs == n_subs;
-        c->m1_total_gen = c->total_gen, c->m1_sheet_gen = c->sheet_gen, c->m1_n_subs = n_subs;
-        c->m1_from_rc = rc_mode != 0;
-        ProfScope ps(c, FRB_K_MATCH);
-        if (c->wide) {  // sweeps over the split idx1 / idx2 words (no candidate tables for wide keys)
-            WideMatchArgs w{a, c->total.keys_hi, c->sheet.fwd_hi, c->sheet.rc_hi};
-            if (!reuse) {
-                CU(c, cudaMemsetAsync(mo.work_n, 0, 8, c->compute));
-                match_idx1_wide_kernel<<<grid_for(n, kMatchThreads, c->sm_count, 8), kMatchThreads,
-                                         static_cast<size_t>(c->rows) * 8 + 16, c->compute>>>(w);
-                c->launches++;
-            } else {
-                CU(c, cudaMemsetAsync(mo.m2, 0xFF, n * 4, c->compute));
-                CU(c, cudaMemsetAsync(mo.srow, 0xFF, n * 4, c->compute));
-                CU(c, cudaMemsetAsync(mo.type, 0, n, c->compute));
-            }
-            match_wide_kernel<<<grid_for(n, kMatchThreads, c->sm_count, 8), kMatchThreads,
-                                static_cast<size_t>(c->rows) * (5 * 8 + 4) + 16, c->compute>>>(w);
-            c->launches++;
-            CU(c, cudaGetLastError());
-        } else {
+        // m1 and the work list describe nothing until this call has succeeded: a failed pass (a key of the wrong
+        // length, a CUDA error) must not be reused by the next one, nor reduced over by frb_demux_ok
+        c->m1_total_gen = ~0ULL, c->m1_from_rc = false;
         // candidate rows from per-part tables instead of a sweep over the sheet, whenever the shape allows
         static const bool sweep_only = getenv("FRB_MATCH") && strcmp(getenv("FRB_MATCH"), "sweep") == 0;
-        const unsigned parts = n_subs + 1;
-        const unsigned slots = static_cast<unsigned long long>(c->rows) * parts * 2 <= 2048 ? 2048u : 4096u;
-        const bool cand = !sweep_only && c->rows > 0 && c->l2 > 0 && parts_usable(c->l1, n_subs, c->rows, slots) &&
-                          parts_usable(c->l2, n_subs, c->rows, slots);
+        MatchPlan plan = match_plan(c->rows, c->l1, c->l2, n_subs, c->wide);
+        if (sweep_only && plan.path == kMatchCand) plan = kSweepPlan;
+        const int grid = grid_for(n, kMatchThreads, c->sm_count, plan.blocks_per_sm);
+        const size_t smem1 = match_smem_idx1(plan, c->rows, n_subs);
+        const size_t smem2 = match_smem_classify(plan, c->rows, n_subs, rc_mode != 0);
+        ProfScope ps(c, FRB_K_MATCH);
         if (!reuse) {
             CU(c, cudaMemsetAsync(mo.work_n, 0, 8, c->compute));
-            if (cand)
-                match_idx1_cand_kernel<<<grid_for(n, kMatchThreads, c->sm_count, 4), kMatchThreads,
-                                         cand_bytes(c->rows, parts, slots) + 16, c->compute>>>(a, slots);
-            else
-                match_idx1_kernel<<<grid_for(n, kMatchThreads, c->sm_count, 8), kMatchThreads,
-                                    static_cast<size_t>(c->rows) * 8 + 16, c->compute>>>(a);
-            c->launches++;
         } else {
             // keys off the work list stay undetermined; m1 is already -1 for them
             CU(c, cudaMemsetAsync(mo.m2, 0xFF, n * 4, c->compute));
             CU(c, cudaMemsetAsync(mo.srow, 0xFF, n * 4, c->compute));
             CU(c, cudaMemsetAsync(mo.type, 0, n, c->compute));
         }
-        if (cand) {
-            const size_t smem = static_cast<size_t>(c->rows) * 24 + 32 + (rc_mode ? 2 : 1) * cand_bytes(c->rows, parts, slots);
-            match_cand_kernel<<<grid_for(n, kMatchThreads, c->sm_count, 4), kMatchThreads, smem, c->compute>>>(a, slots);
+        if (plan.path == kMatchWide) {  // sweeps over the split idx1 / idx2 words (no candidate tables for wide keys)
+            WideMatchArgs w{a, c->total.keys_hi, c->sheet.fwd_hi, c->sheet.rc_hi};
+            if (!reuse) {
+                match_idx1_wide_kernel<<<grid, kMatchThreads, smem1, c->compute>>>(w);
+                c->launches++;
+            }
+            match_wide_kernel<<<grid, kMatchThreads, smem2, c->compute>>>(w);
+        } else if (plan.path == kMatchCand) {
+            if (!reuse) {
+                match_idx1_cand_kernel<<<grid, kMatchThreads, smem1, c->compute>>>(a, plan.slots);
+                c->launches++;
+            }
+            match_cand_kernel<<<grid, kMatchThreads, smem2, c->compute>>>(a, plan.slots);
         } else {
-            const size_t smem = static_cast<size_t>(c->rows) * (4 * 8 + 4) + 16;
-            match_kernel<<<grid_for(n, kMatchThreads, c->sm_count, 8), kMatchThreads, smem, c->compute>>>(a);
+            if (!reuse) {
+                match_idx1_kernel<<<grid, kMatchThreads, smem1, c->compute>>>(a);
+                c->launches++;
+            }
+            match_kernel<<<grid, kMatchThreads, smem2, c->compute>>>(a);
         }
         c->launches++;
         CU(c, cudaGetLastError());
-        }
     }
     if (n) {
         if (m1_row) CU(c, cudaMemcpyAsync(m1_row, mo.m1, n * 4, cudaMemcpyDeviceToHost, c->compute));
@@ -1531,7 +1521,10 @@ int frb_match(frb_ctx* c, uint32_t n_subs, int rc_mode, const uint8_t* use_rc_ro
     if (f_sum && c->rows) CU(c, cudaMemcpyAsync(f_sum, c->sheet.f_sum, c->rows * 8, cudaMemcpyDeviceToHost, c->compute));
     if (rc_sum && c->rows) CU(c, cudaMemcpyAsync(rc_sum, c->sheet.rc_sum, c->rows * 8, cudaMemcpyDeviceToHost, c->compute));
     CU(c, cudaStreamSynchronize(c->compute));
-    return device_error_check(c);
+    TRY(device_error_check(c));
+    // what m1 and the work list now describe
+    if (n) c->m1_total_gen = c->total_gen, c->m1_sheet_gen = c->sheet_gen, c->m1_n_subs = n_subs, c->m1_from_rc = rc_mode != 0;
+    return FRB_OK;
 }
 
 // demux_ok per unique key of the total list + which files hold a key they should not (F:504-564), on the device.

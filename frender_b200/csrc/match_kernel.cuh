@@ -564,4 +564,45 @@ __global__ void __launch_bounds__(kMatchThreads) match_wide_kernel(const WideMat
     flush_group_sums(a, s_f, s_r);
 }
 
+// =================================================================================================
+// Which pair of kernels frb_match launches for a sheet shape, and with how much shared memory.
+// =================================================================================================
+enum MatchPath : int {
+    kMatchCand = 0,   // match_idx1_cand_kernel + match_cand_kernel
+    kMatchSweep = 1,  // match_idx1_kernel + match_kernel
+    kMatchWide = 2,   // match_idx1_wide_kernel + match_wide_kernel
+};
+constexpr int kMatchSmemMax = 200 * 1024;      // dynamic shared memory allowed to match_kernel and both cand kernels
+constexpr int kMatchWideSmemMax = 220 * 1024;  // ... and to match_wide_kernel
+
+struct MatchPlan {
+    MatchPath path;
+    unsigned slots;     // slots of each candidate table (kMatchCand only, else 0)
+    int blocks_per_sm;  // grid of both kernels: at most sm_count * blocks_per_sm blocks of kMatchThreads
+};
+constexpr MatchPlan kSweepPlan{kMatchSweep, 0, 8};
+
+// Candidate tables whenever both indexes can be split into n_subs + 1 parts and the tables fit (2048 slots while
+// rows * parts * 2 <= 2048, else 4096); the sweep for every other narrow shape; wide contexts sweep the split words.
+__host__ inline MatchPlan match_plan(unsigned rows, unsigned l1, unsigned l2, unsigned n_subs, bool wide) {
+    if (wide) return {kMatchWide, 0, 8};
+    const unsigned parts = n_subs + 1;
+    const unsigned slots = static_cast<unsigned long long>(rows) * parts * 2 <= 2048 ? 2048u : 4096u;
+    if (rows > 0 && l2 > 0 && parts_usable(l1, n_subs, rows, slots) && parts_usable(l2, n_subs, rows, slots))
+        return {kMatchCand, slots, 4};
+    return kSweepPlan;
+}
+// dynamic shared memory of kernel 1 (idx1 sweep / table, work list)
+__host__ inline size_t match_smem_idx1(const MatchPlan& p, unsigned rows, unsigned n_subs) {
+    if (p.path == kMatchCand) return cand_bytes(rows, n_subs + 1, p.slots) + 16;
+    return static_cast<size_t>(rows) * 8 + 16;
+}
+// dynamic shared memory of kernel 2 (classification of the work list)
+__host__ inline size_t match_smem_classify(const MatchPlan& p, unsigned rows, unsigned n_subs, bool rc_mode) {
+    if (p.path == kMatchCand)
+        return static_cast<size_t>(rows) * 24 + 32 + (rc_mode ? 2 : 1) * cand_bytes(rows, n_subs + 1, p.slots);
+    if (p.path == kMatchSweep) return static_cast<size_t>(rows) * (4 * 8 + 4) + 16;
+    return static_cast<size_t>(rows) * (5 * 8 + 4) + 16;
+}
+
 }  // namespace frb
